@@ -3,7 +3,7 @@
 Levenberg-Marquardt iterations, i.e. visible observations x accepted LM iterations / second).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--workload c2|c3|c4|c5] [--weak]
-                    [--extras auto|none|c2,c4,c5] [--impl reference]
+                    [--extras auto|none|c2,c4,c5] [--impl reference] [--dump-outputs DIR]
 
 Headline workload: BASELINE.json config 3 (200 cameras x 100 000 points, full visibility -- the
 dense Schur SYRK), one GPU at N = 1 and STRONG-scaled at N > 1: every rank generates its shard of
@@ -27,6 +27,9 @@ solve(s), trial cost, accept), started from the same perturbed-ground-truth stat
 `extra`    N = 1: config 2 (50 x 10k, the small latency-bound case) with its own roofline / e2e;
            N = 8: config 4 (1000 cameras x 1M points, 10 % visibility) strong-scaled with parity and
            the sparsity-aware CPU denominator, and config 5 (1 % outliers) run to convergence.
+
+`--dump-outputs DIR` writes the headline's results after its timed steps (see dump_outputs).  The
+scenes come from fixed seeds, so two builds run with the same arguments can be compared file by file.
 """
 from __future__ import annotations
 
@@ -59,6 +62,8 @@ CHUNK = 10  # LM iterations per run from the perturbed start (see run_iters)
 # all (an unseen camera makes the reference's reduced system singular, :146), and 100 points are 65 GB
 REF_SAMPLE = {"c2": 1_000, "c3": 60, "c4": None, "c5": None}
 PORT_SAMPLE = {"c2": (10_000, 2), "c3": (1_500, 1), "c4": (20_000, 1), "c5": (20_000, 1)}
+DUMP_MAX_BYTES = 64 << 20
+DUMP_SEED = 0
 
 
 def parse_args():
@@ -82,7 +87,15 @@ def parse_args():
     ap.add_argument("--extras", default="auto",
                     help="auto: c2 at N = 1, c4 + c5 at N = 8; none; or a comma list of c2,c4,c5")
     ap.add_argument("--no-parity", action="store_true", help="N > 1: skip the single-GPU parity run")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the headline workload's last step computed "
+                         "(X, K, R, t in the caller's frame and the costs of the last LM run) as DIR/<name>.npy")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "cuda":
+        ap.error("--dump-outputs writes the CUDA arm's outputs")
+    return args
 
 
 def workload_config(name: str) -> dict:
@@ -425,11 +438,52 @@ def single_gpu_trajectory(ctx: Ctx, sc, whole, iters: int, tol: float = TOL_NEVE
     return np.array(E), int(st.solves)
 
 
+def gather_rows_on_rank0(ctx: Ctx, arr: np.ndarray):
+    """Every rank's rows of a float64 array, concatenated in rank order on rank 0 (None elsewhere)."""
+    torch, dist, dev = ctx.torch, ctx.dist, f"cuda:{ctx.local_rank}"
+    counts = torch.empty(ctx.world, dtype=torch.int64, device=dev)
+    dist.all_gather_into_tensor(counts, torch.tensor([arr.shape[0]], dtype=torch.int64, device=dev))
+    counts = counts.cpu().numpy()
+    mine = torch.zeros((int(counts.max()),) + arr.shape[1:], dtype=torch.float64, device=dev)
+    mine[: arr.shape[0]] = torch.from_numpy(np.ascontiguousarray(arr)).to(dev)
+    out = torch.empty((ctx.world,) + tuple(mine.shape), dtype=torch.float64, device=dev)
+    dist.all_gather_into_tensor(out, mine)
+    if ctx.rank != 0:
+        return None
+    return np.concatenate([out[r, : counts[r]].cpu().numpy() for r in range(ctx.world)])
+
+
+def dump_outputs(ctx: Ctx, adj, out_dir: str) -> None:
+    """What the timed path computed in its last step, as optimize() hands it to its caller: X, K, R, t
+    in the caller's frame, and E, the cost before and after every iteration of the last LM run, as
+    out_dir/<name>.npy in float64.  At N > 1 the point shards are gathered on rank 0.  If the files
+    would exceed DUMP_MAX_BYTES, X is a fixed seeded sample of rows, whose indices go to X_rows.npy."""
+    eng = adj.engine
+    X, R, t, f, u = eng.get_state(0)
+    X, R, t = ctx.gauge.denormalize(adj._R0, adj._t0, adj._c0c1_len, X, R, t)
+    recs = eng.lm_records()
+    out = {"K": ctx.gauge.make_K(f, u, adj._f0), "R": R, "t": t,
+           "E": np.array([recs[0].E_prev] + [r.E for r in recs])}
+    if ctx.world > 1:
+        X = gather_rows_on_rank0(ctx, X)
+    if ctx.rank != 0:
+        return
+    budget = DUMP_MAX_BYTES - sum(a.nbytes for a in out.values())
+    if X.nbytes > budget:
+        rows = np.random.default_rng(DUMP_SEED).choice(X.shape[0], budget // (4 * 8), replace=False)
+        rows.sort()
+        X, out["X_rows"] = X[rows], rows.astype(np.float64)
+    out["X"] = X
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), np.ascontiguousarray(a, dtype=np.float64))
+
+
 def measure(ctx: Ctx, name: str, strong: bool, K: int, W: int, *, full_run_tol=None,
-            with_e2e: bool = True, with_parity: bool = True) -> dict | None:
+            with_e2e: bool = True, with_parity: bool = True, dump_dir: str | None = None) -> dict | None:
     """One workload on this invocation's ranks; rank 0 returns the result dict.  `full_run_tol`:
     instead of K steps in chunks, ONE optimize(2.0, tol, max_iter=K) call (config 5's convergence
-    run)."""
+    run).  `dump_dir`: write the outputs of the timed steps there (see dump_outputs)."""
     torch, args, rank, world, local_rank = ctx.torch, ctx.args, ctx.rank, ctx.world, ctx.local_rank
     dist, group, ba_b200 = ctx.dist, ctx.group, ctx.ba
     t_gen = time.perf_counter()
@@ -514,6 +568,8 @@ def measure(ctx: Ctx, name: str, strong: bool, K: int, W: int, *, full_run_tol=N
         steps_done = K
         assert st.count == K, f"ran {st.count} iterations instead of {K}"
     launches = ctx.engine_mod.launch_count() - launches0
+    if dump_dir:
+        dump_outputs(ctx, adj, dump_dir)
     ctx.barrier()
     ms = ctx.max_over_ranks(ev0.elapsed_time(ev1))
     nobs_total = int(ctx.sum_over_ranks(float(sc.nobs)))
@@ -712,9 +768,9 @@ def run_cuda(args, rank: int, world: int, local_rank: int):
         sampler.start()
 
     if name == "c5":
-        out = measure(ctx, name, strong, max(K, 50), W, full_run_tol=1e-8)
+        out = measure(ctx, name, strong, K, W, full_run_tol=1e-8, dump_dir=args.dump_outputs)
     else:
-        out = measure(ctx, name, strong, K, W)
+        out = measure(ctx, name, strong, K, W, dump_dir=args.dump_outputs)
     if rank == 0:
         t_wall0, t_wall1 = out.pop("_wall")
         out["clocks"] = sampler.stop(t_wall0, t_wall1)

@@ -6,6 +6,9 @@ import os
 import subprocess
 import sys
 
+import numpy as np
+import pytest
+
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
@@ -52,3 +55,33 @@ def test_reference_arm_is_not_pinned_to_one_thread_under_torchrun():
     ncpu = len(os.sched_getaffinity(0))
     assert d["cpu_baseline"]["cores"] == ncpu and d["n_gpus"] == 2 and d["scaling"] == "strong"
     assert d["config"]["workload"].startswith("c2")
+
+
+@pytest.mark.gpu
+def test_cuda_arm_times_the_requested_steps_and_dumps_reproducible_outputs(tmp_path):
+    """--steps sets the number of timed LM iterations; --dump-outputs writes what the last of them
+    computed (X, K, R, t and the costs of the last LM run, float64, at most 64 MB), and the same
+    arguments give the same outputs."""
+    def run(steps, name):
+        out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--workload", "c2", "--steps", str(steps),
+                              "--warmup", "1", "--extras", "none", "--no-cpu-baseline", "--dump-outputs",
+                              str(tmp_path / name)], capture_output=True, text=True, timeout=900, cwd=ROOT)
+        assert out.returncode == 0, out.stderr[-2000:]
+        d = json.loads([l for l in out.stdout.splitlines() if l.startswith("{")][0])
+        files = sorted(os.listdir(tmp_path / name))
+        assert files == ["E.npy", "K.npy", "R.npy", "X.npy", "t.npy"]
+        arrays = {f[:-4]: np.load(tmp_path / name / f) for f in files}
+        assert all(a.dtype == np.float64 for a in arrays.values())
+        assert sum(os.path.getsize(tmp_path / name / f) for f in files) <= 64 << 20
+        return d, arrays
+
+    d12, a12 = run(12, "a")
+    assert d12["steps"] == 12 and d12["inner_solves"] >= 12
+    # 12 steps are LM runs of 10 and 2 iterations; E holds the last run's costs
+    assert a12["E"].shape == (3,) and a12["X"].shape == (d12["config"]["n_points"], 3)
+    assert a12["K"].shape == a12["R"].shape == (d12["config"]["n_cams"], 3, 3)
+    d3, a3 = run(3, "b")
+    assert d3["steps"] == 3 and a3["E"].shape == (4,)
+    _, again = run(3, "c")
+    for k in a3:
+        np.testing.assert_allclose(again[k], a3[k], rtol=1e-12, atol=1e-12, err_msg=k)

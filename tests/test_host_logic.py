@@ -108,29 +108,27 @@ def test_scene_generator_properties():
     np.testing.assert_array_equal(sc.obs_xy, sc2.obs_xy)
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/lib"), reason="reference checkout not present")
 def test_scene_conventions_match_reference_camera_module():
-    """look_at / projection against the reference's own lib/camera.py (build container only)."""
-    import sys
-
-    sys.path.insert(0, "/root/reference")
-    try:
-        from lib.camera import Camera, calc_projected_points
-    finally:
-        sys.path.remove("/root/reference")
-    rs = np.random.RandomState(3)
-    pos = scenes.hemisphere_positions(rs, 5, 5.0)
-    tgt = rs.normal(0, 0.5, (5, 3))
+    """look_at / projection against the reference's own lib/camera.py, through the cameras it made
+    for tests/golden/projection.npz (oracle/gen_golden_projection.py): nine
+    ``Camera.create(pos, target, f=1 + 0.1 i, f0=1)`` with the targets drawn from RandomState(7),
+    then N(0, 0.01) noise added to K from the same stream."""
+    g = load_golden("projection")
+    rs = np.random.RandomState(7)
+    tgt = np.array([rs.normal(0, 0.5, 3) for _ in range(9)])
+    K = g["K"] - rs.normal(0, 0.01, g["K"].shape)
+    f = 1.0 + 0.1 * np.arange(9)
+    np.testing.assert_array_equal(K, gauge.make_K(f, np.zeros((9, 2)), 1.0))  # the stream is reproduced
+    pos = g["t"]
     R = scenes.look_at(pos, tgt)
-    X = rs.uniform(-1, 1, (7, 3))
-    for i in range(5):
-        cam = Camera.create(pos[i], tgt[i], f=1.0, f0=1.0)
-        K, Rr, tr = cam.get_parameters()
-        np.testing.assert_allclose(R[i], Rr, atol=1e-14)
-        proj = calc_projected_points(X, K[None], Rr[None], tr[None])[0]
-        mine = scenes.project_obs(X, np.ones(5), np.zeros((5, 2)), R, pos, 1.0,
-                                  np.arange(7), np.full(7, i))
-        np.testing.assert_allclose(mine, proj, atol=1e-13)
+    np.testing.assert_allclose(R, g["R"], atol=1e-14)
+    # the reference's projection of these cameras is pinned by the fixture through the oracle
+    np.testing.assert_allclose(O.project_all(g["X"], g["K"], g["R"], pos), g["x"], rtol=1e-13, atol=1e-14)
+    X = g["X"]
+    proj = O.project_all(X, K, g["R"], pos)
+    for i in range(9):
+        mine = scenes.project_obs(X, f, np.zeros((9, 2)), R, pos, 1.0, np.arange(len(X)), np.full(len(X), i))
+        np.testing.assert_allclose(mine, proj[i], atol=1e-13)
     # the reference's two known-answer projections (lib/camera.py:101-117)
     Xk = np.array([[0, 0, 0], [1, 0, 0], [0, 1, 0], [0, 0, 1]], dtype=float)
     R1 = scenes.look_at(np.array([[0.0, 0, -1]]), np.array([[0.0, 0, 1]]))

@@ -2,7 +2,6 @@
 reduction against the dense NumPy form (which the reference's golden vectors pin), the oracle at the
 full config 2 against two iterations of the UNMODIFIED reference (tests/golden/c2_reference.npz,
 oracle/gen_golden_large.py), and the build-time copy of the reference (oracle/_ref)."""
-import os
 
 import numpy as np
 import pytest
@@ -84,28 +83,36 @@ def test_chunk_seeded_scene_shards_tile_the_whole_scene():
         ba_b200.scenes.make_scene(9, 100, point_range=(0, 10))
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/lib"), reason="reference checkout not present")
-def test_oracle_ref_is_a_byte_for_byte_copy_of_the_reference():
+def _stand_in_reference(root):
+    """A reference checkout in miniature: the lib/ modules load_reference_class() imports and a script."""
+    (root / "lib").mkdir(parents=True)
+    (root / "lib" / "utils.py").write_text("def unit_vec(v):\n    return v\n")
+    (root / "lib" / "bundle_adjustment.py").write_text(
+        "from lib.utils import unit_vec\n\n\nclass BundleAdjuster:\n    def __init__(self, x):\n        self.x = unit_vec(x)\n")
+    (root / "euclidiean_reconstruction.py").write_text("print('script')\n")
+    return root
+
+
+def test_oracle_ref_is_a_byte_for_byte_copy_of_the_reference(tmp_path, monkeypatch):
+    src = _stand_in_reference(tmp_path / "reference")
+    dst = tmp_path / "_ref"
+    monkeypatch.setattr(build_ref, "REF_SRC", str(src))
+    monkeypatch.setattr(build_ref, "REF_DST", str(dst))
     build_ref.build()
     assert build_ref.verify()
-    for name in os.listdir("/root/reference/lib"):
-        if name.endswith(".py"):
-            with open(os.path.join("/root/reference/lib", name), "rb") as a, \
-                    open(os.path.join(build_ref.REF_DST, "lib", name), "rb") as b:
-                assert a.read() == b.read()
+    for name in ["lib/utils.py", "lib/bundle_adjustment.py", "euclidiean_reconstruction.py"]:
+        assert (src / name).read_bytes() == (dst / name).read_bytes()
     # the class bench.py times is the reference's own, not the product's
     cls = build_ref.load_reference_class()
-    assert cls.__module__ == "lib.bundle_adjustment" and "oracle/_ref" in cls.__init__.__code__.co_filename
+    assert cls.__module__ == "lib.bundle_adjustment" and cls.__init__.__code__.co_filename.startswith(str(dst))
+    assert cls is not ba_b200.BundleAdjuster and cls("x").x == "x"
 
 
 def test_reference_copy_detects_modification(tmp_path, monkeypatch):
-    if not build_ref.available():
-        pytest.skip("oracle/_ref not built")
-    import shutil
-
     dst = tmp_path / "_ref"
-    shutil.copytree(build_ref.REF_DST, dst)
+    monkeypatch.setattr(build_ref, "REF_SRC", str(_stand_in_reference(tmp_path / "reference")))
     monkeypatch.setattr(build_ref, "REF_DST", str(dst))
+    build_ref.build()
     assert build_ref.verify()
     with open(dst / "lib" / "utils.py", "a") as f:
         f.write("\n# edited\n")

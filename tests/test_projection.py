@@ -57,26 +57,34 @@ def test_cuda_projection_rejects_bad_shapes():
         ba_b200.calc_projected_points(np.zeros((4, 2)), np.zeros((2, 3, 3)), np.zeros((2, 3, 3)), np.zeros((2, 3)))
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/lib"), reason="needs the reference checkout (build container only)")
-def test_shadow_camera_module_keeps_reference_code_and_swaps_projection():
+def test_shadow_camera_module_keeps_reference_code_and_swaps_projection(tmp_path):
     """With this package's directory before the reference on sys.path, `lib.camera` is the
-    reference's module except for `calc_projected_points` (SURVEY.md section 8b / 8f)."""
+    reference's module except for `calc_projected_points` (SURVEY.md section 8b / 8f); checked with a
+    stand-in for the reference's lib/camera.py, whose names and module-internal calls must survive."""
     import importlib
     import sys
 
     import ba_b200
 
+    ref = tmp_path / "ref" / "lib"
+    ref.mkdir(parents=True)
+    (ref / "camera.py").write_text(
+        "class Camera:\n"
+        "    @staticmethod\n"
+        "    def create(pos, target, f=1, f0=1):\n        return 'reference camera'\n"
+        "def calc_projected_points(X, K, R, t):\n    return 'reference'\n"
+        "def get_camera_parames(cameras):\n    return calc_projected_points(None, None, None, None)\n")
     saved = {k: sys.modules.pop(k) for k in list(sys.modules) if k == "lib" or k.startswith("lib.")}
     saved_path = list(sys.path)
-    sys.path.insert(0, "/root/reference")
+    sys.path.insert(0, str(tmp_path / "ref"))
     sys.path.insert(0, ba_b200.PACKAGE_DIR)
     try:
         mod = importlib.import_module("lib.camera")
         assert mod.calc_projected_points is ba_b200.calc_projected_points
-        cam = mod.Camera.create((0, 0, -1), (0, 0, 1), f=1)  # the reference's own class and self-test (:104-107)
-        X = np.array([[0, 0, 0], [1, 0, 0], [0, 1, 0], [0, 0, 1]], dtype=float)
-        np.testing.assert_array_almost_equal(cam.project_points(X), np.array([[0, 0], [1, 0], [0, 1], [0, 0]]))
+        assert mod.Camera.create((0, 0, -1), (0, 0, 1), f=1) == "reference camera"
         assert mod.get_camera_parames.__module__ == "lib._reference_camera"
+        # the reference's own functions keep calling the reference's projection
+        assert mod.get_camera_parames([]) == "reference"
     finally:
         sys.path[:] = saved_path
         for k in [k for k in sys.modules if k == "lib" or k.startswith("lib.")]:
