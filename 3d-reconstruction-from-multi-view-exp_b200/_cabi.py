@@ -92,6 +92,8 @@ SIGNATURES = {
     "ba_matrix_free": (C.c_int, [_P]),
     "ba_syrk_plan_info": (C.c_int, [C.c_int, C.c_int64, C.c_int, C.c_int, C.POINTER(C.c_int), C.POINTER(C.c_int),
                                     C.POINTER(C.c_double), C.POINTER(C.c_double)]),
+    "ba_syrk_emu_info": (C.c_int, [C.c_int64, C.POINTER(C.c_int32), C.POINTER(C.c_int), C.POINTER(C.c_int)]),
+    "ba_syrk_emulated": (C.c_int, [_P]),
     "ba_projective_depth_primary": (C.c_int, [C.c_int, C.c_int64, C.c_int32, _P, C.c_double, C.c_double, C.c_int,
                                               _P, _P, C.POINTER(C.c_int), C.c_int, _P]),
     "ba_projective_depth_dual": (C.c_int, [C.c_int, C.c_int64, C.c_int32, _P, C.c_double, C.c_double, C.c_int,

@@ -63,8 +63,9 @@ struct CamState {
   double* t = nullptr;  // [M][3]
 };
 
-// "k3" brackets the whole Schur phase; "syrk" only the DMMA kernel inside it (nested scopes
-// use their own event pair).
+// "k3" brackets the whole Schur phase; "syrk" only the dense product inside it (the DMMA kernels, or
+// the INT8 emulation's conversion, product and reconstruction kernels; nested scopes use their own
+// event pair).
 enum ProfGroup { PG_K1 = 0, PG_K2, PG_K3, PG_K4, PG_COST, PG_OTHER, PG_SYRK, PG_CHOL, PG_COMM, PG_COUNT };
 
 // One CTA of the dense Schur product: tile (ti, tj) of P and the k-chunks [c_lo, c_hi) of Y^T.
@@ -72,6 +73,12 @@ struct SyrkItem {
   int ti, tj, c_lo, c_hi;
   int slot2;  // >= 0: a "tall" item also computes the ragged rows below its tile (the thin tile
               // (ti + 1, tj)); their partial results go to this slot of the partial-tile store
+};
+
+// One CTA of the emulated Schur product: modulus `mod`, 128-tile (ti, tj) of P, 128-row k-blocks
+// [kb_lo, kb_hi) of the residue planes.
+struct EmuItem {
+  int mod, ti, tj, kb_lo, kb_hi;
 };
 
 struct Comm;  // peer-memory exchange of a sharded run (comm_peer.cu)
@@ -110,6 +117,14 @@ struct ba_engine {
   int* syrk_tile_first = nullptr;      // [syrk_n_tiles + 1]
   int* syrk_tile_items = nullptr;      // items of each tile in ascending k order
   int64_t k_pad = 0;  // padded 3N (rows of Yt)
+  // dense Schur product emulated on the INT8 tensor cores (k3_schur_syrk.cu): chosen at engine creation
+  int syrk_emu = 0;
+  int emu_bits = 0;                      // b: |scaled entry| <= 2^b, exact CRT lift for k_pad rows
+  int emu_n_items = 0;
+  ba::EmuItem* emu_items = nullptr;      // [emu_n_items] launch order
+  int8_t* Yq = nullptr;                  // [kEmuModuli][n_pad][k_pad] residue planes, K-major
+  uint32_t* Pmod = nullptr;              // [kEmuModuli][lower 128-tiles][128 cols][128 rows] residue sums
+  unsigned long long* colmax = nullptr;  // [n_pad] bit pattern of max |Yt[k][a]| over k
 
   // observations (CSR by point) and camera-major index
   int64_t* obs_ptr = nullptr;
@@ -376,6 +391,7 @@ int launch_k2b(ba_engine* e, bool conditional, double c_host, cudaStream_t s);
 bool dense_matrix_free(const ba_engine* e);  // dense K2b / point update re-derive the Jacobian rows
 int launch_k3(ba_engine* e, bool conditional, cudaStream_t s);
 int syrk_plan_engine(ba_engine* e);
+int syrk_emu_info(int64_t k_pad, int32_t* moduli, int* n_moduli, int* bits);
 int syrk_feed_is_tma();  // 1: the 128-tile SYRK is fed by TMA + mbarriers, 0: by cp.async (BA_SYRK_NO_TMA)
 // Gram matrix P = Yt^T Yt of a k-major operand outside an engine (k3_schur_syrk.cu)
 struct GramWorkspace {

@@ -278,7 +278,7 @@ static void free_engine(ba_engine* e) {
   void* ptrs[] = {e->obs_ptr, e->obs_cam, e->obs_pt, e->obs_xy, e->cam_ptr, e->cm_perm, e->bits, e->PT, e->pair_ptr, e->pair_pts, e->X[0],
                   e->X[1], e->cam[0].f, e->cam[1].f, e->camtab[0], e->camtab[1], e->JP, e->JC, e->V,
                   e->GPT, e->Upart, e->Uloc, e->LINV, e->Z, e->Yt, e->Ysp, e->red_in_window ? nullptr : e->red, e->Spart, e->Lt, e->Winv,
-                  e->dxi, e->cost_part, e->cost_buf, e->ctl, e->rec, e->ywork, e->chol_bar, e->gauge, e->syrk_items, e->syrk_tile_first, e->syrk_tile_items, e->syrk_cta_first};
+                  e->dxi, e->cost_part, e->cost_buf, e->ctl, e->rec, e->ywork, e->chol_bar, e->gauge, e->syrk_items, e->syrk_tile_first, e->syrk_tile_items, e->syrk_cta_first, e->emu_items, e->Yq, e->Pmod, e->colmax};
   for (void* p : ptrs)
     dev_free(p);
   for (int k = 0; k < 2; ++k) {
@@ -936,5 +936,10 @@ int ba_syrk_plan_info(int n_cams, int64_t n_points, int tile, int num_sms, int* 
                       double* makespan_rows, double* ideal_rows) {
   return syrk_plan_selftest(n_cams, n_points, tile, num_sms, n_items, n_tiles, makespan_rows, ideal_rows);
 }
+
+int ba_syrk_emu_info(int64_t k_pad, int32_t* moduli, int* n_moduli, int* bits) {
+  return syrk_emu_info(k_pad, moduli, n_moduli, bits);
+}
+int ba_syrk_emulated(ba_engine* e) { return e && e->dense && e->syrk_emu ? 1 : 0; }
 
 }  // extern "C"

@@ -17,6 +17,13 @@
 //
 // Compute roofline (FP64 tensor): algorithmic flops = 3N * n (n + 1), n = 9M - 7.
 //
+// Large dense products (C3: n_pad^2 k_pad = 9.8e11) run instead on the INT8 tensor cores, FP64-accurate
+// through the modular Ozaki scheme (see "FP64-accurate product on the INT8 tensor cores" below):
+// emu_colmax_kernel and emu_residue_kernel turn Yt into 16 int8 residue planes, syrk_i8_kernel
+// (tcgen05.mma kind::i8) forms one SYRK per modulus, emu_reconstruct_kernel lifts the exact integer
+// products back to FP64 into P.  The DMMA kernels stay for smaller products (C2), the Cholesky's
+// trailing updates and the projective-depth Gram matrix.  BA_SYRK_EMU=0|1 overrides the size rule.
+//
 // Sparse visibility: see k3_schur_sparse.cu (output-stationary, no atomics).
 #include <cuda.h>  // CUtensorMap (types only: the encoder is fetched through cudaGetDriverEntryPoint)
 
@@ -659,6 +666,337 @@ __global__ void stage_camera_blocks_kernel(int n, const double* __restrict__ src
   if (k < n) dst[k] = src[k];
 }
 
+// ---- FP64-accurate product on the INT8 tensor cores (Ozaki scheme II) -------------------------------
+// P = Yt^T Yt from exact integer products (Ozaki, Uchino, Imamura, "Ozaki Scheme II", 2025):
+//  1. every column a is scaled by 2^e_a so that |Yt[k][a]| 2^e_a < 2^b, and rounded to the integer
+//     a' = rint(Yt[k][a] 2^e_a) (|a'| <= 2^b <= 2^53: the rounding error is at most 2^-53 of the
+//     column's largest entry; a zero column gives a' = 0 and an exactly zero row of P);
+//  2. a' is reduced modulo L = 16 pairwise coprime moduli p_i <= 256 into int8 residue planes;
+//  3. one int8 SYRK per modulus on tcgen05 (kind::i8, int32 accumulators in tensor memory) gives
+//     sum_k a'_k b'_k mod p_i exactly -- int32 is exact over <= 131 071 k-rows, longer k ranges are
+//     split into items whose results are reduced mod p_i and summed with integer atomics (exact and
+//     order-independent, so P is bit-reproducible);
+//  4. Garner's mixed-radix conversion and the symmetric lift recover the integer dot product, exact
+//     while k_pad 2^(2b) < prod(p) / 2 (the host picks b accordingly: 53 up to k_pad ~ 2^19.4); it is
+//     converted to double by Horner from the most significant digit (16 fused multiply-adds of
+//     non-negative terms: relative error <= 16 u = 1.8e-15, exact below 2^53) and scaled by
+//     2^-(e_a + e_b), which is exact.
+constexpr int kEmuModuli = 16;
+constexpr int kEmuTile = 128;     // operand tile rows = M = N of the MMA
+constexpr int kEmuKB = 128;       // k-rows per pipeline stage: one 128-byte swizzle row of int8
+constexpr int kEmuStages = 3;     // x 32 KB: two CTAs per SM
+constexpr int kEmuThreads = 128;  // four warps: one per 32-lane quarter of tensor memory
+constexpr unsigned kEmuOpBytes = kEmuTile * kEmuKB;     // 16 384
+constexpr unsigned kEmuStageBytes = 2 * kEmuOpBytes;    // 32 768
+constexpr size_t kEmuSmemBytes = (size_t)kEmuStages * kEmuStageBytes + 1024 /*alignment*/ + 64 /*barriers*/;
+constexpr double kEmuMinWork = 1e11;  // n_pad^2 k_pad from which the emulation is the default
+constexpr int kEmuMaxKB = (int)(((1u << 31) - 1) / (128u * 128u) / kEmuKB);  // 1023 k-blocks: |sum| < 2^31
+// M = 128, S8 x S8 -> S32, both operands K-major (instruction descriptor of tcgen05.mma); N at bits 17..22
+constexpr uint32_t kEmuIdescM128 = (2u << 4) | (1u << 7) | (1u << 10) | ((uint32_t)(kEmuTile >> 4) << 24);
+
+__host__ __device__ constexpr int emu_modulus(int i) {
+  constexpr int p[kEmuModuli] = {256, 255, 253, 251, 247, 241, 239, 233, 229, 227, 223, 217, 211, 199, 197, 193};
+  return p[i];
+}
+
+// Garner's constants: inv[j][i] = p_j^-1 mod p_i (j < i); half[i]: mixed-radix digits of prod(p) / 2
+struct EmuConsts {
+  int inv[kEmuModuli][kEmuModuli];
+  int half[kEmuModuli];
+};
+
+// e_a for a column whose largest |entry| has the bit pattern `maxbits`: max 2^e_a < 2^b
+__device__ __forceinline__ int emu_exponent(unsigned long long maxbits, int b) {
+  if (maxbits == 0) return 0;
+  return b - 1 - ilogb(__longlong_as_double((long long)maxbits));
+}
+
+// Column maxima of |Yt| as bit patterns (the order of an integer max does not matter).
+__global__ void __launch_bounds__(128)
+emu_colmax_kernel(const double* __restrict__ Yt, int64_t k_pad, int n_pad, unsigned long long* __restrict__ colmax,
+                  const ba_lm_state* ctl) {
+  if (ctl && ctl->done) return;
+  const int a = 2 * (blockIdx.x * blockDim.x + threadIdx.x);
+  if (a >= n_pad) return;
+  const int64_t rows = (k_pad + gridDim.y - 1) / gridDim.y;
+  const int64_t k0 = (int64_t)blockIdx.y * rows, k1 = k0 + rows < k_pad ? k0 + rows : k_pad;
+  constexpr unsigned long long kAbs = 0x7FFFFFFFFFFFFFFFull;
+  unsigned long long m0 = 0, m1 = 0;
+#pragma unroll 8
+  for (int64_t k = k0; k < k1; ++k) {
+    const double2 v = __ldg(reinterpret_cast<const double2*>(Yt + k * n_pad + a));
+    m0 = max(m0, (unsigned long long)__double_as_longlong(v.x) & kAbs);
+    m1 = max(m1, (unsigned long long)__double_as_longlong(v.y) & kAbs);
+  }
+  if (m0) atomicMax(colmax + a, m0);
+  if (m1) atomicMax(colmax + a + 1, m1);
+}
+
+// Symmetric residue of the integer v (|v| <= 2^53) modulo p_I as an int in [-128, 127]: q = rint(v / p)
+// through the 1.5 * 2^52 rounding constant (|v / p| < 2^46), r = v - p q exact.  1 / p is rounded, so
+// q can miss the nearest integer by one when v / p lies within 0.0052 of a half: |r| <= 128.8.
+// (Called from fully unrolled loops: p and 1 / p are compile-time constants.)
+__device__ __forceinline__ int emu_residue(double v, int i) {
+  const double p = (double)emu_modulus(i), inv = 1.0 / p, magic = 6755399441055744.0;
+  const double q = __dadd_rn(__fma_rn(v, inv, magic), -magic);
+  const double r = __fma_rn(-p, q, v);
+  const int ri = __double2loint(__dadd_rn(r, magic));
+  return ri > 127 ? ri - (int)p : ri;
+}
+
+// Residue planes Yq[i][a][k] (K-major) from Yt[k][a]: a block converts 64 k-rows x 32 columns,
+// transposing through shared memory -- rows are read as 256-byte segments, plane rows written as
+// 64-byte segments.  48 KB of shared memory and <= 64 registers: four blocks (32 warps) per SM.
+constexpr int kResTK = 64, kResTA = 32, kResThreads = 256;
+constexpr size_t kResSmemBytes = (size_t)kResTK * kResTA * sizeof(double) + (size_t)kEmuModuli * kResTA * kResTK;
+
+__global__ void __launch_bounds__(kResThreads, 4)
+emu_residue_kernel(const double* __restrict__ Yt, int64_t k_pad, int n_pad, const unsigned long long* __restrict__ colmax,
+                   int bits, int8_t* __restrict__ Yq, const ba_lm_state* ctl) {
+  if (ctl && ctl->done) return;
+  extern __shared__ __align__(16) unsigned char res_smem[];
+  double* sIn = reinterpret_cast<double*>(res_smem);  // [64 k][32 a]
+  uint2* sOut = reinterpret_cast<uint2*>(res_smem + kResTK * kResTA * sizeof(double));  // [16][32 a][8 x 8 bytes]
+  const int64_t k0 = (int64_t)blockIdx.x * kResTK;
+  const int a0 = blockIdx.y * kResTA;
+  const int t = threadIdx.x;
+  for (int q = t; q < kResTK * kResTA / 2; q += kResThreads) {
+    const int row = q / (kResTA / 2), cp = q % (kResTA / 2);
+    const int a = a0 + 2 * cp;
+    const int64_t k = k0 + row;
+    double2 v = make_double2(0.0, 0.0);
+    if (k < k_pad && a < n_pad) v = __ldg(reinterpret_cast<const double2*>(Yt + k * n_pad + a));
+    reinterpret_cast<double2*>(sIn)[q] = v;
+  }
+  __syncthreads();
+  // thread: column a0 + lane, k-rows 8 w .. 8 w + 7; its 8 residues of a plane are one 8-byte piece,
+  // stored at piece w ^ (lane & 6) of the column's 64-byte row (the XOR keeps the two pieces of every
+  // 16-byte chunk adjacent and in order, and spreads the stores over the banks)
+  const int lane = t & 31, w = t >> 5;
+  const int e = a0 + lane < n_pad ? emu_exponent(colmax[a0 + lane], bits) : 0;
+  double v[8];
+#pragma unroll
+  for (int j = 0; j < 8; ++j) v[j] = rint(ldexp(sIn[(8 * w + j) * kResTA + lane], e));
+#pragma unroll
+  for (int i = 0; i < kEmuModuli; ++i) {
+    uint32_t word[2];
+#pragma unroll
+    for (int u = 0; u < 2; ++u) {
+      const int r0 = emu_residue(v[4 * u], i), r1 = emu_residue(v[4 * u + 1], i);
+      const int r2 = emu_residue(v[4 * u + 2], i), r3 = emu_residue(v[4 * u + 3], i);
+      word[u] = __byte_perm(__byte_perm(r0, r1, 0x0040), __byte_perm(r2, r3, 0x0040), 0x5410);
+    }
+    sOut[(i * kResTA + lane) * 8 + (w ^ (lane & 6))] = make_uint2(word[0], word[1]);
+  }
+  __syncthreads();
+  // 16-byte chunks: 16 planes x 32 columns x 4 chunks, two planes per pass of the block
+  const int sa = (t >> 2) & 31, c = t & 3, ih = t >> 7;
+  const int ga = a0 + sa;
+  const int64_t gk = k0 + 16 * c;  // k_pad is a multiple of 32: a chunk is all in or all out
+  if (ga >= n_pad || gk >= k_pad) return;
+#pragma unroll
+  for (int i = ih; i < kEmuModuli; i += 2)
+    *reinterpret_cast<uint4*>(Yq + ((size_t)i * n_pad + ga) * k_pad + gk) =
+        *reinterpret_cast<const uint4*>(sOut + (i * kResTA + sa) * 8 + ((2 * c) ^ (sa & 6)));
+}
+
+__device__ __forceinline__ void tma_load_3d(unsigned dst, const CUtensorMap* map, int c0, int c1, int c2, unsigned bar) {
+  asm volatile(
+      "cp.async.bulk.tensor.3d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%2, %3, %4}], [%5];"
+      ::"r"(dst), "l"(map), "r"(c0), "r"(c1), "r"(c2), "r"(bar)
+      : "memory");
+}
+// Shared-memory descriptor of a K-major operand tile written by TMA with SWIZZLE_128B: rows of 128 bytes,
+// 8-row groups 1024 bytes apart (tile 1024-byte aligned); layout 2 = 128-byte swizzle, version 1.
+__device__ __forceinline__ uint64_t umma_desc_sw128(unsigned saddr) {
+  return (uint64_t)((saddr & 0x3FFFFu) >> 4) | ((uint64_t)1 << 16) | ((uint64_t)(1024 >> 4) << 32) |
+         ((uint64_t)1 << 46) | ((uint64_t)2 << 61);
+}
+__device__ __forceinline__ void umma_i8(unsigned tmem, uint64_t da, uint64_t db, uint32_t idesc, int accumulate) {
+  asm volatile(
+      "{\n .reg .pred p;\n setp.ne.b32 p, %4, 0;\n tcgen05.mma.cta_group::1.kind::i8 [%0], %1, %2, %3, p;\n}\n"
+      ::"r"(tmem), "l"(da), "l"(db), "r"(idesc), "r"(accumulate));
+}
+// arrive on the mbarrier once every tcgen05.mma issued so far by this thread has completed
+__device__ __forceinline__ void umma_commit(unsigned bar) {
+  asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(bar) : "memory");
+}
+// 32 consecutive columns of this warp's 32 tensor-memory lanes (one int32 accumulator row per lane)
+__device__ __forceinline__ void tmem_ld32(unsigned taddr, uint32_t (&v)[32]) {
+  asm volatile(
+      "tcgen05.ld.sync.aligned.32x32b.x32.b32 {%0, %1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15, %16, %17, %18, %19, %20, %21, %22, %23, %24, %25, %26, %27, %28, %29, %30, %31}, [%32];\n"
+      "tcgen05.wait::ld.sync.aligned;"
+      : "=r"(v[0]), "=r"(v[1]), "=r"(v[2]), "=r"(v[3]), "=r"(v[4]), "=r"(v[5]), "=r"(v[6]), "=r"(v[7]), "=r"(v[8]), "=r"(v[9]), "=r"(v[10]), "=r"(v[11]), "=r"(v[12]), "=r"(v[13]), "=r"(v[14]), "=r"(v[15]), "=r"(v[16]), "=r"(v[17]), "=r"(v[18]), "=r"(v[19]), "=r"(v[20]), "=r"(v[21]), "=r"(v[22]), "=r"(v[23]), "=r"(v[24]), "=r"(v[25]), "=r"(v[26]), "=r"(v[27]), "=r"(v[28]), "=r"(v[29]), "=r"(v[30]), "=r"(v[31])
+      : "r"(taddr)
+      : "memory");
+}
+
+// One CTA per item: the int8 SYRK of tile (ti, tj) of modulus `mod` over its k-blocks.  A ragged last
+// tile row (16 valid rows at 200 cameras) runs with N = its valid rows rounded up to 16: off the
+// diagonal the operands swap (A = tile tj, B = tile ti), so the MMA computes the transposed block.  Warp 0 lane 0
+// feeds a 3-stage TMA ring (one 3D copy per operand: 128 rows x 128 k of plane `mod`; a diagonal tile
+// loads one operand), warp 1 lane 0 issues four 128 x 128 x 32 MMAs per stage into a 128-column int32
+// accumulator in tensor memory and releases the stage through tcgen05.commit.  The four warps then
+// drain the accumulator (warp w owns rows 32 w ..), reduce it mod p and add it to the tile's residue
+// sums, stored column-major so that the lanes of a warp add to consecutive words.  Two CTAs share an
+// SM, so one CTA's drain overlaps the other's MMAs.
+__global__ void __launch_bounds__(kEmuThreads, 2)
+syrk_i8_kernel(const __grid_constant__ CUtensorMap planes, const EmuItem* __restrict__ items, uint32_t* __restrict__ Pmod,
+               int n_tiles, int n_valid, const ba_lm_state* ctl) {
+  if (ctl && ctl->done) return;
+  extern __shared__ unsigned char smem_raw[];
+  const unsigned base = (smem_u32(smem_raw) + 1023u) & ~1023u;
+  const unsigned bars = base + kEmuStages * kEmuStageBytes;
+  const unsigned done_bar = bars + 16u * kEmuStages, tmem_slot = done_bar + 8u;
+  auto full_bar = [&](int st) { return bars + 8u * st; };
+  auto empty_bar = [&](int st) { return bars + 8u * (kEmuStages + st); };
+  const EmuItem it = items[blockIdx.x];
+  const bool diag = it.ti == it.tj;
+  const int nkb = it.kb_hi - it.kb_lo;
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  const int vr = min(kEmuTile, n_valid - it.ti * kEmuTile);     // valid rows of tile row ti
+  const int c_end = min(kEmuTile, n_valid - it.tj * kEmuTile);  // valid columns of tile column tj
+  const int nN = vr < kEmuTile ? (vr + 15) & ~15 : kEmuTile;
+  const bool swap = nN < kEmuTile && !diag;
+  const int rowA = (swap ? it.tj : it.ti) * kEmuTile, rowB = (swap ? it.ti : it.tj) * kEmuTile;
+
+  if (threadIdx.x == 0) {
+    for (int st = 0; st < kEmuStages; ++st) {
+      mbar_init(full_bar(st), 1);
+      mbar_init(empty_bar(st), 1);
+    }
+    mbar_init(done_bar, 1);
+    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    asm volatile("prefetch.tensormap [%0];" ::"l"(&planes) : "memory");
+  }
+  if (warp == 0) {
+    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(tmem_slot), "r"(kEmuTile)
+                 : "memory");
+    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
+  }
+  asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+  __syncthreads();
+  asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+  unsigned tmem;
+  asm volatile("ld.shared.u32 %0, [%1];" : "=r"(tmem) : "r"(tmem_slot) : "memory");
+
+  if (warp == 0 && lane == 0) {
+    for (int kb = 0; kb < nkb; ++kb) {
+      const int st = kb % kEmuStages;
+      if (kb >= kEmuStages) mbar_wait(empty_bar(st), ((unsigned)(kb / kEmuStages) - 1u) & 1u);
+      const unsigned dst = base + (unsigned)st * kEmuStageBytes;
+      const int k0 = (it.kb_lo + kb) * kEmuKB;
+      mbar_arrive_expect_tx(full_bar(st), diag ? kEmuOpBytes : 2 * kEmuOpBytes);
+      tma_load_3d(dst, &planes, k0, rowA, it.mod, full_bar(st));
+      if (!diag) tma_load_3d(dst + kEmuOpBytes, &planes, k0, rowB, it.mod, full_bar(st));
+    }
+  } else if (warp == 1 && lane == 0) {
+    const uint32_t idesc = kEmuIdescM128 | ((uint32_t)(nN >> 3) << 17);
+    for (int kb = 0; kb < nkb; ++kb) {
+      const int st = kb % kEmuStages;
+      mbar_wait(full_bar(st), (unsigned)(kb / kEmuStages) & 1u);
+      asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+      const unsigned a = base + (unsigned)st * kEmuStageBytes;
+      const uint64_t da = umma_desc_sw128(a), db = diag ? da : umma_desc_sw128(a + kEmuOpBytes);
+#pragma unroll
+      for (int k = 0; k < kEmuKB / 32; ++k)  // 32 bytes of k per MMA: +2 in the 16-byte address field
+        umma_i8(tmem, da + 2u * k, db + 2u * k, idesc, (kb | k) != 0);
+      umma_commit(empty_bar(st));
+    }
+    umma_commit(done_bar);
+  }
+  __syncwarp();
+  mbar_wait(done_bar, 0);
+  asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+
+  const int p = emu_modulus(it.mod);
+  const int lr = warp * 32 + lane;  // accumulator row = tensor-memory lane
+  uint32_t* out = Pmod + ((size_t)it.mod * n_tiles + it.ti * (it.ti + 1) / 2 + it.tj) * (kEmuTile * kEmuTile);
+#pragma unroll 1
+  for (int c0 = 0; c0 < nN; c0 += 32) {
+    uint32_t v[32];
+    tmem_ld32(tmem + ((unsigned)(warp * 32) << 16) + (unsigned)c0, v);
+#pragma unroll
+    for (int j = 0; j < 32; ++j) {
+      const int r = swap ? c0 + j : lr, c = swap ? lr : c0 + j;  // tile-local position in P
+      // valid part of P; on a diagonal tile the pairs the DMMA path's reduce kernel writes
+      if (c0 + j >= nN || r >= vr || c >= c_end || (diag && c > (r | 1))) continue;
+      int m = (int)v[j] % p;
+      if (m < 0) m += p;
+      if (m) atomicAdd(out + (size_t)c * kEmuTile + r, (uint32_t)m);
+    }
+  }
+  asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+  __syncthreads();
+  if (warp == 0) {
+    asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem), "r"(kEmuTile) : "memory");
+  }
+}
+
+// The integer sum_k a'_k b'_k from its residue sums (Garner, symmetric lift) as a double (Horner from
+// the most significant digit; see the bound above).
+__device__ __forceinline__ double emu_lift(const uint32_t (&x)[kEmuModuli], const EmuConsts& C) {
+  int v[kEmuModuli];
+#pragma unroll
+  for (int i = 0; i < kEmuModuli; ++i) {
+    const unsigned p = (unsigned)emu_modulus(i);
+    unsigned t = x[i] % p;
+#pragma unroll
+    for (int j = 0; j < i; ++j) t = (t + 2u * p - (unsigned)v[j]) * (unsigned)C.inv[j][i] % p;
+    v[i] = (int)t;
+  }
+  // value >= prod(p) / 2: negative, -(prod(p) - value); prod(p) - 1 - value has the digits p_i - 1 - v_i
+  int cmp = 0;
+#pragma unroll
+  for (int i = kEmuModuli - 1; i >= 0; --i)
+    if (cmp == 0) cmp = v[i] > C.half[i] ? 1 : (v[i] < C.half[i] ? -1 : 0);
+  const bool neg = cmp >= 0;
+  double acc = 0.0;
+#pragma unroll
+  for (int i = kEmuModuli - 1; i >= 0; --i) {
+    const int d = neg ? emu_modulus(i) - 1 - v[i] + (i == 0 ? 1 : 0) : v[i];
+    acc = __fma_rn(acc, (double)emu_modulus(i), (double)d);
+  }
+  return neg ? -acc : acc;
+}
+
+// P[lower] from the residue sums: a block converts a 32 x 32 piece of a tile (read along the columns
+// of the column-major sums, written along the rows of P through shared memory).
+__global__ void __launch_bounds__(256)
+emu_reconstruct_kernel(const uint32_t* __restrict__ Pmod, int n_tiles, const unsigned long long* __restrict__ colmax,
+                       int bits, double* __restrict__ P, int ld, int n_valid, const EmuConsts C, const ba_lm_state* ctl) {
+  if (ctl && ctl->done) return;
+  __shared__ double s[32][33];
+  const int t = blockIdx.x;
+  int ti, tj;
+  tile_from_linear(t, ti, tj);
+  const int rb = blockIdx.y & 3, cb = blockIdx.y >> 2;
+  if (ti == tj && cb > rb) return;  // above the diagonal
+  const int tx = threadIdx.x & 31, ty = threadIdx.x >> 5;
+  const int R = ti * kEmuTile + rb * 32 + tx;
+  const int er = R < n_valid ? emu_exponent(colmax[R], bits) : 0;
+  for (int cc = ty; cc < 32; cc += 8) {
+    const int c = cb * 32 + cc, Cg = tj * kEmuTile + c;
+    double val = 0.0;
+    if (R < n_valid && Cg < n_valid) {
+      uint32_t x[kEmuModuli];
+#pragma unroll
+      for (int i = 0; i < kEmuModuli; ++i)
+        x[i] = Pmod[((size_t)i * n_tiles + t) * (kEmuTile * kEmuTile) + (size_t)c * kEmuTile + rb * 32 + tx];
+      val = ldexp(emu_lift(x, C), -(er + emu_exponent(colmax[Cg], bits)));
+    }
+    s[cc][tx] = val;
+  }
+  __syncthreads();
+  for (int rr = ty; rr < 32; rr += 8) {
+    const int r = rb * 32 + rr, c = cb * 32 + tx;
+    const int Rg = ti * kEmuTile + r, Cg = tj * kEmuTile + c;
+    if (Rg >= n_valid || Cg >= n_valid || (ti == tj && c > (r | 1))) continue;
+    P[(size_t)Rg * ld + Cg] = s[tx][rr];
+  }
+}
+
 // ---- host side --------------------------------------------------------------------------------
 static inline int syrk_kc(int tile) { return tile == 128 ? 32 : 16; }
 static inline int syrk_occupancy(int tile) { return tile == 128 ? 1 : 4; }
@@ -952,8 +1290,15 @@ static const SyrkPlan& cached_plan(int n_pad, int tile, int64_t k_pad, int num_s
 }
 
 // Plans the dense Schur product of this engine and uploads the work items.
+static int emu_plan_engine(ba_engine* e);
+int emu_bits_for(int64_t k_pad);
+static bool emu_select(const ba_engine* e);
+
 int syrk_plan_engine(ba_engine* e) {
   if (!e->dense) return BA_OK;
+  e->emu_bits = emu_bits_for(e->k_pad);
+  e->syrk_emu = emu_select(e) ? 1 : 0;
+  if (e->syrk_emu) return emu_plan_engine(e);
   const SyrkPlan& plan = cached_plan(e->n_pad, e->syrk_tile, e->k_pad, e->num_sms);
   e->syrk_n_items = (int)plan.items.size();
   e->syrk_n_ctas = plan.cta_first.empty() ? e->syrk_n_items : (int)plan.cta_first.size() - 1;
@@ -1024,6 +1369,148 @@ static bool syrk_use_tma() {
 }
 
 int syrk_feed_is_tma() { return syrk_use_tma() && tensor_map_encoder() != nullptr; }
+
+// ---- emulated product: host side ------------------------------------------------------------------
+static const EmuConsts& emu_consts() {
+  static const EmuConsts c = [] {
+    EmuConsts k{};
+    for (int i = 0; i < kEmuModuli; ++i)
+      for (int j = 0; j < i; ++j) {
+        const int p = emu_modulus(i), a = emu_modulus(j) % p;
+        int x = 1;
+        while (a * x % p != 1) ++x;  // p < 257: a search is enough
+        k.inv[j][i] = x;
+      }
+    unsigned __int128 h = 1;
+    for (int i = 0; i < kEmuModuli; ++i) h *= (unsigned)emu_modulus(i);
+    h /= 2;
+    for (int i = 0; i < kEmuModuli; ++i) {
+      k.half[i] = (int)(h % (unsigned)emu_modulus(i));
+      h /= (unsigned)emu_modulus(i);
+    }
+    return k;
+  }();
+  return c;
+}
+
+// Largest b <= 53 with k_pad 2^(2b) < prod(p) / 2: the CRT lift of a dot product of k_pad terms of
+// magnitude <= 2^b each is then exact.  0 if there is none.
+int emu_bits_for(int64_t k_pad) {
+  unsigned __int128 half = 1;
+  for (int i = 0; i < kEmuModuli; ++i) half *= (unsigned)emu_modulus(i);
+  half /= 2;
+  for (int b = 53; b > 0; --b)
+    if ((unsigned __int128)k_pad < (half >> (2 * b))) return b;  // k_pad 2^(2b) < half, whole multiples of 2^(2b)
+  return 0;
+}
+
+// The emulation is chosen when it is exact to (nearly) full FP64 input precision and the product is
+// large enough for the INT8 tensor cores to pay for the conversion passes.  BA_SYRK_EMU=0|1 overrides
+// the size rule (A/B timing and tests); it is read when an engine is created.
+int syrk_emu_info(int64_t k_pad, int32_t* moduli, int* n_moduli, int* bits) {
+  if (k_pad < 1) { set_error("k_pad must be positive"); return BA_ERR_INVALID; }
+  if (moduli)
+    for (int i = 0; i < kEmuModuli; ++i) moduli[i] = emu_modulus(i);
+  if (n_moduli) *n_moduli = kEmuModuli;
+  if (bits) *bits = emu_bits_for(k_pad);
+  return BA_OK;
+}
+
+static bool emu_select(const ba_engine* e) {
+  if (const char* v = std::getenv("BA_SYRK_EMU")) return std::atoi(v) != 0;
+  return e->emu_bits >= 50 && tensor_map_encoder() != nullptr &&
+         (double)e->n_pad * e->n_pad * (double)e->k_pad >= kEmuMinWork;
+}
+
+// Work items: every (modulus, lower 128-tile) over P equal k pieces of <= kEmuMaxKB blocks.  Every
+// item costs the same per k-block, so the plan only picks P for whole waves of two CTAs per SM, and
+// orders the items k-piece first (as plan_syrk does: the CTAs in flight share one k-slab in the L2).
+static std::vector<EmuItem> plan_emu(int n_pad, int64_t k_pad, int num_sms) {
+  const int nt1 = (n_pad + kEmuTile - 1) / kEmuTile;
+  const int64_t n_tiles = nt1 * (nt1 + 1) / 2;
+  const int64_t nkb = (k_pad + kEmuKB - 1) / kEmuKB;
+  const int64_t slots = 2 * (int64_t)num_sms;
+  const int64_t p_min = (nkb + kEmuMaxKB - 1) / kEmuMaxKB;
+  const double overhead = 16.0;  // k-blocks: pipeline fill and the accumulator drain
+  int64_t best_p = p_min;
+  double best = 1e300;
+  for (int64_t p = p_min; p <= std::min<int64_t>(nkb, p_min + 8); ++p) {
+    const int64_t items = kEmuModuli * n_tiles * p, waves = (items + slots - 1) / slots;
+    const double t = (double)waves * ((double)((nkb + p - 1) / p) + overhead);
+    if (t < best * (1.0 - 1e-9)) { best = t; best_p = p; }
+  }
+  const int64_t per = (nkb + best_p - 1) / best_p;
+  std::vector<EmuItem> items;
+  for (int64_t lo = 0; lo < nkb; lo += per)
+    for (int m = 0; m < kEmuModuli; ++m)
+      for (int ti = 0; ti < nt1; ++ti)
+        for (int tj = 0; tj <= ti; ++tj) items.push_back({m, ti, tj, (int)lo, (int)std::min<int64_t>(nkb, lo + per)});
+  return items;
+}
+
+static int emu_plan_engine(ba_engine* e) {
+  const std::vector<EmuItem> items = plan_emu(e->n_pad, e->k_pad, e->num_sms);
+  const int nt1 = (e->n_pad + kEmuTile - 1) / kEmuTile;
+  e->syrk_n_tiles = nt1 * (nt1 + 1) / 2;
+  e->emu_n_items = (int)items.size();
+  const cudaStream_t s0 = (cudaStream_t)0;
+  BA_CUDA(cudaMallocAsync(reinterpret_cast<void**>(&e->emu_items), items.size() * sizeof(EmuItem), s0));
+  BA_CUDA(cudaMallocAsync(reinterpret_cast<void**>(&e->Yq), (size_t)kEmuModuli * e->n_pad * e->k_pad, s0));
+  BA_CUDA(cudaMallocAsync(reinterpret_cast<void**>(&e->Pmod),
+                          (size_t)kEmuModuli * e->syrk_n_tiles * kEmuTile * kEmuTile * sizeof(uint32_t), s0));
+  BA_CUDA(cudaMallocAsync(reinterpret_cast<void**>(&e->colmax), (size_t)e->n_pad * sizeof(unsigned long long), s0));
+  BA_CUDA(cudaMemcpy(e->emu_items, items.data(), items.size() * sizeof(EmuItem), cudaMemcpyHostToDevice));
+  if (std::getenv("BA_TIMING"))
+    std::fprintf(stderr, "[ba syrk plan] int8 emulation: b = %d, %d tiles x %d moduli, %d items\n", e->emu_bits,
+                 e->syrk_n_tiles, kEmuModuli, e->emu_n_items);
+  return BA_OK;
+}
+
+// The residue planes as one 3D tensor {k, row, plane} of bytes; boxes of 128 k x 128 rows of one plane
+// (rows beyond n_pad are zero-filled), 128-byte swizzle: the canonical K-major operand of tcgen05.mma.
+static int make_plane_map(CUtensorMap* map, const int8_t* Yq, int n_pad, int64_t k_pad) {
+  EncodeTiledFn enc = tensor_map_encoder();
+  if (!enc) { set_error("cuTensorMapEncodeTiled is not available from this driver"); return BA_ERR_CUDA; }
+  const cuuint64_t gdim[3] = {(cuuint64_t)k_pad, (cuuint64_t)n_pad, (cuuint64_t)kEmuModuli};
+  const cuuint64_t gstride[2] = {(cuuint64_t)k_pad, (cuuint64_t)k_pad * n_pad};
+  const cuuint32_t box[3] = {(cuuint32_t)kEmuKB, (cuuint32_t)kEmuTile, 1};
+  const cuuint32_t estride[3] = {1, 1, 1};
+  const CUresult r = enc(map, CU_TENSOR_MAP_DATA_TYPE_UINT8, 3, const_cast<int8_t*>(Yq), gdim, gstride, box, estride,
+                         CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
+                         CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+  if (r != CUDA_SUCCESS) {
+    set_error("cuTensorMapEncodeTiled failed (%d) for %d residue planes of %d x %lld", (int)r, kEmuModuli, n_pad,
+              (long long)k_pad);
+    return BA_ERR_CUDA;
+  }
+  return BA_OK;
+}
+
+static int launch_syrk_emu(ba_engine* e, const ba_lm_state* ctl, cudaStream_t s) {
+  CUtensorMap map;
+  BA_TRY(make_plane_map(&map, e->Yq, e->n_pad, e->k_pad));
+  BA_CUDA(cudaFuncSetAttribute(emu_residue_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kResSmemBytes));
+  BA_CUDA(cudaFuncSetAttribute(syrk_i8_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kEmuSmemBytes));
+  const int n_tiles = e->syrk_n_tiles;
+  ProfScope ps(e, PG_SYRK, s);
+  BA_CUDA(cudaMemsetAsync(e->colmax, 0, (size_t)e->n_pad * sizeof(unsigned long long), s));
+  BA_CUDA(cudaMemsetAsync(e->Pmod, 0, (size_t)kEmuModuli * n_tiles * kEmuTile * kEmuTile * sizeof(uint32_t), s));
+  {
+    const int gx = (e->n_pad / 2 + 127) / 128;
+    const int64_t gy = std::max<int64_t>(1, std::min<int64_t>(e->k_pad / 64, (int64_t)16 * e->num_sms / gx));
+    emu_colmax_kernel<<<dim3(gx, (unsigned)gy), 128, 0, s>>>(e->Yt, e->k_pad, e->n_pad, e->colmax, ctl);
+    BA_LAUNCH_CHECK();
+  }
+  emu_residue_kernel<<<dim3((unsigned)((e->k_pad + kResTK - 1) / kResTK), (e->n_pad + kResTA - 1) / kResTA),
+                       kResThreads, kResSmemBytes, s>>>(e->Yt, e->k_pad, e->n_pad, e->colmax, e->emu_bits, e->Yq, ctl);
+  BA_LAUNCH_CHECK();
+  syrk_i8_kernel<<<e->emu_n_items, kEmuThreads, kEmuSmemBytes, s>>>(map, e->emu_items, e->Pmod, n_tiles, e->n_pad, ctl);
+  BA_LAUNCH_CHECK();
+  emu_reconstruct_kernel<<<dim3(n_tiles, 16), 256, 0, s>>>(e->Pmod, n_tiles, e->colmax, e->emu_bits, e->P(), e->n_pad,
+                                                          e->n_pad, emu_consts(), ctl);
+  BA_LAUNCH_CHECK();
+  return BA_OK;
+}
 
 template <int TILE, int WR, int WC, int KC>
 static int launch_syrk(ba_engine* e, const ba_lm_state* ctl, cudaStream_t s) {
@@ -1117,6 +1604,7 @@ int launch_k3(ba_engine* e, bool conditional, cudaStream_t s) {
     BA_LAUNCH_CHECK();
   }
   if (e->dense) {
+    if (e->syrk_emu) return launch_syrk_emu(e, ctl, s);
     if (e->syrk_tile == 128) return launch_syrk<128, 4, 4, 32>(e, ctl, s);
     return launch_syrk<64, 2, 2, 16>(e, ctl, s);
   }

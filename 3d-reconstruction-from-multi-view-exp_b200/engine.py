@@ -306,6 +306,10 @@ class Engine:
         """Dense scene linearised matrix-free (Jacobian rows re-derived where they are used)."""
         return bool(self._lib.ba_matrix_free(self._h))
 
+    def syrk_emulated(self) -> bool:
+        """Dense Schur product on the INT8 tensor cores (Ozaki scheme II) rather than DMMA."""
+        return bool(self._lib.ba_syrk_emulated(self._h))
+
     def profile(self) -> dict:
         out = {}
         for g in ("k1", "k2", "k3", "k4", "cost", "other", "syrk", "chol", "comm"):
@@ -325,6 +329,16 @@ def fp64_peak(device: int = 0, dmma=True) -> float:
     mode = int(dmma) if isinstance(dmma, int) and not isinstance(dmma, bool) and dmma >= 2 else (1 if dmma else 0)
     _cabi.check(_cabi.load().ba_fp64_peak(device, mode, C.byref(v)))
     return v.value
+
+
+def syrk_emu_info(k_pad: int) -> tuple[list[int], int]:
+    """Moduli of the INT8 emulation of the Schur product and the bits b kept per entry for k_pad rows."""
+    lib = _cabi.load()
+    n, b = C.c_int(), C.c_int()
+    _cabi.check(lib.ba_syrk_emu_info(int(k_pad), None, C.byref(n), None))
+    arr = (C.c_int32 * n.value)()
+    _cabi.check(lib.ba_syrk_emu_info(int(k_pad), arr, C.byref(n), C.byref(b)))
+    return list(arr), b.value
 
 
 def syrk_feed() -> str:

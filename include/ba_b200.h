@@ -263,6 +263,13 @@ int ba_matrix_free(ba_engine* e);
  * the perfectly balanced one (both in k-rows of a full tile per SM). */
 int ba_syrk_plan_info(int n_cams, int64_t n_points, int tile, int num_sms, int* n_items, int* n_tiles,
                       double* makespan_rows, double* ideal_rows);
+/* Host-only: the dense Schur product emulated on the INT8 tensor cores (Ozaki scheme II) -- the
+ * moduli (moduli[0 .. *n_moduli), pass null to query the count) and b, the bits every scaled entry
+ * keeps for a product over k_pad rows (largest b <= 53 with k_pad 2^(2b) < prod(moduli) / 2). */
+int ba_syrk_emu_info(int64_t k_pad, int32_t* moduli, int* n_moduli, int* bits);
+/* 1 when this engine's dense Schur product runs on the INT8 tensor cores (chosen at creation by size,
+ * or by BA_SYRK_EMU=0|1), 0 when on the FP64 tensor cores or sparse. */
+int ba_syrk_emulated(ba_engine* e);
 
 /* ---- next to the path: batched re-projection ------------------------------------------- */
 /* calc_projected_points (reference lib/camera.py:74-81, Camera.project_points :18-32): project
