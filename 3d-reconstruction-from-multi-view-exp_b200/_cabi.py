@@ -23,7 +23,7 @@ BA_AXIS_X_RIGHT, BA_AXIS_X_UP = 0, 1
 AXIS_CODES = {"x-right_z-forward": BA_AXIS_X_RIGHT, "x-up_z-forward": BA_AXIS_X_UP}
 
 BUFFERS = {"JP": 0, "JC": 1, "V": 2, "GPT": 3, "U": 4, "GCAM": 5, "S": 6, "DXI": 7, "LINV": 8,
-           "Z": 9, "REDUCE": 10, "COST": 11}
+           "Z": 9, "REDUCE": 10, "COST": 11, "YT": 12}
 
 
 class Problem(C.Structure):

@@ -75,8 +75,8 @@ struct SyrkItem {
               // (ti + 1, tj)); their partial results go to this slot of the partial-tile store
 };
 
-// One CTA of the emulated Schur product: modulus `mod`, 128-tile (ti, tj) of P, 128-row k-blocks
-// [kb_lo, kb_hi) of the residue planes.
+// One two-CTA cluster of the emulated Schur product: modulus `mod`, 256-tile (ti, tj) of P, 128-row
+// k-blocks [kb_lo, kb_hi) of the residue planes.
 struct EmuItem {
   int mod, ti, tj, kb_lo, kb_hi;
 };
@@ -121,6 +121,7 @@ struct ba_engine {
   int syrk_emu = 0;
   int emu_bits = 0;                      // b: |scaled entry| <= 2^b, exact CRT lift for k_pad rows
   int emu_n_items = 0;
+  int emu_n_full = 0;                    // items of whole 256-row tile rows; the ragged row's items follow
   ba::EmuItem* emu_items = nullptr;      // [emu_n_items] launch order
   int8_t* Yq = nullptr;                  // [kEmuModuli][n_pad][k_pad] residue planes, K-major
   uint32_t* Pmod = nullptr;              // [kEmuModuli][lower 128-tiles][128 cols][128 rows] residue sums

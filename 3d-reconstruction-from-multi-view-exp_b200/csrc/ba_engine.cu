@@ -861,6 +861,9 @@ static int buffer_info(ba_engine* e, int id, const double** p, int64_t* n) {
     case BA_BUF_Z: *p = e->Z; *n = 3 * e->N; break;
     case BA_BUF_REDUCE: *p = e->red; *n = e->red_len; break;
     case BA_BUF_COST: *p = e->cost_buf; *n = 4; break;
+    case BA_BUF_YT:
+      if (!e->dense) { set_error("buffer YT exists on dense engines only"); return BA_ERR_INVALID; }
+      *p = e->Yt; *n = e->k_pad * e->n_pad; break;
     default: set_error("unknown buffer id %d", id); return BA_ERR_INVALID;
   }
   return BA_OK;

@@ -19,8 +19,8 @@
 //
 // Large dense products (C3: n_pad^2 k_pad = 9.8e11) run instead on the INT8 tensor cores, FP64-accurate
 // through the modular Ozaki scheme (see "FP64-accurate product on the INT8 tensor cores" below):
-// emu_colmax_kernel and emu_residue_kernel turn Yt into 16 int8 residue planes, syrk_i8_kernel
-// (tcgen05.mma kind::i8) forms one SYRK per modulus, emu_reconstruct_kernel lifts the exact integer
+// emu_colmax_kernel and emu_residue_kernel turn Yt into 16 int8 residue planes, syrk_i8_pair_kernel
+// (tcgen05.mma kind::i8 on pairs of SMs) forms one SYRK per modulus, emu_reconstruct_kernel lifts the exact integer
 // products back to FP64 into P.  The DMMA kernels stay for smaller products (C2), the Cholesky's
 // trailing updates and the projective-depth Gram matrix.  BA_SYRK_EMU=0|1 overrides the size rule.
 //
@@ -682,17 +682,18 @@ __global__ void stage_camera_blocks_kernel(int n, const double* __restrict__ src
 //     non-negative terms: relative error <= 16 u = 1.8e-15, exact below 2^53) and scaled by
 //     2^-(e_a + e_b), which is exact.
 constexpr int kEmuModuli = 16;
-constexpr int kEmuTile = 128;     // operand tile rows = M = N of the MMA
+constexpr int kEmuTile = 128;     // rows of a residue-sum tile (Pmod) and of one CTA's operand box
+constexpr int kEmuPair = 256;     // rows of a work item's tile: M (and full N) of the two-CTA MMA
 constexpr int kEmuKB = 128;       // k-rows per pipeline stage: one 128-byte swizzle row of int8
-constexpr int kEmuStages = 3;     // x 32 KB: two CTAs per SM
+constexpr int kEmuStages = 3;     // x 32 KB (one CTA's half of a pair's operands): the most that leaves room for two CTAs per SM
 constexpr int kEmuThreads = 128;  // four warps: one per 32-lane quarter of tensor memory
 constexpr unsigned kEmuOpBytes = kEmuTile * kEmuKB;     // 16 384
 constexpr unsigned kEmuStageBytes = 2 * kEmuOpBytes;    // 32 768
 constexpr size_t kEmuSmemBytes = (size_t)kEmuStages * kEmuStageBytes + 1024 /*alignment*/ + 64 /*barriers*/;
 constexpr double kEmuMinWork = 1e11;  // n_pad^2 k_pad from which the emulation is the default
 constexpr int kEmuMaxKB = (int)(((1u << 31) - 1) / (128u * 128u) / kEmuKB);  // 1023 k-blocks: |sum| < 2^31
-// M = 128, S8 x S8 -> S32, both operands K-major (instruction descriptor of tcgen05.mma); N at bits 17..22
-constexpr uint32_t kEmuIdescM128 = (2u << 4) | (1u << 7) | (1u << 10) | ((uint32_t)(kEmuTile >> 4) << 24);
+// M = 256, S8 x S8 -> S32, both operands K-major (instruction descriptor of tcgen05.mma); N at bits 17..22
+constexpr uint32_t kEmuIdescM256 = (2u << 4) | (1u << 7) | (1u << 10) | ((uint32_t)(kEmuPair >> 4) << 24);
 
 __host__ __device__ constexpr int emu_modulus(int i) {
   constexpr int p[kEmuModuli] = {256, 255, 253, 251, 247, 241, 239, 233, 229, 227, 223, 217, 211, 199, 197, 193};
@@ -812,15 +813,6 @@ __device__ __forceinline__ uint64_t umma_desc_sw128(unsigned saddr) {
   return (uint64_t)((saddr & 0x3FFFFu) >> 4) | ((uint64_t)1 << 16) | ((uint64_t)(1024 >> 4) << 32) |
          ((uint64_t)1 << 46) | ((uint64_t)2 << 61);
 }
-__device__ __forceinline__ void umma_i8(unsigned tmem, uint64_t da, uint64_t db, uint32_t idesc, int accumulate) {
-  asm volatile(
-      "{\n .reg .pred p;\n setp.ne.b32 p, %4, 0;\n tcgen05.mma.cta_group::1.kind::i8 [%0], %1, %2, %3, p;\n}\n"
-      ::"r"(tmem), "l"(da), "l"(db), "r"(idesc), "r"(accumulate));
-}
-// arrive on the mbarrier once every tcgen05.mma issued so far by this thread has completed
-__device__ __forceinline__ void umma_commit(unsigned bar) {
-  asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(bar) : "memory");
-}
 // 32 consecutive columns of this warp's 32 tensor-memory lanes (one int32 accumulator row per lane)
 __device__ __forceinline__ void tmem_ld32(unsigned taddr, uint32_t (&v)[32]) {
   asm volatile(
@@ -831,34 +823,81 @@ __device__ __forceinline__ void tmem_ld32(unsigned taddr, uint32_t (&v)[32]) {
       : "memory");
 }
 
-// One CTA per item: the int8 SYRK of tile (ti, tj) of modulus `mod` over its k-blocks.  A ragged last
-// tile row (16 valid rows at 200 cameras) runs with N = its valid rows rounded up to 16: off the
-// diagonal the operands swap (A = tile tj, B = tile ti), so the MMA computes the transposed block.  Warp 0 lane 0
-// feeds a 3-stage TMA ring (one 3D copy per operand: 128 rows x 128 k of plane `mod`; a diagonal tile
-// loads one operand), warp 1 lane 0 issues four 128 x 128 x 32 MMAs per stage into a 128-column int32
-// accumulator in tensor memory and releases the stage through tcgen05.commit.  The four warps then
-// drain the accumulator (warp w owns rows 32 w ..), reduce it mod p and add it to the tile's residue
-// sums, stored column-major so that the lanes of a warp add to consecutive words.  Two CTAs share an
-// SM, so one CTA's drain overlaps the other's MMAs.
-__global__ void __launch_bounds__(kEmuThreads, 2)
-syrk_i8_kernel(const __grid_constant__ CUtensorMap planes, const EmuItem* __restrict__ items, uint32_t* __restrict__ Pmod,
-               int n_tiles, int n_valid, const ba_lm_state* ctl) {
-  if (ctl && ctl->done) return;
+__device__ __forceinline__ unsigned cluster_ctarank() {
+  unsigned r;
+  asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(r));
+  return r;
+}
+// address of the same shared-memory object in CTA `rank` of the cluster
+__device__ __forceinline__ unsigned mapa_shared(unsigned addr, unsigned rank) {
+  unsigned r;
+  asm volatile("mapa.shared::cluster.u32 %0, %1, %2;" : "=r"(r) : "r"(addr), "r"(rank));
+  return r;
+}
+__device__ __forceinline__ void cluster_sync() {
+  asm volatile("barrier.cluster.arrive.release.aligned;\nbarrier.cluster.wait.acquire.aligned;" ::: "memory");
+}
+// Copy into this CTA's shared memory; the bytes complete_tx on `bar`, which may be the peer CTA's mbarrier.
+__device__ __forceinline__ void tma_load_3d_pair(unsigned dst, const CUtensorMap* map, int c0, int c1, int c2,
+                                                 unsigned bar) {
+  asm volatile(
+      "cp.async.bulk.tensor.3d.cta_group::2.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%2, %3, %4}], [%5];"
+      ::"r"(dst), "l"(map), "r"(c0), "r"(c1), "r"(c2), "r"(bar)
+      : "memory");
+}
+__device__ __forceinline__ void umma_i8_pair(unsigned tmem, uint64_t da, uint64_t db, uint32_t idesc, int accumulate) {
+  asm volatile(
+      "{\n .reg .pred p;\n setp.ne.b32 p, %4, 0;\n tcgen05.mma.cta_group::2.kind::i8 [%0], %1, %2, %3, p;\n}\n"
+      ::"r"(tmem), "l"(da), "l"(db), "r"(idesc), "r"(accumulate));
+}
+// arrive on the mbarrier at this offset in both CTAs of the pair once the MMAs issued so far have completed
+__device__ __forceinline__ void umma_commit_pair(unsigned bar) {
+  asm volatile("tcgen05.commit.cta_group::2.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;"
+               ::"r"(bar), "h"((unsigned short)3) : "memory");
+}
+
+// One cluster of two CTAs (one per SM) per item: the int8 SYRK of 256-tile (ti, tj) of modulus `mod`
+// over its k-blocks, as tcgen05.mma.cta_group::2 with M = 256: CTA r of the pair holds rows
+// 128 r .. 128 r + 127 of the A tile and the r-th half of the N rows of B, and its tensor memory
+// receives rows 128 r .. of the 256 x N accumulator.  Per k-block an SM thus reads 32 KB for
+// 128 x 256 products (128 x 128 with one CTA per MMA).
+//   Full tile: A = rows 256 ti.., B = rows 256 tj.., N = 256; on the diagonal the B half of a CTA is
+//     its A rows, so it loads one operand (and the MMA also computes the 128 x 128 block above the
+//     diagonal, which is not stored).
+//   Ragged last tile row (ti = last, rv < 256 valid rows; all of P when n_pad < 256): N = rv rounded up
+//     to 16.  Off the diagonal the operands swap (A = tile tj, B = the ragged rows), so the MMA forms
+//     the transposed block and the few ragged rows cost a thin N instead of a 256-row A operand.
+//     Rows beyond n_pad lie outside the tensor and are zero-filled by the TMA unit.
+//   RAGGED selects the ragged row's items, which run as a launch of their own so that their time can be
+//   told apart (they reread the 256-row A tiles for a 256 x 16 product at C3).
+// Warp 0 lane 0 of each CTA feeds its half of a 3-stage TMA ring; the copies complete on the leader's
+// `full` barrier.  Warp 1 lane 0 of the leader issues four 256 x N x 32 MMAs per stage into an int32
+// accumulator in tensor memory and frees the stage in both CTAs with a multicast tcgen05.commit.  The
+// four warps of each CTA then drain its accumulator rows, reduce them mod p and add them to the residue
+// sums of the 128-tiles they belong to (the Pmod layout does not depend on this kernel's tiling).  Two
+// CTAs of different clusters share an SM, so one cluster's drain overlaps the other's MMAs.
+template <bool RAGGED>
+__global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kEmuThreads, 2)
+syrk_i8_pair_kernel(const __grid_constant__ CUtensorMap planes, const EmuItem* __restrict__ items,
+                    uint32_t* __restrict__ Pmod, int n_tiles, int n_valid, const ba_lm_state* ctl) {
+  if (ctl && ctl->done) return;  // uniform over the cluster
   extern __shared__ unsigned char smem_raw[];
+  // identical offsets in both CTAs: the leader's MMA descriptors address the peer's stages too
   const unsigned base = (smem_u32(smem_raw) + 1023u) & ~1023u;
   const unsigned bars = base + kEmuStages * kEmuStageBytes;
   const unsigned done_bar = bars + 16u * kEmuStages, tmem_slot = done_bar + 8u;
   auto full_bar = [&](int st) { return bars + 8u * st; };
   auto empty_bar = [&](int st) { return bars + 8u * (kEmuStages + st); };
-  const EmuItem it = items[blockIdx.x];
-  const bool diag = it.ti == it.tj;
+  const unsigned rank = cluster_ctarank();
+  const EmuItem it = items[blockIdx.x >> 1];
   const int nkb = it.kb_hi - it.kb_lo;
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const int vr = min(kEmuTile, n_valid - it.ti * kEmuTile);     // valid rows of tile row ti
-  const int c_end = min(kEmuTile, n_valid - it.tj * kEmuTile);  // valid columns of tile column tj
-  const int nN = vr < kEmuTile ? (vr + 15) & ~15 : kEmuTile;
-  const bool swap = nN < kEmuTile && !diag;
-  const int rowA = (swap ? it.tj : it.ti) * kEmuTile, rowB = (swap ? it.ti : it.tj) * kEmuTile;
+  const int rv = RAGGED ? n_valid - it.ti * kEmuPair : kEmuPair;  // valid rows of tile row ti
+  const int nN = (rv + 15) & ~15;
+  const bool swap = nN < kEmuPair && it.ti != it.tj;
+  const bool shared_op = nN == kEmuPair && it.ti == it.tj;  // B half of this CTA = its A rows
+  const int rowA = (swap ? it.tj : it.ti) * kEmuPair, rowB = (swap ? it.ti : it.tj) * kEmuPair;
+  const unsigned op_bytes = shared_op ? kEmuOpBytes : 2 * kEmuOpBytes;
 
   if (threadIdx.x == 0) {
     for (int st = 0; st < kEmuStages; ++st) {
@@ -869,13 +908,13 @@ syrk_i8_kernel(const __grid_constant__ CUtensorMap planes, const EmuItem* __rest
     asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
     asm volatile("prefetch.tensormap [%0];" ::"l"(&planes) : "memory");
   }
-  if (warp == 0) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(tmem_slot), "r"(kEmuTile)
+  if (warp == 0) {  // one warp of each CTA: the pair gets the same columns in both
+    asm volatile("tcgen05.alloc.cta_group::2.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(tmem_slot), "r"(kEmuPair)
                  : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
+    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::2.sync.aligned;" ::: "memory");
   }
   asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-  __syncthreads();
+  cluster_sync();  // barriers of both CTAs initialised before any copy or commit reaches them
   asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
   unsigned tmem;
   asm volatile("ld.shared.u32 %0, [%1];" : "=r"(tmem) : "r"(tmem_slot) : "memory");
@@ -885,52 +924,58 @@ syrk_i8_kernel(const __grid_constant__ CUtensorMap planes, const EmuItem* __rest
       const int st = kb % kEmuStages;
       if (kb >= kEmuStages) mbar_wait(empty_bar(st), ((unsigned)(kb / kEmuStages) - 1u) & 1u);
       const unsigned dst = base + (unsigned)st * kEmuStageBytes;
+      const unsigned full_leader = mapa_shared(full_bar(st), 0);
       const int k0 = (it.kb_lo + kb) * kEmuKB;
-      mbar_arrive_expect_tx(full_bar(st), diag ? kEmuOpBytes : 2 * kEmuOpBytes);
-      tma_load_3d(dst, &planes, k0, rowA, it.mod, full_bar(st));
-      if (!diag) tma_load_3d(dst + kEmuOpBytes, &planes, k0, rowB, it.mod, full_bar(st));
+      if (rank == 0) mbar_arrive_expect_tx(full_bar(st), 2 * op_bytes);  // both CTAs' copies
+      tma_load_3d_pair(dst, &planes, k0, rowA + (int)rank * kEmuTile, it.mod, full_leader);
+      if (!shared_op) tma_load_3d_pair(dst + kEmuOpBytes, &planes, k0, rowB + (int)rank * (nN / 2), it.mod, full_leader);
     }
-  } else if (warp == 1 && lane == 0) {
-    const uint32_t idesc = kEmuIdescM128 | ((uint32_t)(nN >> 3) << 17);
+  } else if (warp == 1 && lane == 0 && rank == 0) {
+    const uint32_t idesc = kEmuIdescM256 | ((uint32_t)(nN >> 3) << 17);
     for (int kb = 0; kb < nkb; ++kb) {
       const int st = kb % kEmuStages;
       mbar_wait(full_bar(st), (unsigned)(kb / kEmuStages) & 1u);
       asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
       const unsigned a = base + (unsigned)st * kEmuStageBytes;
-      const uint64_t da = umma_desc_sw128(a), db = diag ? da : umma_desc_sw128(a + kEmuOpBytes);
+      const uint64_t da = umma_desc_sw128(a), db = shared_op ? da : umma_desc_sw128(a + kEmuOpBytes);
 #pragma unroll
       for (int k = 0; k < kEmuKB / 32; ++k)  // 32 bytes of k per MMA: +2 in the 16-byte address field
-        umma_i8(tmem, da + 2u * k, db + 2u * k, idesc, (kb | k) != 0);
-      umma_commit(empty_bar(st));
+        umma_i8_pair(tmem, da + 2u * k, db + 2u * k, idesc, (kb | k) != 0);
+      umma_commit_pair(empty_bar(st));
     }
-    umma_commit(done_bar);
+    umma_commit_pair(done_bar);
   }
   __syncwarp();
   mbar_wait(done_bar, 0);
   asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
 
   const int p = emu_modulus(it.mod);
-  const int lr = warp * 32 + lane;  // accumulator row = tensor-memory lane
-  uint32_t* out = Pmod + ((size_t)it.mod * n_tiles + it.ti * (it.ti + 1) / 2 + it.tj) * (kEmuTile * kEmuTile);
+  const int lr = (int)rank * kEmuTile + warp * 32 + lane;  // accumulator row of the pair = A row - rowA
 #pragma unroll 1
   for (int c0 = 0; c0 < nN; c0 += 32) {
+    // above the diagonal from here on (unswapped: the columns grow with c0)
+    if (!swap && rowB + c0 > ((rowA + (int)rank * kEmuTile) | (kEmuTile - 1))) break;
     uint32_t v[32];
     tmem_ld32(tmem + ((unsigned)(warp * 32) << 16) + (unsigned)c0, v);
 #pragma unroll
     for (int j = 0; j < 32; ++j) {
-      const int r = swap ? c0 + j : lr, c = swap ? lr : c0 + j;  // tile-local position in P
-      // valid part of P; on a diagonal tile the pairs the DMMA path's reduce kernel writes
-      if (c0 + j >= nN || r >= vr || c >= c_end || (diag && c > (r | 1))) continue;
+      const int R = swap ? rowB + c0 + j : rowA + lr, C = swap ? rowA + lr : rowB + c0 + j;  // position in P
+      const int ti = R / kEmuTile, tj = C / kEmuTile, r = R % kEmuTile, c = C % kEmuTile;
+      // valid part of P; on a diagonal 128-tile the pairs the DMMA path's reduce kernel writes
+      if (c0 + j >= nN || R >= n_valid || C >= n_valid || tj > ti || (ti == tj && c > (r | 1))) continue;
       int m = (int)v[j] % p;
       if (m < 0) m += p;
-      if (m) atomicAdd(out + (size_t)c * kEmuTile + r, (uint32_t)m);
+      if (m)
+        atomicAdd(Pmod + ((size_t)it.mod * n_tiles + ti * (ti + 1) / 2 + tj) * (kEmuTile * kEmuTile) +
+                      (size_t)c * kEmuTile + r,
+                  (uint32_t)m);
     }
   }
   asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-  __syncthreads();
+  cluster_sync();  // both CTAs done with the accumulator columns before they are freed
   if (warp == 0) {
     asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem), "r"(kEmuTile) : "memory");
+    asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, %1;" ::"r"(tmem), "r"(kEmuPair) : "memory");
   }
 }
 
@@ -1422,37 +1467,50 @@ static bool emu_select(const ba_engine* e) {
          (double)e->n_pad * e->n_pad * (double)e->k_pad >= kEmuMinWork;
 }
 
-// Work items: every (modulus, lower 128-tile) over P equal k pieces of <= kEmuMaxKB blocks.  Every
-// item costs the same per k-block, so the plan only picks P for whole waves of two CTAs per SM, and
-// orders the items k-piece first (as plan_syrk does: the CTAs in flight share one k-slab in the L2).
-static std::vector<EmuItem> plan_emu(int n_pad, int64_t k_pad, int num_sms) {
-  const int nt1 = (n_pad + kEmuTile - 1) / kEmuTile;
-  const int64_t n_tiles = nt1 * (nt1 + 1) / 2;
-  const int64_t nkb = (k_pad + kEmuKB - 1) / kEmuKB;
-  const int64_t slots = 2 * (int64_t)num_sms;
+// Work items: every (modulus, lower 256-tile) over P equal k pieces of <= kEmuMaxKB blocks, in two
+// lists: the tiles of whole 256-row tile rows, and those of a ragged last tile row (launched apart).
+// Every item of a list costs about the same per k-block, so the plan only picks P for whole waves of
+// two clusters per pair of SMs, and orders the items k-piece first (as plan_syrk does: the clusters in
+// flight share one k-slab in the L2).
+struct EmuPlan {
+  std::vector<EmuItem> full, ragged;
+};
+static std::vector<EmuItem> plan_emu_list(int row_lo, int row_hi, int64_t nkb, int num_sms) {
+  int64_t n_tiles = 0;
+  for (int ti = row_lo; ti < row_hi; ++ti) n_tiles += ti + 1;
+  std::vector<EmuItem> items;
+  if (n_tiles == 0) return items;
+  const int64_t slots = num_sms;
   const int64_t p_min = (nkb + kEmuMaxKB - 1) / kEmuMaxKB;
   const double overhead = 16.0;  // k-blocks: pipeline fill and the accumulator drain
   int64_t best_p = p_min;
   double best = 1e300;
   for (int64_t p = p_min; p <= std::min<int64_t>(nkb, p_min + 8); ++p) {
-    const int64_t items = kEmuModuli * n_tiles * p, waves = (items + slots - 1) / slots;
+    const int64_t n = kEmuModuli * n_tiles * p, waves = (n + slots - 1) / slots;
     const double t = (double)waves * ((double)((nkb + p - 1) / p) + overhead);
     if (t < best * (1.0 - 1e-9)) { best = t; best_p = p; }
   }
   const int64_t per = (nkb + best_p - 1) / best_p;
-  std::vector<EmuItem> items;
   for (int64_t lo = 0; lo < nkb; lo += per)
     for (int m = 0; m < kEmuModuli; ++m)
-      for (int ti = 0; ti < nt1; ++ti)
+      for (int ti = row_lo; ti < row_hi; ++ti)
         for (int tj = 0; tj <= ti; ++tj) items.push_back({m, ti, tj, (int)lo, (int)std::min<int64_t>(nkb, lo + per)});
   return items;
 }
+static EmuPlan plan_emu(int n_pad, int64_t k_pad, int num_sms) {
+  const int full_rows = n_pad / kEmuPair, nt1 = (n_pad + kEmuPair - 1) / kEmuPair;
+  const int64_t nkb = (k_pad + kEmuKB - 1) / kEmuKB;
+  return {plan_emu_list(0, full_rows, nkb, num_sms), plan_emu_list(full_rows, nt1, nkb, num_sms)};
+}
 
 static int emu_plan_engine(ba_engine* e) {
-  const std::vector<EmuItem> items = plan_emu(e->n_pad, e->k_pad, e->num_sms);
+  const EmuPlan plan = plan_emu(e->n_pad, e->k_pad, e->num_sms);
+  std::vector<EmuItem> items = plan.full;
+  items.insert(items.end(), plan.ragged.begin(), plan.ragged.end());
   const int nt1 = (e->n_pad + kEmuTile - 1) / kEmuTile;
   e->syrk_n_tiles = nt1 * (nt1 + 1) / 2;
   e->emu_n_items = (int)items.size();
+  e->emu_n_full = (int)plan.full.size();
   const cudaStream_t s0 = (cudaStream_t)0;
   BA_CUDA(cudaMallocAsync(reinterpret_cast<void**>(&e->emu_items), items.size() * sizeof(EmuItem), s0));
   BA_CUDA(cudaMallocAsync(reinterpret_cast<void**>(&e->Yq), (size_t)kEmuModuli * e->n_pad * e->k_pad, s0));
@@ -1490,7 +1548,8 @@ static int launch_syrk_emu(ba_engine* e, const ba_lm_state* ctl, cudaStream_t s)
   CUtensorMap map;
   BA_TRY(make_plane_map(&map, e->Yq, e->n_pad, e->k_pad));
   BA_CUDA(cudaFuncSetAttribute(emu_residue_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kResSmemBytes));
-  BA_CUDA(cudaFuncSetAttribute(syrk_i8_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kEmuSmemBytes));
+  BA_CUDA(cudaFuncSetAttribute(syrk_i8_pair_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kEmuSmemBytes));
+  BA_CUDA(cudaFuncSetAttribute(syrk_i8_pair_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kEmuSmemBytes));
   const int n_tiles = e->syrk_n_tiles;
   ProfScope ps(e, PG_SYRK, s);
   BA_CUDA(cudaMemsetAsync(e->colmax, 0, (size_t)e->n_pad * sizeof(unsigned long long), s));
@@ -1504,8 +1563,16 @@ static int launch_syrk_emu(ba_engine* e, const ba_lm_state* ctl, cudaStream_t s)
   emu_residue_kernel<<<dim3((unsigned)((e->k_pad + kResTK - 1) / kResTK), (e->n_pad + kResTA - 1) / kResTA),
                        kResThreads, kResSmemBytes, s>>>(e->Yt, e->k_pad, e->n_pad, e->colmax, e->emu_bits, e->Yq, ctl);
   BA_LAUNCH_CHECK();
-  syrk_i8_kernel<<<e->emu_n_items, kEmuThreads, kEmuSmemBytes, s>>>(map, e->emu_items, e->Pmod, n_tiles, e->n_pad, ctl);
-  BA_LAUNCH_CHECK();
+  if (e->emu_n_full > 0) {
+    syrk_i8_pair_kernel<false><<<2 * e->emu_n_full, kEmuThreads, kEmuSmemBytes, s>>>(map, e->emu_items, e->Pmod,
+                                                                                     n_tiles, e->n_pad, ctl);
+    BA_LAUNCH_CHECK();
+  }
+  if (e->emu_n_items > e->emu_n_full) {
+    syrk_i8_pair_kernel<true><<<2 * (e->emu_n_items - e->emu_n_full), kEmuThreads, kEmuSmemBytes, s>>>(
+        map, e->emu_items + e->emu_n_full, e->Pmod, n_tiles, e->n_pad, ctl);
+    BA_LAUNCH_CHECK();
+  }
   emu_reconstruct_kernel<<<dim3(n_tiles, 16), 256, 0, s>>>(e->Pmod, n_tiles, e->colmax, e->emu_bits, e->P(), e->n_pad,
                                                           e->n_pad, emu_consts(), ctl);
   BA_LAUNCH_CHECK();

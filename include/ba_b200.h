@@ -226,7 +226,8 @@ typedef enum ba_buffer_id {
   BA_BUF_LINV = 8,   /* [n_points][6] inverse Cholesky factor of damped V_j     K2 */
   BA_BUF_Z = 9,      /* [n_points][3] L_j^-1 d_P_j                               K2 */
   BA_BUF_REDUCE = 10,/* the reduce buffer (see ba_reduce_buffer)                    */
-  BA_BUF_COST = 11   /* [4] see ba_cost_buffer                                      */
+  BA_BUF_COST = 11,  /* [4] see ba_cost_buffer                                      */
+  BA_BUF_YT = 12     /* dense: [k_pad][n_pad] Y^T, the operand of the Schur product P = Yt^T Yt */
 } ba_buffer_id;
 int ba_buffer_size(ba_engine* e, int id, int64_t* n_doubles);
 int ba_buffer_read(ba_engine* e, int id, double* host_out, int64_t n_doubles, void* stream);

@@ -5,8 +5,12 @@
 Builds the reduced system of one dense scene `reps` times on an engine created with BA_SYRK_EMU=1,
 under torch.profiler (CUDA activities), and prints one JSON line: mean time per build of every K3
 kernel, the conversion passes' bandwidth (bytes they must move: Yt read twice, the residue planes
-written once) and the int8 rate of syrk_i8_kernel (2 x 128 x N x k ops per MMA tile, N = 128, or 16
-on a ragged last tile row).  Needs a GPU."""
+written once), the int8 rate of both instances of syrk_i8_pair_kernel (whole tile rows, ragged last
+tile row) and the operand bytes their TMA copies deliver to
+shared memory per build.  The rate counts the MMA work the kernel issues: 2 x 256 x N x k per 256-tile
+and modulus, N = 256 (diagonal tiles included: their upper halves are computed too), or the rows of a
+ragged last tile row rounded up to 16.  The bytes are counted from the plan (a 128-row box of 128 k per
+operand and CTA, one operand on a full diagonal tile), not profiled.  Needs a GPU."""
 import argparse
 import json
 import os
@@ -53,19 +57,32 @@ def main():
     ms = {}
     for ev in prof.key_averages():
         name = ev.key
-        for k in ("emu_colmax_kernel", "emu_residue_kernel", "syrk_i8_kernel", "emu_reconstruct_kernel"):
+        if "syrk_i8_pair_kernel" in name:  # two instances: whole tile rows, and the ragged last tile row
+            k = "syrk_i8_pair_kernel<ragged>" if "<true>" in name else "syrk_i8_pair_kernel<full>"
+            ms[k] = ms.get(k, 0.0) + ev.device_time_total / 1e3 / args.reps
+        for k in ("emu_colmax_kernel", "emu_residue_kernel", "emu_reconstruct_kernel"):
             if k in name:
                 ms[k] = ms.get(k, 0.0) + ev.device_time_total / 1e3 / args.reps
         if "emset" in name:
             ms["memset"] = ms.get("memset", 0.0) + ev.device_time_total / 1e3 / args.reps
     n_pad, k_pad = eng.n_pad, (3 * args.points + 31) // 32 * 32
     moduli, bits = ba_b200.submodule("engine").syrk_emu_info(k_pad)
-    nt1 = (n_pad + 127) // 128
-    left = n_pad - (nt1 - 1) * 128
-    thin_n = 128 if left == 128 else (left + 15) // 16 * 16
-    tiles_n = (nt1 - 1) * nt1 // 2 * 128 + nt1 * thin_n  # sum of N over the lower tiles
-    kb = (k_pad + 127) // 128 * 128
-    i8_ops = 2.0 * 128 * tiles_n * kb * len(moduli)
+    nt2 = (n_pad + 255) // 256
+    left = n_pad - (nt2 - 1) * 256
+    thin_n = (left + 15) // 16 * 16
+    full_rows = nt2 if left == 256 else nt2 - 1  # 256-tile rows without a ragged edge
+    kb = (k_pad + 127) // 128
+    scale = 16384.0 * kb * len(moduli)  # one 16 KB box (128 rows x 128 k) per k-block and modulus
+    ops = {"full": 2.0 * 256 * 256 * full_rows * (full_rows + 1) // 2 * kb * 128 * len(moduli),
+           "ragged": 0.0 if left == 256 else 2.0 * 256 * nt2 * thin_n * kb * 128 * len(moduli)}
+    # operand boxes per k-block: off-diagonal 4, full diagonal 2, ragged row 4 (A tile + two B boxes)
+    box_GB = {"full": (4 * (full_rows * (full_rows - 1) // 2) + 2 * full_rows) * scale / 1e9,
+              "ragged": (0 if left == 256 else 4 * nt2) * scale / 1e9}
+    # of which L2 -> SM: rows inside the tensor only (the ragged row's B boxes are mostly zero fill)
+    l2_GB = dict(box_GB)
+    if left != 256:
+        l2_GB["ragged"] = nt2 * (2 * 16384.0 + 2 * 128.0 * min(left, 128)) * kb * len(moduli) / 1e9
+    ki = {"full": "syrk_i8_pair_kernel<full>", "ragged": "syrk_i8_pair_kernel<ragged>"}
     conv_bytes = 2 * 8.0 * k_pad * n_pad + len(moduli) * float(n_pad) * k_pad
     conv_ms = ms.get("emu_colmax_kernel", 0) + ms.get("emu_residue_kernel", 0)
     res = {
@@ -75,8 +92,10 @@ def main():
         "conversion_GBps": conv_bytes / (conv_ms * 1e-3) / 1e9 if conv_ms else None,
         "residue_pass_GBps": (8.0 * k_pad * n_pad + len(moduli) * float(n_pad) * k_pad)
         / (ms["emu_residue_kernel"] * 1e-3) / 1e9 if ms.get("emu_residue_kernel") else None,
-        "i8_TOPS": i8_ops / (ms["syrk_i8_kernel"] * 1e-3) / 1e12 if ms.get("syrk_i8_kernel") else None,
-        "i8_ops": i8_ops,
+        "i8_TOPS": {c: ops[c] / (ms[ki[c]] * 1e-3) / 1e12 for c in ops if ms.get(ki[c])},
+        "i8_ops": ops,
+        "tma_box_GB_per_build": box_GB,
+        "l2_to_sm_GB_per_build": l2_GB,
         "gpu": torch.cuda.get_device_name(0),
     }
     eng.close()
