@@ -111,8 +111,6 @@ struct ba_engine {
   int n_full = 0, rhs_row = 0, n_pad = 0;
   int syrk_tile = 128;
   int syrk_n_items = 0, syrk_n_tiles = 0;
-  int syrk_n_ctas = 0;                 // CTAs of the SYRK launch (= items unless stream-K planned)
-  int* syrk_cta_first = nullptr;       // [syrk_n_ctas + 1] stream-K: first item of every CTA (else null)
   ba::SyrkItem* syrk_items = nullptr;  // [syrk_n_items] launch order
   int* syrk_tile_first = nullptr;      // [syrk_n_tiles + 1]
   int* syrk_tile_items = nullptr;      // items of each tile in ascending k order
@@ -393,7 +391,7 @@ bool dense_matrix_free(const ba_engine* e);  // dense K2b / point update re-deri
 int launch_k3(ba_engine* e, bool conditional, cudaStream_t s);
 int syrk_plan_engine(ba_engine* e);
 int syrk_emu_info(int64_t k_pad, int32_t* moduli, int* n_moduli, int* bits);
-int syrk_feed_is_tma();  // 1: the 128-tile SYRK is fed by TMA + mbarriers, 0: by cp.async (BA_SYRK_NO_TMA)
+int require_tensor_map_encoder();  // BA_ERR_CUDA when the driver lacks cuTensorMapEncodeTiled
 // Gram matrix P = Yt^T Yt of a k-major operand outside an engine (k3_schur_syrk.cu)
 struct GramWorkspace {
   int n_pad = 0, num_sms = 0, n_items = 0, n_tiles = 0;

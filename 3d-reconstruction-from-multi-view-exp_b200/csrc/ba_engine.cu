@@ -278,7 +278,7 @@ static void free_engine(ba_engine* e) {
   void* ptrs[] = {e->obs_ptr, e->obs_cam, e->obs_pt, e->obs_xy, e->cam_ptr, e->cm_perm, e->bits, e->PT, e->pair_ptr, e->pair_pts, e->X[0],
                   e->X[1], e->cam[0].f, e->cam[1].f, e->camtab[0], e->camtab[1], e->JP, e->JC, e->V,
                   e->GPT, e->Upart, e->Uloc, e->LINV, e->Z, e->Yt, e->Ysp, e->red_in_window ? nullptr : e->red, e->Spart, e->Lt, e->Winv,
-                  e->dxi, e->cost_part, e->cost_buf, e->ctl, e->rec, e->ywork, e->chol_bar, e->gauge, e->syrk_items, e->syrk_tile_first, e->syrk_tile_items, e->syrk_cta_first, e->emu_items, e->Yq, e->Pmod, e->colmax};
+                  e->dxi, e->cost_part, e->cost_buf, e->ctl, e->rec, e->ywork, e->chol_bar, e->gauge, e->syrk_items, e->syrk_tile_first, e->syrk_tile_items, e->emu_items, e->Yq, e->Pmod, e->colmax};
   for (void* p : ptrs)
     dev_free(p);
   for (int k = 0; k < 2; ++k) {
@@ -341,6 +341,7 @@ static int create_engine(const ba_problem* p, ba_engine** out) {
     return BA_ERR_INVALID;
   }
   BA_CUDA(cudaSetDevice(p->device));
+  BA_TRY(require_tensor_map_encoder());
   tm.lap("device count / set device");
   BA_TRY(retain_pool_memory(p->device));
   tm.lap("pool attribute");
@@ -356,10 +357,6 @@ static int create_engine(const ba_problem* p, ba_engine** out) {
   e->rhs_row = e->n_full;
   const int n_aug = e->n_full + 1;
   e->syrk_tile = n_aug <= 384 ? 64 : 128;  // C2 (n = 451): 128-tiles 0.283 ms vs 64-tiles 0.302 ms per iteration
-  if (const char* t = std::getenv("BA_SYRK_TILE")) {  // tuning experiments only
-    const int v = std::atoi(t);
-    if (v == 64 || v == 128) e->syrk_tile = v;
-  }
   e->n_pad = round_up(n_aug, 8);  // fragment granularity; edge tiles of the SYRK are partial
   e->k_pad = round_up64(3 * e->N, 32);
   // camera_blocks_kernel: 3 blocks per SM (162 registers); ~8 waves of blocks so that the last,
@@ -932,7 +929,6 @@ int ba_profile_reset(ba_engine* e) {
 
 int ba_fp64_peak(int device, int use_dmma, double* tflops) { return fp64_peak(device, use_dmma, tflops); }
 
-int ba_syrk_feed(void) { return syrk_feed_is_tma(); }
 int ba_matrix_free(ba_engine* e) { return e && dense_matrix_free(e) ? 1 : 0; }
 
 int ba_syrk_plan_info(int n_cams, int64_t n_points, int tile, int num_sms, int* n_items, int* n_tiles,

@@ -11,9 +11,11 @@
 // summed in a fixed order (deterministic; no FP64 atomics).  z_j occupies column `rhs_row` of
 // Yt, so row `rhs_row` of P is the rhs term for free.
 //
-// Pipeline: cp.async (LDGSTS) 16-byte copies, 3 stages of KC k-rows, shared-memory rows padded
-// to TILE+4 doubles (stride = 4 mod 16: the 8-byte fragment loads of a half-warp hit 16
-// distinct bank pairs -- ncu: 0 bank conflicts).
+// Two kernels, one per tile size: 128-tiles (syrk_tma_kernel, one CTA per SM) are fed by TMA
+// tensor copies (see "128-tiles fed by TMA" below); 64-tiles (syrk_dmma_kernel, four CTAs per SM)
+// by cp.async (LDGSTS) 16-byte copies, 3 stages of KC k-rows, shared-memory rows padded to TILE+4
+// doubles (stride = 4 mod 16: the 8-byte fragment loads of a half-warp hit 16 distinct bank pairs
+// -- ncu: 0 bank conflicts).
 //
 // Compute roofline (FP64 tensor): algorithmic flops = 3N * n (n + 1), n = 9M - 7.
 //
@@ -71,6 +73,39 @@ struct SubSplit {
   int rank, world, tile_row0, push_cols;
   double* peer[kMaxRanks];
 };
+
+// Epilogue of one accumulator pair at tile-local (rl, cl), cl even: into the item's partial tile
+// (`part` points at it), or (SUB) subtracted in place from the lower triangle of S (`part`), with
+// the peer stores of a divided update.
+template <int TILE, bool SUB>
+__device__ __forceinline__ void syrk_store_pair(double v0, double v1, int ti, int tj, int rl, int cl, int ld,
+                                                int n_store, double* __restrict__ part, const SubSplit& sp) {
+  if (SUB) {
+    const int r = ti * TILE + rl, c = tj * TILE + cl;
+    if (r >= n_store || c > r) return;
+    const size_t off = (size_t)r * ld + c;
+    double* p = part + off;
+    const bool push = sp.world > 1 && tj * TILE < sp.push_cols;
+    if (c + 1 <= r) {
+      double2 v = *reinterpret_cast<double2*>(p);
+      v.x -= v0;
+      v.y -= v1;
+      *reinterpret_cast<double2*>(p) = v;
+      if (push)
+        for (int q = 0; q < sp.world; ++q)
+          if (q != sp.rank) *reinterpret_cast<double2*>(sp.peer[q] + off) = v;
+    } else {
+      const double v = *p - v0;
+      *p = v;
+      if (push)
+        for (int q = 0; q < sp.world; ++q)
+          if (q != sp.rank) sp.peer[q][off] = v;
+    }
+  } else {
+    // `part` is the item's own partial tile
+    *reinterpret_cast<double2*>(part + (size_t)rl * TILE + cl) = make_double2(v0, v1);
+  }
+}
 
 // TILE x TILE output tile per CTA; WR x WC warps, each owning a (TILE/WR) x (TILE/WC) sub-tile.
 // SUB = false: the tile of this split is written to part[split][tile] (Schur product).
@@ -143,8 +178,7 @@ syrk_dmma_kernel(const double* __restrict__ Yt, int ld, int n_valid, int64_t n_c
   // Sub-tile of this warp.  Off the diagonal: row-major over the WR x WC grid.  On a diagonal
   // tile only the WR (WR + 1) / 2 sub-tiles on or below the diagonal are needed (nothing above
   // the diagonal is read anywhere); they are dealt to warps 0, 1, 2, ... -- consecutive warps sit
-  // on different scheduler partitions, so the 10 (of 16) live warps of a 128-tile load the four
-  // FP64 pipes 3/3/2/2 instead of 4/3/2/1 -- and the remaining warps only help with the copies.
+  // on different scheduler partitions -- and the remaining warps only help with the copies.
   int wr = warp / WC, wc = warp % WC;
   bool live = true;
   if (diag && WR == WC) {
@@ -221,47 +255,17 @@ syrk_dmma_kernel(const double* __restrict__ Yt, int ld, int n_valid, int64_t n_c
   const int orow = wr * WM + (lane >> 2);
   const int ocol = wc * WN + 2 * (lane & 3);
   if (!live) return;  // the sub-tiles above the diagonal of a diagonal tile are never read
-  if (SUB) {
-    // S -= acc on the lower triangle; an accumulator pair sits at (r, c), (r, c + 1), c even
-#pragma unroll
-    for (int i = 0; i < FM; ++i)
-#pragma unroll
-      for (int j = 0; j < FN; ++j) {
-        const int r = ti * TILE + orow + 8 * i, c = tj * TILE + ocol + 8 * j;
-        if (r >= n_store || c > r) continue;
-        const size_t off = (size_t)r * ld + c;
-        double* p = part + off;
-        const bool push = sp.world > 1 && tj * TILE < sp.push_cols;
-        if (c + 1 <= r) {
-          double2 v = *reinterpret_cast<double2*>(p);
-          v.x -= acc[i][j][0];
-          v.y -= acc[i][j][1];
-          *reinterpret_cast<double2*>(p) = v;
-          if (push)
-            for (int q = 0; q < sp.world; ++q)
-              if (q != sp.rank) *reinterpret_cast<double2*>(sp.peer[q] + off) = v;
-        } else {
-          const double v = *p - acc[i][j][0];
-          *p = v;
-          if (push)
-            for (int q = 0; q < sp.world; ++q)
-              if (q != sp.rank) sp.peer[q][off] = v;
-        }
-      }
-    return;
-  }
   // partial tile of this item: part[item][TILE][TILE]
-  double* out = part + (size_t)blockIdx.x * TILE * TILE;
+  double* const out = SUB ? part : part + (size_t)blockIdx.x * TILE * TILE;
 #pragma unroll
   for (int i = 0; i < FM; ++i)
 #pragma unroll
     for (int j = 0; j < FN; ++j)
-      *reinterpret_cast<double2*>(out + (size_t)(orow + 8 * i) * TILE + ocol + 8 * j) =
-          make_double2(acc[i][j][0], acc[i][j][1]);
+      syrk_store_pair<TILE, SUB>(acc[i][j][0], acc[i][j][1], ti, tj, orow + 8 * i, ocol + 8 * j, ld, n_store, out, sp);
 }
 
 // ---- 128-tiles fed by TMA ------------------------------------------------------------------------
-// The same product with a Blackwell-native operand feed.  ncu on the cp.async kernel at C3: every
+// The product with a Blackwell-native operand feed.  ncu on a cp.async-fed 128-tile kernel at C3: every
 // chunk starts with all 16 warps issuing their LDGSTS (128 warp instructions, ~8 LSU cycles each)
 // right behind the block barrier, and the fragment loads of the chunk's first k-steps queue behind
 // them in the same LSU pipe -- ~1000 of every 8192 cycles the FP64 tensor pipes wait (tiles without
@@ -327,76 +331,31 @@ __device__ __forceinline__ void tma_load_2d(unsigned dst, const CUtensorMap* map
       : "memory");
 }
 
-// Epilogue of one accumulator pair at tile-local (rl, cl), cl even: into the item's partial tile
-// (`part` points at it), or (SUB) subtracted in place from the lower triangle of S (`part`), with
-// the peer stores of a divided update.
-template <bool SUB>
-__device__ __forceinline__ void syrk_store_pair(double v0, double v1, int ti, int tj, int rl, int cl, int ld,
-                                                int n_store, double* __restrict__ part, const SubSplit& sp) {
-  constexpr int TILE = kTmaTile;
-  if (SUB) {
-    const int r = ti * TILE + rl, c = tj * TILE + cl;
-    if (r >= n_store || c > r) return;
-    const size_t off = (size_t)r * ld + c;
-    double* p = part + off;
-    const bool push = sp.world > 1 && tj * TILE < sp.push_cols;
-    if (c + 1 <= r) {
-      double2 v = *reinterpret_cast<double2*>(p);
-      v.x -= v0;
-      v.y -= v1;
-      *reinterpret_cast<double2*>(p) = v;
-      if (push)
-        for (int q = 0; q < sp.world; ++q)
-          if (q != sp.rank) *reinterpret_cast<double2*>(sp.peer[q] + off) = v;
-    } else {
-      const double v = *p - v0;
-      *p = v;
-      if (push)
-        for (int q = 0; q < sp.world; ++q)
-          if (q != sp.rank) sp.peer[q][off] = v;
-    }
-  } else {
-    // `part` is the item's own partial tile
-    *reinterpret_cast<double2*>(part + (size_t)rl * TILE + cl) = make_double2(v0, v1);
-  }
-}
-
-// One CTA runs a list of SEGMENTS (work items: tile x k-range), items[cta_first[b] .. cta_first[b + 1])
-// -- one item per CTA when cta_first is null (large operands: the planner cuts whole waves of items
-// in k-major order so that a k-slab stays in the L2), several for small operands (stream-K: every
-// CTA gets the same modelled work, crossing tile boundaries).  The TMA ring runs across segment
-// boundaries: the elected thread keeps its own cursor two to three chunks ahead of the warps, so the
-// pipeline is filled once per CTA, not once per item.  The slot of an item's partial tile is its
-// index in `items`.
+// One CTA runs one work item: a tile and a range of k-chunks (Schur product: items[blockIdx.x], its
+// partial tile goes to slot blockIdx.x), or the whole depth of tile blockIdx.x (trailing update).
+// The elected thread fills the three-stage ring with the item's first chunks and, before chunk kc
+// is computed, refills the stage of chunk kc - 1 with chunk kc + 2.
 template <bool SUB>
 __global__ void __launch_bounds__(kTmaThreads, 1)
 syrk_tma_kernel(const __grid_constant__ CUtensorMap tmapA, const __grid_constant__ CUtensorMap tmapB, int ld,
-                int n_valid, int64_t n_chunks, const SyrkItem* __restrict__ items, const int* __restrict__ cta_first,
-                double* __restrict__ part, const ba_lm_state* ctl, int n_store, SubSplit sp) {
+                int n_valid, int64_t n_chunks, const SyrkItem* __restrict__ items, double* __restrict__ part,
+                const ba_lm_state* ctl, int n_store, SubSplit sp) {
   if (ctl && ctl->done) return;
   constexpr int TILE = kTmaTile, KC = kTmaKC, LDA = kTmaLda, LDB = kTmaLdb, WR = 4, WC = 4;
   constexpr int WM = TILE / WR, WN = TILE / WC, FM = WM / 8, FN = WN / 8;
   extern __shared__ unsigned char smem_raw[];
 
-  int seg_lo = blockIdx.x, seg_hi = blockIdx.x + 1;
-  if (!SUB && cta_first) { seg_lo = cta_first[blockIdx.x]; seg_hi = cta_first[blockIdx.x + 1]; }
-  // segment `seg` -> tile, first chunk, chunks, second slot
-  auto segment = [&](int seg, int& ti, int& tj, int& c_lo, int& nk, int& slot2) {
-    if (SUB) {
-      tile_from_linear(seg, ti, tj);
-      c_lo = 0;
-      nk = (int)n_chunks;
-      slot2 = -1;
-    } else {
-      const SyrkItem it = items[seg];
-      ti = it.ti; tj = it.tj; c_lo = it.c_lo; nk = it.c_hi > it.c_lo ? it.c_hi - it.c_lo : 0; slot2 = it.slot2;
-    }
-  };
+  int ti, tj, c_lo = 0, nk;
+  bool tall = false;
   if (SUB) {
-    int ti, tj;
     tile_from_linear(blockIdx.x, ti, tj);
     if (sp.world > 1 && (sp.tile_row0 + ti) % sp.world != sp.rank) return;  // another rank's tile row
+    nk = (int)n_chunks;
+  } else {
+    const SyrkItem it = items[blockIdx.x];
+    ti = it.ti; tj = it.tj; c_lo = it.c_lo; nk = it.c_hi > it.c_lo ? it.c_hi - it.c_lo : 0; tall = it.slot2 >= 0;
   }
+  const bool diag = ti == tj;
 
   // carve shared memory: operand stages (128-byte aligned for the TMA unit), then the mbarriers
   const unsigned base = (smem_u32(smem_raw) + 127u) & ~127u;
@@ -406,27 +365,13 @@ syrk_tma_kernel(const __grid_constant__ CUtensorMap tmapA, const __grid_constant
   auto full_bar = [&](int st) { return bars + 8u * st; };
   auto empty_bar = [&](int st) { return bars + 8u * (kTmaStages + st); };
 
-  // ---- the elected thread's side of the ring: a cursor over the chunks of all segments ----------
-  int pseg = seg_lo - 1, pkc = 0, pnk = 0;   // cursor: segment, next chunk in it, its chunk count
-  int pti = 0, ptj = 0, pclo = 0;            // ... and its tile / first chunk (kept in registers:
-                                             // the item is read from global memory once per segment)
-  unsigned issued = 0;                       // chunks issued so far = global index of the next one
-  auto issue_next = [&]() {                  // thread 0 only
-    while (pkc >= pnk) {
-      if (++pseg >= seg_hi) { pseg = seg_hi; return; }
-      int slot2;
-      segment(pseg, pti, ptj, pclo, pnk, slot2);
-      pkc = 0;
-    }
-    const int st = (int)(issued % kTmaStages);
+  auto issue = [&](int kc) {  // thread 0 only: chunk kc of the item into stage kc % kTmaStages
+    const int st = kc % kTmaStages;
     const unsigned dst = base + (unsigned)st * kTmaStageBytes;
-    const int row = (pclo + pkc) * KC;
-    const bool dg = pti == ptj;
-    mbar_arrive_expect_tx(full_bar(st), kTmaABytes + (dg ? 0u : kTmaBBytes));
-    tma_load_2d(dst, &tmapA, pti * TILE, row, full_bar(st));
-    if (!dg) tma_load_2d(dst + kTmaABytes, &tmapB, ptj * TILE, row, full_bar(st));
-    ++issued;
-    ++pkc;
+    const int row = (c_lo + kc) * KC;
+    mbar_arrive_expect_tx(full_bar(st), kTmaABytes + (diag ? 0u : kTmaBBytes));
+    tma_load_2d(dst, &tmapA, ti * TILE, row, full_bar(st));
+    if (!diag) tma_load_2d(dst + kTmaABytes, &tmapB, tj * TILE, row, full_bar(st));
   };
 
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
@@ -436,185 +381,180 @@ syrk_tma_kernel(const __grid_constant__ CUtensorMap tmapA, const __grid_constant
       mbar_init(empty_bar(st), kTmaThreads / 32);
     }
     asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    for (int k = 0; k < kTmaStages; ++k) issue_next();
+    for (int kc = 0; kc < kTmaStages && kc < nk; ++kc) issue(kc);
   }
   __syncthreads();
-  // Before global chunk g is computed the elected thread refills the stage of chunk g - 1 with the
-  // next chunk not yet issued (every warp is done with chunk g - 1 or about to be: the wait on
-  // `empty` is short).
-  auto refill = [&](unsigned g) {
+  // Before chunk kc is computed the elected thread refills the stage of chunk kc - 1 with chunk
+  // kc + kTmaStages - 1 (every warp is done with chunk kc - 1 or about to be: the wait on `empty`
+  // is short).
+  auto refill = [&](int kc) {
     if (warp == 0) {
-      if (lane == 0 && g >= 1 && issued == g + kTmaStages - 1) {
-        mbar_wait(empty_bar((int)((g - 1) % kTmaStages)), ((g - 1) / kTmaStages) & 1u);
-        issue_next();
+      if (lane == 0 && kc >= 1 && kc + kTmaStages - 1 < nk) {
+        mbar_wait(empty_bar((kc - 1) % kTmaStages), ((kc - 1) / kTmaStages) & 1u);
+        issue(kc + kTmaStages - 1);
       }
       __syncwarp();
     }
   };
   const int kq = lane & 3;
-  unsigned g = 0;  // global chunk counter of this CTA
+  double* const slot_part = SUB ? part : part + (size_t)blockIdx.x * TILE * TILE;
 
-  for (int seg = seg_lo; seg < seg_hi; ++seg) {
-    int ti, tj, c_lo_unused, nk, slot2;
-    segment(seg, ti, tj, c_lo_unused, nk, slot2);
-    const bool diag = ti == tj;
-    const bool tall = slot2 >= 0;
-    double* const slot_part = SUB ? part : part + (size_t)seg * TILE * TILE;
-
-    if (diag) {
-      // Diagonal tile: only the 136 fragments (8 x 8) on or below the diagonal of the 16 x 16
-      // fragment grid are needed.  Fragment rows r and 15 - r together hold 17 of them; the pair is
-      // shared by two warps, one taking nine fragments (row 15 - r, columns 0..8), the other eight
-      // (the rest of row 15 - r and all of row r); which warp of a pair takes nine alternates so
-      // that every scheduler partition (warp % 4) carries 34 fragments per k-step.
-      const int pr = warp >> 1;
-      const bool nine = (((warp & 1) ^ ((warp >> 2) & 1)) == 0);
-      const int r_hi = 15 - pr, r_lo = pr;
-      const int n_hi = nine ? 9 : 7 - pr;        // fragments this warp takes from row r_hi
-      const int c_hi0 = nine ? 0 : 9;            // ... starting at this column
-      const int nfr = nine ? 9 : 8;
-      const int frag_rows_valid = (n_valid - ti * TILE + 7) / 8;  // ragged last tile
-      int boffj[9];
-      bool usej[9];
-      bool any = false;
+  if (diag) {
+    // Diagonal tile: only the 136 fragments (8 x 8) on or below the diagonal of the 16 x 16
+    // fragment grid are needed.  Fragment rows r and 15 - r together hold 17 of them; the pair is
+    // shared by two warps, one taking nine fragments (row 15 - r, columns 0..8), the other eight
+    // (the rest of row 15 - r and all of row r); which warp of a pair takes nine alternates so
+    // that every scheduler partition (warp % 4) carries 34 fragments per k-step.
+    const int pr = warp >> 1;
+    const bool nine = (((warp & 1) ^ ((warp >> 2) & 1)) == 0);
+    const int r_hi = 15 - pr, r_lo = pr;
+    const int n_hi = nine ? 9 : 7 - pr;        // fragments this warp takes from row r_hi
+    const int c_hi0 = nine ? 0 : 9;            // ... starting at this column
+    const int nfr = nine ? 9 : 8;
+    const int frag_rows_valid = (n_valid - ti * TILE + 7) / 8;  // ragged last tile
+    int boffj[9];
+    bool usej[9];
+    bool any = false;
 #pragma unroll
-      for (int j = 0; j < 9; ++j) {
-        const bool hi = j < n_hi;
-        const int rf = hi ? r_hi : r_lo;
-        const int cf = hi ? c_hi0 + j : j - n_hi;
-        usej[j] = j < nfr && rf < frag_rows_valid;
-        any |= usej[j];
-        boffj[j] = kq * LDA + 8 * cf + (lane >> 2);
-      }
-      const int aoff_hi = kq * LDA + 8 * r_hi + (lane >> 2);
-      const int aoff_lo = kq * LDA + 8 * r_lo + (lane >> 2);
-      double dacc[9][2];
-#pragma unroll
-      for (int j = 0; j < 9; ++j) dacc[j][0] = dacc[j][1] = 0.0;
-      for (int kc = 0; kc < nk; ++kc, ++g) {
-        refill(g);
-        const int st = (int)(g % kTmaStages);
-        mbar_wait(full_bar(st), (g / kTmaStages) & 1u);
-        const double* a = stages + (size_t)st * kStageDoubles;
-        if (any) {
-#pragma unroll
-          for (int kk = 0; kk < KC; kk += 4) {
-            const double fa_hi = a[aoff_hi + kk * LDA], fa_lo = a[aoff_lo + kk * LDA];
-            double fb[9];
-#pragma unroll
-            for (int j = 0; j < 9; ++j) fb[j] = a[boffj[j] + kk * LDA];
-#pragma unroll
-            for (int j = 0; j < 9; ++j)
-              if (usej[j]) dmma884(dacc[j][0], dacc[j][1], j < n_hi ? fa_hi : fa_lo, fb[j]);
-          }
-        }
-        __syncwarp();
-        if (lane == 0) mbar_arrive(empty_bar(st));
-      }
-#pragma unroll
-      for (int j = 0; j < 9; ++j) {
-        if (!usej[j]) continue;
-        const bool hi = j < n_hi;
-        syrk_store_pair<SUB>(dacc[j][0], dacc[j][1], ti, ti, 8 * (hi ? r_hi : r_lo) + (lane >> 2),
-                             8 * (hi ? c_hi0 + j : j - n_hi) + 2 * (lane & 3), ld, n_store, slot_part, sp);
-      }
-      continue;
+    for (int j = 0; j < 9; ++j) {
+      const bool hi = j < n_hi;
+      const int rf = hi ? r_hi : r_lo;
+      const int cf = hi ? c_hi0 + j : j - n_hi;
+      usej[j] = j < nfr && rf < frag_rows_valid;
+      any |= usej[j];
+      boffj[j] = kq * LDA + 8 * cf + (lane >> 2);
     }
-
-    // (A column-per-warp mapping for the thin tiles of a ragged last tile row was tried and dropped:
-    // with only 2 of 16 fragment rows to compute, the warps outrun the three-stage TMA ring and wait
-    // for every chunk -- C3 went from 28.8 to 31.1 ms.  Such rows are folded into tall tiles instead.)
-    const int wr = warp / WC, wc = warp % WC;
-    int vm = 0, vn = 0;
+    const int aoff_hi = kq * LDA + 8 * r_hi + (lane >> 2);
+    const int aoff_lo = kq * LDA + 8 * r_lo + (lane >> 2);
+    double dacc[9][2];
 #pragma unroll
-    for (int i = 0; i < FM; ++i) vm += (ti * TILE + wr * WM + 8 * i) < n_valid;
-#pragma unroll
-    for (int j = 0; j < FN; ++j) vn += (tj * TILE + wc * WN + 8 * j) < n_valid;
-    const bool full = vm == FM && vn == FN;
-    const int aoff = kq * LDA + wr * WM + (lane >> 2);
-    const int boff = kq * LDB + wc * WN + (lane >> 2);
-    // tall item: this warp's two extra fragments -- fragment row 16 + (wr & 1) of A against its B
-    // fragments 2 (wr >> 1) and 2 (wr >> 1) + 1
-    const int xoff = kq * LDA + TILE + 8 * (wr & 1) + (lane >> 2);
-    const int xj = 2 * (wr >> 1);
-    const bool xvalid = tall && (ti + 1) * TILE + 8 * (wr & 1) < n_valid;
-
-    double acc[FM][FN][2], xacc[2][2];
-#pragma unroll
-    for (int i = 0; i < FM; ++i)
-#pragma unroll
-      for (int j = 0; j < FN; ++j) acc[i][j][0] = acc[i][j][1] = 0.0;
-    xacc[0][0] = xacc[0][1] = xacc[1][0] = xacc[1][1] = 0.0;
-
-    for (int kc = 0; kc < nk; ++kc, ++g) {
-      refill(g);
-      const int st = (int)(g % kTmaStages);
-      mbar_wait(full_bar(st), (g / kTmaStages) & 1u);
-      const double* a = stages + (size_t)st * kStageDoubles + aoff;
-      const double* b = stages + (size_t)st * kStageDoubles + kTmaADoubles + boff;
-      if (full && xvalid) {
-        const double* x = stages + (size_t)st * kStageDoubles + xoff;
+    for (int j = 0; j < 9; ++j) dacc[j][0] = dacc[j][1] = 0.0;
+    for (int kc = 0; kc < nk; ++kc) {
+      refill(kc);
+      const int st = kc % kTmaStages;
+      mbar_wait(full_bar(st), (kc / kTmaStages) & 1u);
+      const double* a = stages + (size_t)st * kStageDoubles;
+      if (any) {
 #pragma unroll
         for (int kk = 0; kk < KC; kk += 4) {
-          double fa[FM], fb[FN];
+          const double fa_hi = a[aoff_hi + kk * LDA], fa_lo = a[aoff_lo + kk * LDA];
+          double fb[9];
 #pragma unroll
-          for (int i = 0; i < FM; ++i) fa[i] = a[kk * LDA + 8 * i];
+          for (int j = 0; j < 9; ++j) fb[j] = a[boffj[j] + kk * LDA];
 #pragma unroll
-          for (int j = 0; j < FN; ++j) fb[j] = b[kk * LDB + 8 * j];
-          const double fx = x[kk * LDA];
-#pragma unroll
-          for (int i = 0; i < FM; ++i)
-#pragma unroll
-            for (int j = 0; j < FN; ++j) dmma884(acc[i][j][0], acc[i][j][1], fa[i], fb[j]);
-          dmma884(xacc[0][0], xacc[0][1], fx, xj == 0 ? fb[0] : fb[2]);
-          dmma884(xacc[1][0], xacc[1][1], fx, xj == 0 ? fb[1] : fb[3]);
-        }
-      } else if (full) {
-#pragma unroll
-        for (int kk = 0; kk < KC; kk += 4) {
-          double fa[FM], fb[FN];
-#pragma unroll
-          for (int i = 0; i < FM; ++i) fa[i] = a[kk * LDA + 8 * i];
-#pragma unroll
-          for (int j = 0; j < FN; ++j) fb[j] = b[kk * LDB + 8 * j];
-#pragma unroll
-          for (int i = 0; i < FM; ++i)
-#pragma unroll
-            for (int j = 0; j < FN; ++j) dmma884(acc[i][j][0], acc[i][j][1], fa[i], fb[j]);
-        }
-      } else if (vm > 0 && vn > 0) {
-#pragma unroll
-        for (int kk = 0; kk < KC; kk += 4) {
-          double fa[FM], fb[FN];
-#pragma unroll
-          for (int i = 0; i < FM; ++i) fa[i] = a[kk * LDA + 8 * i];
-#pragma unroll
-          for (int j = 0; j < FN; ++j) fb[j] = b[kk * LDB + 8 * j];
-#pragma unroll
-          for (int i = 0; i < FM; ++i)
-#pragma unroll
-            for (int j = 0; j < FN; ++j)
-              if (i < vm && j < vn) dmma884(acc[i][j][0], acc[i][j][1], fa[i], fb[j]);
+          for (int j = 0; j < 9; ++j)
+            if (usej[j]) dmma884(dacc[j][0], dacc[j][1], j < n_hi ? fa_hi : fa_lo, fb[j]);
         }
       }
       __syncwarp();
-      if (lane == 0) mbar_arrive(empty_bar(st));  // this warp has read the stage
+      if (lane == 0) mbar_arrive(empty_bar(st));
     }
+#pragma unroll
+    for (int j = 0; j < 9; ++j) {
+      if (!usej[j]) continue;
+      const bool hi = j < n_hi;
+      syrk_store_pair<TILE, SUB>(dacc[j][0], dacc[j][1], ti, ti, 8 * (hi ? r_hi : r_lo) + (lane >> 2),
+                                 8 * (hi ? c_hi0 + j : j - n_hi) + 2 * (lane & 3), ld, n_store, slot_part, sp);
+    }
+    return;
+  }
 
-    const int orow = wr * WM + (lane >> 2);
-    const int ocol = wc * WN + 2 * (lane & 3);
+  // (A column-per-warp mapping for the thin tiles of a ragged last tile row was tried and dropped:
+  // with only 2 of 16 fragment rows to compute, the warps outrun the three-stage TMA ring and wait
+  // for every chunk -- C3 went from 28.8 to 31.1 ms.  Such rows are folded into tall tiles instead.)
+  const int wr = warp / WC, wc = warp % WC;
+  int vm = 0, vn = 0;
 #pragma unroll
-    for (int i = 0; i < FM; ++i)
+  for (int i = 0; i < FM; ++i) vm += (ti * TILE + wr * WM + 8 * i) < n_valid;
 #pragma unroll
-      for (int j = 0; j < FN; ++j)
-        syrk_store_pair<SUB>(acc[i][j][0], acc[i][j][1], ti, tj, orow + 8 * i, ocol + 8 * j, ld, n_store, slot_part, sp);
-    if (xvalid) {
-      // the ragged rows below the tile: rows 0.. of the thin tile's partial slot (never with SUB)
-      double* xp = part + (size_t)slot2 * TILE * TILE + (size_t)(8 * (wr & 1) + (lane >> 2)) * TILE;
+  for (int j = 0; j < FN; ++j) vn += (tj * TILE + wc * WN + 8 * j) < n_valid;
+  const bool full = vm == FM && vn == FN;
+  const int aoff = kq * LDA + wr * WM + (lane >> 2);
+  const int boff = kq * LDB + wc * WN + (lane >> 2);
+  // tall item: this warp's two extra fragments -- fragment row 16 + (wr & 1) of A against its B
+  // fragments 2 (wr >> 1) and 2 (wr >> 1) + 1
+  const int xoff = kq * LDA + TILE + 8 * (wr & 1) + (lane >> 2);
+  const int xj = 2 * (wr >> 1);
+  const bool xvalid = tall && (ti + 1) * TILE + 8 * (wr & 1) < n_valid;
+
+  double acc[FM][FN][2], xacc[2][2];
 #pragma unroll
-      for (int e = 0; e < 2; ++e)
-        *reinterpret_cast<double2*>(xp + wc * WN + 8 * (xj + e) + 2 * (lane & 3)) = make_double2(xacc[e][0], xacc[e][1]);
+  for (int i = 0; i < FM; ++i)
+#pragma unroll
+    for (int j = 0; j < FN; ++j) acc[i][j][0] = acc[i][j][1] = 0.0;
+  xacc[0][0] = xacc[0][1] = xacc[1][0] = xacc[1][1] = 0.0;
+
+  for (int kc = 0; kc < nk; ++kc) {
+    refill(kc);
+    const int st = kc % kTmaStages;
+    mbar_wait(full_bar(st), (kc / kTmaStages) & 1u);
+    const double* a = stages + (size_t)st * kStageDoubles + aoff;
+    const double* b = stages + (size_t)st * kStageDoubles + kTmaADoubles + boff;
+    if (full && xvalid) {
+      const double* x = stages + (size_t)st * kStageDoubles + xoff;
+#pragma unroll
+      for (int kk = 0; kk < KC; kk += 4) {
+        double fa[FM], fb[FN];
+#pragma unroll
+        for (int i = 0; i < FM; ++i) fa[i] = a[kk * LDA + 8 * i];
+#pragma unroll
+        for (int j = 0; j < FN; ++j) fb[j] = b[kk * LDB + 8 * j];
+        const double fx = x[kk * LDA];
+#pragma unroll
+        for (int i = 0; i < FM; ++i)
+#pragma unroll
+          for (int j = 0; j < FN; ++j) dmma884(acc[i][j][0], acc[i][j][1], fa[i], fb[j]);
+        dmma884(xacc[0][0], xacc[0][1], fx, xj == 0 ? fb[0] : fb[2]);
+        dmma884(xacc[1][0], xacc[1][1], fx, xj == 0 ? fb[1] : fb[3]);
+      }
+    } else if (full) {
+#pragma unroll
+      for (int kk = 0; kk < KC; kk += 4) {
+        double fa[FM], fb[FN];
+#pragma unroll
+        for (int i = 0; i < FM; ++i) fa[i] = a[kk * LDA + 8 * i];
+#pragma unroll
+        for (int j = 0; j < FN; ++j) fb[j] = b[kk * LDB + 8 * j];
+#pragma unroll
+        for (int i = 0; i < FM; ++i)
+#pragma unroll
+          for (int j = 0; j < FN; ++j) dmma884(acc[i][j][0], acc[i][j][1], fa[i], fb[j]);
+      }
+    } else if (vm > 0 && vn > 0) {
+#pragma unroll
+      for (int kk = 0; kk < KC; kk += 4) {
+        double fa[FM], fb[FN];
+#pragma unroll
+        for (int i = 0; i < FM; ++i) fa[i] = a[kk * LDA + 8 * i];
+#pragma unroll
+        for (int j = 0; j < FN; ++j) fb[j] = b[kk * LDB + 8 * j];
+#pragma unroll
+        for (int i = 0; i < FM; ++i)
+#pragma unroll
+          for (int j = 0; j < FN; ++j)
+            if (i < vm && j < vn) dmma884(acc[i][j][0], acc[i][j][1], fa[i], fb[j]);
+      }
     }
+    __syncwarp();
+    if (lane == 0) mbar_arrive(empty_bar(st));  // this warp has read the stage
+  }
+
+  const int orow = wr * WM + (lane >> 2);
+  const int ocol = wc * WN + 2 * (lane & 3);
+#pragma unroll
+  for (int i = 0; i < FM; ++i)
+#pragma unroll
+    for (int j = 0; j < FN; ++j)
+      syrk_store_pair<TILE, SUB>(acc[i][j][0], acc[i][j][1], ti, tj, orow + 8 * i, ocol + 8 * j, ld, n_store, slot_part, sp);
+  if (xvalid) {
+    // the ragged rows below the tile: rows 0.. of the thin tile's partial slot (never with SUB).  The
+    // slot is read again here (a volatile load, which is not merged with the first one): kept live
+    // through the k-loop it would be spilled at 128 registers.
+    const int slot2 = __ldcv(&items[blockIdx.x].slot2);
+    double* xp = part + (size_t)slot2 * TILE * TILE + (size_t)(8 * (wr & 1) + (lane >> 2)) * TILE;
+#pragma unroll
+    for (int e = 0; e < 2; ++e)
+      *reinterpret_cast<double2*>(xp + wc * WN + 8 * (xj + e) + 2 * (lane & 3)) = make_double2(xacc[e][0], xacc[e][1]);
   }
 }
 
@@ -1046,14 +986,6 @@ emu_reconstruct_kernel(const uint32_t* __restrict__ Pmod, int n_tiles, const uns
 static inline int syrk_kc(int tile) { return tile == 128 ? 32 : 16; }
 static inline int syrk_occupancy(int tile) { return tile == 128 ? 1 : 4; }
 
-int syrk_feed_is_tma();
-// The planner's view of the feed: BA_SYRK_PLAN_ASSUME_TMA=1 lets the host-only self-check of the
-// plan (ba_syrk_plan_info, run on CPU boxes) exercise the TMA kernel's tile shapes.
-static bool plan_for_tma() {
-  static const bool assume = std::getenv("BA_SYRK_PLAN_ASSUME_TMA") != nullptr;
-  return assume || syrk_feed_is_tma();
-}
-
 // Relative duration of a tile per k-row (1 = full tile), mirroring the kernel's warp mapping:
 // edge tiles skip the 8x8 fragments beyond n_valid, diagonal tiles the sub-tiles above the
 // diagonal.  A warp sits on scheduler partition (warp % 4) with its own FP64 pipe: a CTA that has
@@ -1063,8 +995,7 @@ static double tile_weight(int TILE, int WR, int WC, int occ, int ti, int tj, int
                           double floor_override = -1.0) {
   const int WM = TILE / WR, WN = TILE / WC, FM = WM / 8, FN = WN / 8;
   double load[4] = {0, 0, 0, 0};
-  const bool tma_tile = TILE == kTmaTile && occ == 1 && plan_for_tma();
-  const bool folded_diag = ti == tj && tma_tile;
+  const bool folded_diag = ti == tj && TILE == kTmaTile;
 
   if (folded_diag) {
     // the TMA kernel's diagonal mapping: fragment rows r and 15 - r shared by two warps (9 + 8)
@@ -1099,17 +1030,15 @@ static double tile_weight(int TILE, int WR, int WC, int occ, int ti, int tj, int
   // A CTA pays for every k-row it streams whatever it computes on it (copies, barrier, pipeline
   // bookkeeping): tiles with little tensor work are bounded by that floor, not by their DMMA count.
   // Measured at C2 (50 x 10k): the 64-tile kernel (four CTAs per SM) is fastest with uniform cuts
-  // (floor 1.0: 0.302 ms per iteration, 0.75: 0.309, 0.5: 0.344, 0.35: 0.430); the 128-tile
-  // kernel with floor 0.75 (1.0: 0.326, 0.75: 0.283, 0.5: 0.343, 0.35: 0.355).
-  // The TMA-fed kernel has no per-row copy instructions to pay for: a thin tile costs what its
+  // (floor 1.0: 0.302 ms per iteration, 0.75: 0.309, 0.5: 0.344, 0.35: 0.430).
+  // The TMA-fed 128-tile kernel has no per-row copy instructions to pay for: a thin tile costs what its
   // fragments cost, down to the rate at which the TMA unit streams the rows (measured floor ~0.3).
   // Measured with the TMA kernel (B200): C3 (4.3 GB operand, ~3300-row pieces) floor 0.5: 28.79 ms,
   // 0.3: 28.86, 0.15: 28.86, 0.75: 29.42; C2 (108 MB operand, two waves of ~730-row pieces) floor
   // 1.0: 0.286 ms, 0.5: 0.298, 0.3: 0.311 -- with two waves the schedule is decided by whole items,
   // and uniform cuts pack them best.
   const bool small_operand = k_pad > 0 && (double)k_pad * n_valid * 8.0 <= 256.0 * 1024 * 1024;
-  double floor_w = occ == 1 ? (plan_for_tma() ? (small_operand ? 1.0 : 0.5) : 0.75) : 1.0;
-  if (const char* f = std::getenv("BA_SYRK_FLOOR")) floor_w = std::atof(f);  // tuning experiments only
+  double floor_w = occ == 1 && !small_operand ? 0.5 : 1.0;
   if (floor_override >= 0.0) floor_w = floor_override;
   return w > floor_w ? w : floor_w;
 }
@@ -1118,19 +1047,17 @@ struct SyrkPlan {
   std::vector<SyrkItem> items;       // launch order: ascending k range, then tile
   std::vector<int> tile_first;       // [n_tiles + 1]
   std::vector<int> tile_items;       // partial-tile slot per (tile, piece), pieces in ascending k order
-  std::vector<int> cta_first;        // stream-K plans: [n_ctas + 1] first item of every CTA (else empty)
   int n_slots = 0;                   // partial tiles: one per item + one per tall item (its thin tile below)
   int tall_row = -1;                 // tile row whose off-diagonal tiles also compute the ragged rows below
   double makespan = 0.0;             // modelled duration in k-rows of a full tile on one SM slot
 };
 
-// The ragged last tile row is folded into the row above (see kTmaTallRows) when the TMA kernel runs
-// and at most kTmaTallRows rows are left over: returns that row (nt1 - 2), else -1.
-static int tall_tile_row(int n_pad, int TILE, int occ) {
-  static const bool off = std::getenv("BA_SYRK_NO_TALL") != nullptr;  // A/B timing only
+// The ragged last tile row of 128-tiles is folded into the row above (see kTmaTallRows) when at most
+// kTmaTallRows rows are left over: returns that row (nt1 - 2), else -1.
+static int tall_tile_row(int n_pad, int TILE) {
   const int nt1 = (n_pad + TILE - 1) / TILE;
   const int left = n_pad - (nt1 - 1) * TILE;
-  if (off || TILE != kTmaTile || occ != 1 || !plan_for_tma() || nt1 < 3 || left > kTmaTallRows) return -1;
+  if (TILE != kTmaTile || nt1 < 3 || left > kTmaTallRows) return -1;
   return nt1 - 2;
 }
 
@@ -1148,10 +1075,9 @@ static SyrkPlan plan_syrk(int n_pad, int TILE, int WR, int WC, int64_t k_pad, in
   const int64_t n_chunks = k_pad / KC;
   const int slots = num_sms * occ;
   std::vector<double> w(n_tiles), w_run(n_tiles);  // w: decides the cuts; w_run: the modelled duration per k-row
-  static const char* lpt_env = std::getenv("BA_SYRK_LPT");  // "0" / "1": A/B timing
-  const bool lpt = lpt_env ? std::atoi(lpt_env) != 0 : (double)k_pad * n_pad * 8.0 <= 116.0 * 1024 * 1024;
-  static const double run_floor = std::getenv("BA_SYRK_RUN_FLOOR") ? std::atof(std::getenv("BA_SYRK_RUN_FLOOR")) : 0.5;
-  const int tall_row = tall_tile_row(n_pad, TILE, occ);
+  const bool lpt = (double)k_pad * n_pad * 8.0 <= 116.0 * 1024 * 1024;
+  const double run_floor = 0.5;
+  const int tall_row = tall_tile_row(n_pad, TILE);
   // absorbed[t]: thin tile (nt1 - 1, tj), tj < tall_row: computed by the tall tile (tall_row, tj)
   std::vector<char> absorbed(n_tiles, 0), is_tall(n_tiles, 0);
   for (int t = 0, ti = 0; ti < nt1; ++ti)
@@ -1248,75 +1174,6 @@ static SyrkPlan plan_syrk(int n_pad, int TILE, int WR, int WC, int64_t k_pad, in
   return plan;
 }
 
-// Small operands (the whole of Y^T stays in the 126 MB L2, so the order in which k-ranges are
-// visited does not matter): stream-K.  With whole items the C2 product is two waves of ~1000-row
-// items on 148 SMs -- the schedule, not the kernel, bounds it at 0.55 of the DMMA peak.  Here the
-// modelled work (tile weight x chunks, tile by tile) is dealt to one CTA per SM in equal shares,
-// crossing tile boundaries; a CTA's segments run through one TMA ring (syrk_tma_kernel), so the
-// pipeline is filled once per CTA.  Every segment still writes its own partial tile, and the tiles
-// are summed in ascending k order as before: deterministic.
-static SyrkPlan plan_streamk(int n_pad, int64_t k_pad, int num_sms) {
-  constexpr int TILE = kTmaTile, KC = kTmaKC;
-  const int nt1 = (n_pad + TILE - 1) / TILE;
-  const int n_tiles = nt1 * (nt1 + 1) / 2;
-  const int64_t n_chunks = k_pad / KC;
-  std::vector<double> w(n_tiles);
-  for (int t = 0, ti = 0; ti < nt1; ++ti)
-    for (int tj = 0; tj <= ti; ++tj, ++t) {
-      // executed 8 x 8 fragments per k-step against the 256 of a full tile; a thin tile is bound by
-      // the ring's latency instead (measured ~0.3)
-      const int rows = std::min(16, (n_pad - ti * TILE + 7) / 8);
-      const double frags = ti == tj ? rows * (rows + 1) / 2.0 : rows * 16.0;
-      w[t] = std::max(0.3, frags / 256.0);
-    }
-  const int64_t min_seg = 4;       // chunks
-  const double seg_cost = 1.5;     // chunks of a full tile: accumulator hand-over and the partial-tile store
-  double total = 0.0;
-  for (int t = 0; t < n_tiles; ++t) total += w[t] * (double)n_chunks + seg_cost;
-  const int G = num_sms;
-  const double budget = total / G + seg_cost;
-  SyrkPlan plan;
-  plan.tile_first.assign(n_tiles + 1, 0);
-  plan.cta_first.assign(1, 0);
-  int cta = 0;
-  double left = budget;
-  auto next_cta = [&]() {
-    plan.cta_first.push_back((int)plan.items.size());
-    ++cta;
-    left = budget;
-  };
-  for (int t = 0, ti = 0; ti < nt1; ++ti)
-    for (int tj = 0; tj <= ti; ++tj, ++t) {
-      int64_t pos = 0;
-      while (pos < n_chunks) {
-        const int64_t rem = n_chunks - pos;
-        int64_t can = (int64_t)std::floor((left - seg_cost) / w[t]);
-        if (cta == G - 1) can = rem;  // the last CTA takes whatever is left
-        if (can < min_seg && cta < G - 1) { next_cta(); continue; }
-        int64_t take = std::min<int64_t>(rem, std::max<int64_t>(can, min_seg));
-        if (rem - take < min_seg) take = rem;  // no crumbs
-        plan.tile_items.push_back((int)plan.items.size());
-        plan.items.push_back({ti, tj, (int)pos, (int)(pos + take), -1});
-        pos += take;
-        left -= (double)take * w[t] + seg_cost;
-      }
-      plan.tile_first[t + 1] = (int)plan.items.size();
-    }
-  while ((int)plan.cta_first.size() < G + 1) plan.cta_first.push_back((int)plan.items.size());
-  plan.n_slots = (int)plan.items.size();
-  plan.makespan = budget * KC;
-  return plan;
-}
-
-// Measured on B200 (C2, 50 cameras x 10k points): 0.82 ms against 0.29 ms with whole items in k-major
-// order -- with every CTA streaming its own (tile, k-range) nothing is shared between the SMs any
-// more and the thin tiles' long k-ranges become the makespan.  The plan and the multi-segment kernel
-// are kept behind BA_SYRK_STREAMK=1 for the next attempt (k-major dealing of equal shares).
-static bool use_streamk(int n_pad, int tile, int64_t k_pad) {
-  static const bool on = std::getenv("BA_SYRK_STREAMK") != nullptr;
-  return on && tile == kTmaTile && plan_for_tma() && (double)k_pad * n_pad * 8.0 <= 128.0 * 1024 * 1024;
-}
-
 // Plans are kept for the life of the process: the schedule search costs milliseconds of host
 // time, more than a small adjustment, and callers adjust scene after scene of the same shape.
 static const SyrkPlan& cached_plan(int n_pad, int tile, int64_t k_pad, int num_sms) {
@@ -1327,9 +1184,8 @@ static const SyrkPlan& cached_plan(int n_pad, int tile, int64_t k_pad, int num_s
   for (auto& kv : cache)
     if (kv.first.n_pad == n_pad && kv.first.tile == tile && kv.first.k_pad == k_pad && kv.first.sms == num_sms)
       return *kv.second;
-  SyrkPlan* p = new SyrkPlan(use_streamk(n_pad, tile, k_pad) ? plan_streamk(n_pad, k_pad, num_sms)
-                             : tile == 128 ? plan_syrk(n_pad, 128, 4, 4, k_pad, num_sms)
-                                           : plan_syrk(n_pad, 64, 2, 2, k_pad, num_sms));
+  SyrkPlan* p = new SyrkPlan(tile == 128 ? plan_syrk(n_pad, 128, 4, 4, k_pad, num_sms)
+                                         : plan_syrk(n_pad, 64, 2, 2, k_pad, num_sms));
   cache.push_back({Key{n_pad, tile, k_pad, num_sms}, p});
   return *p;
 }
@@ -1346,11 +1202,6 @@ int syrk_plan_engine(ba_engine* e) {
   if (e->syrk_emu) return emu_plan_engine(e);
   const SyrkPlan& plan = cached_plan(e->n_pad, e->syrk_tile, e->k_pad, e->num_sms);
   e->syrk_n_items = (int)plan.items.size();
-  e->syrk_n_ctas = plan.cta_first.empty() ? e->syrk_n_items : (int)plan.cta_first.size() - 1;
-  if (!plan.cta_first.empty()) {
-    BA_CUDA(cudaMallocAsync(reinterpret_cast<void**>(&e->syrk_cta_first), plan.cta_first.size() * sizeof(int), (cudaStream_t)0));
-    BA_CUDA(cudaMemcpy(e->syrk_cta_first, plan.cta_first.data(), plan.cta_first.size() * sizeof(int), cudaMemcpyHostToDevice));
-  }
   const int nt1 = (e->n_pad + e->syrk_tile - 1) / e->syrk_tile;
   e->syrk_n_tiles = nt1 * (nt1 + 1) / 2;
   const size_t tt = (size_t)e->syrk_tile * e->syrk_tile;
@@ -1407,13 +1258,13 @@ static int make_operand_map(CUtensorMap* map, const double* base, int cols, int6
   return BA_OK;
 }
 
-// BA_SYRK_NO_TMA=1 keeps the cp.async kernel (A/B timing).
-static bool syrk_use_tma() {
-  static const bool on = std::getenv("BA_SYRK_NO_TMA") == nullptr;
-  return on;
+// The 128-tile product, the wide Cholesky updates and the INT8 emulation are all fed by TMA; every
+// driver that runs sm_100a code offers the encoder, so an engine checks for it once when created.
+int require_tensor_map_encoder() {
+  if (tensor_map_encoder()) return BA_OK;
+  set_error("cuTensorMapEncodeTiled is not available from this driver (the TMA-fed kernels need it)");
+  return BA_ERR_CUDA;
 }
-
-int syrk_feed_is_tma() { return syrk_use_tma() && tensor_map_encoder() != nullptr; }
 
 // ---- emulated product: host side ------------------------------------------------------------------
 static const EmuConsts& emu_consts() {
@@ -1463,8 +1314,7 @@ int syrk_emu_info(int64_t k_pad, int32_t* moduli, int* n_moduli, int* bits) {
 
 static bool emu_select(const ba_engine* e) {
   if (const char* v = std::getenv("BA_SYRK_EMU")) return std::atoi(v) != 0;
-  return e->emu_bits >= 50 && tensor_map_encoder() != nullptr &&
-         (double)e->n_pad * e->n_pad * (double)e->k_pad >= kEmuMinWork;
+  return e->emu_bits >= 50 && (double)e->n_pad * e->n_pad * (double)e->k_pad >= kEmuMinWork;
 }
 
 // Work items: every (modulus, lower 256-tile) over P equal k pieces of <= kEmuMaxKB blocks, in two
@@ -1582,16 +1432,16 @@ static int launch_syrk_emu(ba_engine* e, const ba_lm_state* ctl, cudaStream_t s)
 template <int TILE, int WR, int WC, int KC>
 static int launch_syrk(ba_engine* e, const ba_lm_state* ctl, cudaStream_t s) {
   const int64_t n_chunks = e->k_pad / KC;
-  if (TILE == kTmaTile && KC == kTmaKC && syrk_use_tma()) {
+  if constexpr (TILE == kTmaTile) {
+    static_assert(KC == kTmaKC, "the 128-tile product runs on the TMA kernel");
     CUtensorMap mapA, mapB;
     BA_TRY(make_operand_map(&mapA, e->Yt, e->n_pad, e->k_pad, e->n_pad, kTmaLda));
     BA_TRY(make_operand_map(&mapB, e->Yt, e->n_pad, e->k_pad, e->n_pad, kTmaLdb));
     BA_CUDA(cudaFuncSetAttribute(syrk_tma_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                  (int)kTmaSmemBytes));
     ProfScope ps(e, PG_SYRK, s);
-    syrk_tma_kernel<false><<<e->syrk_n_ctas, kTmaThreads, kTmaSmemBytes, s>>>(
-        mapA, mapB, e->n_pad, e->n_pad, n_chunks, e->syrk_items, e->syrk_cta_first, e->Spart, ctl, 0,
-        SubSplit{0, 1, 0, 0, {}});
+    syrk_tma_kernel<false><<<e->syrk_n_items, kTmaThreads, kTmaSmemBytes, s>>>(
+        mapA, mapB, e->n_pad, e->n_pad, n_chunks, e->syrk_items, e->Spart, ctl, 0, SubSplit{0, 1, 0, 0, {}});
     BA_LAUNCH_CHECK();
   } else {
     const size_t smem = (size_t)2 * kStages * KC * (TILE + 4) * sizeof(double);
@@ -1625,9 +1475,6 @@ static int launch_syrk_sub(double* S, int ld, int n_rows, int t0, const double* 
   const int nt1 = (n_valid + TILE - 1) / TILE;
   const int n_tiles = nt1 * (nt1 + 1) / 2;
   const int n_chunks = depth / KC;
-  const size_t smem = (size_t)2 * kStages * KC * (TILE + 4) * sizeof(double);
-  BA_CUDA(cudaFuncSetAttribute(syrk_dmma_kernel<TILE, WR, WC, KC, true>,
-                               cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   const size_t origin = (size_t)t0 * ld + t0;
   SubSplit sp{0, 1, 0, 0, {}};
   if (split && split->world > 1) {
@@ -1637,19 +1484,22 @@ static int launch_syrk_sub(double* S, int ld, int n_rows, int t0, const double* 
     sp.push_cols = split->push_cols;
     for (int q = 0; q < split->world; ++q) sp.peer[q] = split->S_peer[q] + origin;
   }
-  if (TILE == kTmaTile && KC == kTmaKC && syrk_use_tma()) {
+  if constexpr (TILE == kTmaTile) {
+    static_assert(KC == kTmaKC, "the 128-tile update runs on the TMA kernel");
     CUtensorMap mapA, mapB;
     BA_TRY(make_operand_map(&mapA, Lt + t0, n_valid, depth, ld, kTmaLda));
     BA_TRY(make_operand_map(&mapB, Lt + t0, n_valid, depth, ld, kTmaLdb));
     BA_CUDA(cudaFuncSetAttribute(syrk_tma_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                  (int)kTmaSmemBytes));
     syrk_tma_kernel<true><<<n_tiles, kTmaThreads, kTmaSmemBytes, s>>>(mapA, mapB, ld, n_valid, n_chunks, nullptr,
-                                                                      nullptr, S + origin, ctl, n_store, sp);
-    BA_LAUNCH_CHECK();
-    return BA_OK;
+                                                                      S + origin, ctl, n_store, sp);
+  } else {
+    const size_t smem = (size_t)2 * kStages * KC * (TILE + 4) * sizeof(double);
+    BA_CUDA(cudaFuncSetAttribute(syrk_dmma_kernel<TILE, WR, WC, KC, true>,
+                                 cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    syrk_dmma_kernel<TILE, WR, WC, KC, true><<<n_tiles, WR * WC * 32, smem, s>>>(
+        Lt + t0, ld, n_valid, n_chunks, nullptr, S + origin, ctl, n_store, sp);
   }
-  syrk_dmma_kernel<TILE, WR, WC, KC, true><<<n_tiles, WR * WC * 32, smem, s>>>(
-      Lt + t0, ld, n_valid, n_chunks, nullptr, S + origin, ctl, n_store, sp);
   BA_LAUNCH_CHECK();
   return BA_OK;
 }

@@ -342,5 +342,6 @@ def syrk_emu_info(k_pad: int) -> tuple[list[int], int]:
 
 
 def syrk_feed() -> str:
-    """Operand feed of the 128-tile SYRK kernel: "tma" (cp.async.bulk.tensor + mbarriers) or "cp.async"."""
-    return "tma" if _cabi.load().ba_syrk_feed() else "cp.async"
+    """Operand feed of the 128-tile SYRK kernel, which bench.py reports as `operand_feed`: always
+    "tma" (cp.async.bulk.tensor + mbarriers), the only feed that kernel has."""
+    return "tma"

@@ -248,10 +248,6 @@ int ba_profile_reset(ba_engine* e);
  * 0: DFMA, 2: both interleaved with equal FMA counts (do they share the FP64 datapath?), 100 + w:
  * the DFMA loop with w warps per SM (rate at low occupancy). */
 int ba_fp64_peak(int device, int use_dmma, double* tflops);
-/* How the 128-tile Schur SYRK / Cholesky trailing update gets its operands: 1 = TMA tensor copies +
- * mbarriers with a producer warp (cp.async.bulk.tensor, SASS UTMALDG), 0 = cp.async (LDGSTS; set
- * BA_SYRK_NO_TMA=1 for A/B timing, or the driver does not offer cuTensorMapEncodeTiled). */
-int ba_syrk_feed(void);
 /* 1 when this engine linearises matrix-free: a dense scene whose camera table fits shared memory
  * (<= 361 cameras) re-derives the Jacobian rows in K2a, the camera blocks, K2b and the point update
  * instead of storing them in K1 and reading them back (reference :309-427 evaluated where used);

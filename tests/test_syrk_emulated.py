@@ -136,6 +136,7 @@ DENSE_SHAPES = [
     (17, 333, "x-up_z-forward"),
     (260, 300, "x-right_z-forward"),
     (40, 50_000, "x-up_z-forward"),   # K = 150 000 > 131 071: two k pieces per tile
+    (200, 300, "x-up_z-forward"),     # n_pad = 14 x 128 + 16: the DMMA reference runs tall 128-tiles
 ]
 
 

@@ -1,10 +1,11 @@
-"""Time the dense Schur product (K3: syrk_dmma_kernel + syrk_reduce_kernel) alone on one scene.
+"""Time the dense Schur product (K3) alone on one scene: the "syrk" profile group, i.e. the DMMA
+kernels (syrk_tma_kernel for 128-tiles, syrk_dmma_kernel for 64-tiles) and syrk_reduce_kernel, or
+the INT8 emulation's kernels when the engine picks it.
 
     python tools/syrk_sweep.py --cams 200 --points 100000 [--reps 5]
 
 Prints the SYRK kernel's average launch time, the algorithmic TFLOP/s (3 N n (n + 1), n = 9 M - 7)
-and its fraction of the DMMA peak measured on the same GPU.  Planner experiments go through the
-library's environment switches (BA_SYRK_TILE, BA_SYRK_FLOOR, ...), one process per setting.
+and its fraction of the DMMA peak measured on the same GPU.
 """
 import argparse
 import json
