@@ -117,8 +117,7 @@ static bool upload_pool_ready(int device) {
 }
 
 static bool staged_upload(void* dst, const void* src, size_t bytes, cudaStream_t s) {
-  static const bool off = std::getenv("BA_NO_STAGED_UPLOAD") != nullptr;  // A/B timing
-  if (off || bytes < kUpMin) return false;
+  if (bytes < kUpMin) return false;
   cudaPointerAttributes attr;
   if (cudaPointerGetAttributes(&attr, src) != cudaSuccess) { cudaGetLastError(); return false; }
   if (attr.type != cudaMemoryTypeUnregistered) return false;  // pinned / managed: the DMA engine reads it directly

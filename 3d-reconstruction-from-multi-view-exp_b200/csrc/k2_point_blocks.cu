@@ -22,8 +22,6 @@
 // from the camera table, X_j and the observed point instead of reading what K1 stored -- the same
 // pinned arithmetic, the same summation orders, hence the same bits; K1 then stores nothing, k2a and
 // cam read 16 B/obs, k2b only writes its 216 B/obs.
-#include <cstdlib>
-
 #include "ba_common.cuh"
 
 namespace ba {
@@ -403,11 +401,9 @@ k2b_point_solve_kernel(int64_t N, int M, int axis, const int64_t* __restrict__ o
   }
 }
 
-// Dense scenes whose camera table fits next to the staging rows re-derive the Jacobian rows
-// (BA_NO_MATRIX_FREE: read them back as the sparse path does -- A/B timing).
+// Dense scenes whose camera table fits next to the staging rows re-derive the Jacobian rows.
 bool dense_matrix_free(const ba_engine* e) {
-  static const bool off = std::getenv("BA_NO_MATRIX_FREE") != nullptr;
-  return !off && e->dense && tab_smem_doubles(e->M) * sizeof(double) <= 48 * 1024;
+  return e->dense && tab_smem_doubles(e->M) * sizeof(double) <= 48 * 1024;
 }
 
 int launch_k2b(ba_engine* e, bool conditional, double c_host, cudaStream_t s) {

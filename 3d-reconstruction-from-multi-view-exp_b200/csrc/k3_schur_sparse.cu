@@ -22,20 +22,22 @@
 // No shared-memory or global read-modify-write; the per-lane sums meet once per pair in a fixed order.
 // Order of summation depends on the data only: runs are bit-reproducible.
 //
-// Where the common points come from, and who adds up (history and measurements: DESIGN.md section 3b):
-//   * build_pair_index      once per engine: bitmaps per camera and -- memory permitting -- the STATIC
-//                           PAIR LISTS: the ascending ids of the points every pair shares
-//                           (pair_count_kernel, exclusive sum, pair_fill_kernel; 4 B per pair-point).
-//                           Visibility does not change between iterations; intersecting the bitmaps
-//                           and compacting the hits every solve was more than half of the kernel.
-//   * schur_pairs_reg_kernel<LIST = true>   the default: 32 ids per round with one coalesced load; the
-//                           pair's 9 x 9 block lives in 81 FP64 registers per lane (144 DFMAs per point).
-//   * schur_pairs_kernel<MINB, LIST>        the variant with the leading 8 x 8 of the block on DMMA.8x8x4
-//                           (operands transposed through shared memory); with LIST = false it scans
-//                           the bitmaps itself (4096 points per step, warp prefix sum, ring queue):
-//                           the path taken when the lists do not fit the memory budget.
-//   * schur_pairs_reg_kernel<LIST = false>  register accumulators with a lane-autonomous bitmap scan
-//                           (claimed 256-point groups); A/B runs only (BA_PAIRS_REG with BA_PAIRS_NO_LIST).
+// Two pair kernels; where the common points come from decides which one runs (measurements: DESIGN.md
+// section 3b):
+//   * build_pair_index        once per engine: bitmaps per camera and -- memory permitting -- the STATIC
+//                             PAIR LISTS: the ascending ids of the points every pair shares
+//                             (pair_count_kernel, exclusive sum, pair_fill_kernel; 4 B per pair-point).
+//                             Visibility does not change between iterations; intersecting the bitmaps
+//                             and compacting the hits every solve was more than half of the kernel.
+//   * schur_pairs_reg_kernel  when the lists exist: 32 ids per round with one coalesced load; the pair's
+//                             9 x 9 block lives in 81 FP64 registers per lane (144 DFMAs per point).
+//   * schur_pairs_kernel      when the lists do not fit a third of the free memory (or BA_PAIRS_NO_LIST
+//                             is set): it scans the bitmaps itself (4096 points per step, warp prefix sum,
+//                             ring queue) and sums the leading 8 x 8 of the block on DMMA.8x8x4 (operands
+//                             transposed through shared memory).  Register accumulators lose with the scan
+//                             (40.0 against 35.9 ms at 1000 x 200k): at 255 registers two warps per
+//                             scheduler cannot overlap the scan's serial phases.  Without the scan they
+//                             win (27.0 against 27.8 ms).
 //
 // Bound: FP64 pipe (~316 instructions per pair-point; sum_j m_j (m_j - 1) / 2 pair-points).  DMMA runs
 // on the same FP64 datapath as DFMA on this GPU (fp64_peak.cu, mode 2), so the tensor form buys no
@@ -138,8 +140,8 @@ int build_pair_index(ba_engine* e, cudaStream_t s) {
   BA_CUDA(cudaMemsetAsync(e->PT, 0, (size_t)e->N * kPT * sizeof(double), s));
   bitmap_fill_kernel<<<e->num_sms * 8, 256, 0, s>>>(e->nobs, e->Wp, e->obs_cam, e->obs_pt, e->bits);
   BA_LAUNCH_CHECK();
-  static const bool no_lists = std::getenv("BA_PAIRS_NO_LIST") != nullptr;  // A/B timing: scan the bitmaps every solve
-  if (no_lists) return BA_OK;
+  // BA_PAIRS_NO_LIST: no lists, the pair kernel scans the bitmaps every solve (tests of that fallback)
+  if (std::getenv("BA_PAIRS_NO_LIST")) return BA_OK;
   const int nt = (e->M + kPairTile - 1) / kPairTile;
   const int64_t n_items = (int64_t)nt * (nt + 1) / 2 * kPairTile * kPairTile;
   if (n_items >= ((int64_t)1 << 31)) return BA_OK;
@@ -248,14 +250,14 @@ __device__ __forceinline__ SideJac side_jacobian(const double* __restrict__ c, d
   return s;
 }
 
-// LIST: the pair's common points come from the static lists (build_pair_index) -- one coalesced load of
-// 32 ids per round, fetched a round ahead -- instead of the bitmap scan with its queue.
-template <int MINB, bool LIST>
-__global__ void __launch_bounds__(32, MINB)
+// ---- bitmap scan (no pair lists) ------------------------------------------------------------------
+// The lanes intersect the two cameras' bitmaps 128 points each per step, a warp prefix sum of the hit
+// counts gives their slots in a ring queue of point ids, and every 32 queued ids make a round.
+// 12 warps per SM at 168 registers.
+__global__ void __launch_bounds__(32, 12)
 schur_pairs_kernel(int M, int axis, int64_t Wp, const uint32_t* __restrict__ bits,
                    const double* __restrict__ camtab, double f0, const double* __restrict__ PT,
-                   double* __restrict__ P, int ld, const ba_lm_state* ctl,
-                   const int64_t* __restrict__ pair_ptr, const int32_t* __restrict__ pair_pts) {
+                   double* __restrict__ P, int ld, const ba_lm_state* ctl) {
   if (ctl && ctl->done) return;
   int i, k;
   if (!pair_from_linear(blockIdx.x, M, i, k)) return;
@@ -417,34 +419,6 @@ schur_pairs_kernel(int M, int axis, int64_t Wp, const uint32_t* __restrict__ bit
     ++rounds;
   };
 
-  if (LIST) {
-    const int64_t lo = pair_ptr[blockIdx.x], hi = pair_ptr[blockIdx.x + 1];
-    int jnext = lo + lane < hi ? pair_pts[lo + lane] : -1;  // the ids of the first round
-    for (int64_t base = lo; base < hi; base += 32) {
-      const int cnt = hi - base < 32 ? (int)(hi - base) : 32;
-      const int jcur = jnext;
-      if (base + 32 < hi) jnext = base + 32 + lane < hi ? pair_pts[base + 32 + lane] : -1;
-      // gather of this round: five consecutive lanes per row
-      const uint32_t sa = s_addr + (uint32_t)(rounds & 1) * (32 * kPS * 8);
-#pragma unroll
-      for (int u = 0; u < kPieces; ++u) {
-        const int p = lane + 32 * u;
-        const int row = (p * 205) >> 10;  // p / 5 for p < 160
-        const int piece = p - kPieces * row;
-        const int jr = __shfl_sync(0xffffffffu, jcur, row);
-        if (row < cnt) cp_async16(sa + (row * kPS + 2 * piece) * 8, PT + (size_t)jr * kPT + 2 * piece);
-      }
-      cp_commit();
-      if (rounds > 0) {
-        cp_wait<1>();
-        __syncwarp();
-        compute((rounds & 1) ^ 1, cnt_prev);
-      }
-      __syncwarp();
-      cnt_prev = cnt;
-      ++rounds;
-    }
-  } else {
   // bitmap words are fetched one batch ahead
   uint4 wi = bi[0], wk = bk[0];
   for (int64_t w0 = 0; w0 < Wp; w0 += 128) {
@@ -483,7 +457,6 @@ schur_pairs_kernel(int M, int axis, int64_t Wp, const uint32_t* __restrict__ bit
     }
   }
   if (qn > 0) round(qn);
-  }
   if (rounds > 0) {
     cp_wait<0>();
     __syncwarp();
@@ -521,38 +494,24 @@ schur_pairs_kernel(int M, int axis, int64_t Wp, const uint32_t* __restrict__ bit
   }
 }
 
-// ---- register-accumulator variant (the default when the static pair lists exist) -------------------
-// What ncu said about the kernel above (profiles/r2_pairs_*): DMMA shares the FP64 datapath with DFMA
-// (fp64_peak mode 2: 32 TF/s in sum), so the tensor instructions buy no arithmetic, and building
-// their fragments costs 128 shared-memory wavefronts per 32 pair-points; and, by stall samples, 60 %
-// of the time went into finding the common points -- the warp-wide prefix scan, the divergent
-// bit-extraction loops, the queue and the index arithmetic of the gather (~400 integer instructions
-// per round) -- not into the products.  This variant changes both:
-//   * every lane keeps the whole 9 x 9 block of the pair in 81 FP64 registers and adds its point's
-//     Jc_i^T (G Jc_k) with 144 DFMAs (the structural zeros of Jc_i skipped): no fragments, no
-//     shuffles, 255 registers, eight warps per SM, independent accumulator chains;
-//   * every lane scans the bitmaps ON ITS OWN: the point range is cut into groups of 256 points that
-//     the lanes claim one at a time, a lane holds the AND of its current group in four
-//     64-bit registers, takes its next common point with one find-first-set, and computes the point
-//     it took one round earlier (the 32 rows of a round are gathered by the warp together, five
-//     consecutive lanes per row, with 16-byte cp.async).  No queue, no prefix sums, no warp-level compaction; the next
-//     group's bitmap words are prefetched into a private shared-memory slot by cp.async as well.
-//     A lane whose new group is empty idles for that round (3 % at 10 % visibility).
+// ---- pair lists: register accumulators ------------------------------------------------------------
+// DMMA shares the FP64 datapath with DFMA (fp64_peak mode 2: 32 TF/s in sum), so the tensor
+// instructions of the kernel above buy no arithmetic, and building their fragments costs 128
+// shared-memory wavefronts per 32 pair-points.  Here every lane keeps the whole 9 x 9 block of the pair
+// in 81 FP64 registers and adds its point's Jc_i^T (G Jc_k) with 144 DFMAs (the structural zeros of
+// Jc_i skipped): no fragments, no shuffles, 255 registers, eight warps per SM, independent accumulator
+// chains.  The ids of a round come from the static lists (build_pair_index): 32 with one coalesced
+// load, fetched a round ahead.
 // The 81 per-lane sums meet once per pair, through shared memory (the staging rows, free by then),
 // in lane order.  Order of summation depends on the data only: bit-reproducible.
-constexpr int kGroupWords = 8;  // 256 points per lane and group
-
 struct PairRegSmem {
-  double stage[2][32 * kPS];  // [parity][lane][kPS] private rows; reduction scratch [27][33] at the end
-  uint4 slot[2][4][32];       // [parity][camera i lo, i hi, camera k lo, k hi][lane]: prefetched bitmap group
+  double stage[2][32 * kPS];  // [parity][lane][kPS] the rows of the round's points; reduction scratch [27][33] at the end
   double cam[2][20];
 };
 static_assert(27 * 33 <= 2 * 32 * kPS, "reduction scratch must fit the staging buffers");
 
-template <bool LIST>
 __global__ void __launch_bounds__(32, 8)
-schur_pairs_reg_kernel(int M, int axis, int64_t Wp, const uint32_t* __restrict__ bits,
-                       const double* __restrict__ camtab, double f0, const double* __restrict__ PT,
+schur_pairs_reg_kernel(int M, int axis, const double* __restrict__ camtab, double f0, const double* __restrict__ PT,
                        double* __restrict__ P, int ld, const ba_lm_state* ctl,
                        const int64_t* __restrict__ pair_ptr, const int32_t* __restrict__ pair_pts) {
   if (ctl && ctl->done) return;
@@ -646,127 +605,37 @@ schur_pairs_reg_kernel(int M, int axis, int64_t Wp, const uint32_t* __restrict__
     }
   };
 
-  if (LIST) {
-    // static pair lists (build_pair_index): 32 ids per round with one coalesced load, a round ahead
-    const uint32_t stage0 = (uint32_t)__cvta_generic_to_shared(sm.stage[0]);
-    const int64_t lo = pair_ptr[blockIdx.x], hi = pair_ptr[blockIdx.x + 1];
-    int jnext = lo + lane < hi ? pair_pts[lo + lane] : -1;
-    int rounds = 0, cnt_prev = 0;
-    for (int64_t base = lo; base < hi; base += 32) {
-      const int cnt = hi - base < 32 ? (int)(hi - base) : 32;
-      const int jcur = jnext;
-      if (base + 32 < hi) jnext = base + 32 + lane < hi ? pair_pts[base + 32 + lane] : -1;
-      const uint32_t dst = stage0 + (uint32_t)(rounds & 1) * (32 * kPS * 8);
+  const uint32_t stage0 = (uint32_t)__cvta_generic_to_shared(sm.stage[0]);
+  const int64_t lo = pair_ptr[blockIdx.x], hi = pair_ptr[blockIdx.x + 1];
+  int jnext = lo + lane < hi ? pair_pts[lo + lane] : -1;
+  int rounds = 0, cnt_prev = 0;
+  for (int64_t base = lo; base < hi; base += 32) {
+    const int cnt = hi - base < 32 ? (int)(hi - base) : 32;
+    const int jcur = jnext;
+    if (base + 32 < hi) jnext = base + 32 + lane < hi ? pair_pts[base + 32 + lane] : -1;
+    const uint32_t dst = stage0 + (uint32_t)(rounds & 1) * (32 * kPS * 8);
 #pragma unroll
-      for (int u = 0; u < kPieces; ++u) {
-        const int p = lane + 32 * u;
-        const int row = (p * 205) >> 10;  // p / 5 for p < 160
-        const int piece = p - kPieces * row;
-        const int jr = __shfl_sync(0xffffffffu, jcur, row);
-        if (row < cnt) cp_async16(dst + (uint32_t)(row * kPS + 2 * piece) * 8u, PT + (size_t)jr * kPT + 2 * piece);
-      }
-      cp_commit();
-      if (rounds > 0) {
-        cp_wait<1>();
-        __syncwarp();
-        if (lane < cnt_prev) compute((rounds & 1) ^ 1);
-      }
-      __syncwarp();
-      cnt_prev = cnt;
-      ++rounds;
-    }
-    if (rounds > 0) {
-      cp_wait<0>();
-      __syncwarp();
-      if (lane < cnt_prev) compute((rounds - 1) & 1);
-    }
-  } else {
-  // ---- the lanes' walk over the groups -----------------------------------------------------------
-  // Groups are CLAIMED, not owned: a lane that has moved its waiting group into its registers takes
-  // the next unclaimed group (ballot + popc, warp-uniform counter) and starts its prefetch.  Every
-  // lane thus always has one group in flight behind the one it is working on, and the lanes finish
-  // within one group of each other (with fixed ownership the warp waits for its unluckiest lane:
-  // +2 sigma of a Poisson count, 28 % of all rounds at 10^5 points).  The claim order depends on
-  // the bitmaps only: still bit-reproducible.
-  const int n_groups = (int)(Wp / kGroupWords);
-  const uint32_t slot_addr = (uint32_t)__cvta_generic_to_shared(&sm.slot[0][0][lane]);
-  const uint32_t stage_addr0 = (uint32_t)__cvta_generic_to_shared(sm.stage[0]);
-  const uint32_t* gi = bits + (size_t)i * Wp;
-  const uint32_t* gk = bits + (size_t)k * Wp;
-  const uint32_t lt_mask = (1u << lane) - 1u;
-  uint64_t m0 = 0ull, m1 = 0ull, m2 = 0ull, m3 = 0ull;  // common points of the current group, not taken yet
-  int base = 0;          // point id of the current group's bit 0
-  int next = 0;          // first unclaimed group (warp-uniform)
-  int slot_g = -1;       // group waiting (or arriving) in this lane's slot, -1: none
-  int par = 0;           // which of the lane's two slots the next claim uses
-  bool prev = false;     // the lane took a point in the previous round
-  for (int r = 0;; ++r) {
-    cp_wait<0>();  // the previous round's point rows (copied by five lanes each) and bitmap groups
-    __syncwarp();
-    if ((m0 | m1 | m2 | m3) == 0ull && slot_g >= 0) {
-      const uint4* sl = &sm.slot[par ^ 1][0][lane];
-      const uint4 a0 = sl[0], a1 = sl[32], b0 = sl[64], b1 = sl[96];
-      m0 = ((uint64_t)(a0.y & b0.y) << 32) | (a0.x & b0.x);
-      m1 = ((uint64_t)(a0.w & b0.w) << 32) | (a0.z & b0.z);
-      m2 = ((uint64_t)(a1.y & b1.y) << 32) | (a1.x & b1.x);
-      m3 = ((uint64_t)(a1.w & b1.w) << 32) | (a1.z & b1.z);
-      base = slot_g * (32 * kGroupWords);
-      slot_g = -1;
-    }
-    {
-      const uint32_t need = __ballot_sync(0xffffffffu, slot_g < 0);
-      const int g = next + __popc(need & lt_mask);
-      if (slot_g < 0 && g < n_groups) {
-        const uint32_t dst = slot_addr + (uint32_t)par * (uint32_t)sizeof(sm.slot[0]);
-        const size_t off = (size_t)g * kGroupWords;
-        cp_async16(dst, gi + off);
-        cp_async16(dst + 512u, gi + off + 4);
-        cp_async16(dst + 1024u, gk + off);
-        cp_async16(dst + 1536u, gk + off + 4);
-        slot_g = g;
-        par ^= 1;
-      }
-      next += __popc(need);
-      if (next > n_groups) next = n_groups;
-    }
-    const bool hit = (m0 | m1 | m2 | m3) != 0ull;
-    int jhit = -1;
-    if (hit) {
-      int b;
-      if (m0 != 0ull) {
-        b = __ffsll((long long)m0) - 1;
-        m0 &= m0 - 1;
-      } else if (m1 != 0ull) {
-        b = 64 + __ffsll((long long)m1) - 1;
-        m1 &= m1 - 1;
-      } else if (m2 != 0ull) {
-        b = 128 + __ffsll((long long)m2) - 1;
-        m2 &= m2 - 1;
-      } else {
-        b = 192 + __ffsll((long long)m3) - 1;
-        m3 &= m3 - 1;
-      }
-      jhit = base + b;
-    }
-    // The 32 point rows are gathered by the warp together, five consecutive lanes per row: one
-    // instruction then touches ~7 rows instead of 32 (the L1 takes ~2 cycles per 128-byte line an
-    // instruction touches: lane-private gathers cost more than the arithmetic of the round).
-    {
-      const uint32_t dst = stage_addr0 + (uint32_t)(r & 1) * (32 * kPS * 8);
-#pragma unroll
-      for (int u = 0; u < kPieces; ++u) {
-        const int p = lane + 32 * u;
-        const int row = (p * 205) >> 10;  // p / 5 for p < 160
-        const int piece = p - kPieces * row;
-        const int jr = __shfl_sync(0xffffffffu, jhit, row);
-        if (jr >= 0) cp_async16(dst + (uint32_t)(row * kPS + 2 * piece) * 8u, PT + (size_t)jr * kPT + 2 * piece);
-      }
+    for (int u = 0; u < kPieces; ++u) {
+      const int p = lane + 32 * u;
+      const int row = (p * 205) >> 10;  // p / 5 for p < 160
+      const int piece = p - kPieces * row;
+      const int jr = __shfl_sync(0xffffffffu, jcur, row);
+      if (row < cnt) cp_async16(dst + (uint32_t)(row * kPS + 2 * piece) * 8u, PT + (size_t)jr * kPT + 2 * piece);
     }
     cp_commit();
-    if (prev) compute((r & 1) ^ 1);
-    prev = hit;
-    if (!__any_sync(0xffffffffu, hit || slot_g >= 0)) break;  // `hit` lanes still owe one compute
+    if (rounds > 0) {
+      cp_wait<1>();
+      __syncwarp();
+      if (lane < cnt_prev) compute((rounds & 1) ^ 1);
+    }
+    __syncwarp();
+    cnt_prev = cnt;
+    ++rounds;
   }
+  if (rounds > 0) {
+    cp_wait<0>();
+    __syncwarp();
+    if (lane < cnt_prev) compute((rounds - 1) & 1);
   }
   __syncwarp();
 
@@ -882,29 +751,16 @@ int launch_schur_sparse(ba_engine* e, const ba_lm_state* ctl, cudaStream_t s) {
     set_error("too many camera pairs for one launch (M=%d)", e->M);
     return BA_ERR_INVALID;
   }
-  // Variant: with the static pair lists the register-accumulator kernel is the faster one (27.0 against
-  // 27.8 ms at 1000 x 200k), with the bitmap scan the DMMA kernel (35.9 against 40.0).  BA_PAIRS_REG /
-  // BA_PAIRS_DMMA force one of them (A/B timing).
-  static const bool force_reg = std::getenv("BA_PAIRS_REG") != nullptr;
-  static const bool force_dmma = std::getenv("BA_PAIRS_DMMA") != nullptr;
-  const bool have_lists = e->pair_ptr != nullptr && e->pair_pts != nullptr;
-  const bool use_reg = force_reg || (have_lists && !force_dmma);
-  if (!use_reg) {
-    // 12 warps per SM at 168 registers; BA_PAIRS_OCC15: 128 registers (A/B timing with a 14 KB variant of the
-    // shared-memory layout, 15 warps per SM: 39.3 against 38.5 ms at 1000 x 200k -- not occupancy-bound)
-    static const bool occ15 = std::getenv("BA_PAIRS_OCC15") != nullptr;
-    const bool lists = e->pair_ptr != nullptr && e->pair_pts != nullptr;
-    auto kern = lists ? schur_pairs_kernel<12, true> : occ15 ? schur_pairs_kernel<15, false> : schur_pairs_kernel<12, false>;
-    BA_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributePreferredSharedMemoryCarveout,
+  if (e->pair_ptr != nullptr && e->pair_pts != nullptr) {
+    BA_CUDA(cudaFuncSetAttribute(schur_pairs_reg_kernel, cudaFuncAttributePreferredSharedMemoryCarveout,
                                  (int)cudaSharedmemCarveoutMaxShared));
-    kern<<<(unsigned)n_items, 32, 0, s>>>(e->M, e->axis, e->Wp, e->bits, e->camtab[0], e->f0, e->PT, e->P(),
-                                         e->n_pad, ctl, e->pair_ptr, e->pair_pts);
+    schur_pairs_reg_kernel<<<(unsigned)n_items, 32, 0, s>>>(e->M, e->axis, e->camtab[0], e->f0, e->PT, e->P(), e->n_pad,
+                                                           ctl, e->pair_ptr, e->pair_pts);
   } else {
-    const bool lists = e->pair_ptr != nullptr && e->pair_pts != nullptr;
-    auto kern = lists ? schur_pairs_reg_kernel<true> : schur_pairs_reg_kernel<false>;
-    BA_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributePreferredSharedMemoryCarveout, (int)cudaSharedmemCarveoutMaxShared));
-    kern<<<(unsigned)n_items, 32, 0, s>>>(e->M, e->axis, e->Wp, e->bits, e->camtab[0], e->f0, e->PT, e->P(), e->n_pad, ctl,
-                                         e->pair_ptr, e->pair_pts);
+    BA_CUDA(cudaFuncSetAttribute(schur_pairs_kernel, cudaFuncAttributePreferredSharedMemoryCarveout,
+                                 (int)cudaSharedmemCarveoutMaxShared));
+    schur_pairs_kernel<<<(unsigned)n_items, 32, 0, s>>>(e->M, e->axis, e->Wp, e->bits, e->camtab[0], e->f0, e->PT,
+                                                       e->P(), e->n_pad, ctl);
   }
   BA_LAUNCH_CHECK();
   return BA_OK;

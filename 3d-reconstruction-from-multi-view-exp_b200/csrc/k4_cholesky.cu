@@ -7,11 +7,13 @@
 // right-hand side and is swept along as one more row, so after the factorisation it holds
 // y = L^-1 b.  Only L^T x = y is left for chol_backsolve_kernel.
 //
-// Three regimes by size: n < 2048 -- the whole factorisation in ONE persistent cooperative launch
-// (chol_fused_kernel: the steps of chol_step_kernel with a grid barrier between them); n >= 2048 --
-// two-level blocking, per 64-column panel the two launches below and one rank-256 update on the
-// FP64 tensor cores per outer block (launch_chol_wide_update, divided over the ranks of a sharded
-// run).  Back substitution: one CTA (n < 1024), one 8-CTA cluster over distributed shared memory
+// Two regimes by size, n_rows = n + 1 counting the right-hand-side row:
+//   n_rows < 2048  the whole factorisation in ONE persistent cooperative launch (chol_fused_kernel:
+//                  one step per 64-column panel, a grid barrier between the steps);
+//   larger         two-level blocking: per 64-column panel the two launches below, and per 256-wide
+//                  outer block one rank-256 update on the FP64 tensor cores (launch_chol_wide_update,
+//                  divided over the ranks of a sharded run).
+// Back substitution: one CTA (n < 1024), one 8-CTA cluster over distributed shared memory
 // (n < 2048), the whole grid (larger).
 //
 // Large systems, per 64-column panel two launches:
@@ -23,8 +25,6 @@
 //                       Writes L rows in place and a k-major copy Lt for the update.
 //   chol_update_kernel  trailing update S -= L_panel L_panel^T on 64x64 tiles.
 #include <cooperative_groups.h>
-
-#include <cstdlib>
 
 #include "ba_common.cuh"
 
@@ -180,9 +180,8 @@ chol_panel_kernel(double* __restrict__ S, int ld, int n_rows, int k0, int nb,
 // Trailing update S[r][c] -= sum_m L[r][k0+m] L[c][k0+m] on 64x64 tiles of the lower triangle
 // (rows >= cols >= k0+nb, rows < n_rows, cols < c_end).  The diagonal blocks of S keep their
 // pre-factor content: nothing reads L_D from S afterwards (the back substitution uses W = L_D^-T).
-// Small systems: c_end = n_rows, the whole trailing matrix after every panel.  Large systems
-// (two-level blocking): only the columns of the current 256-wide outer block; the rest of the
-// trailing matrix waits for the rank-256 update on the tensor cores (launch_chol_wide_update).
+// c_end closes the current 256-wide outer block: the rest of the trailing matrix waits for the
+// rank-256 update on the tensor cores (launch_chol_wide_update).
 __global__ void __launch_bounds__(256)
 chol_update_kernel(double* __restrict__ S, int ld, int n_rows, int c_end, int k0, int nb,
                    const double* __restrict__ Lt, const ba_lm_state* ctl, int use_ctl) {
@@ -243,17 +242,16 @@ chol_update_kernel(double* __restrict__ S, int ld, int n_rows, int c_end, int k0
     }
 }
 
-// ---- small systems: one launch per panel ------------------------------------------------------
-// For n < 2048 the factorisation is a chain of latency-bound launches (C2, n = 451: 8 panels x
-// (panel 17 us + update 12 us) = 0.23 ms of a 0.70 ms solve).  chol_step_kernel takes the trailing
-// update off that chain: launch p runs
+// ---- small systems: one step per panel -----------------------------------------------------------
+// The factorisation of a small system is a chain of latency-bound panels.  Step p of chol_fused_kernel
+// takes the trailing update off that chain:
 //   * panel blocks   -- as chol_panel_kernel, but each first applies the PREVIOUS panel's update
 //                       to its own 128 x 64 slice (diagonal block + its rows of block column p):
 //                       T -= Lp^T Lp on the FP64 tensor cores, operands staged k-major in shared
 //                       memory next to T (about 2 us), then the elimination;
 //   * update blocks  -- the rest of the previous panel's trailing update (64 x 64 tiles of the
-//                       columns beyond block column p), which nothing in this launch reads.
-// Launch p + 1 needs both, and gets them by stream order.  Lt alternates between two 64-row
+//                       columns beyond block column p), which nothing in step p reads.
+// Step p + 1 needs both and gets them after the grid barrier.  Lt alternates between two 64-row
 // buffers so the previous panel stays readable while the current one is written.
 __device__ __forceinline__ void step_dmma884(double& c0, double& c1, double a, double b) {
   asm volatile("mma.sync.aligned.m8n8k4.row.col.f64.f64.f64.f64 {%0,%1}, {%2}, {%3}, {%0,%1};\n"
@@ -282,8 +280,8 @@ __device__ __forceinline__ void panel_product(const double* __restrict__ A, cons
 }
 
 // One virtual block `vb` of step p (vb < p_blocks: panel block, else update tile vb - p_blocks).
-// S and Lp are read with ld.global.cg: in the persistent kernel below other SMs wrote them within the
-// same launch, and the L1 is not coherent.
+// S and Lp are read with ld.global.cg: other SMs wrote them earlier in the same launch, and the L1 is
+// not coherent.
 __device__ __forceinline__ void chol_step_body(int vb, double* S, int ld, int n_rows, int k0, int nb, int p_blocks,
                                                double* Lt, const double* Lp, double* W, ba_lm_state* ctl,
                                                double* psm) {
@@ -455,15 +453,6 @@ __device__ __forceinline__ void chol_step_body(int vb, double* S, int ld, int n_
   }
 }
 
-
-__global__ void __launch_bounds__(kPanelThreads)
-chol_step_kernel(double* S, int ld, int n_rows, int k0, int nb, int p_blocks, double* Lt, const double* Lp,
-                 double* W, ba_lm_state* ctl, int use_ctl) {
-  if (use_ctl && ctl->done) return;
-  extern __shared__ double psm[];
-  chol_step_body((int)blockIdx.x, S, ld, n_rows, k0, nb, p_blocks, Lt, Lp, W, ctl, psm);
-}
-
 // Back substitution L^T x = y (y = row rhs_row of the factor) by 64-column blocks from the
 // last one: rhs_B = y_B - L[below, B]^T x_below (GEMV), x_B = W_B rhs_B with W_B = L_BB^-T from
 // the panel kernel.  One block; x lives in shared memory.
@@ -565,13 +554,11 @@ __device__ __forceinline__ void grid_barrier(unsigned int* bar, unsigned int tar
 }
 
 // ---- small systems: the whole factorisation in ONE persistent launch ------------------------------
-// The chain of chol_step_kernel launches (one per 64-column panel) spends a third of its time between
-// kernels: launch, drain, the first loads of the next launch (C3, n = 1793: 29 launches, 0.62 ms).
-// chol_fused_kernel runs the same steps -- the same virtual blocks, the same arithmetic in the same
-// order, so the factor is bit-identical -- inside one cooperative launch, with a grid barrier where a
-// launch boundary was.  Panel blocks go to the first CTAs; the update tiles of the previous panel,
-// which nothing in the step waits for, are dealt to the CTAs that hold no panel block, so that the
-// CTAs on the critical path (slice update, elimination) reach the barrier first.
+// All steps run in one cooperative launch, a grid barrier between them, so the latency-bound panel
+// chain pays no launch, drain and first loads per panel.  Panel blocks go to the first CTAs; the
+// update tiles of the previous panel, which nothing in the step waits for, are dealt to the CTAs that
+// hold no panel block, so that the CTAs on the critical path (slice update, elimination) reach the
+// barrier first.
 __global__ void __launch_bounds__(kPanelThreads)
 chol_fused_kernel(double* S, int ld, int n, int n_rows, double* Lt, double* Winv, unsigned int* bar,
                   ba_lm_state* ctl, int use_ctl) {
@@ -694,7 +681,13 @@ chol_backsolve_grid_kernel(const double* __restrict__ S, int ld, int n, int rhs_
 // updates its own chunks; the factor rows and W of the next step are static and fetched before the
 // barrier.  Fixed summation order: deterministic.
 constexpr int kBsCluster = 8;
-constexpr int kBsMaxOwn = 4;  // chunks per CTA: n < 2048 -> at most 32 chunks
+constexpr int kBsMaxOwn = 4;  // chunks per CTA
+// The cluster from n = 1024: against one CTA it measured 8 us slower at 7 blocks (C2), 37 us faster
+// at 29 blocks (C3).
+constexpr int kBsClusterMinN = 1024;
+constexpr int kBsGridMinN = 2048;  // from here the grid-wide kernel
+static_assert((kBsGridMinN - 1 + NB - 1) / NB <= kBsCluster * kBsMaxOwn,
+              "every 64-block of an n < kBsGridMinN system needs a chunk slot in the cluster");
 
 __global__ void __launch_bounds__(256)
 chol_backsolve_cluster_kernel(const double* __restrict__ S, int ld, int n, int rhs_row,
@@ -790,143 +783,114 @@ chol_backsolve_cluster_kernel(const double* __restrict__ S, int ld, int n, int r
   }
 }
 
+// Rows (with the right-hand-side row) from which the factorisation is two-level.
+constexpr int kCholTwoLevelRows = 2048;
+
 int launch_cholesky_solve(ba_engine* e, bool conditional, cudaStream_t s) {
   const int use_ctl = conditional ? 1 : 0;
-  constexpr size_t kPanelSmem = (2 * NB * (NB + 1) + 5 * NB) * sizeof(double);
-  BA_CUDA(cudaFuncSetAttribute(chol_panel_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                               (int)kPanelSmem));
-  constexpr size_t kUpdateSmem = 2 * NB * 65 * sizeof(double);
-  BA_CUDA(cudaFuncSetAttribute(chol_update_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                               (int)kUpdateSmem));
   const int n = e->n_full, n_rows = e->rhs_row + 1, ld = e->n_pad;
-  // Small systems: after every 64-panel the whole trailing matrix is updated (FMA 64-tiles).
-  // Large systems: two-level blocking.  Inside a 256-wide outer block the panels update only the
-  // block's own columns; the rest of the trailing matrix then gets ONE rank-256 update on the
-  // FP64 tensor cores (the SYRK kernel of K3 with a subtracting epilogue), which reads and writes
-  // S a quarter as often and keeps the DMMA pipe fed from a 3-stage cp.async pipeline.
-  static const bool one_level = std::getenv("BA_CHOL_ONE_LEVEL") != nullptr;  // A/B timing only
-  static const bool no_fused = std::getenv("BA_CHOL_NO_FUSED_STEP") != nullptr;  // A/B timing only
-  const int OB = (n_rows >= 2048 && !one_level) ? kCholOB : NB;
-  CholSplit split;
-  comm_chol_split(e, &split);
-  if (std::getenv("BA_CHOL_NO_SPLIT")) split.world = 1;  // A/B timing only (set on every rank)
-  if (OB == NB && !no_fused) {
-    // small systems: one launch per panel, the previous panel's update rides along
+  if (n_rows < kCholTwoLevelRows) {
     constexpr size_t kStepSmem = (2 * NB * (NB + 1) + 5 * NB + 2 * NB * kSLD) * sizeof(double);
-    BA_CUDA(cudaFuncSetAttribute(chol_step_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kStepSmem));
-    static const bool no_persist = std::getenv("BA_CHOL_NO_PERSIST") != nullptr;  // A/B timing: one launch per panel
     // the persistent kernel needs its CTAs co-resident (cooperative launch): ask once how many fit
     static int fused_ctas_per_sm = -1;
     if (fused_ctas_per_sm < 0) {
       BA_CUDA(cudaFuncSetAttribute(chol_fused_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kStepSmem));
       int per_sm = 0;
-      if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, chol_fused_kernel, kPanelThreads, kStepSmem) != cudaSuccess) {
-        cudaGetLastError();
-        per_sm = 0;
-      }
+      BA_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, chol_fused_kernel, kPanelThreads, kStepSmem));
       fused_ctas_per_sm = per_sm;
     }
-    if (!no_persist && fused_ctas_per_sm > 0) {
-      // grid: enough CTAs for the busiest step (panel blocks + the tiles of the previous panel's update)
-      int want = 1;
-      {
-        int panel = 0;
-        for (int k0 = 0; k0 < n; k0 += NB, ++panel) {
-          const int nb = n - k0 < NB ? n - k0 : NB;
-          const int below = n_rows - (k0 + nb);
-          int blocks = 1 + (below + NB - 1) / NB;
-          const int rest = n_rows - (k0 + NB);
-          if (panel > 0 && rest > 0) {
-            const int nt = (rest + NB - 1) / NB;
-            blocks += nt * (nt + 1) / 2;
-          }
-          if (blocks > want) want = blocks;
-        }
-      }
-      const int fit = e->num_sms * fused_ctas_per_sm;
-      const int G = want < fit ? want : fit;
-      BA_CUDA(cudaMemsetAsync(e->chol_bar, 0, sizeof(unsigned int), s));
-      cudaLaunchConfig_t cfg = {};
-      cfg.gridDim = dim3(G);
-      cfg.blockDim = dim3(kPanelThreads);
-      cfg.dynamicSmemBytes = kStepSmem;
-      cfg.stream = s;
-      cudaLaunchAttribute attr[1];
-      attr[0].id = cudaLaunchAttributeCooperative;
-      attr[0].val.cooperative = 1;
-      cfg.attrs = attr;
-      cfg.numAttrs = 1;
-      BA_CUDA(cudaLaunchKernelEx(&cfg, chol_fused_kernel, e->P(), ld, n, n_rows, e->Lt, e->Winv, e->chol_bar, e->ctl,
-                                 use_ctl));
-      BA_LAUNCH_CHECK();
-    } else {
-    int panel = 0;
-    for (int k0 = 0; k0 < n; k0 += NB, ++panel) {
-      const int nb = n - k0 < NB ? n - k0 : NB;
-      const int below = n_rows - (k0 + nb);
-      const int p_blocks = 1 + (below + NB - 1) / NB;
-      int u_blocks = 0;
-      if (panel > 0) {
-        const int rest = n_rows - (k0 + NB);  // rows / columns beyond block column `panel`
-        if (rest > 0) {
+    if (fused_ctas_per_sm == 0) {
+      set_error("chol_fused_kernel does not fit on an SM (%d threads, %zu B of shared memory)", kPanelThreads,
+                kStepSmem);
+      return BA_ERR_CUDA;
+    }
+    // grid: enough CTAs for the busiest step (panel blocks + the tiles of the previous panel's update)
+    int want = 1;
+    {
+      int panel = 0;
+      for (int k0 = 0; k0 < n; k0 += NB, ++panel) {
+        const int nb = n - k0 < NB ? n - k0 : NB;
+        const int below = n_rows - (k0 + nb);
+        int blocks = 1 + (below + NB - 1) / NB;
+        const int rest = n_rows - (k0 + NB);
+        if (panel > 0 && rest > 0) {
           const int nt = (rest + NB - 1) / NB;
-          u_blocks = nt * (nt + 1) / 2;
+          blocks += nt * (nt + 1) / 2;
+        }
+        if (blocks > want) want = blocks;
+      }
+    }
+    const int fit = e->num_sms * fused_ctas_per_sm;
+    const int G = want < fit ? want : fit;
+    BA_CUDA(cudaMemsetAsync(e->chol_bar, 0, sizeof(unsigned int), s));
+    cudaLaunchConfig_t cfg = {};
+    cfg.gridDim = dim3(G);
+    cfg.blockDim = dim3(kPanelThreads);
+    cfg.dynamicSmemBytes = kStepSmem;
+    cfg.stream = s;
+    cudaLaunchAttribute attr[1];
+    attr[0].id = cudaLaunchAttributeCooperative;
+    attr[0].val.cooperative = 1;
+    cfg.attrs = attr;
+    cfg.numAttrs = 1;
+    BA_CUDA(cudaLaunchKernelEx(&cfg, chol_fused_kernel, e->P(), ld, n, n_rows, e->Lt, e->Winv, e->chol_bar, e->ctl,
+                               use_ctl));
+    BA_LAUNCH_CHECK();
+  } else {
+    // Two-level blocking.  Inside a 256-wide outer block the panels update only the block's own
+    // columns; the rest of the trailing matrix then gets ONE rank-256 update on the FP64 tensor cores
+    // (the SYRK kernel of K3 with a subtracting epilogue), which reads and writes S a quarter as often.
+    constexpr int OB = kCholOB;
+    constexpr size_t kPanelSmem = (2 * NB * (NB + 1) + 5 * NB) * sizeof(double);
+    BA_CUDA(cudaFuncSetAttribute(chol_panel_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kPanelSmem));
+    constexpr size_t kUpdateSmem = 2 * NB * 65 * sizeof(double);
+    BA_CUDA(cudaFuncSetAttribute(chol_update_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kUpdateSmem));
+    CholSplit split;
+    comm_chol_split(e, &split);
+    int panel = 0;
+    for (int K0 = 0; K0 < n; K0 += OB) {
+      // columns the panels of this block update themselves
+      const int c_end = K0 + OB < n_rows ? K0 + OB : n_rows;
+      for (int k0 = K0; k0 < K0 + OB && k0 < n; k0 += NB, ++panel) {
+        const int nb = n - k0 < NB ? n - k0 : NB;
+        const int below = n_rows - (k0 + nb);
+        const int pblocks = 1 + (below + NB - 1) / NB;
+        double* Lt = e->Lt + (size_t)(k0 - K0) * ld;  // k-rows of this panel inside the block column
+        chol_panel_kernel<<<pblocks, kPanelThreads, kPanelSmem, s>>>(e->P(), ld, n_rows, k0, nb, Lt,
+                                                                     e->Winv + (size_t)panel * NB * NB, e->ctl, use_ctl);
+        BA_LAUNCH_CHECK();
+        if (below <= 0 || k0 + nb >= c_end) continue;
+        dim3 grid((c_end - (k0 + nb) + 63) / 64, (below + 63) / 64);
+        chol_update_kernel<<<grid, 256, kUpdateSmem, s>>>(e->P(), ld, n_rows, c_end, k0, nb, Lt, e->ctl, use_ctl);
+        BA_LAUNCH_CHECK();
+      }
+      if (K0 + OB < n_rows) {  // all four panels of the block are full here
+        const int t0 = K0 + OB, remaining = n_rows - t0;
+        if (split.world > 1 && remaining >= kCholSplitMinRows) {
+          // sharded run: every rank updates its own tile rows and sends the part the next panels
+          // read -- the next block column, or everything that is left when the following update
+          // will not be divided any more -- to all ranks; one flag exchange closes the step
+          const bool next_divided = t0 + OB < n_rows && n_rows - (t0 + OB) >= kCholSplitMinRows;
+          split.push_cols = next_divided ? OB : (remaining + 127) / 128 * 128;
+          // Before the FIRST divided update nothing has ordered the ranks since the sum of `red`:
+          // a rank that is ahead would store into a peer's matrix while that peer is still
+          // assembling it in place.  One more flag exchange closes the window (the later steps are
+          // ordered by the exchange that ends the step before).
+          if (K0 == 0) BA_TRY(launch_comm_chol_sync(e, conditional, s));
+          BA_TRY(launch_chol_wide_update(e->P(), ld, n_rows, t0, e->Lt, OB, e->ctl, s, &split));
+          BA_TRY(launch_comm_chol_sync(e, conditional, s));
+        } else {
+          BA_TRY(launch_chol_wide_update(e->P(), ld, n_rows, t0, e->Lt, OB, e->ctl, s, nullptr));
         }
       }
-      double* Lt_cur = e->Lt + (size_t)(panel & 1) * NB * ld;
-      const double* Lt_prev = panel > 0 ? e->Lt + (size_t)((panel - 1) & 1) * NB * ld : nullptr;
-      chol_step_kernel<<<p_blocks + u_blocks, kPanelThreads, kStepSmem, s>>>(
-          e->P(), ld, n_rows, k0, nb, p_blocks, Lt_cur, Lt_prev, e->Winv + (size_t)panel * NB * NB, e->ctl, use_ctl);
-      BA_LAUNCH_CHECK();
-    }
-    }
-  } else {
-  int panel = 0;
-  for (int K0 = 0; K0 < n; K0 += OB) {
-    // columns the panels of this block update themselves
-    const int c_end = (OB == NB || K0 + OB > n_rows) ? n_rows : K0 + OB;
-    for (int k0 = K0; k0 < K0 + OB && k0 < n; k0 += NB, ++panel) {
-      const int nb = n - k0 < NB ? n - k0 : NB;
-      const int below = n_rows - (k0 + nb);
-      const int pblocks = 1 + (below + NB - 1) / NB;
-      double* Lt = e->Lt + (size_t)(k0 - K0) * ld;  // k-rows of this panel inside the block column
-      chol_panel_kernel<<<pblocks, kPanelThreads, kPanelSmem, s>>>(e->P(), ld, n_rows, k0, nb, Lt,
-                                                e->Winv + (size_t)panel * NB * NB, e->ctl, use_ctl);
-      BA_LAUNCH_CHECK();
-      if (below <= 0 || k0 + nb >= c_end) continue;
-      dim3 grid((c_end - (k0 + nb) + 63) / 64, (below + 63) / 64);
-      chol_update_kernel<<<grid, 256, kUpdateSmem, s>>>(e->P(), ld, n_rows, c_end, k0, nb, Lt, e->ctl, use_ctl);
-      BA_LAUNCH_CHECK();
-    }
-    if (OB > NB && K0 + OB < n_rows) {  // all four panels of the block are full here
-      const int t0 = K0 + OB, remaining = n_rows - t0;
-      if (split.world > 1 && remaining >= kCholSplitMinRows) {
-        // sharded run: every rank updates its own tile rows and sends the part the next panels
-        // read -- the next block column, or everything that is left when the following update
-        // will not be divided any more -- to all ranks; one flag exchange closes the step
-        const bool next_divided = t0 + OB < n_rows && n_rows - (t0 + OB) >= kCholSplitMinRows;
-        split.push_cols = next_divided ? OB : (remaining + 127) / 128 * 128;
-        // Before the FIRST divided update nothing has ordered the ranks since the sum of `red`:
-        // a rank that is ahead would store into a peer's matrix while that peer is still
-        // assembling it in place.  One more flag exchange closes the window (the later steps are
-        // ordered by the exchange that ends the step before).
-        if (K0 == 0) BA_TRY(launch_comm_chol_sync(e, conditional, s));
-        BA_TRY(launch_chol_wide_update(e->P(), ld, n_rows, t0, e->Lt, OB, e->ctl, s, &split));
-        BA_TRY(launch_comm_chol_sync(e, conditional, s));
-      } else {
-        BA_TRY(launch_chol_wide_update(e->P(), ld, n_rows, t0, e->Lt, OB, e->ctl, s, nullptr));
-      }
     }
   }
-  }
-  static const int grid_min = std::getenv("BA_CHOL_BACKSOLVE_GRID_MIN") ? std::atoi(std::getenv("BA_CHOL_BACKSOLVE_GRID_MIN")) : 2048;
-  if (n >= grid_min && !std::getenv("BA_CHOL_BACKSOLVE_1CTA")) {
+  if (n >= kBsGridMinN) {
     const int nblk = (n + NB - 1) / NB;
     const int G = nblk < e->num_sms ? nblk : e->num_sms;
     BA_CUDA(cudaMemsetAsync(e->chol_bar, 0, sizeof(unsigned int), s));
     // cooperative launch: the driver admits the grid only if all G CTAs can be resident together,
-    // whatever else the device is running (BA_CHOL_NO_COOP: plain launch, for A/B runs)
-    static const bool no_coop = std::getenv("BA_CHOL_NO_COOP") != nullptr;
+    // whatever else the device is running
     cudaLaunchConfig_t cfg = {};
     cfg.gridDim = dim3(G);
     cfg.blockDim = dim3(256);
@@ -936,14 +900,13 @@ int launch_cholesky_solve(ba_engine* e, bool conditional, cudaStream_t s) {
     attr[0].id = cudaLaunchAttributeCooperative;
     attr[0].val.cooperative = 1;
     cfg.attrs = attr;
-    cfg.numAttrs = no_coop ? 0 : 1;
+    cfg.numAttrs = 1;
     BA_CUDA(cudaLaunchKernelEx(&cfg, chol_backsolve_grid_kernel, (const double*)e->P(), ld, n, e->rhs_row,
                                (const double*)e->Winv, e->ywork, e->dxi, e->chol_bar, e->ctl, use_ctl));
     BA_LAUNCH_CHECK();
     return BA_OK;
   }
-  static const int cluster_min = std::getenv("BA_CHOL_BACKSOLVE_CLUSTER_MIN") ? std::atoi(std::getenv("BA_CHOL_BACKSOLVE_CLUSTER_MIN")) : 1024;  // measured: 7 blocks (C2) 8 us slower, 29 blocks (C3) 37 us faster than one CTA
-  if (n >= cluster_min && (n + NB - 1) / NB <= kBsCluster * kBsMaxOwn && !std::getenv("BA_CHOL_BACKSOLVE_1CTA")) {
+  if (n >= kBsClusterMinN) {
     cudaLaunchConfig_t cfg = {};
     cfg.gridDim = dim3(kBsCluster);
     cfg.blockDim = dim3(256);
@@ -961,11 +924,7 @@ int launch_cholesky_solve(ba_engine* e, bool conditional, cudaStream_t s) {
     BA_LAUNCH_CHECK();
     return BA_OK;
   }
-  const size_t smem = ((size_t)n + 16 * 64 + 64) * sizeof(double);
-  if (smem > 220 * 1024) {
-    set_error("reduced system too large for the single-block back substitution (n=%d)", n);
-    return BA_ERR_INVALID;
-  }
+  const size_t smem = ((size_t)n + 16 * 64 + 64) * sizeof(double);  // n < 1024: at most 17 KB
   BA_CUDA(cudaFuncSetAttribute(chol_backsolve_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                (int)smem));
   chol_backsolve_kernel<<<1, 1024, smem, s>>>(e->P(), ld, n, e->rhs_row, e->Winv, e->dxi, e->ctl,

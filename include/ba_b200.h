@@ -251,7 +251,7 @@ int ba_fp64_peak(int device, int use_dmma, double* tflops);
 /* 1 when this engine linearises matrix-free: a dense scene whose camera table fits shared memory
  * (<= 361 cameras) re-derives the Jacobian rows in K2a, the camera blocks, K2b and the point update
  * instead of storing them in K1 and reading them back (reference :309-427 evaluated where used);
- * 0 otherwise (sparse visibility, more cameras, or BA_NO_MATRIX_FREE=1).  ba_buffer_read of the
+ * 0 otherwise (sparse visibility or more cameras).  ba_buffer_read of the
  * JP / JC rows still works: K1 writes them for that read. */
 int ba_matrix_free(ba_engine* e);
 /* Host-only (no device): plan the dense Schur product (K3) of an n_cams x n_points scene for a GPU

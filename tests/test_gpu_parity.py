@@ -108,7 +108,7 @@ def _check_one_linearisation(ba, obs, X, R, t, f, u, f0, axis, dense, c=1e-4):
     E_trial = float(eng.cost_values()[1])
     assert E_trial == pytest.approx(O.cost(obs, rX, rf, ru, rR, rt, f0), rel=1e-8)
     eng.close()
-    return E_trial
+    return E_trial, red
 
 
 @pytest.mark.parametrize("name", SMALL_CASES)
@@ -118,31 +118,54 @@ def test_kernels_match_oracle_on_golden_cases(ba, name):
     obs = O.ObsList.from_dense(x, vis)
     X, R, t = O.normalize_gauge(X0, R0, t0, axis)
     f, u = K0[:, 0, 0].copy(), K0[:, :2, 2].copy()
-    E_trial = _check_one_linearisation(ba, obs, X, R, t, f, u, f0, axis, dense=vis is None)
+    E_trial, _ = _check_one_linearisation(ba, obs, X, R, t, f, u, f0, axis, dense=vis is None)
     # and against the reference's own first trial cost
     assert E_trial == pytest.approx(float(g["lin_E_trial"]), rel=1e-8)
 
 
-@pytest.mark.parametrize("n_cams,n_points,visibility,axis", [
-    (30, 1500, 1.0, "x-up_z-forward"),      # dense, 64-wide SYRK tiles, several k splits
-    (120, 900, 1.0, "x-right_z-forward"),   # dense, 128-wide SYRK tiles, multi-panel Cholesky
-    (40, 2000, 0.3, "x-up_z-forward"),      # sparse path
-    (17, 333, 1.0, "x-up_z-forward"),       # ragged sizes (nothing a multiple of anything)
-    (70, 3000, 0.9, "x-up_z-forward"),      # sparse path, nearly full bitmaps: multi-pass hit queue, 3 x 3 pair tiles
-    (33, 200, 0.5, "x-right_z-forward"),    # sparse path, one camera beyond a pair tile, single bitmap batch
-    (5, 9000, 0.7, "x-up_z-forward"),       # sparse path, few cameras, several bitmap batches per pair
-    (320, 450, 0.3, "x-up_z-forward"),      # n = 2880: two-level Cholesky (rank-256 DMMA updates, 128- and 64-tiles), grid-wide back substitution
-    (260, 300, 1.0, "x-right_z-forward"),   # n = 2340, dense: same with 64-tiles only, edge tiles cut by n_rows
-    (1000, 1500, 0.1, "x-up_z-forward"),    # C4's camera count: n = 8993, 35 outer blocks of the two-level Cholesky,
-                                            # 141-CTA back substitution, 31 x 31 pair tiles (oracle: ~25 s of LU)
-])
-def test_kernels_match_oracle_on_random_scenes(ba, n_cams, n_points, visibility, axis):
+def _check_random_scene(ba, n_cams, n_points, visibility, axis):
     sc = ba.scenes.make_scene(n_cams, n_points, seed=n_cams, visibility=visibility, axis=axis)
     obs = O.ObsList(sc.n_points, sc.n_cams, np.repeat(np.arange(sc.n_points), np.diff(sc.obs_ptr)),
                     sc.obs_cam.astype(np.int64), sc.obs_xy, sc.obs_ptr)
     X, R, t = O.normalize_gauge(sc.X0, sc.R0, sc.t0, axis)
     f, u = sc.K0[:, 0, 0].copy(), sc.K0[:, :2, 2].copy()
-    _check_one_linearisation(ba, obs, X, R, t, f, u, sc.f0, axis, dense=sc.dense)
+    return _check_one_linearisation(ba, obs, X, R, t, f, u, sc.f0, axis, dense=sc.dense)
+
+
+# Sparse scenes run twice: with the static pair lists (schur_pairs_reg_kernel) and with
+# BA_PAIRS_NO_LIST (schur_pairs_kernel scans the bitmaps: the path of scenes whose lists do not fit).
+@pytest.mark.parametrize("n_cams,n_points,visibility,axis,lists", [
+    (30, 1500, 1.0, "x-up_z-forward", True),      # dense, 64-wide SYRK tiles, several k splits
+    (120, 900, 1.0, "x-right_z-forward", True),   # dense, 128-wide SYRK tiles, multi-panel Cholesky
+    (40, 2000, 0.3, "x-up_z-forward", True),      # sparse path
+    (40, 2000, 0.3, "x-up_z-forward", False),
+    (17, 333, 1.0, "x-up_z-forward", True),       # ragged sizes (nothing a multiple of anything)
+    (70, 3000, 0.9, "x-up_z-forward", True),      # sparse path, nearly full bitmaps, 3 x 3 pair tiles
+    (70, 3000, 0.9, "x-up_z-forward", False),     # bitmap scan: multi-pass hit queue
+    (33, 200, 0.5, "x-right_z-forward", True),    # sparse path, one camera beyond a pair tile
+    (33, 200, 0.5, "x-right_z-forward", False),   # bitmap scan: single bitmap batch
+    (5, 9000, 0.7, "x-up_z-forward", True),       # sparse path, few cameras, long pair lists
+    (5, 9000, 0.7, "x-up_z-forward", False),      # bitmap scan: several bitmap batches per pair
+    (320, 450, 0.3, "x-up_z-forward", True),      # n = 2880: two-level Cholesky (rank-256 DMMA updates, 128- and 64-tiles), grid-wide back substitution
+    (320, 450, 0.3, "x-up_z-forward", False),
+    (260, 300, 1.0, "x-right_z-forward", True),   # n = 2340, dense: same with 64-tiles only, edge tiles cut by n_rows
+    (1000, 1500, 0.1, "x-up_z-forward", True),    # C4's camera count: n = 8993, 35 outer blocks of the two-level Cholesky,
+                                                  # 141-CTA back substitution, 31 x 31 pair tiles (oracle: ~25 s of LU)
+])
+def test_kernels_match_oracle_on_random_scenes(ba, monkeypatch, n_cams, n_points, visibility, axis, lists):
+    if not lists:
+        monkeypatch.setenv("BA_PAIRS_NO_LIST", "1")
+    _check_random_scene(ba, n_cams, n_points, visibility, axis)
+
+
+def test_bitmap_scan_pair_kernel_is_the_one_that_ran(ba, monkeypatch):
+    """BA_PAIRS_NO_LIST really switches the pair kernel: the list kernel sums on per-lane FMA chains, the
+    bitmap scan on DMMA fragments, so the two reduced systems differ in the last bits somewhere, and
+    both match the oracle."""
+    _, red_lists = _check_random_scene(ba, 70, 3000, 0.9, "x-up_z-forward")
+    monkeypatch.setenv("BA_PAIRS_NO_LIST", "1")
+    _, red_scan = _check_random_scene(ba, 70, 3000, 0.9, "x-up_z-forward")
+    assert not np.array_equal(red_lists, red_scan)
 
 
 @pytest.mark.parametrize("n_cams,n_points,axis", [(30, 1500, "x-up_z-forward"), (120, 900, "x-right_z-forward"),

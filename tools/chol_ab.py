@@ -1,6 +1,7 @@
 """A/B of the small-system Cholesky: prints a hash of dxi and per-phase times for one scene.
+Run it from two builds of the library and compare the hashes and the times.
 
-    [BA_CHOL_NO_PERSIST=1] python tools/chol_ab.py --cams 50 --points 10000
+    python tools/chol_ab.py --cams 50 --points 10000
 """
 import argparse
 import hashlib
