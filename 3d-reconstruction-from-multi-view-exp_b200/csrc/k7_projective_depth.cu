@@ -193,10 +193,12 @@ subspace_eig_kernel(int n, const double* __restrict__ G, double* __restrict__ U4
 // Parallel cyclic Jacobi in one CTA.  The n indices (padded to an even count with a dummy) are
 // paired round-robin, n/2 disjoint rotations per step, n - 1 steps per sweep: each step computes
 // the rotation angles, rotates the columns of G and V, then the rows of G.  Fixed order, fixed
-// stopping rule: bit-reproducible.  G and V live in global memory (L1/L2 resident: n <= 192).
+// stopping rule: bit-reproducible.  The rotations work on G, a copy of Gin (which the callers still
+// need), made after the early return: a converged subspace iteration costs no copy.  G and V live in
+// global memory (L1/L2 resident: n <= 192).
 __global__ void __launch_bounds__(256)
-jacobi_eig_kernel(int n, double* __restrict__ G, double* __restrict__ V, double* __restrict__ U4,
-                  double* __restrict__ evals4, const int* __restrict__ status) {
+jacobi_eig_kernel(int n, const double* __restrict__ Gin, double* __restrict__ G, double* __restrict__ V,
+                  double* __restrict__ U4, double* __restrict__ evals4, const int* __restrict__ status) {
   if (status && status[0] == 1) return;  // the subspace iteration already delivered U4
   extern __shared__ double jsm[];
   const int ne = n + (n & 1), h = ne / 2;
@@ -206,7 +208,10 @@ jacobi_eig_kernel(int n, double* __restrict__ G, double* __restrict__ V, double*
   __shared__ double scratch[32];
   __shared__ int s_done;
   const int tid = threadIdx.x, nt = blockDim.x;
-  for (int k = tid; k < n * n; k += nt) V[k] = (k / n == k % n) ? 1.0 : 0.0;
+  for (int k = tid; k < n * n; k += nt) {
+    G[k] = Gin[k];
+    V[k] = (k / n == k % n) ? 1.0 : 0.0;
+  }
   for (int k = tid; k < ne; k += nt) pl[k] = k;
   __syncthreads();
   for (int sweep = 0; sweep < 40; ++sweep) {
@@ -910,109 +915,206 @@ struct DevBufs {
     return BA_OK;
   }
   ~DevBufs() {
+    if (ptrs.empty()) return;  // the call was rejected before it touched the device
     for (void* p : ptrs) cudaFreeAsync(p, s);
     cudaStreamSynchronize(s);
   }
 };
 
-static int leading_subspace(int n, int ld, int64_t k_pad, const GramWorkspace* ws, const double* Wk, double* P,
-                            double* G, double* V, double* U4, double* ev, int* status, bool warm, cudaStream_t s) {
-  static const bool force_jacobi = std::getenv("BA_DEPTH_JACOBI") != nullptr;
-  BA_TRY(gram_launch(ws, Wk, P, s));
-  gram_symmetrize_kernel<<<(n * n + 255) / 256, 256, 0, s>>>(n, ld, P, G);
-  if (!force_jacobi)
-    subspace_eig_kernel<<<1, 256, (size_t)8 * n * sizeof(double), s>>>(n, G, U4, warm ? 1 : 0, 2000, status);
-  const size_t jac_smem = (size_t)(2 * ((n + 1) / 2)) * sizeof(double) + (size_t)2 * (n + 1) * sizeof(int) + 16;
-  // the Jacobi fallback rotates its matrix in place and G is still needed afterwards: it works on
-  // a copy (V is the eigenvector store, the copy lives behind it)
-  BA_CUDA(cudaMemcpyAsync(V + (size_t)n * n, G, (size_t)n * n * sizeof(double), cudaMemcpyDeviceToDevice, s));
-  jacobi_eig_kernel<<<1, 256, jac_smem, s>>>(n, V + (size_t)n * n, V, U4, ev, force_jacobi ? nullptr : status);
-  g_launch_count += 3;
-  (void)k_pad;
-  return BA_OK;
+static int check_launches(const char* what) {
+  if (cudaGetLastError() == cudaSuccess) return BA_OK;
+  set_error("%s: a kernel launch failed", what);
+  return BA_ERR_CUDA;
+}
+
+// What the two depth methods and the factorisation share: the device, the k-major operand Wk
+// [k_pad][ld] (one row per point, n entries used), its Gram matrix and leading eigenspace, the input
+// (x or W) staged on the device and the output (z or S).  Every buffer is in `bufs` and the Gram
+// workspace is released by the destructor, so every exit path frees everything.
+struct DepthCall {
+  cudaStream_t s;
+  DevBufs bufs;
+  GramWorkspace ws;
+  int num_sms = 0, n = 0, ld = 0, grid = 0, mem = BA_MEM_HOST;
+  int64_t N = 0, k_pad = 0;
+  bool force_jacobi = false;
+  const double* in = nullptr;
+  double *out = nullptr, *out_user = nullptr;
+  size_t out_count = 0;
+  double *Wk = nullptr, *P = nullptr, *G = nullptr, *V = nullptr, *U4 = nullptr, *ev = nullptr;
+  int* status = nullptr;
+
+  explicit DepthCall(void* stream) : s((cudaStream_t)stream), bufs(s) {}
+  ~DepthCall() { gram_release(&ws, s); }
+
+  // `args_ok` and `usage`: the entry point's own argument rule and its message.  Wk gets N_ rows (points,
+  // or columns of W) of n_ entries; in / out hold in_count / out_count doubles, on the device with
+  // BA_MEM_DEVICE.
+  int open(bool args_ok, const char* what, const char* usage, int device, int64_t N_, int n_,
+           const double* in_, size_t in_count, double* out_, size_t out_count_, int mem_) {
+    int ndev = 0;
+    if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0) {
+      set_error("no CUDA device: %s has no CPU path", what);
+      return BA_ERR_NO_DEVICE;
+    }
+    if (!args_ok || device < 0 || device >= ndev) {
+      set_error("%s", usage);
+      return BA_ERR_INVALID;
+    }
+    BA_CUDA(cudaSetDevice(device));
+    BA_CUDA(cudaDeviceGetAttribute(&num_sms, cudaDevAttrMultiProcessorCount, device));
+    N = N_;
+    n = n_;
+    ld = (n + 7) / 8 * 8;
+    k_pad = (N + 31) / 32 * 32;
+    grid = balanced_blocks((N + 7) / 8, (int64_t)num_sms * 8);
+    force_jacobi = std::getenv("BA_DEPTH_JACOBI") != nullptr;  // tests: the fallback path
+    mem = mem_;
+    out_user = out_;
+    out_count = out_count_;
+    BA_TRY(bufs.alloc(&Wk, (size_t)k_pad * ld));
+    BA_TRY(bufs.alloc(&P, (size_t)ld * ld));
+    BA_TRY(bufs.alloc(&G, (size_t)n * n));
+    BA_TRY(bufs.alloc(&V, (size_t)2 * n * n));
+    BA_TRY(bufs.alloc(&U4, (size_t)4 * n));
+    BA_TRY(bufs.alloc(&ev, 4));
+    BA_TRY(bufs.alloc(&status, 1));
+    if (mem == BA_MEM_DEVICE) {
+      in = in_;
+      out = out_;
+    } else {
+      double* din = nullptr;
+      BA_TRY(bufs.alloc(&din, in_count));
+      BA_TRY(bufs.alloc(&out, out_count));
+      BA_CUDA(cudaMemcpyAsync(din, in_, in_count * sizeof(double), cudaMemcpyHostToDevice, s));
+      in = din;
+    }
+    BA_CUDA(cudaMemsetAsync(Wk, 0, (size_t)k_pad * ld * sizeof(double), s));
+    BA_CUDA(cudaMemsetAsync(P, 0, (size_t)ld * ld * sizeof(double), s));
+    BA_CUDA(cudaMemsetAsync(status, 0, sizeof(int), s));
+    return gram_prepare(&ws, ld, k_pad, num_sms, s);
+  }
+
+  // U4 = a basis of the leading four-dimensional eigenspace of G = Wk^T Wk, which stays intact: the
+  // subspace iteration (warm-started from U4), then the Jacobi solver if that did not converge.
+  int leading_subspace(bool warm) {
+    BA_TRY(gram_launch(&ws, Wk, P, s));
+    gram_symmetrize_kernel<<<(n * n + 255) / 256, 256, 0, s>>>(n, ld, P, G);
+    if (!force_jacobi)
+      subspace_eig_kernel<<<1, 256, (size_t)8 * n * sizeof(double), s>>>(n, G, U4, warm ? 1 : 0, 2000, status);
+    const size_t jac_smem = (size_t)(2 * ((n + 1) / 2)) * sizeof(double) + (size_t)2 * (n + 1) * sizeof(int) + 16;
+    // V [2][n][n]: the eigenvectors, then the Jacobi solver's copy of G
+    jacobi_eig_kernel<<<1, 256, jac_smem, s>>>(n, G, V + (size_t)n * n, V, U4, ev, force_jacobi ? nullptr : status);
+    g_launch_count += 3;
+    return BA_OK;
+  }
+
+  // with BA_MEM_HOST: the result to the caller's buffer (with BA_MEM_DEVICE the kernels wrote it there)
+  cudaError_t copy_out() const {
+    if (mem == BA_MEM_DEVICE) return cudaSuccess;
+    return cudaMemcpyAsync(out_user, out, out_count * sizeof(double), cudaMemcpyDeviceToHost, s);
+  }
+};
+
+// The pass loop of both depth methods.  z starts at 1 (:80, :160); pass(it) enqueues one pass, which
+// updates z and leaves its reprojection error in dE; the host reads E and stops when E < tolerance or
+// after max_iter passes (:138-142, :228-229).
+template <class Pass>
+static int run_passes(DepthCall& c, const char* what, const double* dE, double tolerance, int max_iter,
+                      double* errors, int* n_iter, Pass pass) {
+  {
+    std::vector<double> ones(c.out_count, 1.0);
+    BA_CUDA(cudaMemcpyAsync(c.out, ones.data(), ones.size() * sizeof(double), cudaMemcpyHostToDevice, c.s));
+    BA_CUDA(cudaStreamSynchronize(c.s));
+  }
+  int st = BA_OK, it = 0;
+  for (;;) {
+    st = pass(it);
+    if (st == BA_OK) st = check_launches(what);
+    if (st != BA_OK) break;
+    double E = 0.0;
+    if (cudaMemcpyAsync(&E, dE, sizeof(double), cudaMemcpyDeviceToHost, c.s) != cudaSuccess ||
+        cudaStreamSynchronize(c.s) != cudaSuccess) {
+      set_error("%s: %s", what, cudaGetErrorString(cudaGetLastError()));
+      st = BA_ERR_CUDA;
+      break;
+    }
+    if (errors) errors[it] = E;
+    ++it;
+    if (E < tolerance || it >= max_iter) break;
+  }
+  *n_iter = it;
+  if (st == BA_OK && c.copy_out() != cudaSuccess) st = BA_ERR_CUDA;
+  return st;
 }
 
 }  // namespace ba
 
 using namespace ba;
 
+extern "C" int ba_projective_depth_primary(int device, int64_t n_points, int32_t n_images, const double* x,
+                                           double f0, double tolerance, int max_iter, double* z,
+                                           double* errors, int* n_iter, int mem, void* stream) {
+  DepthCall c(stream);
+  BA_TRY(c.open(x && z && n_iter && n_points >= 4 && n_images >= 2 && n_images <= 64 && max_iter >= 1,
+                "the projective-depth iteration",
+                "projective depth: need >= 4 points, 2..64 images, max_iter >= 1 and valid pointers", device,
+                n_points, 3 * n_images, x, (size_t)n_points * n_images * 3, z, (size_t)n_points * n_images, mem));
+  const int64_t N = n_points;
+  const int M = n_images, grid = c.grid;
+  cudaStream_t s = c.s;
+  const double* dx = c.in;
+  double* dz = c.out;
+  double *part = nullptr, *dE = nullptr;
+  BA_TRY(c.bufs.alloc(&part, (size_t)grid));
+  BA_TRY(c.bufs.alloc(&dE, 1));
+  auto pass = [&](int it) -> int {
+    depth_scale_kernel<<<grid, 256, 0, s>>>(N, M, c.ld, dx, dz, c.Wk);
+    BA_TRY(c.leading_subspace(it > 0));
+    depth_update_kernel<<<grid, 256, (size_t)12 * M * sizeof(double), s>>>(N, M, c.ld, dx, c.Wk, c.U4, dz, part);
+    depth_error_kernel<<<1, 256, 0, s>>>(part, grid, (double)N * (double)M, f0, dE);
+    g_launch_count += 3;
+    return BA_OK;
+  };
+  return run_passes(c, "projective depth", dE, tolerance, max_iter, errors, n_iter, pass);
+}
+
 static double* const* g_dual_probe = nullptr;
 
 extern "C" int ba_projective_depth_dual(int device, int64_t n_points, int32_t n_images, const double* x, double f0,
                                         double tolerance, int max_iter, double* z, double* errors, int* n_iter,
                                         int mem, void* stream) {
-  int ndev = 0;
-  if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0) {
-    set_error("no CUDA device: the projective-depth iteration has no CPU path");
-    return BA_ERR_NO_DEVICE;
-  }
-  if (!x || !z || !n_iter || n_points < 4 || n_images < 2 || n_images > 32 * kMaxImageSlots || device < 0 ||
-      device >= ndev) {
-    set_error("projective depth (dual): need >= 4 points, 2..64 images and valid pointers");
-    return BA_ERR_INVALID;
-  }
+  DepthCall c(stream);
+  BA_TRY(c.open(x && z && n_iter && n_points >= 4 && n_images >= 2 && n_images <= 32 * kMaxImageSlots,
+                "the projective-depth iteration",
+                "projective depth (dual): need >= 4 points, 2..64 images and valid pointers", device, n_points,
+                3 * n_images, x, (size_t)n_points * n_images * 3, z, (size_t)n_points * n_images, mem));
   if (max_iter < 1) max_iter = 1;  // the reference runs at least one pass (:162-231)
-  cudaStream_t s = (cudaStream_t)stream;
-  BA_CUDA(cudaSetDevice(device));
-  int num_sms = 148;
-  BA_CUDA(cudaDeviceGetAttribute(&num_sms, cudaDevAttrMultiProcessorCount, device));
   const int64_t N = n_points;
-  const int M = n_images, n = 3 * M;
-  const int ld = (n + 7) / 8 * 8;
-  const int64_t k_pad = (N + 31) / 32 * 32;
-  const size_t d = sizeof(double);
-  const int grid = balanced_blocks((N + 7) / 8, (int64_t)num_sms * 8);
+  const int M = n_images, n = c.n, grid = c.grid;
   const int64_t nwarps = (int64_t)grid * 8;
-  DevBufs bufs(s);
-  double *dx = nullptr, *dz = nullptr, *Wn = nullptr, *P = nullptr, *G = nullptr, *V = nullptr, *U4 = nullptr,
-         *ev = nullptr, *part = nullptr, *sums = nullptr, *small = nullptr, *V4 = nullptr, *R60 = nullptr,
-         *W12 = nullptr, *ebuf = nullptr, *errp = nullptr, *dE = nullptr;
-  int* status = nullptr;
-  BA_TRY(bufs.alloc(&Wn, (size_t)k_pad * ld));
-  BA_TRY(bufs.alloc(&P, (size_t)ld * ld));
-  BA_TRY(bufs.alloc(&G, (size_t)n * n));
-  BA_TRY(bufs.alloc(&V, (size_t)2 * n * n));
-  BA_TRY(bufs.alloc(&U4, (size_t)4 * n));
-  BA_TRY(bufs.alloc(&ev, 4));
-  BA_TRY(bufs.alloc(&part, (size_t)nwarps * M * 60));
-  BA_TRY(bufs.alloc(&sums, (size_t)2 * M));
-  BA_TRY(bufs.alloc(&small, 32));
-  BA_TRY(bufs.alloc(&V4, (size_t)4 * N));
-  BA_TRY(bufs.alloc(&R60, (size_t)60 * M));
-  BA_TRY(bufs.alloc(&W12, (size_t)12 * M));
-  BA_TRY(bufs.alloc(&ebuf, (size_t)N * M));
-  BA_TRY(bufs.alloc(&errp, (size_t)grid));
-  BA_TRY(bufs.alloc(&dE, 1));
-  BA_TRY(bufs.alloc(&status, 1));
-  if (mem == BA_MEM_DEVICE) {
-    dx = const_cast<double*>(x);
-    dz = z;
-  } else {
-    BA_TRY(bufs.alloc(&dx, (size_t)N * M * 3));
-    BA_TRY(bufs.alloc(&dz, (size_t)N * M));
-    BA_CUDA(cudaMemcpyAsync(dx, x, (size_t)N * M * 3 * d, cudaMemcpyHostToDevice, s));
-  }
-  BA_CUDA(cudaMemsetAsync(Wn, 0, (size_t)k_pad * ld * d, s));
-  BA_CUDA(cudaMemsetAsync(P, 0, (size_t)ld * ld * d, s));
-  BA_CUDA(cudaMemsetAsync(status, 0, sizeof(int), s));
-  {
-    std::vector<double> ones((size_t)N * M, 1.0);  // :160  z = 1
-    BA_CUDA(cudaMemcpyAsync(dz, ones.data(), ones.size() * d, cudaMemcpyHostToDevice, s));
-    BA_CUDA(cudaStreamSynchronize(s));
-  }
-  GramWorkspace ws;
-  int st = gram_prepare(&ws, ld, k_pad, num_sms, s);
-  int it = 0;
-  double E = 0.0;
-  while (st == BA_OK) {
+  const size_t d = sizeof(double);
+  cudaStream_t s = c.s;
+  double *part = nullptr, *sums = nullptr, *small = nullptr, *V4 = nullptr, *R60 = nullptr, *W12 = nullptr,
+         *ebuf = nullptr, *errp = nullptr, *dE = nullptr;
+  BA_TRY(c.bufs.alloc(&part, (size_t)nwarps * M * 60));
+  BA_TRY(c.bufs.alloc(&sums, (size_t)2 * M));
+  BA_TRY(c.bufs.alloc(&small, 32));
+  BA_TRY(c.bufs.alloc(&V4, (size_t)4 * N));
+  BA_TRY(c.bufs.alloc(&R60, (size_t)60 * M));
+  BA_TRY(c.bufs.alloc(&W12, (size_t)12 * M));
+  BA_TRY(c.bufs.alloc(&ebuf, (size_t)N * M));
+  BA_TRY(c.bufs.alloc(&errp, (size_t)grid));
+  BA_TRY(c.bufs.alloc(&dE, 1));
+  const double* dx = c.in;
+  double* dz = c.out;
+  auto pass = [&](int it) -> int {
     dual_norm_kernel<<<grid, 256, 0, s>>>(N, M, dx, dz, part);
     colsum_finish_kernel<<<(M + 63) / 64, 64, 0, s>>>(part, nwarps, M, sums);
-    dual_scale_kernel<<<grid, 256, 0, s>>>(N, M, ld, dx, dz, sums, Wn);
-    // the Jacobi fallback needs its own copy of G (see leading_subspace)
-    st = leading_subspace(n, ld, k_pad, &ws, Wn, P, G, V, U4, ev, status, it > 0, s);
-    if (st != BA_OK) break;
-    dual_small_kernel<<<1, 256, (size_t)4 * n * d, s>>>(n, G, U4, small, 0);
-    dual_v_kernel<<<grid, 256, (size_t)12 * M * d, s>>>(N, M, ld, dx, Wn, U4, small, V4, errp);
+    dual_scale_kernel<<<grid, 256, 0, s>>>(N, M, c.ld, dx, dz, sums, c.Wk);
+    BA_TRY(c.leading_subspace(it > 0));
+    dual_small_kernel<<<1, 256, (size_t)4 * n * d, s>>>(n, c.G, c.U4, small, 0);
+    dual_v_kernel<<<grid, 256, (size_t)12 * M * d, s>>>(N, M, c.ld, dx, c.Wk, c.U4, small, V4, errp);
     depth_error_kernel<<<1, 256, 0, s>>>(errp, grid, (double)N * (double)M, f0, dE);
     dual_outer_kernel<<<grid, 256, 0, s>>>(N, M, dx, V4, part);
     colsum_finish_kernel<<<(60 * M + 127) / 128, 128, 0, s>>>(part, nwarps, 60 * M, R60);
@@ -1021,36 +1123,19 @@ extern "C" int ba_projective_depth_dual(int device, int64_t n_points, int32_t n_
     colsum_finish_kernel<<<(2 * M + 63) / 64, 64, 0, s>>>(part, nwarps, 2 * M, sums);
     dual_z_kernel<<<grid, 256, 0, s>>>(N, M, dx, ebuf, sums, dz);
     g_launch_count += 12;
-    if (cudaGetLastError() != cudaSuccess) {
-      set_error("projective depth (dual): a kernel launch failed");
-      st = BA_ERR_CUDA;
-      break;
-    }
-    if (cudaMemcpyAsync(&E, dE, d, cudaMemcpyDeviceToHost, s) != cudaSuccess ||
-        cudaStreamSynchronize(s) != cudaSuccess) {
-      set_error("projective depth (dual): %s", cudaGetErrorString(cudaGetLastError()));
-      st = BA_ERR_CUDA;
-      break;
-    }
-    if (errors) errors[it] = E;
-    ++it;
-    if (E < tolerance || it >= max_iter) break;  // :228-229
-  }
-  *n_iter = it;
-  if (st == BA_OK && mem != BA_MEM_DEVICE &&
-      cudaMemcpyAsync(z, dz, (size_t)N * M * d, cudaMemcpyDeviceToHost, s) != cudaSuccess)
-    st = BA_ERR_CUDA;
+    return BA_OK;
+  };
+  const int st = run_passes(c, "projective depth (dual)", dE, tolerance, max_iter, errors, n_iter, pass);
   if (st == BA_OK && g_dual_probe) {
     // intermediates of the LAST pass for the tests (host buffers registered by ba_depth_dual_probe)
     double* const* pr = g_dual_probe;
-    const double* src[6] = {V4, R60, W12, ebuf, sums, U4};
+    const double* src[6] = {V4, R60, W12, ebuf, sums, c.U4};
     const size_t cnt[6] = {(size_t)4 * N, (size_t)60 * M, (size_t)12 * M, (size_t)N * M, (size_t)2 * M, (size_t)4 * n};
     for (int k = 0; k < 6; ++k)
       if (pr[k]) cudaMemcpyAsync(pr[k], src[k], cnt[k] * d, cudaMemcpyDeviceToHost, s);
     cudaStreamSynchronize(s);
   }
-  gram_release(&ws, s);
-  return st;  // ~DevBufs frees everything and synchronises the stream
+  return st;  // ~DepthCall releases the Gram workspace, frees everything and synchronises the stream
 }
 
 // Tests only: host buffers that the next ba_projective_depth_dual call fills with the intermediates
@@ -1066,82 +1151,43 @@ extern "C" int ba_depth_dual_probe(double* V4, double* R60, double* W12, double*
 static int factorize_rank4_impl(int device, int64_t n_cols, int32_t n_rows, const double* Wt, bool centre,
                                 double* mean_out, double* M_out, double* S_out, double* sigma_out, int mem,
                                 void* stream) {
-  int ndev = 0;
-  if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0) {
-    set_error("no CUDA device: the factorisation has no CPU path");
-    return BA_ERR_NO_DEVICE;
-  }
-  if (!Wt || !M_out || !S_out || n_cols < 4 || n_rows < 4 || n_rows > 192 || device < 0 || device >= ndev) {
-    set_error("factorisation: need >= 4 columns, 4..192 rows and valid pointers");
-    return BA_ERR_INVALID;
-  }
-  cudaStream_t s = (cudaStream_t)stream;
-  BA_CUDA(cudaSetDevice(device));
-  int num_sms = 148;
-  BA_CUDA(cudaDeviceGetAttribute(&num_sms, cudaDevAttrMultiProcessorCount, device));
+  DepthCall c(stream);
+  BA_TRY(c.open(Wt && M_out && S_out && n_cols >= 4 && n_rows >= 4 && n_rows <= 192, "the factorisation",
+                "factorisation: need >= 4 columns, 4..192 rows and valid pointers", device, n_cols, n_rows, Wt,
+                (size_t)n_cols * n_rows, S_out, (size_t)4 * n_cols, mem));
   const int64_t N = n_cols;
-  const int n = n_rows;
-  const int ld = (n + 7) / 8 * 8;
-  const int64_t k_pad = (N + 31) / 32 * 32;
+  const int n = n_rows, grid = c.grid;
   const size_t d = sizeof(double);
-  const int grid = balanced_blocks((N + 7) / 8, (int64_t)num_sms * 8);
-  DevBufs bufs(s);
-  double *dW = nullptr, *Wk = nullptr, *P = nullptr, *G = nullptr, *V = nullptr, *U4 = nullptr, *ev = nullptr,
-         *small = nullptr, *dS = nullptr;
-  int* status = nullptr;
-  BA_TRY(bufs.alloc(&Wk, (size_t)k_pad * ld));
-  BA_TRY(bufs.alloc(&P, (size_t)ld * ld));
-  BA_TRY(bufs.alloc(&G, (size_t)n * n));
-  BA_TRY(bufs.alloc(&V, (size_t)2 * n * n));
-  BA_TRY(bufs.alloc(&U4, (size_t)4 * n));
-  BA_TRY(bufs.alloc(&ev, 4));
-  BA_TRY(bufs.alloc(&small, 32));
-  BA_TRY(bufs.alloc(&status, 1));
-  if (mem == BA_MEM_DEVICE) {
-    dW = const_cast<double*>(Wt);
-    dS = S_out;
-  } else {
-    BA_TRY(bufs.alloc(&dW, (size_t)N * n));
-    BA_TRY(bufs.alloc(&dS, (size_t)4 * N));
-    BA_CUDA(cudaMemcpyAsync(dW, Wt, (size_t)N * n * d, cudaMemcpyHostToDevice, s));
-  }
-  BA_CUDA(cudaMemsetAsync(Wk, 0, (size_t)k_pad * ld * d, s));
-  BA_CUDA(cudaMemsetAsync(P, 0, (size_t)ld * ld * d, s));
-  BA_CUDA(cudaMemsetAsync(status, 0, sizeof(int), s));
+  cudaStream_t s = c.s;
+  const cudaMemcpyKind kind = mem == BA_MEM_DEVICE ? cudaMemcpyDeviceToDevice : cudaMemcpyDeviceToHost;
+  double* small = nullptr;
+  BA_TRY(c.bufs.alloc(&small, 32));
   if (centre) {
     double *part = nullptr, *colsum = nullptr, *mean = nullptr;
     const int64_t warps = (int64_t)grid * 8;
-    BA_TRY(bufs.alloc(&part, (size_t)warps * n));
-    BA_TRY(bufs.alloc(&colsum, (size_t)n));
-    BA_TRY(bufs.alloc(&mean, (size_t)n));
-    col_partial_kernel<<<grid, 256, 0, s>>>(N, n, dW, part);
+    BA_TRY(c.bufs.alloc(&part, (size_t)warps * n));
+    BA_TRY(c.bufs.alloc(&colsum, (size_t)n));
+    BA_TRY(c.bufs.alloc(&mean, (size_t)n));
+    col_partial_kernel<<<grid, 256, 0, s>>>(N, n, c.in, part);
     colsum_finish_kernel<<<(n + 63) / 64, 64, 0, s>>>(part, warps, n, colsum);
-    pad_rows_centred_kernel<<<grid, 256, 0, s>>>(N, n, ld, dW, colsum, mean, Wk);
+    pad_rows_centred_kernel<<<grid, 256, 0, s>>>(N, n, c.ld, c.in, colsum, mean, c.Wk);
     g_launch_count += 2;
-    if (mean_out)
-      BA_CUDA(cudaMemcpyAsync(mean_out, mean, (size_t)n * d,
-                              mem == BA_MEM_DEVICE ? cudaMemcpyDeviceToDevice : cudaMemcpyDeviceToHost, s));
+    if (mean_out) BA_CUDA(cudaMemcpyAsync(mean_out, mean, (size_t)n * d, kind, s));
   } else {
-    pad_rows_kernel<<<grid, 256, 0, s>>>(N, n, ld, dW, Wk);
+    pad_rows_kernel<<<grid, 256, 0, s>>>(N, n, c.ld, c.in, c.Wk);
   }
-  GramWorkspace ws;
-  int st = gram_prepare(&ws, ld, k_pad, num_sms, s);
-  if (st == BA_OK) st = leading_subspace(n, ld, k_pad, &ws, Wk, P, G, V, U4, ev, status, false, s);
-  if (st == BA_OK) {
-    dual_small_kernel<<<1, 256, (size_t)4 * n * d, s>>>(n, G, U4, small, 1);
-    factor_shape_kernel<<<grid, 256, (size_t)4 * n * d, s>>>(N, n, ld, Wk, U4, dS);
-    g_launch_count += 3;
-    const cudaMemcpyKind kind = mem == BA_MEM_DEVICE ? cudaMemcpyDeviceToDevice : cudaMemcpyDeviceToHost;
-    if (cudaMemcpyAsync(M_out, U4, (size_t)4 * n * d, kind, s) != cudaSuccess ||
-        (sigma_out && cudaMemcpyAsync(sigma_out, small + 16, 4 * d, kind, s) != cudaSuccess) ||
-        (mem != BA_MEM_DEVICE && cudaMemcpyAsync(S_out, dS, (size_t)4 * N * d, cudaMemcpyDeviceToHost, s) != cudaSuccess) ||
-        cudaStreamSynchronize(s) != cudaSuccess) {
-      set_error("factorisation: %s", cudaGetErrorString(cudaGetLastError()));
-      st = BA_ERR_CUDA;
-    }
+  BA_TRY(c.leading_subspace(false));
+  dual_small_kernel<<<1, 256, (size_t)4 * n * d, s>>>(n, c.G, c.U4, small, 1);
+  factor_shape_kernel<<<grid, 256, (size_t)4 * n * d, s>>>(N, n, c.ld, c.Wk, c.U4, c.out);
+  g_launch_count += 3;
+  BA_TRY(check_launches("factorisation"));
+  if (cudaMemcpyAsync(M_out, c.U4, (size_t)4 * n * d, kind, s) != cudaSuccess ||
+      (sigma_out && cudaMemcpyAsync(sigma_out, small + 16, 4 * d, kind, s) != cudaSuccess) ||
+      c.copy_out() != cudaSuccess || cudaStreamSynchronize(s) != cudaSuccess) {
+    set_error("factorisation: %s", cudaGetErrorString(cudaGetLastError()));
+    return BA_ERR_CUDA;
   }
-  gram_release(&ws, s);
-  return st;
+  return BA_OK;
 }
 
 extern "C" int ba_factorize_rank4(int device, int64_t n_cols, int32_t n_rows, const double* Wt, double* M_out,
@@ -1153,96 +1199,4 @@ extern "C" int ba_factorize_centred_rank4(int device, int64_t n_cols, int32_t n_
                                           double* mean_out, double* M_out, double* S_out, double* sigma_out,
                                           int mem, void* stream) {
   return factorize_rank4_impl(device, n_cols, n_rows, Wt, true, mean_out, M_out, S_out, sigma_out, mem, stream);
-}
-
-extern "C" int ba_projective_depth_primary(int device, int64_t n_points, int32_t n_images, const double* x,
-                                           double f0, double tolerance, int max_iter, double* z,
-                                           double* errors, int* n_iter, int mem, void* stream) {
-  int ndev = 0;
-  if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0) {
-    set_error("no CUDA device: the projective-depth iteration has no CPU path");
-    return BA_ERR_NO_DEVICE;
-  }
-  if (!x || !z || !n_iter || n_points < 4 || n_images < 2 || n_images > 64 || max_iter < 1 || device < 0 ||
-      device >= ndev) {
-    set_error("projective depth: need >= 4 points, 2..64 images, max_iter >= 1 and valid pointers");
-    return BA_ERR_INVALID;
-  }
-  cudaStream_t s = (cudaStream_t)stream;
-  BA_CUDA(cudaSetDevice(device));
-  int num_sms = 148;
-  BA_CUDA(cudaDeviceGetAttribute(&num_sms, cudaDevAttrMultiProcessorCount, device));
-  const int64_t N = n_points;
-  const int M = n_images, n = 3 * M;
-  const int ld = (n + 7) / 8 * 8;
-  const int64_t k_pad = (N + 31) / 32 * 32;
-  const size_t d = sizeof(double);
-  double *dx = nullptr, *dz = nullptr, *Wn = nullptr, *P = nullptr, *G = nullptr, *V = nullptr, *U4 = nullptr,
-         *ev = nullptr, *part = nullptr, *dE = nullptr;
-  const int64_t blocks64 = (N + 7) / 8;
-  const int grid = balanced_blocks(blocks64, (int64_t)num_sms * 8);
-  BA_CUDA(cudaMallocAsync(reinterpret_cast<void**>(&Wn), (size_t)k_pad * ld * d, s));
-  BA_CUDA(cudaMallocAsync(reinterpret_cast<void**>(&P), (size_t)ld * ld * d, s));
-  BA_CUDA(cudaMallocAsync(reinterpret_cast<void**>(&G), (size_t)n * n * d, s));
-  BA_CUDA(cudaMallocAsync(reinterpret_cast<void**>(&V), (size_t)n * n * d, s));
-  BA_CUDA(cudaMallocAsync(reinterpret_cast<void**>(&U4), (size_t)4 * n * d, s));
-  BA_CUDA(cudaMallocAsync(reinterpret_cast<void**>(&ev), 4 * d, s));
-  BA_CUDA(cudaMallocAsync(reinterpret_cast<void**>(&part), (size_t)grid * d, s));
-  BA_CUDA(cudaMallocAsync(reinterpret_cast<void**>(&dE), d, s));
-  if (mem == BA_MEM_DEVICE) {
-    dx = const_cast<double*>(x);
-    dz = z;
-  } else {
-    BA_CUDA(cudaMallocAsync(reinterpret_cast<void**>(&dx), (size_t)N * M * 3 * d, s));
-    BA_CUDA(cudaMallocAsync(reinterpret_cast<void**>(&dz), (size_t)N * M * d, s));
-    BA_CUDA(cudaMemcpyAsync(dx, x, (size_t)N * M * 3 * d, cudaMemcpyHostToDevice, s));
-  }
-  BA_CUDA(cudaMemsetAsync(Wn, 0, (size_t)k_pad * ld * d, s));
-  BA_CUDA(cudaMemsetAsync(P, 0, (size_t)ld * ld * d, s));
-  {
-    std::vector<double> ones((size_t)N * M, 1.0);  // :80  z = 1
-    BA_CUDA(cudaMemcpyAsync(dz, ones.data(), ones.size() * d, cudaMemcpyHostToDevice, s));
-    BA_CUDA(cudaStreamSynchronize(s));
-  }
-  int* status = nullptr;
-  BA_CUDA(cudaMallocAsync(reinterpret_cast<void**>(&status), sizeof(int), s));
-  BA_CUDA(cudaMemsetAsync(status, 0, sizeof(int), s));
-  static const bool force_jacobi = std::getenv("BA_DEPTH_JACOBI") != nullptr;  // tests: the fallback path
-  GramWorkspace ws;
-  int st = gram_prepare(&ws, ld, k_pad, num_sms, s);
-  const size_t jac_smem = (size_t)(2 * ((n + 1) / 2)) * d + (size_t)2 * (n + 1) * sizeof(int) + 16;
-  int it = 0;
-  double E = 0.0;
-  while (st == BA_OK) {
-    depth_scale_kernel<<<grid, 256, 0, s>>>(N, M, ld, dx, dz, Wn);
-    st = gram_launch(&ws, Wn, P, s);
-    if (st != BA_OK) break;
-    gram_symmetrize_kernel<<<(n * n + 255) / 256, 256, 0, s>>>(n, ld, P, G);
-    if (!force_jacobi)
-      subspace_eig_kernel<<<1, 256, (size_t)8 * n * d, s>>>(n, G, U4, it > 0 ? 1 : 0, 2000, status);
-    jacobi_eig_kernel<<<1, 256, jac_smem, s>>>(n, G, V, U4, ev, force_jacobi ? nullptr : status);
-    depth_update_kernel<<<grid, 256, (size_t)12 * M * d, s>>>(N, M, ld, dx, Wn, U4, dz, part);
-    depth_error_kernel<<<1, 256, 0, s>>>(part, grid, (double)N * (double)M, f0, dE);
-    g_launch_count += 6;
-    if (cudaMemcpyAsync(&E, dE, d, cudaMemcpyDeviceToHost, s) != cudaSuccess ||
-        cudaStreamSynchronize(s) != cudaSuccess) {
-      set_error("projective depth: %s", cudaGetErrorString(cudaGetLastError()));
-      st = BA_ERR_CUDA;
-      break;
-    }
-    if (errors) errors[it] = E;
-    ++it;
-    if (E < tolerance || it >= max_iter) break;  // :138-142
-  }
-  *n_iter = it;
-  if (st == BA_OK && mem != BA_MEM_DEVICE) {
-    if (cudaMemcpyAsync(z, dz, (size_t)N * M * d, cudaMemcpyDeviceToHost, s) != cudaSuccess) st = BA_ERR_CUDA;
-  }
-  gram_release(&ws, s);
-  void* frees[] = {Wn, P, G, V, U4, ev, part, dE, status, mem == BA_MEM_DEVICE ? nullptr : dx,
-                   mem == BA_MEM_DEVICE ? nullptr : dz};
-  for (void* p : frees)
-    if (p) cudaFreeAsync(p, s);
-  cudaStreamSynchronize(s);
-  return st;
 }

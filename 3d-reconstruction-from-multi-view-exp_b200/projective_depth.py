@@ -19,21 +19,25 @@ from . import _cabi
 from .bundle_adjuster import _default_device
 
 
-def projective_depth_primary(x, f0: float, tolerance: float, max_iter: int = 200, device: int | None = None):
-    """``(z, errors)``: depths ``(n_points, n_images)`` and the reprojection error of every iteration."""
+def _depth(symbol: str, x, f0: float, tolerance: float, max_iter: int, device: int | None):
+    """``(z, errors)`` of the C entry point ``symbol`` (the primary or the dual method)."""
     x = np.ascontiguousarray(x, dtype=np.float64)
     if x.ndim != 3 or x.shape[2] != 3:
         raise ValueError("x must be (n_points, n_images, 3)")
     N, M = x.shape[:2]
     z = np.empty((N, M), dtype=np.float64)
-    errors = np.empty(int(max_iter), dtype=np.float64)
+    errors = np.empty(max(int(max_iter), 1), dtype=np.float64)  # the dual method runs one pass at least
     n_iter = C.c_int(0)
-    lib = _cabi.load()
+    fn = getattr(_cabi.load(), symbol)
     dev = _default_device() if device is None else int(device)
-    _cabi.check(lib.ba_projective_depth_primary(dev, N, M, x.ctypes.data, float(f0), float(tolerance), int(max_iter),
-                                                z.ctypes.data, errors.ctypes.data, C.byref(n_iter),
-                                                _cabi.BA_MEM_HOST, None))
+    _cabi.check(fn(dev, N, M, x.ctypes.data, float(f0), float(tolerance), int(max_iter), z.ctypes.data,
+                   errors.ctypes.data, C.byref(n_iter), _cabi.BA_MEM_HOST, None))
     return z, errors[: n_iter.value].copy()
+
+
+def projective_depth_primary(x, f0: float, tolerance: float, max_iter: int = 200, device: int | None = None):
+    """``(z, errors)``: depths ``(n_points, n_images)`` and the reprojection error of every iteration."""
+    return _depth("ba_projective_depth_primary", x, f0, tolerance, max_iter, device)
 
 
 def compute_projective_depth_primary_method(x, f0: float, tolerance: float, max_iter: int = 200):
@@ -51,19 +55,7 @@ MAX_IMAGES = 64  # the kernels keep one or two images per lane / a (3 M)^2 Gram 
 
 def projective_depth_dual(x, f0: float, tolerance: float, max_iter: int = 50, device: int | None = None):
     """``(z, errors)`` of the dual method (:147-235) in O(n_images x n_points) memory."""
-    x = np.ascontiguousarray(x, dtype=np.float64)
-    if x.ndim != 3 or x.shape[2] != 3:
-        raise ValueError("x must be (n_points, n_images, 3)")
-    N, M = x.shape[:2]
-    z = np.empty((N, M), dtype=np.float64)
-    errors = np.empty(max(int(max_iter), 1), dtype=np.float64)
-    n_iter = C.c_int(0)
-    lib = _cabi.load()
-    dev = _default_device() if device is None else int(device)
-    _cabi.check(lib.ba_projective_depth_dual(dev, N, M, x.ctypes.data, float(f0), float(tolerance), int(max_iter),
-                                             z.ctypes.data, errors.ctypes.data, C.byref(n_iter),
-                                             _cabi.BA_MEM_HOST, None))
-    return z, errors[: n_iter.value].copy()
+    return _depth("ba_projective_depth_dual", x, f0, tolerance, max_iter, device)
 
 
 def compute_projective_depth_dual_method(x, f0: float, tolerance: float, max_iter: int = 50):
