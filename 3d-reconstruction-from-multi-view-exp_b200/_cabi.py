@@ -87,6 +87,7 @@ SIGNATURES = {
     "ba_profile_enable": (C.c_int, [_P, C.c_int]),
     "ba_profile_get": (C.c_int, [_P, C.c_char_p, C.POINTER(C.c_double), C.POINTER(C.c_int64)]),
     "ba_profile_reset": (C.c_int, [_P]),
+    "ba_covariance": (C.c_int, [_P, _P, _P, C.POINTER(C.c_double), C.c_int, _P]),
     "ba_fp64_peak": (C.c_int, [C.c_int, C.c_int, C.POINTER(C.c_double)]),
     "ba_matrix_free": (C.c_int, [_P]),
     "ba_syrk_plan_info": (C.c_int, [C.c_int, C.c_int64, C.c_int, C.c_int, C.POINTER(C.c_int), C.POINTER(C.c_int),

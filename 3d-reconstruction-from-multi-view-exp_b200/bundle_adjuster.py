@@ -175,6 +175,18 @@ class BundleAdjuster:
                                                       self._X, self._R, self._t)
         return self._X, gauge.make_K(self._f, self._u, self._f0), self._R, self._t
 
+    def covariance(self):
+        """Marginal covariances at the current state (after ``optimize``: the solution), in the
+        caller's frame that ``optimize`` returns: ``(cov_X (N, 3, 3), cov_cam (M, 9, 9), sigma2)``,
+        cameras in the order (f, u0, v0, t, w).  sigma2 = E / (2 n_obs - n_unknowns) scales
+        (J^T J)^-1; the 7 gauge-pinned camera parameters have zero rows and columns.  Raises
+        ``numpy.linalg.LinAlgError`` for a point seen fewer than twice or an indefinite system."""
+        if self._group is not None:
+            raise RuntimeError("covariance of a sharded adjuster is not supported")
+        cov_X, cov_cam, sigma2 = self._engine.covariance()
+        cov_X, cov_cam = gauge.covariance_to_caller(self._R0, self._c0c1_len, cov_X, cov_cam)
+        return cov_X, cov_cam, sigma2
+
     def get_log(self):
         """Per-iteration points / camera log in the normalised frame (:204-206)."""
         return self._log

@@ -274,6 +274,25 @@ __device__ __forceinline__ double block_sum(double v, double* scratch) {
 #endif
 
 #ifdef __CUDACC__
+// 16-byte cp.async (LDGSTS) through L2; src_bytes < 16 zero-fills the rest of the destination
+__device__ __forceinline__ void cp_async16_zfill(void* smem, const void* gmem, int src_bytes) {
+  const unsigned sa = (unsigned)__cvta_generic_to_shared(smem);
+  asm volatile("cp.async.cg.shared.global [%0], [%1], 16, %2;\n" ::"r"(sa), "l"(gmem), "r"(src_bytes));
+}
+__device__ __forceinline__ void cp_async_commit() { asm volatile("cp.async.commit_group;\n" ::); }
+template <int N>
+__device__ __forceinline__ void cp_async_wait() {
+  asm volatile("cp.async.wait_group %0;\n" ::"n"(N));
+}
+
+// One FP64 tensor-core step (DMMA.8x8x4): C[8x8] += A[8x4] B[4x8].  Lane l holds A[l / 4][l % 4],
+// B[l % 4][l / 4] and C[l / 4][2 (l % 4) + {0, 1}].
+__device__ __forceinline__ void dmma884(double& c0, double& c1, double a, double b) {
+  asm volatile("mma.sync.aligned.m8n8k4.row.col.f64.f64.f64.f64 {%0,%1}, {%2}, {%3}, {%0,%1};\n"
+               : "+d"(c0), "+d"(c1)
+               : "d"(a), "d"(b));
+}
+
 // Shared-memory copy of a camera table: rows padded to 17 doubles (conflict-free when the lanes of a
 // warp read one column of 32 consecutive rows, the dense-visibility pattern).
 constexpr int kTabStride = kCamTab + 1;
@@ -429,6 +448,7 @@ int build_camera_major_index(ba_engine* e, cudaStream_t s);
 int build_pair_index(ba_engine* e, cudaStream_t s);
 int launch_schur_sparse(ba_engine* e, const ba_lm_state* ctl, cudaStream_t s);
 int fp64_peak(int device, int use_dmma, double* tflops);
+int covariance(ba_engine* e, double* point_cov, double* cam_cov, double* sigma2, int mem, cudaStream_t s);
 int launch_comm_allreduce_red(ba_engine* e, bool conditional, cudaStream_t s);
 int launch_comm_allreduce_cost(ba_engine* e, int slot, bool conditional, cudaStream_t s);
 void comm_free(ba_engine* e);

@@ -926,6 +926,11 @@ int ba_profile_reset(ba_engine* e) {
   return BA_OK;
 }
 
+int ba_covariance(ba_engine* e, double* point_cov, double* cam_cov, double* sigma2, int mem, void* stream) {
+  BA_TRY(check_ready(e));
+  return covariance(e, point_cov, cam_cov, sigma2, mem, (cudaStream_t)stream);
+}
+
 int ba_fp64_peak(int device, int use_dmma, double* tflops) { return fp64_peak(device, use_dmma, tflops); }
 
 int ba_matrix_free(ba_engine* e) { return e && dense_matrix_free(e) ? 1 : 0; }

@@ -15,7 +15,8 @@ PKG = os.path.dirname(HERE)
 ROOT = os.path.dirname(PKG)
 OUT = os.path.join(PKG, "libba_b200.so")
 SOURCES = ["ba_engine.cu", "k1_residual_jacobian.cu", "k2_point_blocks.cu", "k3_schur_syrk.cu", "k3_schur_sparse.cu",
-           "k4_cholesky_solve.cu", "k4_cholesky.cu", "k5_project.cu", "fp64_peak.cu", "comm_peer.cu", "k6_gauge.cu", "k7_projective_depth.cu"]
+           "k4_cholesky_solve.cu", "k4_cholesky.cu", "k5_project.cu", "fp64_peak.cu", "comm_peer.cu", "k6_gauge.cu", "k7_projective_depth.cu",
+           "k8_covariance.cu"]
 HEADERS = ["ba_common.cuh", os.path.join(ROOT, "include", "ba_b200.h")]
 ARCH = ["-gencode", "arch=compute_100a,code=sm_100a"]
 

@@ -43,22 +43,6 @@ namespace ba {
 
 constexpr int kStages = 3;
 
-__device__ __forceinline__ void cp_async16_zfill(void* smem, const void* gmem, int src_bytes) {
-  const unsigned sa = (unsigned)__cvta_generic_to_shared(smem);
-  asm volatile("cp.async.cg.shared.global [%0], [%1], 16, %2;\n" ::"r"(sa), "l"(gmem), "r"(src_bytes));
-}
-__device__ __forceinline__ void cp_async_commit() { asm volatile("cp.async.commit_group;\n" ::); }
-template <int N>
-__device__ __forceinline__ void cp_async_wait() {
-  asm volatile("cp.async.wait_group %0;\n" ::"n"(N));
-}
-
-__device__ __forceinline__ void dmma884(double& c0, double& c1, double a, double b) {
-  asm volatile("mma.sync.aligned.m8n8k4.row.col.f64.f64.f64.f64 {%0,%1}, {%2}, {%3}, {%0,%1};\n"
-               : "+d"(c0), "+d"(c1)
-               : "d"(a), "d"(b));
-}
-
 __device__ __forceinline__ void tile_from_linear(int t, int& ti, int& tj) {
   ti = (int)((sqrt(8.0 * t + 1.0) - 1.0) * 0.5);
   while ((ti + 1) * (ti + 2) / 2 <= t) ++ti;

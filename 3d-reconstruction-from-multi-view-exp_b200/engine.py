@@ -185,6 +185,16 @@ class Engine:
     def solve_trial(self, c: float):
         _cabi.check(self._lib.ba_solve_trial(self._h, float(c), self.stream))
 
+    def covariance(self, points: bool = True):
+        """(point_cov (N,3,3) or None, cam_cov (M,9,9), sigma2) at the current state, undamped, in the
+        normalised frame and the parameter order (f, u0, v0, t, w); see ``ba_covariance``."""
+        pc = np.empty((self.n_points, 3, 3)) if points else None
+        cc = np.empty((self.n_cams, 9, 9))
+        s2 = C.c_double()
+        _cabi.check(self._lib.ba_covariance(self._h, None if pc is None else pc.ctypes.data, cc.ctypes.data,
+                                            C.byref(s2), _cabi.BA_MEM_HOST, self.stream))
+        return pc, cc, s2.value
+
     # -- LM loop ------------------------------------------------------------------------------
     def lm_begin(self, scale_factor, delta_tol, max_iter, max_retries=200):
         _cabi.check(self._lib.ba_lm_begin(self._h, float(scale_factor), float(delta_tol), int(max_iter),

@@ -54,3 +54,23 @@ def make_K(f, u, f0):
     K[:, 1, 2] = u[:, 1]
     K[:, 2, 2] = f0
     return K
+
+
+def covariance_jacobians(R0, length):
+    """Jacobians of ``denormalize`` at the solution: points ``length R0``, cameras
+    T = blockdiag(I_3, length R0, R0) over (f, u0, v0, t, w).  The rotation update is
+    R <- exp([w]x) R, so R0 exp([w]x) R = exp([R0 w]x) R0 R maps w by R0.  The sign of the
+    divisor (``normalize``) cancels in T S T^T."""
+    Jx = length * np.asarray(R0)
+    T = np.zeros((9, 9))
+    T[:3, :3] = np.eye(3)
+    T[3:6, 3:6] = Jx
+    T[6:, 6:] = R0
+    return Jx, T
+
+
+def covariance_to_caller(R0, length, cov_X, cov_cam):
+    """Normalised-frame covariances -> the caller's frame: Jx S Jx^T per point, T S T^T per camera."""
+    Jx, T = covariance_jacobians(R0, length)
+    out_X = None if cov_X is None else Jx @ cov_X @ Jx.T
+    return out_X, T @ cov_cam @ T.T

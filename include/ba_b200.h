@@ -234,6 +234,25 @@ int ba_buffer_read(ba_engine* e, int id, double* host_out, int64_t n_doubles, vo
 /* Layout facts the host needs: padded order of the reduced system and its rhs row. */
 int ba_reduced_layout(ba_engine* e, int32_t* n_pad, int32_t* n_full, int32_t* rhs_row);
 
+/* ---- uncertainty ------------------------------------------------------------------- */
+/* Marginal covariances at the current state (slot 0), undamped, gauge unknowns pinned, in the
+ * normalised frame and the parameter order (f, u0, v0, t, w) of ba_get_state:
+ *   sigma2      = E / (2 n_obs - (3 n_points + 9 n_cams - 7)), E the cost of the state;
+ *   H           = 2 J^T J (the engine's Gauss-Newton Hessian), S its reduced camera system, S = L L^T;
+ *   cam_cov[i]  = 2 sigma2 S^-1[9i..9i+8][9i..9i+8], S^-1[a][b] = <L^-1 e_a, L^-1 e_b>; the rows and
+ *                 columns of the 7 pinned parameters (camera 0: t, w; camera 1: the baseline
+ *                 component) are exactly 0;
+ *   point_cov[j] = 2 sigma2 L_j^-T (I_3 + Q_j) L_j^-1, V_j = L_j L_j^T the point block and
+ *                 Q_j[d][e] = <L^-1 y_{3j+d}, L^-1 y_{3j+e}> with Y_j = W_j^T L_j^-T.
+ * point_cov is [n_points][3][3], cam_cov [n_cams][9][9]; either may be NULL to skip that pass.
+ * mem = BA_MEM_HOST / BA_MEM_DEVICE for both.  The LM state, the control block and the records are
+ * left as they were: a later ba_lm_run gives the same results as without this call.
+ * Errors: BA_ERR_INVALID when there are no more residuals than unknowns; BA_ERR_SINGULAR when a
+ * point has fewer than two views, a point block or the reduced system is not positive definite
+ * (e.g. a camera without observations); BA_ERR_STATE on an engine with a peer exchange. */
+int ba_covariance(ba_engine* e, double* point_cov, double* cam_cov, double* sigma2, int mem,
+                  void* stream);
+
 /* ---- profiling helpers ------------------------------------------------------------ */
 /* Number of kernels this library launched since ba_create (all engines of the process). */
 int64_t ba_launch_count(void);
