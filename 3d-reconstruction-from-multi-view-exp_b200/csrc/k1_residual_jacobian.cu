@@ -206,9 +206,11 @@ int launch_cost(ba_engine* e, int which, int slot, cudaStream_t s) {
   const size_t smem = tab_smem_bytes(e);
   const double2* xy = reinterpret_cast<const double2*>(e->obs_xy);
   const int grid = e->cost_blocks;
+  // the 48 KB default limit counts the static block_sum scratch too: at 360 and 361 cameras the table
+  // alone fits under it, table and scratch do not
 #define BA_COST_LAUNCH(D, T)                                                                   \
   do {                                                                                         \
-    if (smem > 48 * 1024)                                                                      \
+    if (smem + 32 * sizeof(double) > 48 * 1024)                                                \
       BA_CUDA(cudaFuncSetAttribute(cost_kernel<D, T>, cudaFuncAttributeMaxDynamicSharedMemorySize, \
                                    (int)smem));                                                \
     cost_kernel<D, T><<<grid, 256, smem, s>>>(e->nobs, e->M, e->obs_cam, e->obs_pt, xy,        \

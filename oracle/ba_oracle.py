@@ -301,14 +301,17 @@ def schur_flops_sparse(obs: ObsList) -> float:
 
 
 def solve_damped(obs: ObsList, lin: Linearization, c: float, axis: str, chunk_points: int = 4096,
-                 schur: str = "dense", solver: str = "lu"):
+                 schur: str = "dense", solver: str = "lu", reduced=None):
     """One inner LM solve: returns (delta_xi_full (M,9), delta_X (N,3), A_red, b_red).
 
     ``schur="sparse"`` uses the sparsity-aware C restatement; ``solver="cholesky"`` replaces the
     reference's LU (:146) by LAPACK ``dposv`` -- half the flops at n = 8993, and SURVEY.md section 6
-    measured the effect on the cost trajectory at <= 3e-14 relative (A is SPD)."""
+    measured the effect on the cost trajectory at <= 3e-14 relative (A is SPD).  ``reduced``: the
+    (A_full, b_full, Vinv) of this ``lin`` and ``c`` when the caller has formed it already."""
     _, kept = gauge_indices(obs.n_cams, axis)
-    if schur == "sparse":
+    if reduced is not None:
+        A, b, Vinv = reduced
+    elif schur == "sparse":
         A, b, Vinv = reduced_system_sparse(obs, lin, c)
     else:
         A, b, Vinv = reduced_system(obs, lin, c, chunk_points)

@@ -177,11 +177,14 @@ def test_golden_runs_against_full_inverse(ba, name):
 
 
 # n = 9M: 180 (one CTA back substitution, ragged), 576 (whole 64-blocks), 1350 (cluster regime,
-# ragged), 2250 (two-level factorisation).  The seeds give cond(S) = 1.4e6, 2.0e6, 4.7e6 and 4.8e6;
-# at the initial state of some seeds a camera is barely constrained (150 cameras, seed 150:
-# cond(S) = 5.4e10), where both routes stay within cond(S) eps but not within 1e-9 of each other.
+# ragged), 2250 (two-level factorisation), 3600 (a dense engine above 361 cameras: stored Jacobian
+# rows, 128-tile updates).  The seeds give cond(S) = 1.4e6, 2.0e6, 4.7e6, 4.8e6 and 1.3e7; at the
+# initial state of some seeds a camera is barely constrained (150 cameras, seed 150: cond(S) = 5.4e10;
+# 400 cameras x 700 points, seeds 1 to 5 and 10 to 15: 1.5e7 .. 7e13), where both routes stay within
+# cond(S) eps but not within 1e-9 of each other.
 @pytest.mark.gpu
-@pytest.mark.parametrize("M,N,seed", [(20, 300, 20), (64, 400, 64), (150, 600, 3), (250, 2000, 250)])
+@pytest.mark.parametrize("M,N,seed", [(20, 300, 20), (64, 400, 64), (150, 600, 3), (250, 2000, 250),
+                                      (400, 700, 403)])
 def test_each_factorisation_regime(ba, M, N, seed):
     sc, obs, X, R, t, f, u = _scene(ba, M, N, seed=seed)
     eng = _engine(ba, obs, X, R, t, f, u, sc.f0, sc.axis, dense=True)

@@ -37,7 +37,9 @@ def _close(a, b, rel, what):
     assert err <= rel, f"{what}: max err / scale = {err:.3e} > {rel:.1e}"
 
 
-def _check_one_linearisation(ba, obs, X, R, t, f, u, f0, axis, dense, c=1e-4):
+def _check_linearisation(ba, obs, X, R, t, f, u, f0, axis, dense):
+    """cost(0), K1 and K2 against the oracle; returns the linearised engine and the oracle's
+    linearisation."""
     N, M = obs.n_points, obs.n_cams
     eng = _engine_for(ba, obs, X, R, t, f, u, f0, axis, dense)
     lin = O.linearize(obs, X, f, u, R, t, f0)
@@ -60,40 +62,53 @@ def _check_one_linearisation(ba, obs, X, R, t, f, u, f0, axis, dense, c=1e-4):
     _close(V, lin.V[:, iu[0], iu[1]], 1e-12, "V_j")
     _close(eng.buffer("GPT").reshape(N, 3), lin.g_pt, 1e-11, "d_P")
     removed, kept = O.gauge_indices(M, axis)
+    # the diagonal blocks U_i, entries in kept rows and columns (block by block: the 9M x 9M block
+    # diagonal is a gigabyte from 1250 cameras on)
+    keep = np.zeros(9 * M, dtype=bool)
+    keep[kept] = True
+    keep = keep.reshape(M, 9)
+    keep = keep[:, :, None] & keep[:, None, :]
     U = eng.buffer("U").reshape(M, 9, 9)
-    Ufull = np.zeros((9 * M, 9 * M))
-    Uref = np.zeros((9 * M, 9 * M))
-    for i in range(M):
-        Ufull[9 * i: 9 * i + 9, 9 * i: 9 * i + 9] = U[i]
-        Uref[9 * i: 9 * i + 9, 9 * i: 9 * i + 9] = lin.U[i]
-    _close(Ufull[np.ix_(kept, kept)], Uref[np.ix_(kept, kept)], 1e-12, "U_i")
-    assert np.all(Ufull[removed] == 0) and np.all(Ufull[:, removed] == 0)
+    _close(U[keep], lin.U[keep], 1e-12, "U_i")
+    assert np.all(U[~keep] == 0)
     g = eng.buffer("GCAM")
     _close(g[kept], lin.g_cam.ravel()[kept], 1e-11, "d_F")
     assert np.all(g[removed] == 0)
+    return eng, lin
 
-    # K2b + K3: partial reduced system P = sum Y Y^T with the rhs row
-    A_ref, b_ref, Vinv = O.reduced_system(obs, lin, c)
+
+def _check_one_linearisation(ba, obs, X, R, t, f, u, f0, axis, dense, c=1e-4):
+    M = obs.n_cams
+    eng, lin = _check_linearisation(ba, obs, X, R, t, f, u, f0, axis, dense)
+    removed, kept = O.gauge_indices(M, axis)
+
+    # K2b + K3: partial reduced system P = sum Y Y^T with the rhs row.  From n ~ 10^4 the oracle forms
+    # the reduced system with its C restatement and solves it by Cholesky (the dense route and LU take
+    # minutes there); either way it is formed once and the solve below reuses it.
+    schur, solver = ("sparse", "cholesky") if 9 * M > 10_000 else ("dense", "lu")
+    reduced = O.reduced_system_sparse(obs, lin, c) if schur == "sparse" else O.reduced_system(obs, lin, c)
+    A_ref, b_ref, _ = reduced
     eng.build_reduced(c)
     red = eng.buffer("REDUCE")
     npad, nfull, rhs = eng.n_pad, eng.n_full, eng.rhs_row
     P = red[: npad * npad].reshape(npad, npad)
-    Plow = np.tril(P[:nfull, :nfull])
-    Psym = Plow + np.tril(Plow, -1).T
-    Ublk = np.zeros((nfull, nfull))
+    b_gpu = P[rhs, :nfull] - red[npad * npad + 81 * M:]
+    _close(b_gpu[kept], b_ref[kept], 1e-10, "reduced rhs b")
+    # A = blockdiag(U_i with the diagonal scaled by 1 + c) - P, formed in place (n^2 doubles at a time)
+    A_gpu = np.tril(P[:nfull, :nfull])
+    A_gpu += np.tril(A_gpu, -1).T
+    assert np.all(A_gpu[removed] == 0)
+    np.negative(A_gpu, out=A_gpu)
     Ured = red[npad * npad: npad * npad + 81 * M].reshape(M, 9, 9)
     for i in range(M):
         blk = Ured[i].copy()
         blk[np.arange(9), np.arange(9)] *= 1 + c
-        Ublk[9 * i: 9 * i + 9, 9 * i: 9 * i + 9] = blk
-    A_gpu = Ublk - Psym
+        A_gpu[9 * i: 9 * i + 9, 9 * i: 9 * i + 9] += blk
     _close(A_gpu[np.ix_(kept, kept)], A_ref[np.ix_(kept, kept)], 1e-11, "reduced system A")
-    b_gpu = P[rhs, :nfull] - red[npad * npad + 81 * M:]
-    _close(b_gpu[kept], b_ref[kept], 1e-10, "reduced rhs b")
-    assert np.all(Psym[removed] == 0)
+    del P, A_gpu
 
     # K4: solve, update, trial cost
-    dxi_ref, dX_ref, _, _ = O.solve_damped(obs, lin, c, axis)
+    dxi_ref, dX_ref, _, _ = O.solve_damped(obs, lin, c, axis, solver=solver, reduced=reduced)
     eng.solve_trial(c)
     dxi = eng.buffer("DXI").reshape(M, 9)
     _close(dxi, dxi_ref, 1e-8, "camera step")
@@ -132,6 +147,21 @@ def _check_random_scene(ba, n_cams, n_points, visibility, axis):
     return _check_one_linearisation(ba, obs, X, R, t, f, u, sc.f0, axis, dense=sc.dense)
 
 
+# (cameras, points, visibility) past the camera-count thresholds that select kernel instances
+# (test_camera_count_limits.py checks that these scenes reach every instance).  Seed = cameras;
+# cond(S) at the initial state and c = 1e-4: 9.9e4, 3.9e5, 1.1e5, 1.1e5.  1253 cameras because seed
+# 1250 leaves a camera barely constrained (cond(S) = 3.5e8).
+CAMERA_COUNT_SCENES = [
+    (361, 500, 1.0),    # the largest matrix-free dense engine: 48 KB camera table, 121 KB of shared
+                        # memory in the point update
+    (400, 700, 1.0),    # dense on stored rows (K1 writes them), camera table in shared memory,
+                        # 128-tile DMMA SYRK, two-level Cholesky with 128-tile updates
+    (1253, 300, 1.0),   # dense, camera table in global memory, emulated SYRK at n >> k (n_pad = 11 280,
+                        # k_pad = 928), 177 64-blocks on at most 148 back-substitution CTAs
+    (1253, 2000, 0.1),  # the same for the list engine and its pair lists
+]
+
+
 # Sparse scenes run twice: with the static pair lists (schur_pairs_reg_kernel) and with
 # BA_PAIRS_NO_LIST (schur_pairs_kernel scans the bitmaps: the path of scenes whose lists do not fit).
 @pytest.mark.parametrize("n_cams,n_points,visibility,axis,lists", [
@@ -151,6 +181,7 @@ def _check_random_scene(ba, n_cams, n_points, visibility, axis):
     (260, 300, 1.0, "x-right_z-forward", True),   # n = 2340, dense: same with 64-tiles only, edge tiles cut by n_rows
     (1000, 1500, 0.1, "x-up_z-forward", True),    # C4's camera count: n = 8993, 35 outer blocks of the two-level Cholesky,
                                                   # 141-CTA back substitution, 31 x 31 pair tiles (oracle: ~25 s of LU)
+    *[(m, n, v, "x-up_z-forward", True) for m, n, v in CAMERA_COUNT_SCENES],
 ])
 def test_kernels_match_oracle_on_random_scenes(ba, monkeypatch, n_cams, n_points, visibility, axis, lists):
     if not lists:
@@ -168,46 +199,51 @@ def test_bitmap_scan_pair_kernel_is_the_one_that_ran(ba, monkeypatch):
     assert not np.array_equal(red_lists, red_scan)
 
 
-@pytest.mark.parametrize("n_cams,n_points,axis", [(30, 1500, "x-up_z-forward"), (120, 900, "x-right_z-forward"),
-                                                  (17, 333, "x-up_z-forward")])
+@pytest.mark.parametrize("n_cams,n_points,axis", [
+    (30, 1500, "x-up_z-forward"),
+    (120, 900, "x-right_z-forward"),
+    (17, 333, "x-up_z-forward"),
+    (400, 700, "x-up_z-forward"),    # dense engine on stored rows, camera table in shared memory
+    (1250, 300, "x-up_z-forward"),   # both engines read the camera table from global memory; seed 1253:
+                                     # cond(S) = 1.1e5 at c = 1e-4
+])
 def test_matrix_free_linearisation_is_bitwise_the_stored_row_one(ba, n_cams, n_points, axis):
-    """A dense engine re-derives the Jacobian rows in K2a, the camera blocks, K2b and the point update
-    (ba_matrix_free); an engine built from the same observations as a LIST stores them in K1 and
-    reads them back.  The arithmetic is shared and pinned (obs_jacobian, scaled_point_rows, y_entry,
-    pair_accumulate in ba_common.cuh) and the summation orders coincide for full visibility, so
-    V, d_P, U, d_F, L^-1 and z must agree bit for bit -- as must the rows that the matrix-free engine
-    writes on request (JP / JC buffer reads)."""
+    """A dense engine of at most 361 cameras re-derives the Jacobian rows in K2a, the camera blocks,
+    K2b and the point update (ba_matrix_free); a larger one stores them in K1 and reads them back, as
+    an engine built from the same observations as a LIST always does.  The arithmetic is shared and
+    pinned (obs_jacobian, scaled_point_rows, y_entry, pair_accumulate in ba_common.cuh) and the
+    summation orders coincide for full visibility, so V, d_P, U, d_F, L^-1 and z must agree bit for
+    bit -- as must the rows that the matrix-free engine writes on request (JP / JC buffer reads)."""
     sc = ba.scenes.make_scene(n_cams, n_points, seed=3 + n_cams, visibility=1.0, axis=axis)
     assert sc.dense
     obs = O.ObsList(sc.n_points, sc.n_cams, np.repeat(np.arange(sc.n_points), np.diff(sc.obs_ptr)),
                     sc.obs_cam.astype(np.int64), sc.obs_xy, sc.obs_ptr)
     X, R, t = O.normalize_gauge(sc.X0, sc.R0, sc.t0, axis)
     f, u = sc.K0[:, 0, 0].copy(), sc.K0[:, :2, 2].copy()
-    mf = _engine_for(ba, obs, X, R, t, f, u, sc.f0, axis, dense=True)
-    st = _engine_for(ba, obs, X, R, t, f, u, sc.f0, axis, dense=False)
-    assert mf.matrix_free() and not st.matrix_free()
-    for eng in (mf, st):
+    dn = _engine_for(ba, obs, X, R, t, f, u, sc.f0, axis, dense=True)
+    ls = _engine_for(ba, obs, X, R, t, f, u, sc.f0, axis, dense=False)
+    assert dn.matrix_free() == (n_cams <= 361) and not ls.matrix_free()
+    for eng in (dn, ls):
         eng.linearize()
         eng.build_reduced(1e-3)
     for name in ("V", "GPT", "U", "GCAM", "LINV", "Z", "JP", "JC"):
-        a, b = mf.buffer(name), st.buffer(name)
+        a, b = dn.buffer(name), ls.buffer(name)
         assert np.array_equal(a, b), f"{name}: {np.abs(a - b).max():.3e}"
     # the reduced systems come from different Schur kernels (SYRK / pair products): equal to rounding;
     # the dense engine keeps P = Y Y^T with the rhs in row 9M, the list engine the same layout
-    npad, n, rhs = mf.n_pad, mf.n_full, mf.rhs_row
-    assert (npad, n, rhs) == (st.n_pad, st.n_full, st.rhs_row)
-    Pa = mf.buffer("REDUCE")[: npad * npad].reshape(npad, npad)
-    Pb = st.buffer("REDUCE")[: npad * npad].reshape(npad, npad)
-    low = np.tril_indices(n)
-    _close(Pa[:n, :n][low], Pb[:n, :n][low], 1e-12, "P (lower triangle)")
+    npad, n, rhs = dn.n_pad, dn.n_full, dn.rhs_row
+    assert (npad, n, rhs) == (ls.n_pad, ls.n_full, ls.rhs_row)
+    Pa = dn.buffer("REDUCE")[: npad * npad].reshape(npad, npad)
+    Pb = ls.buffer("REDUCE")[: npad * npad].reshape(npad, npad)
+    _close(np.tril(Pa[:n, :n]), np.tril(Pb[:n, :n]), 1e-12, "P (lower triangle)")
     _close(Pa[rhs, :n], Pb[rhs, :n], 1e-12, "rhs row")
-    # one step: the same trial state (the dense point update re-derives Y, the list one reads it)
-    for eng in (mf, st):
+    # one step: the same trial state (the matrix-free point update re-derives Y, the others read it)
+    for eng in (dn, ls):
         eng.solve_trial(1e-3)
-    for got, ref, what in zip(mf.get_state(1), st.get_state(1), ("X", "R", "t", "f", "u")):
+    for got, ref, what in zip(dn.get_state(1), ls.get_state(1), ("X", "R", "t", "f", "u")):
         _close(got, ref, 1e-11, f"trial {what}")
-    mf.close()
-    st.close()
+    dn.close()
+    ls.close()
 
 
 @pytest.mark.parametrize("name", RUN_CASES)
@@ -599,6 +635,31 @@ def test_thousand_camera_trajectory_matches_the_oracle(ba):
     np.testing.assert_allclose(K, g["K"], rtol=0, atol=1e-6)
     np.testing.assert_allclose(R, g["R"], rtol=0, atol=1e-6)
     np.testing.assert_allclose(t, g["t"], rtol=0, atol=1e-6)
+
+
+def test_global_camera_table_run_matches_the_oracle(ba):
+    """1253 cameras (camera table in global memory, 177 64-blocks in the back substitution on at most
+    148 CTAs), 10 % visibility: three LM iterations through the CUDA-graph loop against the oracle's
+    (sparse Schur product, Cholesky solve) -- the bars of the thousand-camera trajectory.  Seed 1253:
+    cond(S) = 1.1e5 at the initial state and c = 1e-4."""
+    sc = ba.scenes.make_scene(1253, 2000, seed=1253, visibility=0.1)
+    adj = ba.BundleAdjuster.from_observations(sc.obs_ptr, sc.obs_cam, sc.obs_xy, sc.X0, sc.K0, sc.R0, sc.t0,
+                                              f0=sc.f0, axis=sc.axis)
+    with contextlib.redirect_stdout(io.StringIO()):
+        X, K, R, t = adj.optimize(2.0, -1.0, max_iter=3)
+    E = np.array([adj.records[0]["E_prev"]] + [r["E"] for r in adj.records])
+    solves = np.array([0] + [r["solves"] for r in adj.records])
+    adj.engine.close()
+    obs = O.ObsList(sc.n_points, sc.n_cams, np.repeat(np.arange(sc.n_points), np.diff(sc.obs_ptr)),
+                    sc.obs_cam.astype(np.int64), sc.obs_xy, sc.obs_ptr)
+    ora = O.OracleBundleAdjuster(None, sc.X0, sc.K0, sc.R0, sc.t0, f0=sc.f0, axis=sc.axis, obs=obs)
+    Xo, Ko, Ro, to = ora.optimize(2.0, -1.0, max_iter=3, verbose=False, schur="sparse", solver="cholesky")
+    assert len(E) == len(ora.trace) == 4
+    np.testing.assert_allclose(E, [r["E"] for r in ora.trace], rtol=1e-9, atol=0)
+    assert np.array_equal(solves, [r["solves"] for r in ora.trace])
+    np.testing.assert_allclose(K, Ko, rtol=0, atol=1e-6)
+    np.testing.assert_allclose(R, Ro, rtol=0, atol=1e-6)
+    np.testing.assert_allclose(t, to, rtol=0, atol=1e-6)
 
 
 def test_outlier_scene_converges_to_the_oracles_rms(ba):

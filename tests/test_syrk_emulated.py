@@ -137,6 +137,9 @@ DENSE_SHAPES = [
     (260, 300, "x-right_z-forward"),
     (40, 50_000, "x-up_z-forward"),   # K = 150 000 > 131 071: two k pieces per tile
     (200, 300, "x-up_z-forward"),     # n_pad = 14 x 128 + 16: the DMMA reference runs tall 128-tiles
+    (400, 700, "x-up_z-forward"),     # n_pad = 3608, k_pad = 2112: 128-tile DMMA reference
+    (1250, 300, "x-up_z-forward"),    # n >> k (n_pad = 11 256, k_pad = 928): 43 full 256-tile rows and a
+                                      # ragged row of 248, as the emulation is selected by default there
 ]
 
 

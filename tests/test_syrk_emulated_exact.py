@@ -119,6 +119,8 @@ EXACT_SHAPES = [
     (256, 120),      # n = 2305 = 9 x 256 + 1 (1 row past the last full tile row); n_pad 2312: ragged row of 8
     (200, 150),      # n = 1801 = 7 x 256 + 9; n_pad 1808: the headline shape's ragged row of 16
     (45, 44_000),    # n = 406 = 256 + 150 (> 128 rows); K = 132 000 > 131 071: two int32 runs per tile
+    (1250, 300),     # n >> k, where the emulation is the default: n_pad = 11 256 = 43 x 256 + 248, k_pad = 928
+                     # (2.2e6 entries checked: every 128-boundary row and column, ~15 s on the host)
 ]
 
 
