@@ -98,7 +98,6 @@ SIGNATURES = {
                                               _P, _P, C.POINTER(C.c_int), C.c_int, _P]),
     "ba_projective_depth_dual": (C.c_int, [C.c_int, C.c_int64, C.c_int32, _P, C.c_double, C.c_double, C.c_int,
                                            _P, _P, C.POINTER(C.c_int), C.c_int, _P]),
-    "ba_depth_dual_probe": (C.c_int, [_P, _P, _P, _P, _P, _P]),
     "ba_factorize_rank4": (C.c_int, [C.c_int, C.c_int64, C.c_int32, _P, _P, _P, _P, C.c_int, _P]),
     "ba_factorize_centred_rank4": (C.c_int, [C.c_int, C.c_int64, C.c_int32, _P, _P, _P, _P, _P, C.c_int, _P]),
     "ba_project_points": (C.c_int, [C.c_int, C.c_int64, C.c_int32, _P, _P, _P, _P, _P, C.c_int, _P]),

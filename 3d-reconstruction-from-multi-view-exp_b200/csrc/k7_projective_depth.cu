@@ -747,7 +747,7 @@ __device__ __forceinline__ int sym_pair(int a, int b, int n) {  // index of (a, 
 // shared memory, lane r owns row r of the column rotation and column r of the row rotation.
 // (A single-thread version on local-memory arrays -- the straightforward code, fine on the host -- is
 // miscompiled by nvcc 12.9 for sm_100a at K = 12: it stops converging after the first sweep;
-// tools/gpu/jac_test.cu reproduces it next to this version.)  Returns with the eigenvalues on the
+// tools/jac_test.cu reproduces it next to this version.)  Returns with the eigenvalues on the
 // diagonal of a; fixed order of operations.
 template <int K>
 __device__ void jacobi_warp(double* a, double* e) {
@@ -1079,8 +1079,6 @@ extern "C" int ba_projective_depth_primary(int device, int64_t n_points, int32_t
   return run_passes(c, "projective depth", dE, tolerance, max_iter, errors, n_iter, pass);
 }
 
-static double* const* g_dual_probe = nullptr;
-
 extern "C" int ba_projective_depth_dual(int device, int64_t n_points, int32_t n_images, const double* x, double f0,
                                         double tolerance, int max_iter, double* z, double* errors, int* n_iter,
                                         int mem, void* stream) {
@@ -1125,27 +1123,7 @@ extern "C" int ba_projective_depth_dual(int device, int64_t n_points, int32_t n_
     g_launch_count += 12;
     return BA_OK;
   };
-  const int st = run_passes(c, "projective depth (dual)", dE, tolerance, max_iter, errors, n_iter, pass);
-  if (st == BA_OK && g_dual_probe) {
-    // intermediates of the LAST pass for the tests (host buffers registered by ba_depth_dual_probe)
-    double* const* pr = g_dual_probe;
-    const double* src[6] = {V4, R60, W12, ebuf, sums, c.U4};
-    const size_t cnt[6] = {(size_t)4 * N, (size_t)60 * M, (size_t)12 * M, (size_t)N * M, (size_t)2 * M, (size_t)4 * n};
-    for (int k = 0; k < 6; ++k)
-      if (pr[k]) cudaMemcpyAsync(pr[k], src[k], cnt[k] * d, cudaMemcpyDeviceToHost, s);
-    cudaStreamSynchronize(s);
-  }
-  return st;  // ~DepthCall releases the Gram workspace, frees everything and synchronises the stream
-}
-
-// Tests only: host buffers that the next ba_projective_depth_dual call fills with the intermediates
-// of its last pass -- V4 [N][4], R60 [M][60], W12 [M][12], e [N][M], sums [2][M], U4 [3M][4]; any may
-// be NULL; pass all NULL to switch the probe off again.
-extern "C" int ba_depth_dual_probe(double* V4, double* R60, double* W12, double* e, double* sums, double* U4) {
-  static double* slots[6];
-  slots[0] = V4; slots[1] = R60; slots[2] = W12; slots[3] = e; slots[4] = sums; slots[5] = U4;
-  g_dual_probe = (V4 || R60 || W12 || e || sums || U4) ? slots : nullptr;
-  return BA_OK;
+  return run_passes(c, "projective depth (dual)", dE, tolerance, max_iter, errors, n_iter, pass);
 }
 
 static int factorize_rank4_impl(int device, int64_t n_cols, int32_t n_rows, const double* Wt, bool centre,

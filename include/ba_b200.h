@@ -319,11 +319,6 @@ int ba_projective_depth_dual(int device, int64_t n_points, int32_t n_images, con
                              double tolerance, int max_iter, double* z, double* errors, int* n_iter,
                              int mem, void* stream);
 
-/* Tests only: register host buffers that the next ba_projective_depth_dual call fills with the
- * intermediates of its last pass (V4 [N][4], R60 [M][60], W12 [M][12], e [N][M], sums [2][M],
- * U4 [3M][4]); any may be NULL, all NULL switches the probe off. */
-int ba_depth_dual_probe(double* V4, double* R60, double* W12, double* e, double* sums, double* U4);
-
 /* factorization_method(W, n_rank=4) (reference lib/factorization.py:5-15), the step between the
  * projective depths and the Euclidean upgrade (lib/perspective_camera_calibration.py:533): rank-4
  * truncated SVD W ~ M S of the (n_rows x n_cols) matrix, n_rows = 3 n_images <= 192.  Wt is W
