@@ -123,7 +123,7 @@ struct ba_engine {
   ba::EmuItem* emu_items = nullptr;      // [emu_n_items] launch order
   int8_t* Yq = nullptr;                  // [kEmuModuli][n_pad][k_pad] residue planes, K-major
   uint32_t* Pmod = nullptr;              // [kEmuModuli][lower 128-tiles][128 cols][128 rows] residue sums
-  unsigned long long* colmax = nullptr;  // [n_pad] bit pattern of max |Yt[k][a]| over k
+  unsigned long long* colmax = nullptr;  // [n_pad] max |Yt[k][a]| over k, to its exponent (K2b gathers it)
 
   // observations (CSR by point) and camera-major index
   int64_t* obs_ptr = nullptr;

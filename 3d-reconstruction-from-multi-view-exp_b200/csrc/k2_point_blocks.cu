@@ -240,6 +240,29 @@ int launch_camera_blocks(ba_engine* e, cudaStream_t s, bool conditional) {
 // MF (dense scenes, camera table small enough for shared memory): matrix-free -- the Jacobian rows
 // are re-derived from the camera table and X_j (obs_jacobian, the arithmetic K1 stored them with:
 // the same bits) instead of being read back, 224 B per observation; the kernel then only writes.
+//
+// colmax (dense, when K3 runs on the INT8 emulation; nullptr otherwise): the column maxima of |Yt| that
+// set the emulation's column exponents, gathered as Yt is written.  Only ilogb of a maximum is used,
+// and for a normal double that is its exponent field: a CTA keeps the largest top 16 bits (exponent and
+// four mantissa bits) of every column in shared memory (2 bytes per column: room for the stored-row
+// kernel's three CTAs per SM up to n_pad 10 752, for the matrix-free one's two at every M it takes),
+// then raises colmax[a] to them << 48 with one atomicMax per column.  A subnormal entry (exponent field
+// 0) goes straight to colmax with its full bit pattern, so ilogb of colmax[a] is that of max |Yt[k][a]|
+// in every case, and an all-zero column keeps 0.
+__device__ __forceinline__ unsigned colmax_top16(double y, unsigned long long* __restrict__ colmax, int col) {
+  const unsigned long long u = (unsigned long long)__double_as_longlong(y) & 0x7FFFFFFFFFFFFFFFull;
+  if (u != 0 && u < (1ull << 52)) atomicMax(colmax + col, u);  // subnormal: rare
+  return (unsigned)(u >> 48);
+}
+__device__ __forceinline__ void colmax_smem_max(unsigned short* cm, int col, unsigned v) {
+  unsigned short old = *reinterpret_cast<volatile unsigned short*>(cm + col);
+  while (v > old) {  // the maximum rarely grows after a CTA's first points: mostly one load
+    const unsigned short prev = atomicCAS(cm + col, old, (unsigned short)v);
+    if (prev == old) break;
+    old = prev;
+  }
+}
+
 template <bool DENSE, bool MF>
 __global__ void __launch_bounds__(256, MF ? 2 : 3)
 k2b_point_solve_kernel(int64_t N, int M, int axis, const int64_t* __restrict__ obs_ptr,
@@ -249,7 +272,7 @@ k2b_point_solve_kernel(int64_t N, int M, int axis, const int64_t* __restrict__ o
                        int use_ctl, double* __restrict__ LINV, double* __restrict__ Z,
                        double* __restrict__ Yt, int ld, int rhs_col, double* __restrict__ Ysp,
                        const double* __restrict__ X, double* __restrict__ PT,
-                       const double* __restrict__ camtab, double f0) {
+                       const double* __restrict__ camtab, double f0, unsigned long long* __restrict__ colmax) {
   static_assert(DENSE || !MF, "the matrix-free variant is the dense one");
   if (use_ctl && ctl->done) return;
   const double c = use_ctl ? ctl->c : c_host;
@@ -257,11 +280,14 @@ k2b_point_solve_kernel(int64_t N, int M, int axis, const int64_t* __restrict__ o
   const int lane = threadIdx.x & 31;
   extern __shared__ double k2b_stage[];
   double* tab = k2b_stage;  // MF: the camera table, rows padded to kTabStride
-  if (MF) {
+  double* st0 = k2b_stage + (MF ? tab_smem_doubles(M) : 0);
+  unsigned short* cm = reinterpret_cast<unsigned short*>(st0 + 8 * 864);  // colmax: [ld] top 16 bits
+  if (DENSE && colmax)
+    for (int k = threadIdx.x; k < ld; k += blockDim.x) cm[k] = 0;
+  if (MF)
     for (int k = threadIdx.x; k < M * kCamTab; k += blockDim.x) tab[(k >> 4) * kTabStride + (k & 15)] = camtab[k];
-    __syncthreads();
-  }
-  double* st = k2b_stage + (MF ? tab_smem_doubles(M) : 0) + (threadIdx.x >> 5) * 864;  // 32 observations x 27 doubles per warp
+  if (MF || (DENSE && colmax)) __syncthreads();
+  double* st = st0 + (threadIdx.x >> 5) * 864;  // 32 observations x 27 doubles per warp
   const int64_t warp = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
   const int64_t nwarps = ((int64_t)gridDim.x * blockDim.x) >> 5;
   for (int64_t j = warp; j < N; j += nwarps) {
@@ -311,6 +337,11 @@ k2b_point_solve_kernel(int64_t N, int M, int axis, const int64_t* __restrict__ o
         Yt[(size_t)(3 * j + 0) * ld + rhs_col] = z0;
         Yt[(size_t)(3 * j + 1) * ld + rhs_col] = z1;
         Yt[(size_t)(3 * j + 2) * ld + rhs_col] = z2;
+        if (colmax) {
+          const unsigned h0 = colmax_top16(z0, colmax, rhs_col), h1 = colmax_top16(z1, colmax, rhs_col),
+                         h2 = colmax_top16(z2, colmax, rhs_col);
+          colmax_smem_max(cm, rhs_col, max(max(h0, h1), h2));
+        }
       }
     }
     const int64_t lo = DENSE ? j * M : obs_ptr[j];
@@ -386,11 +417,18 @@ k2b_point_solve_kernel(int64_t N, int M, int axis, const int64_t* __restrict__ o
       }
       __syncwarp();
       if (DENSE) {
-        const size_t col0 = 9 * (size_t)(o0 - lo);
-#pragma unroll
-        for (int d = 0; d < 3; ++d) {
-          double* dst = Yt + (size_t)(3 * j + d) * ld + col0;
-          for (int k = lane; k < 9 * cnt; k += 32) dst[k] = st[288 * d + k];
+        const int col0 = 9 * (int)(o0 - lo);
+        double* dst = Yt + (size_t)(3 * j) * ld + col0;
+        for (int k = lane; k < 9 * cnt; k += 32) {
+          const double y0 = st[k], y1 = st[288 + k], y2 = st[576 + k];
+          dst[k] = y0;
+          dst[(size_t)ld + k] = y1;
+          dst[2 * (size_t)ld + k] = y2;
+          if (colmax) {
+            const unsigned h0 = colmax_top16(y0, colmax, col0 + k), h1 = colmax_top16(y1, colmax, col0 + k),
+                           h2 = colmax_top16(y2, colmax, col0 + k);
+            colmax_smem_max(cm, col0 + k, max(max(h0, h1), h2));
+          }
         }
       } else {
         double* dst = Ysp + (size_t)o0 * 27;
@@ -399,6 +437,11 @@ k2b_point_solve_kernel(int64_t N, int M, int axis, const int64_t* __restrict__ o
       __syncwarp();
     }
   }
+  if (DENSE && colmax) {
+    __syncthreads();
+    for (int k = threadIdx.x; k < ld; k += blockDim.x)
+      if (cm[k]) atomicMax(colmax + k, (unsigned long long)cm[k] << 48);
+  }
 }
 
 // Dense scenes whose camera table fits next to the staging rows re-derive the Jacobian rows.
@@ -406,10 +449,15 @@ bool dense_matrix_free(const ba_engine* e) {
   return e->dense && tab_smem_doubles(e->M) * sizeof(double) <= 48 * 1024;
 }
 
+// Every path that runs K2b (LM graph, eager loop, covariance, sharded phases) comes through here, so the
+// column maxima are reset before each launch that gathers them.
 int launch_k2b(ba_engine* e, bool conditional, double c_host, cudaStream_t s) {
   const int use_ctl = conditional ? 1 : 0;
   const bool mf = dense_matrix_free(e);
-  const size_t kStage = 8 * 864 * sizeof(double) + (mf ? tab_smem_doubles(e->M) * sizeof(double) : 0);
+  unsigned long long* colmax = e->dense && e->syrk_emu ? e->colmax : nullptr;
+  if (colmax) BA_CUDA(cudaMemsetAsync(colmax, 0, (size_t)e->n_pad * sizeof(unsigned long long), s));
+  const size_t kStage = 8 * 864 * sizeof(double) + (mf ? tab_smem_doubles(e->M) * sizeof(double) : 0) +
+                        (colmax ? ((size_t)e->n_pad * sizeof(unsigned short) + 15) / 16 * 16 : 0);
   const int grid = balanced_blocks((e->N + 7) / 8, (int64_t)e->num_sms * 16);
 #define BA_K2B_LAUNCH(D, F)                                                                                  \
   do {                                                                                                       \
@@ -417,7 +465,7 @@ int launch_k2b(ba_engine* e, bool conditional, double c_host, cudaStream_t s) {
                                  (int)kStage));                                                              \
     k2b_point_solve_kernel<D, F><<<grid, 256, kStage, s>>>(                                                  \
         e->N, e->M, e->axis, e->obs_ptr, e->obs_cam, e->JP, e->JC, e->V, e->GPT, c_host, e->ctl, use_ctl,   \
-        e->LINV, e->Z, e->Yt, e->n_pad, e->rhs_row, e->Ysp, e->X[0], e->PT, e->camtab[0], e->f0);            \
+        e->LINV, e->Z, e->Yt, e->n_pad, e->rhs_row, e->Ysp, e->X[0], e->PT, e->camtab[0], e->f0, colmax);    \
   } while (0)
   if (mf) BA_K2B_LAUNCH(true, true);
   else if (e->dense) BA_K2B_LAUNCH(true, false);

@@ -21,9 +21,9 @@
 //
 // Large dense products (C3: n_pad^2 k_pad = 9.8e11) run instead on the INT8 tensor cores, FP64-accurate
 // through the modular Ozaki scheme (see "FP64-accurate product on the INT8 tensor cores" below):
-// emu_colmax_kernel and emu_residue_kernel turn Yt into 16 int8 residue planes, syrk_i8_pair_kernel
-// (tcgen05.mma kind::i8 on pairs of SMs) forms one SYRK per modulus, emu_reconstruct_kernel lifts the exact integer
-// products back to FP64 into P.  The DMMA kernels stay for smaller products (C2), the Cholesky's
+// emu_residue_kernel turns Yt into 16 int8 residue planes (with the column maxima K2b gathers as it
+// writes Yt), syrk_i8_pair_kernel (tcgen05.mma kind::i8 on pairs of SMs) forms one SYRK per modulus,
+// emu_reconstruct_kernel lifts the exact integer products back to FP64 into P.  The DMMA kernels stay for smaller products (C2), the Cholesky's
 // trailing updates and the projective-depth Gram matrix.  BA_SYRK_EMU=0|1 overrides the size rule.
 //
 // Sparse visibility: see k3_schur_sparse.cu (output-stationary, no atomics).
@@ -630,99 +630,115 @@ struct EmuConsts {
   int half[kEmuModuli];
 };
 
-// e_a for a column whose largest |entry| has the bit pattern `maxbits`: max 2^e_a < 2^b
+// e_a for a column whose largest |entry| has the exponent of the bit pattern `maxbits`: max 2^e_a < 2^b
 __device__ __forceinline__ int emu_exponent(unsigned long long maxbits, int b) {
   if (maxbits == 0) return 0;
   return b - 1 - ilogb(__longlong_as_double((long long)maxbits));
 }
 
-// Column maxima of |Yt| as bit patterns (the order of an integer max does not matter).
-__global__ void __launch_bounds__(128)
-emu_colmax_kernel(const double* __restrict__ Yt, int64_t k_pad, int n_pad, unsigned long long* __restrict__ colmax,
-                  const ba_lm_state* ctl) {
-  if (ctl && ctl->done) return;
-  const int a = 2 * (blockIdx.x * blockDim.x + threadIdx.x);
-  if (a >= n_pad) return;
-  const int64_t rows = (k_pad + gridDim.y - 1) / gridDim.y;
-  const int64_t k0 = (int64_t)blockIdx.y * rows, k1 = k0 + rows < k_pad ? k0 + rows : k_pad;
-  constexpr unsigned long long kAbs = 0x7FFFFFFFFFFFFFFFull;
-  unsigned long long m0 = 0, m1 = 0;
-#pragma unroll 8
-  for (int64_t k = k0; k < k1; ++k) {
-    const double2 v = __ldg(reinterpret_cast<const double2*>(Yt + k * n_pad + a));
-    m0 = max(m0, (unsigned long long)__double_as_longlong(v.x) & kAbs);
-    m1 = max(m1, (unsigned long long)__double_as_longlong(v.y) & kAbs);
+// Residue planes Yq[i][a][k] (K-major) from Yt[k][a], with the column maxima K2b gathered (colmax).
+// A thread converts 16 consecutive k-rows of one column: 16 loads in flight, then for every modulus one
+// 16-byte store; the 8 threads of a column in a warp write whole 128-byte lines of a plane row, and its
+// loads read 32-byte pieces (4 columns) of 8 k-rows.  Per element, a' = rint(x 2^e_a) is formed once as
+// an int64 (two exact power-of-two multiplications: 2^e_a alone is not a normal double for all e_a),
+// and biased by 2^55 so that its seven low bytes u_0..u_6 are unsigned digits of a' + 2^55.  Then per
+// modulus p, without FP64:
+//   f = 2^23 + c_p + sum_k u_k (256^k mod p)   two dp4a; c_p = (-2^23 - 2^55) mod p, so f = a' (mod p),
+//                                              and the accumulator starts at the bit pattern of 2^23 + c_p:
+//                                              it is f as a float (f < 2^23 + 2^19, exact)
+//   q = rint(f / p)                             one FFMA with the float 1 / p and the 1.5 * 2^23 rounding
+//                                              constant; exact for every f in range (checked exhaustively
+//                                              by tests/test_emu_residue_digits.py) except p = 255,
+//                                              which takes q from f - 2^23 (< 2^11) instead
+//   r = f - p q                                 one IMAD on the bit patterns; every constant it carries is a
+//                                              multiple of 256, so its low byte is that of r in [-127, 127]
+// p = 256 is the low byte of a'.  Any representative of a' mod p gives the same residue sums, P is
+// unchanged.
+constexpr int kResK = 16;                      // k-rows per thread
+constexpr int kResTK = 8 * kResK;              // k-rows of a block: one 128-byte line per plane row
+constexpr int kResTA = 32;                     // columns of a block: 4 per warp
+constexpr int kResThreads = 8 * kResTA;
+constexpr float kResRound = 12582912.0f;       // 1.5 * 2^23
+constexpr unsigned kResFloat23 = 0x4B000000u;  // bit pattern of 2^23
+
+__host__ __device__ constexpr unsigned emu_pow256_mod(int k, int p) {
+  unsigned r = 1;
+  for (int i = 0; i < k; ++i) r = r * 256u % (unsigned)p;
+  return r;
+}
+__host__ __device__ constexpr unsigned emu_digit_weights(int k0, int p) {  // bytes 256^(k0 + j) mod p
+  return emu_pow256_mod(k0, p) | emu_pow256_mod(k0 + 1, p) << 8 | emu_pow256_mod(k0 + 2, p) << 16 |
+         (k0 + 3 < 7 ? emu_pow256_mod(k0 + 3, p) << 24 : 0u);
+}
+__host__ __device__ constexpr unsigned emu_digit_bias(int p) {  // c_p = (-2^23 - 2^55) mod p
+  return (unsigned)((2u * (unsigned)p - emu_pow256_mod(6, p) * 128u % (unsigned)p - (1u << 23) % (unsigned)p) %
+                    (unsigned)p);
+}
+
+// Low byte: a' mod p_I (lo, hi: the words of a' + 2^55)
+template <int I>
+__device__ __forceinline__ unsigned emu_residue_byte(unsigned lo, unsigned hi) {
+  constexpr int p = emu_modulus(I);
+  if constexpr (p == 256) {
+    return lo;
+  } else {
+    constexpr bool small = p == 255;
+    const unsigned acc = __dp4a(hi, emu_digit_weights(4, p),
+                                __dp4a(lo, emu_digit_weights(0, p), kResFloat23 + emu_digit_bias(p) + (small ? (1u << 23) % p : 0u)));
+    float f = __uint_as_float(acc);
+    if (small) f = __fadd_rn(f, -8388608.0f);
+    const float q = __fmaf_rn(f, 1.0f / (float)p, kResRound);
+    return acc - (unsigned)p * __float_as_uint(q);
   }
-  if (m0) atomicMax(colmax + a, m0);
-  if (m1) atomicMax(colmax + a + 1, m1);
 }
 
-// Symmetric residue of the integer v (|v| <= 2^53) modulo p_I as an int in [-128, 127]: q = rint(v / p)
-// through the 1.5 * 2^52 rounding constant (|v / p| < 2^46), r = v - p q exact.  1 / p is rounded, so
-// q can miss the nearest integer by one when v / p lies within 0.0052 of a half: |r| <= 128.8.
-// (Called from fully unrolled loops: p and 1 / p are compile-time constants.)
-__device__ __forceinline__ int emu_residue(double v, int i) {
-  const double p = (double)emu_modulus(i), inv = 1.0 / p, magic = 6755399441055744.0;
-  const double q = __dadd_rn(__fma_rn(v, inv, magic), -magic);
-  const double r = __fma_rn(-p, q, v);
-  const int ri = __double2loint(__dadd_rn(r, magic));
-  return ri > 127 ? ri - (int)p : ri;
+template <int I>
+__device__ __forceinline__ uint4 emu_plane_piece(const unsigned (&lo)[kResK], const unsigned (&hi)[kResK]) {
+  unsigned w[4];
+#pragma unroll
+  for (int g = 0; g < 4; ++g) {
+    const unsigned r0 = emu_residue_byte<I>(lo[4 * g], hi[4 * g]), r1 = emu_residue_byte<I>(lo[4 * g + 1], hi[4 * g + 1]);
+    const unsigned r2 = emu_residue_byte<I>(lo[4 * g + 2], hi[4 * g + 2]), r3 = emu_residue_byte<I>(lo[4 * g + 3], hi[4 * g + 3]);
+    w[g] = __byte_perm(__byte_perm(r0, r1, 0x0040), __byte_perm(r2, r3, 0x0040), 0x5410);
+  }
+  return make_uint4(w[0], w[1], w[2], w[3]);
+}
+template <int I>
+__device__ __forceinline__ void emu_store_planes(int8_t* __restrict__ dst, size_t plane_stride, const unsigned (&lo)[kResK],
+                                                 const unsigned (&hi)[kResK]) {
+  if constexpr (I < kEmuModuli) {
+    *reinterpret_cast<uint4*>(dst + I * plane_stride) = emu_plane_piece<I>(lo, hi);
+    emu_store_planes<I + 1>(dst, plane_stride, lo, hi);
+  }
 }
 
-// Residue planes Yq[i][a][k] (K-major) from Yt[k][a]: a block converts 64 k-rows x 32 columns,
-// transposing through shared memory -- rows are read as 256-byte segments, plane rows written as
-// 64-byte segments.  48 KB of shared memory and <= 64 registers: four blocks (32 warps) per SM.
-constexpr int kResTK = 64, kResTA = 32, kResThreads = 256;
-constexpr size_t kResSmemBytes = (size_t)kResTK * kResTA * sizeof(double) + (size_t)kEmuModuli * kResTA * kResTK;
-
-__global__ void __launch_bounds__(kResThreads, 4)
+__global__ void __launch_bounds__(kResThreads, 3)
 emu_residue_kernel(const double* __restrict__ Yt, int64_t k_pad, int n_pad, const unsigned long long* __restrict__ colmax,
                    int bits, int8_t* __restrict__ Yq, const ba_lm_state* ctl) {
   if (ctl && ctl->done) return;
-  extern __shared__ __align__(16) unsigned char res_smem[];
-  double* sIn = reinterpret_cast<double*>(res_smem);  // [64 k][32 a]
-  uint2* sOut = reinterpret_cast<uint2*>(res_smem + kResTK * kResTA * sizeof(double));  // [16][32 a][8 x 8 bytes]
-  const int64_t k0 = (int64_t)blockIdx.x * kResTK;
-  const int a0 = blockIdx.y * kResTA;
-  const int t = threadIdx.x;
-  for (int q = t; q < kResTK * kResTA / 2; q += kResThreads) {
-    const int row = q / (kResTA / 2), cp = q % (kResTA / 2);
-    const int a = a0 + 2 * cp;
-    const int64_t k = k0 + row;
-    double2 v = make_double2(0.0, 0.0);
-    if (k < k_pad && a < n_pad) v = __ldg(reinterpret_cast<const double2*>(Yt + k * n_pad + a));
-    reinterpret_cast<double2*>(sIn)[q] = v;
-  }
-  __syncthreads();
-  // thread: column a0 + lane, k-rows 8 w .. 8 w + 7; its 8 residues of a plane are one 8-byte piece,
-  // stored at piece w ^ (lane & 6) of the column's 64-byte row (the XOR keeps the two pieces of every
-  // 16-byte chunk adjacent and in order, and spreads the stores over the banks)
-  const int lane = t & 31, w = t >> 5;
-  const int e = a0 + lane < n_pad ? emu_exponent(colmax[a0 + lane], bits) : 0;
-  double v[8];
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  const int a = blockIdx.x * kResTA + 4 * warp + (lane & 3);
+  if (a >= n_pad) return;
+  // 2^e_a = s1 s2, each an exact double (e_a > 1023 only for columns whose maximum is below 2^-971)
+  const int e = emu_exponent(colmax[a], bits);
+  const int e1 = e < 1023 ? e : 1023;
+  const double s1 = ldexp(1.0, e1), s2 = ldexp(1.0, e - e1);
+  const size_t plane_stride = (size_t)n_pad * k_pad;
+  for (int64_t k0 = (int64_t)blockIdx.y * kResTK + kResK * (lane >> 2); k0 < k_pad; k0 += (int64_t)gridDim.y * kResTK) {
+    // k_pad is a multiple of 32: a thread's 16 rows are all in or all out
+    const double* src = Yt + k0 * n_pad + a;
+    double x[kResK];
 #pragma unroll
-  for (int j = 0; j < 8; ++j) v[j] = rint(ldexp(sIn[(8 * w + j) * kResTA + lane], e));
+    for (int j = 0; j < kResK; ++j) x[j] = __ldcs(src + (size_t)j * n_pad);
+    unsigned lo[kResK], hi[kResK];
 #pragma unroll
-  for (int i = 0; i < kEmuModuli; ++i) {
-    uint32_t word[2];
-#pragma unroll
-    for (int u = 0; u < 2; ++u) {
-      const int r0 = emu_residue(v[4 * u], i), r1 = emu_residue(v[4 * u + 1], i);
-      const int r2 = emu_residue(v[4 * u + 2], i), r3 = emu_residue(v[4 * u + 3], i);
-      word[u] = __byte_perm(__byte_perm(r0, r1, 0x0040), __byte_perm(r2, r3, 0x0040), 0x5410);
+    for (int j = 0; j < kResK; ++j) {
+      const long long v = __double2ll_rn(__dmul_rn(__dmul_rn(x[j], s1), s2));  // a' = rint(x 2^e_a), |a'| <= 2^53
+      lo[j] = (unsigned)v;
+      hi[j] = (unsigned)(v >> 32) + (1u << 23);  // + 2^55
     }
-    sOut[(i * kResTA + lane) * 8 + (w ^ (lane & 6))] = make_uint2(word[0], word[1]);
+    emu_store_planes<0>(Yq + (size_t)a * k_pad + k0, plane_stride, lo, hi);
   }
-  __syncthreads();
-  // 16-byte chunks: 16 planes x 32 columns x 4 chunks, two planes per pass of the block
-  const int sa = (t >> 2) & 31, c = t & 3, ih = t >> 7;
-  const int ga = a0 + sa;
-  const int64_t gk = k0 + 16 * c;  // k_pad is a multiple of 32: a chunk is all in or all out
-  if (ga >= n_pad || gk >= k_pad) return;
-#pragma unroll
-  for (int i = ih; i < kEmuModuli; i += 2)
-    *reinterpret_cast<uint4*>(Yq + ((size_t)i * n_pad + ga) * k_pad + gk) =
-        *reinterpret_cast<const uint4*>(sOut + (i * kResTA + sa) * 8 + ((2 * c) ^ (sa & 6)));
 }
 
 __device__ __forceinline__ void tma_load_3d(unsigned dst, const CUtensorMap* map, int c0, int c1, int c2, unsigned bar) {
@@ -1381,22 +1397,18 @@ static int make_plane_map(CUtensorMap* map, const int8_t* Yq, int n_pad, int64_t
 static int launch_syrk_emu(ba_engine* e, const ba_lm_state* ctl, cudaStream_t s) {
   CUtensorMap map;
   BA_TRY(make_plane_map(&map, e->Yq, e->n_pad, e->k_pad));
-  BA_CUDA(cudaFuncSetAttribute(emu_residue_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kResSmemBytes));
   BA_CUDA(cudaFuncSetAttribute(syrk_i8_pair_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kEmuSmemBytes));
   BA_CUDA(cudaFuncSetAttribute(syrk_i8_pair_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kEmuSmemBytes));
   const int n_tiles = e->syrk_n_tiles;
   ProfScope ps(e, PG_SYRK, s);
-  BA_CUDA(cudaMemsetAsync(e->colmax, 0, (size_t)e->n_pad * sizeof(unsigned long long), s));
+  // colmax was gathered by K2b (launch_k2b resets it before every launch)
   BA_CUDA(cudaMemsetAsync(e->Pmod, 0, (size_t)kEmuModuli * n_tiles * kEmuTile * kEmuTile * sizeof(uint32_t), s));
   {
-    const int gx = (e->n_pad / 2 + 127) / 128;
-    const int64_t gy = std::max<int64_t>(1, std::min<int64_t>(e->k_pad / 64, (int64_t)16 * e->num_sms / gx));
-    emu_colmax_kernel<<<dim3(gx, (unsigned)gy), 128, 0, s>>>(e->Yt, e->k_pad, e->n_pad, e->colmax, ctl);
+    const int64_t k_tiles = (e->k_pad + kResTK - 1) / kResTK;
+    emu_residue_kernel<<<dim3((e->n_pad + kResTA - 1) / kResTA, (unsigned)std::min<int64_t>(k_tiles, 65535)),
+                         kResThreads, 0, s>>>(e->Yt, e->k_pad, e->n_pad, e->colmax, e->emu_bits, e->Yq, ctl);
     BA_LAUNCH_CHECK();
   }
-  emu_residue_kernel<<<dim3((unsigned)((e->k_pad + kResTK - 1) / kResTK), (e->n_pad + kResTA - 1) / kResTA),
-                       kResThreads, kResSmemBytes, s>>>(e->Yt, e->k_pad, e->n_pad, e->colmax, e->emu_bits, e->Yq, ctl);
-  BA_LAUNCH_CHECK();
   if (e->emu_n_full > 0) {
     syrk_i8_pair_kernel<false><<<2 * e->emu_n_full, kEmuThreads, kEmuSmemBytes, s>>>(map, e->emu_items, e->Pmod,
                                                                                      n_tiles, e->n_pad, ctl);

@@ -4,8 +4,9 @@
 
 Builds the reduced system of one dense scene `reps` times on an engine created with BA_SYRK_EMU=1,
 under torch.profiler (CUDA activities), and prints one JSON line: mean time per build of every K3
-kernel, the conversion passes' bandwidth (bytes they must move: Yt read twice, the residue planes
-written once), the int8 rate of both instances of syrk_i8_pair_kernel (whole tile rows, ragged last
+kernel and of K2b (k2b_point_solve_kernel, which gathers the column maxima the conversion needs; run
+on a build before that change for K2b without them), the residue conversion's bandwidth (bytes it must
+move: Yt read once, the residue planes written once), the int8 rate of both instances of syrk_i8_pair_kernel (whole tile rows, ragged last
 tile row) and the operand bytes their TMA copies deliver to
 shared memory per build.  The rate counts the MMA work the kernel issues: 2 x 256 x N x k per 256-tile
 and modulus, N = 256 (diagonal tiles included: their upper halves are computed too), or the rows of a
@@ -20,6 +21,16 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
+
+
+def _smi(field):
+    import subprocess
+    try:
+        out = subprocess.run(["nvidia-smi", f"--query-gpu={field}", "--format=csv,noheader,nounits", "-i", "0"],
+                             capture_output=True, text=True, timeout=30).stdout.strip()
+        return float(out)
+    except (OSError, ValueError, subprocess.SubprocessError):
+        return None
 
 
 def main():
@@ -60,7 +71,7 @@ def main():
         if "syrk_i8_pair_kernel" in name:  # two instances: whole tile rows, and the ragged last tile row
             k = "syrk_i8_pair_kernel<ragged>" if "<true>" in name else "syrk_i8_pair_kernel<full>"
             ms[k] = ms.get(k, 0.0) + ev.device_time_total / 1e3 / args.reps
-        for k in ("emu_colmax_kernel", "emu_residue_kernel", "emu_reconstruct_kernel"):
+        for k in ("emu_colmax_kernel", "emu_residue_kernel", "emu_reconstruct_kernel", "k2b_point_solve_kernel"):
             if k in name:
                 ms[k] = ms.get(k, 0.0) + ev.device_time_total / 1e3 / args.reps
         if "emset" in name:
@@ -83,20 +94,22 @@ def main():
     if left != 256:
         l2_GB["ragged"] = nt2 * (2 * 16384.0 + 2 * 128.0 * min(left, 128)) * kb * len(moduli) / 1e9
     ki = {"full": "syrk_i8_pair_kernel<full>", "ragged": "syrk_i8_pair_kernel<ragged>"}
-    conv_bytes = 2 * 8.0 * k_pad * n_pad + len(moduli) * float(n_pad) * k_pad
+    conv_bytes = 8.0 * k_pad * n_pad + len(moduli) * float(n_pad) * k_pad
     conv_ms = ms.get("emu_colmax_kernel", 0) + ms.get("emu_residue_kernel", 0)
+    k2b_ms = ms.pop("k2b_point_solve_kernel", None)
     res = {
         "scene": f"{args.cams} x {args.points}", "n_pad": n_pad, "k_pad": k_pad, "bits": bits, "moduli": len(moduli),
         "ms_per_build": ms,
         "syrk_total_ms": sum(ms.values()),
+        "k2b_ms": k2b_ms,
+        "conversion_bytes": conv_bytes,
         "conversion_GBps": conv_bytes / (conv_ms * 1e-3) / 1e9 if conv_ms else None,
-        "residue_pass_GBps": (8.0 * k_pad * n_pad + len(moduli) * float(n_pad) * k_pad)
-        / (ms["emu_residue_kernel"] * 1e-3) / 1e9 if ms.get("emu_residue_kernel") else None,
         "i8_TOPS": {c: ops[c] / (ms[ki[c]] * 1e-3) / 1e12 for c in ops if ms.get(ki[c])},
         "i8_ops": ops,
         "tma_box_GB_per_build": box_GB,
         "l2_to_sm_GB_per_build": l2_GB,
         "gpu": torch.cuda.get_device_name(0),
+        "power_limit_W": _smi("power.limit"), "sm_clock_MHz": _smi("clocks.sm"),
     }
     eng.close()
     print(json.dumps(res))
