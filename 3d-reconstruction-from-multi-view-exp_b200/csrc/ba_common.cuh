@@ -81,6 +81,36 @@ struct EmuItem {
   int mod, ti, tj, kb_lo, kb_hi;
 };
 
+// A planned dense product P = Yt^T Yt (lower triangle) of a k-major operand Yt [k_pad][n_pad]
+// (k3_schur_syrk.cu): which kernels compute it, their work items on the device and their scratch.
+// The engine holds one for its Schur product, the projective-depth solver one for its Gram matrix.
+enum SyrkKind {
+  SYRK_AUTO = 0,   // syrk_prepare chooses by size (and BA_SYRK_EMU)
+  SYRK_TILE64,     // FP64 tensor cores, 64-tiles (syrk_dmma_kernel)
+  SYRK_TILE128,    // FP64 tensor cores, 128-tiles fed by TMA (syrk_tma_kernel)
+  SYRK_EMULATED,   // INT8 tensor cores, FP64-accurate (Ozaki scheme II)
+};
+struct SyrkProduct {
+  SyrkKind kind = SYRK_AUTO;
+  int n_pad = 0, num_sms = 0;
+  int64_t k_pad = 0;
+  int n_tiles = 0;  // lower tiles of P: of the FP64 tile size, or 128-tiles of the residue sums
+  // FP64 tiles
+  int n_items = 0;
+  SyrkItem* items = nullptr;  // [n_items] launch order
+  int* tile_first = nullptr;  // [n_tiles + 1]
+  int* tile_items = nullptr;  // partial-tile slots of each tile in ascending k order
+  double* part = nullptr;     // partial tiles, one per item (and one per tall item's ragged rows)
+  // INT8 emulation
+  int emu_bits = 0;                      // b: |scaled entry| <= 2^b, exact CRT lift for k_pad rows
+  int emu_n_items = 0;
+  int emu_n_ragged = 0;                  // the last items: those of a ragged last 256-row tile row
+  EmuItem* emu_items = nullptr;          // [emu_n_items] launch order
+  int8_t* Yq = nullptr;                  // [kEmuModuli][n_pad][k_pad] residue planes, K-major
+  uint32_t* Pmod = nullptr;              // [kEmuModuli][n_tiles][128 cols][128 rows] residue sums
+  unsigned long long* colmax = nullptr;  // [n_pad] max |Yt[k][a]| over k, to its exponent (K2b gathers it)
+};
+
 struct Comm;  // peer-memory exchange of a sharded run (comm_peer.cu)
 
 struct ProfSlot {
@@ -109,21 +139,8 @@ struct ba_engine {
   // reduced system layout: n_full = 9M unknown slots (gauge entries pinned, not deleted),
   // row rhs_row = 9M carries the right-hand side, n_pad = padded order = leading dimension
   int n_full = 0, rhs_row = 0, n_pad = 0;
-  int syrk_tile = 128;
-  int syrk_n_items = 0, syrk_n_tiles = 0;
-  ba::SyrkItem* syrk_items = nullptr;  // [syrk_n_items] launch order
-  int* syrk_tile_first = nullptr;      // [syrk_n_tiles + 1]
-  int* syrk_tile_items = nullptr;      // items of each tile in ascending k order
   int64_t k_pad = 0;  // padded 3N (rows of Yt)
-  // dense Schur product emulated on the INT8 tensor cores (k3_schur_syrk.cu): chosen at engine creation
-  int syrk_emu = 0;
-  int emu_bits = 0;                      // b: |scaled entry| <= 2^b, exact CRT lift for k_pad rows
-  int emu_n_items = 0;
-  int emu_n_full = 0;                    // items of whole 256-row tile rows; the ragged row's items follow
-  ba::EmuItem* emu_items = nullptr;      // [emu_n_items] launch order
-  int8_t* Yq = nullptr;                  // [kEmuModuli][n_pad][k_pad] residue planes, K-major
-  uint32_t* Pmod = nullptr;              // [kEmuModuli][lower 128-tiles][128 cols][128 rows] residue sums
-  unsigned long long* colmax = nullptr;  // [n_pad] max |Yt[k][a]| over k, to its exponent (K2b gathers it)
+  ba::SyrkProduct syrk;  // dense: the Schur product P = Yt^T Yt, chosen at engine creation
 
   // observations (CSR by point) and camera-major index
   int64_t* obs_ptr = nullptr;
@@ -164,7 +181,6 @@ struct ba_engine {
   int64_t red_len = 0;
   bool red_in_window = false;  // red lives in the exchange window (freed with it)
   ba::Comm* comm = nullptr;    // non-null: sharded run, sums go through peer memory
-  double* Spart = nullptr;  // partial tiles, one per work item of the Schur product
   double* Lt = nullptr;     // Cholesky block column, k-major copy [kCholOB][n_pad]
   double* ywork = nullptr;  // [n_pad] running right-hand side of the grid-wide back substitution
   unsigned int* chol_bar = nullptr;  // grid barrier counter of that kernel
@@ -408,21 +424,15 @@ int launch_camera_blocks(ba_engine* e, cudaStream_t s, bool conditional);
 int launch_k2b(ba_engine* e, bool conditional, double c_host, cudaStream_t s);
 bool dense_matrix_free(const ba_engine* e);  // dense K2b / point update re-derive the Jacobian rows
 int launch_k3(ba_engine* e, bool conditional, cudaStream_t s);
-int syrk_plan_engine(ba_engine* e);
+// The dense product: plan `kind` (SYRK_AUTO: chosen here) and allocate and upload on s, which is
+// synchronised; compute P [n_pad][n_pad] from Yt (skipped when ctl->done; with `prof`, timed in that
+// engine's "syrk" group); free everything on s.
+int syrk_prepare(SyrkProduct* p, SyrkKind kind, int n_pad, int64_t k_pad, int num_sms, cudaStream_t s);
+int syrk_launch(const SyrkProduct* p, const double* Yt, double* P, const ba_lm_state* ctl, cudaStream_t s,
+                ba_engine* prof);
+void syrk_release(SyrkProduct* p, cudaStream_t s);
 int syrk_emu_info(int64_t k_pad, int32_t* moduli, int* n_moduli, int* bits);
 int require_tensor_map_encoder();  // BA_ERR_CUDA when the driver lacks cuTensorMapEncodeTiled
-// Gram matrix P = Yt^T Yt of a k-major operand outside an engine (k3_schur_syrk.cu)
-struct GramWorkspace {
-  int n_pad = 0, num_sms = 0, n_items = 0, n_tiles = 0;
-  int64_t k_pad = 0;
-  SyrkItem* items = nullptr;
-  int* tile_first = nullptr;
-  int* tile_items = nullptr;
-  double* Spart = nullptr;
-};
-int gram_prepare(GramWorkspace* ws, int n_pad, int64_t k_pad, int num_sms, cudaStream_t s);
-int gram_launch(const GramWorkspace* ws, const double* Yt, double* P, cudaStream_t s);
-void gram_release(GramWorkspace* ws, cudaStream_t s);
 int syrk_plan_selftest(int n_cams, int64_t n_points, int tile, int num_sms, int* n_items, int* n_tiles,
                        double* makespan_rows, double* ideal_rows);
 int launch_assemble(ba_engine* e, bool conditional, double c_host, cudaStream_t s);

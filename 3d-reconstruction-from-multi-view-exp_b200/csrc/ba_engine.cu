@@ -276,10 +276,11 @@ static void free_engine(ba_engine* e) {
   comm_free(e);  // closes the peers' windows and frees this rank's (which holds red)
   void* ptrs[] = {e->obs_ptr, e->obs_cam, e->obs_pt, e->obs_xy, e->cam_ptr, e->cm_perm, e->bits, e->PT, e->pair_ptr, e->pair_pts, e->X[0],
                   e->X[1], e->cam[0].f, e->cam[1].f, e->camtab[0], e->camtab[1], e->JP, e->JC, e->V,
-                  e->GPT, e->Upart, e->Uloc, e->LINV, e->Z, e->Yt, e->Ysp, e->red_in_window ? nullptr : e->red, e->Spart, e->Lt, e->Winv,
-                  e->dxi, e->cost_part, e->cost_buf, e->ctl, e->rec, e->ywork, e->chol_bar, e->gauge, e->syrk_items, e->syrk_tile_first, e->syrk_tile_items, e->emu_items, e->Yq, e->Pmod, e->colmax};
+                  e->GPT, e->Upart, e->Uloc, e->LINV, e->Z, e->Yt, e->Ysp, e->red_in_window ? nullptr : e->red, e->Lt, e->Winv,
+                  e->dxi, e->cost_part, e->cost_buf, e->ctl, e->rec, e->ywork, e->chol_bar, e->gauge};
   for (void* p : ptrs)
     dev_free(p);
+  syrk_release(&e->syrk, (cudaStream_t)0);
   for (int k = 0; k < 2; ++k) {
     if (e->solve_graph[k]) cudaGraphExecDestroy(e->solve_graph[k]);
     if (e->solve_ev[k]) cudaEventDestroy(e->solve_ev[k]);
@@ -355,7 +356,6 @@ static int create_engine(const ba_problem* p, ba_engine** out) {
   e->n_full = 9 * e->M;
   e->rhs_row = e->n_full;
   const int n_aug = e->n_full + 1;
-  e->syrk_tile = n_aug <= 384 ? 64 : 128;  // C2 (n = 451): 128-tiles 0.283 ms vs 64-tiles 0.302 ms per iteration
   e->n_pad = round_up(n_aug, 8);  // fragment granularity; edge tiles of the SYRK are partial
   e->k_pad = round_up64(3 * e->N, 32);
   // camera_blocks_kernel: 3 blocks per SM (162 registers); ~8 waves of blocks so that the last,
@@ -404,7 +404,7 @@ static int create_engine(const ba_problem* p, ba_engine** out) {
   A(dev_alloc(&e->red, (size_t)e->red_len));
   if (e->dense) {
     A(dev_alloc(&e->Yt, (size_t)e->k_pad * e->n_pad));
-    A(syrk_plan_engine(e));
+    A(syrk_prepare(&e->syrk, SYRK_AUTO, e->n_pad, e->k_pad, e->num_sms, (cudaStream_t)0));
   } else {
     A(dev_alloc(&e->Ysp, (size_t)e->nobs * 27));
   }
@@ -943,6 +943,6 @@ int ba_syrk_plan_info(int n_cams, int64_t n_points, int tile, int num_sms, int* 
 int ba_syrk_emu_info(int64_t k_pad, int32_t* moduli, int* n_moduli, int* bits) {
   return syrk_emu_info(k_pad, moduli, n_moduli, bits);
 }
-int ba_syrk_emulated(ba_engine* e) { return e && e->dense && e->syrk_emu ? 1 : 0; }
+int ba_syrk_emulated(ba_engine* e) { return e && e->syrk.kind == SYRK_EMULATED ? 1 : 0; }
 
 }  // extern "C"

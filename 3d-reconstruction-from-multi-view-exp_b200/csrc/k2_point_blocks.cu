@@ -454,7 +454,7 @@ bool dense_matrix_free(const ba_engine* e) {
 int launch_k2b(ba_engine* e, bool conditional, double c_host, cudaStream_t s) {
   const int use_ctl = conditional ? 1 : 0;
   const bool mf = dense_matrix_free(e);
-  unsigned long long* colmax = e->dense && e->syrk_emu ? e->colmax : nullptr;
+  unsigned long long* colmax = e->syrk.colmax;  // null unless the dense product is emulated
   if (colmax) BA_CUDA(cudaMemsetAsync(colmax, 0, (size_t)e->n_pad * sizeof(unsigned long long), s));
   const size_t kStage = 8 * 864 * sizeof(double) + (mf ? tab_smem_doubles(e->M) * sizeof(double) : 0) +
                         (colmax ? ((size_t)e->n_pad * sizeof(unsigned short) + 15) / 16 * 16 : 0);

@@ -34,6 +34,7 @@
 #include <cstdlib>
 #include <functional>
 #include <mutex>
+#include <optional>
 #include <queue>
 #include <vector>
 
@@ -91,18 +92,24 @@ __device__ __forceinline__ void syrk_store_pair(double v0, double v1, int ti, in
   }
 }
 
+// 64-tiles: 2 x 2 warps, each owning a 32 x 32 sub-tile, KC k-rows per stage; four CTAs per SM.
+constexpr int kDmmaTile = 64, kDmmaWR = 2, kDmmaWC = 2, kDmmaKC = 16;
+constexpr int kDmmaThreads = kDmmaWR * kDmmaWC * 32;
+constexpr size_t kDmmaSmemBytes = (size_t)2 * kStages * kDmmaKC * (kDmmaTile + 4) * sizeof(double);
+
 // TILE x TILE output tile per CTA; WR x WC warps, each owning a (TILE/WR) x (TILE/WC) sub-tile.
 // SUB = false: the tile of this split is written to part[split][tile] (Schur product).
 // SUB = true:  one split; the tile is subtracted in place from the lower triangle of the n_store x
 //              n_store matrix `part` (leading dimension ld) -- the rank-k trailing update of the
 //              blocked Cholesky (k4_cholesky.cu), where Yt is the k-major copy of a block column.
-template <int TILE, int WR, int WC, int KC, bool SUB>
-__global__ void __launch_bounds__(WR* WC * 32)
+template <bool SUB>
+__global__ void __launch_bounds__(kDmmaThreads)
 syrk_dmma_kernel(const double* __restrict__ Yt, int ld, int n_valid, int64_t n_chunks,
                  const SyrkItem* __restrict__ items, double* __restrict__ part,
                  const ba_lm_state* ctl, int n_store, SubSplit sp) {
   if (ctl && ctl->done) return;
-  constexpr int NT = WR * WC * 32;
+  constexpr int TILE = kDmmaTile, WR = kDmmaWR, WC = kDmmaWC, KC = kDmmaKC;
+  constexpr int NT = kDmmaThreads;
   constexpr int LDS = TILE + 4;
   constexpr int WM = TILE / WR, WN = TILE / WC;
   constexpr int FM = WM / 8, FN = WN / 8;
@@ -983,16 +990,17 @@ emu_reconstruct_kernel(const uint32_t* __restrict__ Pmod, int n_tiles, const uns
 }
 
 // ---- host side --------------------------------------------------------------------------------
-static inline int syrk_kc(int tile) { return tile == 128 ? 32 : 16; }
-static inline int syrk_occupancy(int tile) { return tile == 128 ? 1 : 4; }
+static inline int syrk_kc(int tile) { return tile == kTmaTile ? kTmaKC : kDmmaKC; }
+static inline int syrk_occupancy(int tile) { return tile == kTmaTile ? 1 : 4; }
 
 // Relative duration of a tile per k-row (1 = full tile), mirroring the kernel's warp mapping:
 // edge tiles skip the 8x8 fragments beyond n_valid, diagonal tiles the sub-tiles above the
 // diagonal.  A warp sits on scheduler partition (warp % 4) with its own FP64 pipe: a CTA that has
 // an SM to itself takes as long as its busiest partition; with several CTAs per SM the partitions
 // even out and the mean counts.
-static double tile_weight(int TILE, int WR, int WC, int occ, int ti, int tj, int n_valid, int64_t k_pad = 0,
-                          double floor_override = -1.0) {
+static double tile_weight(int TILE, int ti, int tj, int n_valid, int64_t k_pad = 0, double floor_override = -1.0) {
+  const int WR = TILE == kTmaTile ? 4 : kDmmaWR, WC = TILE == kTmaTile ? 4 : kDmmaWC;  // syrk_tma_kernel: 4 x 4 warps
+  const int occ = syrk_occupancy(TILE);
   const int WM = TILE / WR, WN = TILE / WC, FM = WM / 8, FN = WN / 8;
   double load[4] = {0, 0, 0, 0};
   const bool folded_diag = ti == tj && TILE == kTmaTile;
@@ -1068,7 +1076,7 @@ static int tall_tile_row(int n_pad, int TILE) {
 // and the partial-tile write stay small against it), and -- L2 residency -- the k-slab that the
 // CTAs of one "column" of the schedule share should stay below 48 MB: ncu showed 18.6 GB of DRAM
 // reads for the 4.3 GB operand of C3 when 271 MB slabs were streamed by tiles drifting apart.
-static SyrkPlan plan_syrk(int n_pad, int TILE, int WR, int WC, int64_t k_pad, int num_sms) {
+static SyrkPlan plan_syrk(int n_pad, int TILE, int64_t k_pad, int num_sms) {
   const int KC = syrk_kc(TILE), occ = syrk_occupancy(TILE);
   const int nt1 = (n_pad + TILE - 1) / TILE;
   const int n_tiles = nt1 * (nt1 + 1) / 2;
@@ -1082,10 +1090,10 @@ static SyrkPlan plan_syrk(int n_pad, int TILE, int WR, int WC, int64_t k_pad, in
   std::vector<char> absorbed(n_tiles, 0), is_tall(n_tiles, 0);
   for (int t = 0, ti = 0; ti < nt1; ++ti)
     for (int tj = 0; tj <= ti; ++tj, ++t) {
-      w[t] = tile_weight(TILE, WR, WC, occ, ti, tj, n_pad, k_pad);
+      w[t] = tile_weight(TILE, ti, tj, n_pad, k_pad);
       // longest-first schedules are simulated with what a tile really costs (its fragments, down to
       // the rate of the TMA ring), not with the weight that decides the cuts
-      w_run[t] = lpt ? tile_weight(TILE, WR, WC, occ, ti, tj, n_pad, k_pad, run_floor) : w[t];
+      w_run[t] = lpt ? tile_weight(TILE, ti, tj, n_pad, k_pad, run_floor) : w[t];
       if (tall_row >= 0 && tj < tall_row) {
         if (ti == tall_row) { is_tall[t] = 1; w[t] *= 1.0 + 2.0 / 16.0; w_run[t] *= 1.0 + 2.0 / 16.0; }  // two more fragments per warp
         if (ti == nt1 - 1) absorbed[t] = 1;
@@ -1184,39 +1192,9 @@ static const SyrkPlan& cached_plan(int n_pad, int tile, int64_t k_pad, int num_s
   for (auto& kv : cache)
     if (kv.first.n_pad == n_pad && kv.first.tile == tile && kv.first.k_pad == k_pad && kv.first.sms == num_sms)
       return *kv.second;
-  SyrkPlan* p = new SyrkPlan(tile == 128 ? plan_syrk(n_pad, 128, 4, 4, k_pad, num_sms)
-                                         : plan_syrk(n_pad, 64, 2, 2, k_pad, num_sms));
+  SyrkPlan* p = new SyrkPlan(plan_syrk(n_pad, tile, k_pad, num_sms));
   cache.push_back({Key{n_pad, tile, k_pad, num_sms}, p});
   return *p;
-}
-
-// Plans the dense Schur product of this engine and uploads the work items.
-static int emu_plan_engine(ba_engine* e);
-int emu_bits_for(int64_t k_pad);
-static bool emu_select(const ba_engine* e);
-
-int syrk_plan_engine(ba_engine* e) {
-  if (!e->dense) return BA_OK;
-  e->emu_bits = emu_bits_for(e->k_pad);
-  e->syrk_emu = emu_select(e) ? 1 : 0;
-  if (e->syrk_emu) return emu_plan_engine(e);
-  const SyrkPlan& plan = cached_plan(e->n_pad, e->syrk_tile, e->k_pad, e->num_sms);
-  e->syrk_n_items = (int)plan.items.size();
-  const int nt1 = (e->n_pad + e->syrk_tile - 1) / e->syrk_tile;
-  e->syrk_n_tiles = nt1 * (nt1 + 1) / 2;
-  const size_t tt = (size_t)e->syrk_tile * e->syrk_tile;
-  BA_CUDA(cudaMallocAsync(reinterpret_cast<void**>(&e->syrk_items), plan.items.size() * sizeof(SyrkItem), (cudaStream_t)0));
-  BA_CUDA(cudaMallocAsync(reinterpret_cast<void**>(&e->syrk_tile_first), plan.tile_first.size() * sizeof(int), (cudaStream_t)0));
-  BA_CUDA(cudaMallocAsync(reinterpret_cast<void**>(&e->syrk_tile_items), plan.tile_items.size() * sizeof(int), (cudaStream_t)0));
-  BA_CUDA(cudaMallocAsync(reinterpret_cast<void**>(&e->Spart), (size_t)plan.n_slots * tt * sizeof(double), (cudaStream_t)0));
-  BA_CUDA(cudaMemcpy(e->syrk_items, plan.items.data(), plan.items.size() * sizeof(SyrkItem), cudaMemcpyHostToDevice));
-  BA_CUDA(cudaMemcpy(e->syrk_tile_first, plan.tile_first.data(), plan.tile_first.size() * sizeof(int), cudaMemcpyHostToDevice));
-  BA_CUDA(cudaMemcpy(e->syrk_tile_items, plan.tile_items.data(), plan.tile_items.size() * sizeof(int), cudaMemcpyHostToDevice));
-  if (std::getenv("BA_TIMING"))
-    std::fprintf(stderr, "[ba syrk plan] tile %d: %d tiles, %d items on %d slots, modelled %.0f k-rows (ideal %.0f)\n",
-                 e->syrk_tile, e->syrk_n_tiles, e->syrk_n_items, e->num_sms * syrk_occupancy(e->syrk_tile),
-                 plan.makespan, 0.0);
-  return BA_OK;
 }
 
 // ---- tensor maps (host) ---------------------------------------------------------------------------
@@ -1291,7 +1269,7 @@ static const EmuConsts& emu_consts() {
 
 // Largest b <= 53 with k_pad 2^(2b) < prod(p) / 2: the CRT lift of a dot product of k_pad terms of
 // magnitude <= 2^b each is then exact.  0 if there is none.
-int emu_bits_for(int64_t k_pad) {
+static int emu_bits_for(int64_t k_pad) {
   unsigned __int128 half = 1;
   for (int i = 0; i < kEmuModuli; ++i) half *= (unsigned)emu_modulus(i);
   half /= 2;
@@ -1300,9 +1278,6 @@ int emu_bits_for(int64_t k_pad) {
   return 0;
 }
 
-// The emulation is chosen when it is exact to (nearly) full FP64 input precision and the product is
-// large enough for the INT8 tensor cores to pay for the conversion passes.  BA_SYRK_EMU=0|1 overrides
-// the size rule (A/B timing and tests); it is read when an engine is created.
 int syrk_emu_info(int64_t k_pad, int32_t* moduli, int* n_moduli, int* bits) {
   if (k_pad < 1) { set_error("k_pad must be positive"); return BA_ERR_INVALID; }
   if (moduli)
@@ -1310,11 +1285,6 @@ int syrk_emu_info(int64_t k_pad, int32_t* moduli, int* n_moduli, int* bits) {
   if (n_moduli) *n_moduli = kEmuModuli;
   if (bits) *bits = emu_bits_for(k_pad);
   return BA_OK;
-}
-
-static bool emu_select(const ba_engine* e) {
-  if (const char* v = std::getenv("BA_SYRK_EMU")) return std::atoi(v) != 0;
-  return e->emu_bits >= 50 && (double)e->n_pad * e->n_pad * (double)e->k_pad >= kEmuMinWork;
 }
 
 // Work items: every (modulus, lower 256-tile) over P equal k pieces of <= kEmuMaxKB blocks, in two
@@ -1353,25 +1323,70 @@ static EmuPlan plan_emu(int n_pad, int64_t k_pad, int num_sms) {
   return {plan_emu_list(0, full_rows, nkb, num_sms), plan_emu_list(full_rows, nt1, nkb, num_sms)};
 }
 
-static int emu_plan_engine(ba_engine* e) {
-  const EmuPlan plan = plan_emu(e->n_pad, e->k_pad, e->num_sms);
-  std::vector<EmuItem> items = plan.full;
-  items.insert(items.end(), plan.ragged.begin(), plan.ragged.end());
-  const int nt1 = (e->n_pad + kEmuTile - 1) / kEmuTile;
-  e->syrk_n_tiles = nt1 * (nt1 + 1) / 2;
-  e->emu_n_items = (int)items.size();
-  e->emu_n_full = (int)plan.full.size();
-  const cudaStream_t s0 = (cudaStream_t)0;
-  BA_CUDA(cudaMallocAsync(reinterpret_cast<void**>(&e->emu_items), items.size() * sizeof(EmuItem), s0));
-  BA_CUDA(cudaMallocAsync(reinterpret_cast<void**>(&e->Yq), (size_t)kEmuModuli * e->n_pad * e->k_pad, s0));
-  BA_CUDA(cudaMallocAsync(reinterpret_cast<void**>(&e->Pmod),
-                          (size_t)kEmuModuli * e->syrk_n_tiles * kEmuTile * kEmuTile * sizeof(uint32_t), s0));
-  BA_CUDA(cudaMallocAsync(reinterpret_cast<void**>(&e->colmax), (size_t)e->n_pad * sizeof(unsigned long long), s0));
-  BA_CUDA(cudaMemcpy(e->emu_items, items.data(), items.size() * sizeof(EmuItem), cudaMemcpyHostToDevice));
-  if (std::getenv("BA_TIMING"))
-    std::fprintf(stderr, "[ba syrk plan] int8 emulation: b = %d, %d tiles x %d moduli, %d items\n", e->emu_bits,
-                 e->syrk_n_tiles, kEmuModuli, e->emu_n_items);
+// ---- the planned product: choice, upload, launch ---------------------------------------------------
+template <typename T>
+static int dev_upload(T** dst, const std::vector<T>& src, cudaStream_t s) {
+  BA_CUDA(cudaMallocAsync(reinterpret_cast<void**>(dst), src.size() * sizeof(T), s));
+  BA_CUDA(cudaMemcpyAsync(*dst, src.data(), src.size() * sizeof(T), cudaMemcpyHostToDevice, s));
   return BA_OK;
+}
+
+int syrk_prepare(SyrkProduct* p, SyrkKind kind, int n_pad, int64_t k_pad, int num_sms, cudaStream_t s) {
+  *p = SyrkProduct();
+  p->n_pad = n_pad;
+  p->k_pad = k_pad;
+  p->num_sms = num_sms;
+  p->emu_bits = emu_bits_for(k_pad);
+  if (kind == SYRK_AUTO) {
+    // The emulation is chosen when it is exact to (nearly) full FP64 input precision and the product
+    // is large enough for the INT8 tensor cores to pay for the conversion passes; BA_SYRK_EMU=0|1
+    // overrides the size rule (A/B timing and tests).  FP64 64-tiles up to n_pad = 384 (C2, n = 451:
+    // 128-tiles 0.283 ms vs 64-tiles 0.302 ms per iteration).
+    const char* v = std::getenv("BA_SYRK_EMU");
+    const bool emu = v ? std::atoi(v) != 0 : p->emu_bits >= 50 && (double)n_pad * n_pad * (double)k_pad >= kEmuMinWork;
+    kind = emu ? SYRK_EMULATED : n_pad <= 384 ? SYRK_TILE64 : SYRK_TILE128;
+  }
+  p->kind = kind;
+  const bool timing = std::getenv("BA_TIMING") != nullptr;
+  if (kind == SYRK_EMULATED) {
+    const EmuPlan plan = plan_emu(n_pad, k_pad, num_sms);
+    std::vector<EmuItem> items = plan.full;
+    items.insert(items.end(), plan.ragged.begin(), plan.ragged.end());
+    const int nt1 = (n_pad + kEmuTile - 1) / kEmuTile;
+    p->n_tiles = nt1 * (nt1 + 1) / 2;
+    p->emu_n_items = (int)items.size();
+    p->emu_n_ragged = (int)plan.ragged.size();
+    BA_TRY(dev_upload(&p->emu_items, items, s));
+    BA_CUDA(cudaMallocAsync(reinterpret_cast<void**>(&p->Yq), (size_t)kEmuModuli * n_pad * k_pad, s));
+    BA_CUDA(cudaMallocAsync(reinterpret_cast<void**>(&p->Pmod),
+                            (size_t)kEmuModuli * p->n_tiles * kEmuTile * kEmuTile * sizeof(uint32_t), s));
+    BA_CUDA(cudaMallocAsync(reinterpret_cast<void**>(&p->colmax), (size_t)n_pad * sizeof(unsigned long long), s));
+    if (timing)
+      std::fprintf(stderr, "[ba syrk plan] int8 emulation: b = %d, %d tiles x %d moduli, %d items\n", p->emu_bits,
+                   p->n_tiles, kEmuModuli, p->emu_n_items);
+  } else {
+    const int tile = kind == SYRK_TILE128 ? kTmaTile : kDmmaTile;
+    const SyrkPlan& plan = cached_plan(n_pad, tile, k_pad, num_sms);
+    const int nt1 = (n_pad + tile - 1) / tile;
+    p->n_tiles = nt1 * (nt1 + 1) / 2;
+    p->n_items = (int)plan.items.size();
+    BA_TRY(dev_upload(&p->items, plan.items, s));
+    BA_TRY(dev_upload(&p->tile_first, plan.tile_first, s));
+    BA_TRY(dev_upload(&p->tile_items, plan.tile_items, s));
+    BA_CUDA(cudaMallocAsync(reinterpret_cast<void**>(&p->part), (size_t)plan.n_slots * tile * tile * sizeof(double), s));
+    if (timing)
+      std::fprintf(stderr, "[ba syrk plan] tile %d: %d tiles, %d items on %d slots, modelled %.0f k-rows (ideal %.0f)\n",
+                   tile, p->n_tiles, p->n_items, num_sms * syrk_occupancy(tile), plan.makespan, 0.0);
+  }
+  BA_CUDA(cudaStreamSynchronize(s));  // allocated and filled on s, used on whatever stream launches the product
+  return BA_OK;
+}
+
+void syrk_release(SyrkProduct* p, cudaStream_t s) {
+  void* ptrs[] = {p->items, p->tile_first, p->tile_items, p->part, p->emu_items, p->Yq, p->Pmod, p->colmax};
+  for (void* q : ptrs)
+    if (q) cudaFreeAsync(q, s);
+  *p = SyrkProduct();
 }
 
 // The residue planes as one 3D tensor {k, row, plane} of bytes; boxes of 128 k x 128 rows of one plane
@@ -1394,94 +1409,105 @@ static int make_plane_map(CUtensorMap* map, const int8_t* Yq, int n_pad, int64_t
   return BA_OK;
 }
 
-static int launch_syrk_emu(ba_engine* e, const ba_lm_state* ctl, cudaStream_t s) {
+// Emulated product: residue planes of Yt, one int8 SYRK per modulus into the residue sums, P from them.
+static int launch_emulated(const SyrkProduct* p, const double* Yt, double* P, const ba_lm_state* ctl, cudaStream_t s,
+                           ba_engine* prof) {
   CUtensorMap map;
-  BA_TRY(make_plane_map(&map, e->Yq, e->n_pad, e->k_pad));
+  BA_TRY(make_plane_map(&map, p->Yq, p->n_pad, p->k_pad));
   BA_CUDA(cudaFuncSetAttribute(syrk_i8_pair_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kEmuSmemBytes));
   BA_CUDA(cudaFuncSetAttribute(syrk_i8_pair_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kEmuSmemBytes));
-  const int n_tiles = e->syrk_n_tiles;
-  ProfScope ps(e, PG_SYRK, s);
+  const int n_tiles = p->n_tiles;
+  std::optional<ProfScope> ps;
+  if (prof) ps.emplace(prof, PG_SYRK, s);
   // colmax was gathered by K2b (launch_k2b resets it before every launch)
-  BA_CUDA(cudaMemsetAsync(e->Pmod, 0, (size_t)kEmuModuli * n_tiles * kEmuTile * kEmuTile * sizeof(uint32_t), s));
+  BA_CUDA(cudaMemsetAsync(p->Pmod, 0, (size_t)kEmuModuli * n_tiles * kEmuTile * kEmuTile * sizeof(uint32_t), s));
   {
-    const int64_t k_tiles = (e->k_pad + kResTK - 1) / kResTK;
-    emu_residue_kernel<<<dim3((e->n_pad + kResTA - 1) / kResTA, (unsigned)std::min<int64_t>(k_tiles, 65535)),
-                         kResThreads, 0, s>>>(e->Yt, e->k_pad, e->n_pad, e->colmax, e->emu_bits, e->Yq, ctl);
+    const int64_t k_tiles = (p->k_pad + kResTK - 1) / kResTK;
+    emu_residue_kernel<<<dim3((p->n_pad + kResTA - 1) / kResTA, (unsigned)std::min<int64_t>(k_tiles, 65535)),
+                         kResThreads, 0, s>>>(Yt, p->k_pad, p->n_pad, p->colmax, p->emu_bits, p->Yq, ctl);
     BA_LAUNCH_CHECK();
   }
-  if (e->emu_n_full > 0) {
-    syrk_i8_pair_kernel<false><<<2 * e->emu_n_full, kEmuThreads, kEmuSmemBytes, s>>>(map, e->emu_items, e->Pmod,
-                                                                                     n_tiles, e->n_pad, ctl);
+  const int n_full = p->emu_n_items - p->emu_n_ragged;
+  if (n_full > 0) {
+    syrk_i8_pair_kernel<false><<<2 * n_full, kEmuThreads, kEmuSmemBytes, s>>>(map, p->emu_items, p->Pmod, n_tiles,
+                                                                              p->n_pad, ctl);
     BA_LAUNCH_CHECK();
   }
-  if (e->emu_n_items > e->emu_n_full) {
-    syrk_i8_pair_kernel<true><<<2 * (e->emu_n_items - e->emu_n_full), kEmuThreads, kEmuSmemBytes, s>>>(
-        map, e->emu_items + e->emu_n_full, e->Pmod, n_tiles, e->n_pad, ctl);
+  if (p->emu_n_ragged > 0) {
+    syrk_i8_pair_kernel<true><<<2 * p->emu_n_ragged, kEmuThreads, kEmuSmemBytes, s>>>(
+        map, p->emu_items + n_full, p->Pmod, n_tiles, p->n_pad, ctl);
     BA_LAUNCH_CHECK();
   }
-  emu_reconstruct_kernel<<<dim3(n_tiles, 16), 256, 0, s>>>(e->Pmod, n_tiles, e->colmax, e->emu_bits, e->P(), e->n_pad,
-                                                          e->n_pad, emu_consts(), ctl);
+  emu_reconstruct_kernel<<<dim3(n_tiles, 16), 256, 0, s>>>(p->Pmod, n_tiles, p->colmax, p->emu_bits, P, p->n_pad,
+                                                          p->n_pad, emu_consts(), ctl);
   BA_LAUNCH_CHECK();
   return BA_OK;
 }
 
-template <int TILE, int WR, int WC, int KC>
-static int launch_syrk(ba_engine* e, const ba_lm_state* ctl, cudaStream_t s) {
-  const int64_t n_chunks = e->k_pad / KC;
-  if constexpr (TILE == kTmaTile) {
-    static_assert(KC == kTmaKC, "the 128-tile product runs on the TMA kernel");
-    CUtensorMap mapA, mapB;
-    BA_TRY(make_operand_map(&mapA, e->Yt, e->n_pad, e->k_pad, e->n_pad, kTmaLda));
-    BA_TRY(make_operand_map(&mapB, e->Yt, e->n_pad, e->k_pad, e->n_pad, kTmaLdb));
+int syrk_launch(const SyrkProduct* p, const double* Yt, double* P, const ba_lm_state* ctl, cudaStream_t s,
+                ba_engine* prof) {
+  if (p->kind == SYRK_EMULATED) return launch_emulated(p, Yt, P, ctl, s, prof);
+  const bool tma = p->kind == SYRK_TILE128;
+  const int tile = tma ? kTmaTile : kDmmaTile;
+  const int64_t n_chunks = p->k_pad / syrk_kc(tile);
+  const SubSplit none{0, 1, 0, 0, {}};
+  CUtensorMap mapA, mapB;
+  if (tma) {
+    BA_TRY(make_operand_map(&mapA, Yt, p->n_pad, p->k_pad, p->n_pad, kTmaLda));
+    BA_TRY(make_operand_map(&mapB, Yt, p->n_pad, p->k_pad, p->n_pad, kTmaLdb));
     BA_CUDA(cudaFuncSetAttribute(syrk_tma_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                  (int)kTmaSmemBytes));
-    ProfScope ps(e, PG_SYRK, s);
-    syrk_tma_kernel<false><<<e->syrk_n_items, kTmaThreads, kTmaSmemBytes, s>>>(
-        mapA, mapB, e->n_pad, e->n_pad, n_chunks, e->syrk_items, e->Spart, ctl, 0, SubSplit{0, 1, 0, 0, {}});
-    BA_LAUNCH_CHECK();
   } else {
-    const size_t smem = (size_t)2 * kStages * KC * (TILE + 4) * sizeof(double);
-    BA_CUDA(cudaFuncSetAttribute(syrk_dmma_kernel<TILE, WR, WC, KC, false>,
-                                 cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    ProfScope ps(e, PG_SYRK, s);
-    syrk_dmma_kernel<TILE, WR, WC, KC, false><<<e->syrk_n_items, WR * WC * 32, smem, s>>>(
-        e->Yt, e->n_pad, e->n_pad, n_chunks, e->syrk_items, e->Spart, ctl, 0, SubSplit{0, 1, 0, 0, {}});
-    BA_LAUNCH_CHECK();
+    BA_CUDA(cudaFuncSetAttribute(syrk_dmma_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                 (int)kDmmaSmemBytes));
   }
-  const int n_tiles = e->syrk_n_tiles;
+  std::optional<ProfScope> ps;  // the "syrk" scope: the tile kernel, not the sums of its partial tiles
+  if (prof) ps.emplace(prof, PG_SYRK, s);
+  if (tma)
+    syrk_tma_kernel<false><<<p->n_items, kTmaThreads, kTmaSmemBytes, s>>>(mapA, mapB, p->n_pad, p->n_pad, n_chunks,
+                                                                          p->items, p->part, ctl, 0, none);
+  else
+    syrk_dmma_kernel<false><<<p->n_items, kDmmaThreads, kDmmaSmemBytes, s>>>(Yt, p->n_pad, p->n_pad, n_chunks,
+                                                                             p->items, p->part, ctl, 0, none);
+  BA_LAUNCH_CHECK();
+  ps.reset();
   // enough blocks to fill the GPU (C2: 10 tiles x 8 slabs = 80 blocks took 33 us for 38 MB), at
   // least one pair of doubles per thread
-  const int slabs_max = TILE * TILE / 2 / 256;
+  const int slabs_max = tile * tile / 2 / 256;
   int slabs = 1;
-  while (slabs < slabs_max && n_tiles * slabs < 4 * e->num_sms) slabs *= 2;
-  syrk_reduce_kernel<TILE><<<dim3(n_tiles, slabs), 256, 0, s>>>(e->Spart, e->syrk_tile_first,
-                                                               e->syrk_tile_items, e->P(), e->n_pad,
-                                                               e->n_pad, ctl);
+  while (slabs < slabs_max && p->n_tiles * slabs < 4 * p->num_sms) slabs *= 2;
+  const dim3 grid(p->n_tiles, slabs);
+  if (tma)
+    syrk_reduce_kernel<kTmaTile><<<grid, 256, 0, s>>>(p->part, p->tile_first, p->tile_items, P, p->n_pad, p->n_pad, ctl);
+  else
+    syrk_reduce_kernel<kDmmaTile><<<grid, 256, 0, s>>>(p->part, p->tile_first, p->tile_items, P, p->n_pad, p->n_pad, ctl);
   BA_LAUNCH_CHECK();
   return BA_OK;
 }
 
 // S[t0:, t0:] -= Lt[:, t0:]^T Lt[:, t0:]  (lower triangle, rows < n_rows) with Lt k-major
-// [depth][ld]: the wide trailing update of the two-level blocked Cholesky.
-template <int TILE, int WR, int WC, int KC>
-static int launch_syrk_sub(double* S, int ld, int n_rows, int t0, const double* Lt, int depth,
-                           const ba_lm_state* ctl, cudaStream_t s, const CholSplit* split) {
+// [depth][ld]: the wide trailing update of the two-level blocked Cholesky.  128-tiles (one CTA per
+// SM) once there are enough of them, 64-tiles (four per SM) below.  Only the 128-tile form is
+// divided over the ranks of a sharded run.
+int launch_chol_wide_update(double* S, int ld, int n_rows, int t0, const double* Lt, int depth,
+                            const ba_lm_state* ctl, cudaStream_t s, const CholSplit* split) {
+  const bool tma = n_rows - t0 >= kCholSplitMinRows;
+  const int tile = tma ? kTmaTile : kDmmaTile;
   const int n_store = n_rows - t0;
   const int n_valid = (n_store + 7) / 8 * 8;  // <= ld - t0: ld is a multiple of 8, t0 of 64
-  const int nt1 = (n_valid + TILE - 1) / TILE;
+  const int nt1 = (n_valid + tile - 1) / tile;
   const int n_tiles = nt1 * (nt1 + 1) / 2;
-  const int n_chunks = depth / KC;
+  const int n_chunks = depth / syrk_kc(tile);
   const size_t origin = (size_t)t0 * ld + t0;
   SubSplit sp{0, 1, 0, 0, {}};
-  if (split && split->world > 1) {
+  if (tma && split && split->world > 1) {
     sp.rank = split->rank;
     sp.world = split->world;
-    sp.tile_row0 = t0 / TILE;
+    sp.tile_row0 = t0 / tile;
     sp.push_cols = split->push_cols;
     for (int q = 0; q < split->world; ++q) sp.peer[q] = split->S_peer[q] + origin;
   }
-  if constexpr (TILE == kTmaTile) {
-    static_assert(KC == kTmaKC, "the 128-tile update runs on the TMA kernel");
+  if (tma) {
     CUtensorMap mapA, mapB;
     BA_TRY(make_operand_map(&mapA, Lt + t0, n_valid, depth, ld, kTmaLda));
     BA_TRY(make_operand_map(&mapB, Lt + t0, n_valid, depth, ld, kTmaLdb));
@@ -1490,23 +1516,13 @@ static int launch_syrk_sub(double* S, int ld, int n_rows, int t0, const double* 
     syrk_tma_kernel<true><<<n_tiles, kTmaThreads, kTmaSmemBytes, s>>>(mapA, mapB, ld, n_valid, n_chunks, nullptr,
                                                                       S + origin, ctl, n_store, sp);
   } else {
-    const size_t smem = (size_t)2 * kStages * KC * (TILE + 4) * sizeof(double);
-    BA_CUDA(cudaFuncSetAttribute(syrk_dmma_kernel<TILE, WR, WC, KC, true>,
-                                 cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    syrk_dmma_kernel<TILE, WR, WC, KC, true><<<n_tiles, WR * WC * 32, smem, s>>>(
-        Lt + t0, ld, n_valid, n_chunks, nullptr, S + origin, ctl, n_store, sp);
+    BA_CUDA(cudaFuncSetAttribute(syrk_dmma_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                 (int)kDmmaSmemBytes));
+    syrk_dmma_kernel<true><<<n_tiles, kDmmaThreads, kDmmaSmemBytes, s>>>(Lt + t0, ld, n_valid, n_chunks, nullptr,
+                                                                         S + origin, ctl, n_store, sp);
   }
   BA_LAUNCH_CHECK();
   return BA_OK;
-}
-
-// 128-tiles (one CTA per SM) once there are enough of them, 64-tiles (four per SM) below.  Only
-// the 128-tile form is divided over the ranks of a sharded run.
-int launch_chol_wide_update(double* S, int ld, int n_rows, int t0, const double* Lt, int depth,
-                            const ba_lm_state* ctl, cudaStream_t s, const CholSplit* split) {
-  if (n_rows - t0 >= kCholSplitMinRows)
-    return launch_syrk_sub<128, 4, 4, 32>(S, ld, n_rows, t0, Lt, depth, ctl, s, split);
-  return launch_syrk_sub<64, 2, 2, 16>(S, ld, n_rows, t0, Lt, depth, ctl, s, nullptr);
 }
 
 int launch_k3(ba_engine* e, bool conditional, cudaStream_t s) {
@@ -1516,58 +1532,8 @@ int launch_k3(ba_engine* e, bool conditional, cudaStream_t s) {
     stage_camera_blocks_kernel<<<(n + 255) / 256, 256, 0, s>>>(n, e->Uloc, e->U(), ctl);
     BA_LAUNCH_CHECK();
   }
-  if (e->dense) {
-    if (e->syrk_emu) return launch_syrk_emu(e, ctl, s);
-    if (e->syrk_tile == 128) return launch_syrk<128, 4, 4, 32>(e, ctl, s);
-    return launch_syrk<64, 2, 2, 16>(e, ctl, s);
-  }
+  if (e->dense) return syrk_launch(&e->syrk, e->Yt, e->P(), ctl, s, e);
   return launch_schur_sparse(e, ctl, s);
-}
-
-// ---- Gram matrix of an arbitrary k-major operand (used by the projective-depth iteration) --------
-// P = Yt^T Yt (lower triangle incl. the diagonal pairs) for Yt [k_pad][n_pad], with the 64-tile
-// kernel and the same planner as the Schur product.
-int gram_prepare(GramWorkspace* ws, int n_pad, int64_t k_pad, int num_sms, cudaStream_t s) {
-  *ws = GramWorkspace();
-  const SyrkPlan& plan = cached_plan(n_pad, 64, k_pad, num_sms);
-  ws->n_pad = n_pad;
-  ws->k_pad = k_pad;
-  ws->num_sms = num_sms;
-  ws->n_items = (int)plan.items.size();
-  const int nt1 = (n_pad + 63) / 64;
-  ws->n_tiles = nt1 * (nt1 + 1) / 2;
-  BA_CUDA(cudaMallocAsync(reinterpret_cast<void**>(&ws->items), plan.items.size() * sizeof(SyrkItem), s));
-  BA_CUDA(cudaMallocAsync(reinterpret_cast<void**>(&ws->tile_first), plan.tile_first.size() * sizeof(int), s));
-  BA_CUDA(cudaMallocAsync(reinterpret_cast<void**>(&ws->tile_items), plan.tile_items.size() * sizeof(int), s));
-  BA_CUDA(cudaMallocAsync(reinterpret_cast<void**>(&ws->Spart), plan.items.size() * (size_t)64 * 64 * sizeof(double), s));
-  BA_CUDA(cudaMemcpyAsync(ws->items, plan.items.data(), plan.items.size() * sizeof(SyrkItem), cudaMemcpyHostToDevice, s));
-  BA_CUDA(cudaMemcpyAsync(ws->tile_first, plan.tile_first.data(), plan.tile_first.size() * sizeof(int), cudaMemcpyHostToDevice, s));
-  BA_CUDA(cudaMemcpyAsync(ws->tile_items, plan.tile_items.data(), plan.tile_items.size() * sizeof(int), cudaMemcpyHostToDevice, s));
-  BA_CUDA(cudaStreamSynchronize(s));  // the plan's host vectors are cached, but keep the copies simple
-  return BA_OK;
-}
-
-int gram_launch(const GramWorkspace* ws, const double* Yt, double* P, cudaStream_t s) {
-  constexpr int TILE = 64, KC = 16;
-  const size_t smem = (size_t)2 * kStages * KC * (TILE + 4) * sizeof(double);
-  BA_CUDA(cudaFuncSetAttribute(syrk_dmma_kernel<TILE, 2, 2, KC, false>,
-                               cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-  syrk_dmma_kernel<TILE, 2, 2, KC, false><<<ws->n_items, 128, smem, s>>>(
-      Yt, ws->n_pad, ws->n_pad, ws->k_pad / KC, ws->items, ws->Spart, nullptr, 0, SubSplit{0, 1, 0, 0, {}});
-  BA_LAUNCH_CHECK();
-  int slabs = 1;
-  while (slabs < TILE * TILE / 2 / 256 && ws->n_tiles * slabs < 4 * ws->num_sms) slabs *= 2;
-  syrk_reduce_kernel<TILE><<<dim3(ws->n_tiles, slabs), 256, 0, s>>>(ws->Spart, ws->tile_first, ws->tile_items, P,
-                                                                  ws->n_pad, ws->n_pad, nullptr);
-  BA_LAUNCH_CHECK();
-  return BA_OK;
-}
-
-void gram_release(GramWorkspace* ws, cudaStream_t s) {
-  void* ptrs[] = {ws->items, ws->tile_first, ws->tile_items, ws->Spart};
-  for (void* p : ptrs)
-    if (p) cudaFreeAsync(p, s);
-  *ws = GramWorkspace();
 }
 
 // Host-only check of the planner (no device needed): every tile's pieces must tile [0, n_chunks)
@@ -1614,7 +1580,7 @@ int syrk_plan_selftest(int n_cams, int64_t n_points, int tile, int num_sms, int*
     if (pos != n_chunks) { set_error("plan: tile %d ends at chunk %lld of %lld", t, (long long)pos, (long long)n_chunks); return BA_ERR_STATE; }
     int ti = 0;
     while ((ti + 1) * (ti + 2) / 2 <= t) ++ti;
-    work += tile_weight(tile, tile == 128 ? 4 : 2, tile == 128 ? 4 : 2, syrk_occupancy(tile), ti, t - ti * (ti + 1) / 2, n_pad, k_pad) * (double)k_pad;
+    work += tile_weight(tile, ti, t - ti * (ti + 1) / 2, n_pad, k_pad) * (double)k_pad;
   }
   if (n_items) *n_items = (int)plan.items.size();
   if (n_tiles) *n_tiles = nt;

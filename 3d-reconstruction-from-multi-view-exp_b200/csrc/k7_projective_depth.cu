@@ -930,11 +930,11 @@ static int check_launches(const char* what) {
 // What the two depth methods and the factorisation share: the device, the k-major operand Wk
 // [k_pad][ld] (one row per point, n entries used), its Gram matrix and leading eigenspace, the input
 // (x or W) staged on the device and the output (z or S).  Every buffer is in `bufs` and the Gram
-// workspace is released by the destructor, so every exit path frees everything.
+// product is released by the destructor, so every exit path frees everything.
 struct DepthCall {
   cudaStream_t s;
   DevBufs bufs;
-  GramWorkspace ws;
+  SyrkProduct gram;  // FP64 64-tiles
   int num_sms = 0, n = 0, ld = 0, grid = 0, mem = BA_MEM_HOST;
   int64_t N = 0, k_pad = 0;
   bool force_jacobi = false;
@@ -945,7 +945,7 @@ struct DepthCall {
   int* status = nullptr;
 
   explicit DepthCall(void* stream) : s((cudaStream_t)stream), bufs(s) {}
-  ~DepthCall() { gram_release(&ws, s); }
+  ~DepthCall() { syrk_release(&gram, s); }
 
   // `args_ok` and `usage`: the entry point's own argument rule and its message.  Wk gets N_ rows (points,
   // or columns of W) of n_ entries; in / out hold in_count / out_count doubles, on the device with
@@ -992,13 +992,13 @@ struct DepthCall {
     BA_CUDA(cudaMemsetAsync(Wk, 0, (size_t)k_pad * ld * sizeof(double), s));
     BA_CUDA(cudaMemsetAsync(P, 0, (size_t)ld * ld * sizeof(double), s));
     BA_CUDA(cudaMemsetAsync(status, 0, sizeof(int), s));
-    return gram_prepare(&ws, ld, k_pad, num_sms, s);
+    return syrk_prepare(&gram, SYRK_TILE64, ld, k_pad, num_sms, s);
   }
 
   // U4 = a basis of the leading four-dimensional eigenspace of G = Wk^T Wk, which stays intact: the
   // subspace iteration (warm-started from U4), then the Jacobi solver if that did not converge.
   int leading_subspace(bool warm) {
-    BA_TRY(gram_launch(&ws, Wk, P, s));
+    BA_TRY(syrk_launch(&gram, Wk, P, nullptr, s, nullptr));
     gram_symmetrize_kernel<<<(n * n + 255) / 256, 256, 0, s>>>(n, ld, P, G);
     if (!force_jacobi)
       subspace_eig_kernel<<<1, 256, (size_t)8 * n * sizeof(double), s>>>(n, G, U4, warm ? 1 : 0, 2000, status);

@@ -71,7 +71,7 @@ def main():
         if "syrk_i8_pair_kernel" in name:  # two instances: whole tile rows, and the ragged last tile row
             k = "syrk_i8_pair_kernel<ragged>" if "<true>" in name else "syrk_i8_pair_kernel<full>"
             ms[k] = ms.get(k, 0.0) + ev.device_time_total / 1e3 / args.reps
-        for k in ("emu_colmax_kernel", "emu_residue_kernel", "emu_reconstruct_kernel", "k2b_point_solve_kernel"):
+        for k in ("emu_residue_kernel", "emu_reconstruct_kernel", "k2b_point_solve_kernel"):
             if k in name:
                 ms[k] = ms.get(k, 0.0) + ev.device_time_total / 1e3 / args.reps
         if "emset" in name:
@@ -95,7 +95,7 @@ def main():
         l2_GB["ragged"] = nt2 * (2 * 16384.0 + 2 * 128.0 * min(left, 128)) * kb * len(moduli) / 1e9
     ki = {"full": "syrk_i8_pair_kernel<full>", "ragged": "syrk_i8_pair_kernel<ragged>"}
     conv_bytes = 8.0 * k_pad * n_pad + len(moduli) * float(n_pad) * k_pad
-    conv_ms = ms.get("emu_colmax_kernel", 0) + ms.get("emu_residue_kernel", 0)
+    conv_ms = ms.get("emu_residue_kernel", 0)
     k2b_ms = ms.pop("k2b_point_solve_kernel", None)
     res = {
         "scene": f"{args.cams} x {args.points}", "n_pad": n_pad, "k_pad": k_pad, "bits": bits, "moduli": len(moduli),
