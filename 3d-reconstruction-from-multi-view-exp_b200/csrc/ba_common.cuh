@@ -111,6 +111,24 @@ struct SyrkProduct {
   unsigned long long* colmax = nullptr;  // [n_pad] max |Yt[k][a]| over k, to its exponent (K2b gathers it)
 };
 
+// The camera-pair half of the sparse Schur product (k3_schur_sparse.cu): which pair kernel runs and the
+// device memory it reads.  List engines hold one.
+enum PairKind {
+  PAIRS_LISTS,  // schur_pairs_reg_kernel: the static lists of the points every camera pair shares
+  PAIRS_SCAN,   // schur_pairs_kernel: scans the bitmaps (the lists would not fit, or BA_PAIRS_NO_LIST)
+};
+struct PairProduct {
+  PairKind kind = PAIRS_SCAN;
+  int M = 0;
+  int64_t N = 0;
+  int64_t n_items = 0;          // pair items: one block of a pair kernel each (whole tiles of camera pairs)
+  int64_t Wp = 0;               // words per camera bitmap, padded to a multiple of 256
+  uint32_t* bits = nullptr;     // [M][Wp] per camera: bitmap over points
+  double* PT = nullptr;         // [N][kPT] point table (X, damped V^-1), written by K2b
+  int64_t* pair_ptr = nullptr;  // [n_items + 1] (lists only)
+  int32_t* pair_pts = nullptr;  // ascending point ids of each pair item's common points (lists only)
+};
+
 struct Comm;  // peer-memory exchange of a sharded run (comm_peer.cu)
 
 struct ProfSlot {
@@ -140,7 +158,8 @@ struct ba_engine {
   // row rhs_row = 9M carries the right-hand side, n_pad = padded order = leading dimension
   int n_full = 0, rhs_row = 0, n_pad = 0;
   int64_t k_pad = 0;  // padded 3N (rows of Yt)
-  ba::SyrkProduct syrk;  // dense: the Schur product P = Yt^T Yt, chosen at engine creation
+  ba::SyrkProduct syrk;   // dense: the Schur product P = Yt^T Yt, chosen at engine creation
+  ba::PairProduct pairs;  // sparse: the camera-pair blocks of P, indexed with the observations
 
   // observations (CSR by point) and camera-major index
   int64_t* obs_ptr = nullptr;
@@ -149,8 +168,6 @@ struct ba_engine {
   double* obs_xy = nullptr;
   int64_t* cam_ptr = nullptr;  // [M+1] (sparse)
   int32_t* cm_perm = nullptr;  // [nobs] observation ids sorted by camera (sparse)
-  uint32_t* bits = nullptr;    // [M][Wp] per camera: bitmap over points (sparse)
-  int64_t Wp = 0;              // words per camera bitmap, padded to a multiple of 256
   bool have_obs = false, have_state = false;
 
   // state: [0] current, [1] trial
@@ -170,13 +187,6 @@ struct ba_engine {
   double *LINV = nullptr, *Z = nullptr;
   double* Yt = nullptr;   // dense: [k_pad][n_pad]
   double* Ysp = nullptr;  // sparse: [nobs][27]
-  double* PT = nullptr;   // sparse: [N][kPT] point table of the pair kernel (X, damped V^-1)
-  // sparse: the common points of every camera pair, compacted once per engine (visibility does not
-  // change between iterations): pair_ptr [n_pair_items + 1], pair_pts [pair_total] ascending point ids;
-  // null when the lists would not fit the memory budget (the pair kernel then scans the bitmaps)
-  int64_t* pair_ptr = nullptr;
-  int32_t* pair_pts = nullptr;
-  int64_t pair_total = 0;
   double* red = nullptr;  // [n_pad*n_pad | M*81 | M*9]
   int64_t red_len = 0;
   bool red_in_window = false;  // red lives in the exchange window (freed with it)
@@ -455,7 +465,16 @@ int launch_decide(ba_engine* e, cudaStream_t s);
 int launch_lm_begin(ba_engine* e, double scale, double tol, int max_iter, int max_retries,
                     cudaStream_t s);
 int build_camera_major_index(ba_engine* e, cudaStream_t s);
-int build_pair_index(ba_engine* e, cudaStream_t s);
+// The camera-pair product: size it for M cameras and N points and allocate the bitmaps and the point
+// table on s (BA_ERR_INVALID past the launch limit on pair items); index the observations into the
+// bitmaps and, memory permitting, the pair lists (replacing those of an earlier call); compute the
+// off-diagonal blocks of P (skipped when ctl->done); free everything on s.
+int pairs_prepare(PairProduct* p, int M, int64_t N, cudaStream_t s);
+int pairs_index(PairProduct* p, int64_t nobs, const int32_t* obs_cam, const int32_t* obs_pt, int num_sms,
+                cudaStream_t s);
+int pairs_launch(const PairProduct* p, const double* camtab, double f0, int axis, double* P, int ld,
+                 const ba_lm_state* ctl, cudaStream_t s);
+void pairs_release(PairProduct* p, cudaStream_t s);
 int launch_schur_sparse(ba_engine* e, const ba_lm_state* ctl, cudaStream_t s);
 int fp64_peak(int device, int use_dmma, double* tflops);
 int covariance(ba_engine* e, double* point_cov, double* cam_cov, double* sigma2, int mem, cudaStream_t s);

@@ -274,13 +274,14 @@ static void free_engine(ba_engine* e) {
   if (e->own_stream) cudaStreamSynchronize(e->own_stream);
   prof_resolve(e, false);
   comm_free(e);  // closes the peers' windows and frees this rank's (which holds red)
-  void* ptrs[] = {e->obs_ptr, e->obs_cam, e->obs_pt, e->obs_xy, e->cam_ptr, e->cm_perm, e->bits, e->PT, e->pair_ptr, e->pair_pts, e->X[0],
+  void* ptrs[] = {e->obs_ptr, e->obs_cam, e->obs_pt, e->obs_xy, e->cam_ptr, e->cm_perm, e->X[0],
                   e->X[1], e->cam[0].f, e->cam[1].f, e->camtab[0], e->camtab[1], e->JP, e->JC, e->V,
                   e->GPT, e->Upart, e->Uloc, e->LINV, e->Z, e->Yt, e->Ysp, e->red_in_window ? nullptr : e->red, e->Lt, e->Winv,
                   e->dxi, e->cost_part, e->cost_buf, e->ctl, e->rec, e->ywork, e->chol_bar, e->gauge};
   for (void* p : ptrs)
     dev_free(p);
   syrk_release(&e->syrk, (cudaStream_t)0);
+  pairs_release(&e->pairs, (cudaStream_t)0);
   for (int k = 0; k < 2; ++k) {
     if (e->solve_graph[k]) cudaGraphExecDestroy(e->solve_graph[k]);
     if (e->solve_ev[k]) cudaEventDestroy(e->solve_ev[k]);
@@ -375,6 +376,8 @@ static int create_engine(const ba_problem* p, ba_engine** out) {
 
   int st = BA_OK;
 #define A(expr) if (st == BA_OK) st = (expr)
+  // first: a camera count past the pair kernels' launch limit is refused before anything is allocated
+  if (!e->dense) A(pairs_prepare(&e->pairs, e->M, e->N, (cudaStream_t)0));
   A(dev_alloc(&e->obs_ptr, (size_t)e->N + 1));
   A(dev_alloc(&e->obs_xy, (size_t)e->nobs * 2));
   if (!e->dense) {
@@ -382,9 +385,6 @@ static int create_engine(const ba_problem* p, ba_engine** out) {
     A(dev_alloc(&e->obs_pt, (size_t)e->nobs));
     A(dev_alloc(&e->cm_perm, (size_t)e->nobs));
     A(dev_alloc(&e->cam_ptr, (size_t)e->M + 1));
-    e->Wp = round_up64((e->N + 31) / 32, 256);  // whole groups of 256 words: 32 lanes x 8 words (pair kernels)
-    A(dev_alloc(&e->bits, (size_t)e->M * e->Wp));
-    A(dev_alloc(&e->PT, (size_t)e->N * kPT));
   }
   for (int w = 0; w < 2; ++w) {
     A(dev_alloc(&e->X[w], (size_t)3 * e->N));
@@ -560,7 +560,14 @@ int ba_set_observations(ba_engine* e, const int64_t* obs_ptr, const int32_t* obs
     fill_obs_pt_kernel<<<e->num_sms * 8, 256, 0, s>>>(e->N, e->obs_ptr, e->obs_pt);
     BA_LAUNCH_CHECK();
     BA_TRY(build_camera_major_index(e, s));
-    BA_TRY(build_pair_index(e, s));
+    // captured solves launch the pair kernel of the previous index, on lists pairs_index frees:
+    // ba_lm_run captures them again
+    for (int k = 0; k < 2; ++k)
+      if (e->solve_graph[k]) {
+        BA_CUDA(cudaGraphExecDestroy(e->solve_graph[k]));
+        e->solve_graph[k] = nullptr;
+      }
+    BA_TRY(pairs_index(&e->pairs, e->nobs, e->obs_cam, e->obs_pt, e->num_sms, s));
   }
   BA_CUDA(cudaStreamSynchronize(s));
   e->have_obs = true;

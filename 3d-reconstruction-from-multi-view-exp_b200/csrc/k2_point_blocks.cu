@@ -465,7 +465,8 @@ int launch_k2b(ba_engine* e, bool conditional, double c_host, cudaStream_t s) {
                                  (int)kStage));                                                              \
     k2b_point_solve_kernel<D, F><<<grid, 256, kStage, s>>>(                                                  \
         e->N, e->M, e->axis, e->obs_ptr, e->obs_cam, e->JP, e->JC, e->V, e->GPT, c_host, e->ctl, use_ctl,   \
-        e->LINV, e->Z, e->Yt, e->n_pad, e->rhs_row, e->Ysp, e->X[0], e->PT, e->camtab[0], e->f0, colmax);    \
+        e->LINV, e->Z, e->Yt, e->n_pad, e->rhs_row, e->Ysp, e->X[0], e->pairs.PT, e->camtab[0], e->f0,        \
+        colmax);                                                                                             \
   } while (0)
   if (mf) BA_K2B_LAUNCH(true, true);
   else if (e->dense) BA_K2B_LAUNCH(true, false);

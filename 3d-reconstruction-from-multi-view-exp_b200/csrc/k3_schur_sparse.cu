@@ -22,22 +22,25 @@
 // No shared-memory or global read-modify-write; the per-lane sums meet once per pair in a fixed order.
 // Order of summation depends on the data only: runs are bit-reproducible.
 //
-// Two pair kernels; where the common points come from decides which one runs (measurements: DESIGN.md
-// section 3b):
-//   * build_pair_index        once per engine: bitmaps per camera and -- memory permitting -- the STATIC
-//                             PAIR LISTS: the ascending ids of the points every pair shares
+// The camera-pair product is one PairProduct (ba_common.cuh) of the engine; two pair kernels, and where
+// the common points come from decides which one runs (its `kind`; measurements: DESIGN.md section 3b):
+//   * pairs_prepare           at engine creation: the pair-item count (refused past the launch limit),
+//                             the bitmaps and the point table PT.
+//   * pairs_index             with the observations: bitmaps per camera and -- memory permitting -- the
+//                             STATIC PAIR LISTS: the ascending ids of the points every pair shares
 //                             (pair_count_kernel, exclusive sum, pair_fill_kernel; 4 B per pair-point).
 //                             Visibility does not change between iterations; intersecting the bitmaps
 //                             and compacting the hits every solve was more than half of the kernel.
-//   * schur_pairs_reg_kernel  when the lists exist: 32 ids per round with one coalesced load; the pair's
-//                             9 x 9 block lives in 81 FP64 registers per lane (144 DFMAs per point).
-//   * schur_pairs_kernel      when the lists do not fit a third of the free memory (or BA_PAIRS_NO_LIST
-//                             is set): it scans the bitmaps itself (4096 points per step, warp prefix sum,
-//                             ring queue) and sums the leading 8 x 8 of the block on DMMA.8x8x4 (operands
-//                             transposed through shared memory).  Register accumulators lose with the scan
-//                             (40.0 against 35.9 ms at 1000 x 200k): at 255 registers two warps per
-//                             scheduler cannot overlap the scan's serial phases.  Without the scan they
-//                             win (27.0 against 27.8 ms).
+//   * schur_pairs_reg_kernel  PAIRS_LISTS: 32 ids per round with one coalesced load; the pair's 9 x 9
+//                             block lives in 81 FP64 registers per lane (144 DFMAs per point).
+//   * schur_pairs_kernel      PAIRS_SCAN, when the lists do not fit a third of the free memory (or
+//                             BA_PAIRS_NO_LIST is set): it scans the bitmaps itself (4096 points per step,
+//                             warp prefix sum, ring queue) and sums the leading 8 x 8 of the block on
+//                             DMMA.8x8x4 (operands transposed through shared memory).  Register
+//                             accumulators lose with the scan (40.0 against 35.9 ms at 1000 x 200k): at
+//                             255 registers two warps per scheduler cannot overlap the scan's serial
+//                             phases.  Without the scan they win (27.0 against 27.8 ms).
+// Both take their per-point arithmetic from pair_point, so they differ only in how they sum.
 //
 // Bound: FP64 pipe (~316 instructions per pair-point; sum_j m_j (m_j - 1) / 2 pair-points).  DMMA runs
 // on the same FP64 datapath as DFMA on this GPU (fp64_peak.cu, mode 2), so the tensor form buys no
@@ -76,7 +79,7 @@ __global__ void bitmap_fill_kernel(int64_t nobs, int64_t Wp, const int32_t* __re
 // section 3b) -- every solve.  The intersection is therefore done ONCE per engine: pair_count_kernel
 // counts the common points of every pair item, an exclusive sum gives the offsets, pair_fill_kernel
 // writes the ascending point ids.  4 B per pair-point (C4: 19.8 GB of the 180 GB); if that exceeds a
-// third of the free memory the lists are not built and the pair kernel scans the bitmaps as before.
+// third of the free memory the lists are not built and the pair kernel scans the bitmaps instead.
 __device__ __forceinline__ bool pair_from_linear(int64_t t, int M, int& i, int& k);
 
 __global__ void __launch_bounds__(256)
@@ -133,54 +136,6 @@ pair_fill_kernel(int M, int64_t Wp, int64_t n_items, const uint32_t* __restrict_
     }
     running += total;
   }
-}
-
-int build_pair_index(ba_engine* e, cudaStream_t s) {
-  BA_CUDA(cudaMemsetAsync(e->bits, 0, (size_t)e->M * e->Wp * sizeof(uint32_t), s));
-  BA_CUDA(cudaMemsetAsync(e->PT, 0, (size_t)e->N * kPT * sizeof(double), s));
-  bitmap_fill_kernel<<<e->num_sms * 8, 256, 0, s>>>(e->nobs, e->Wp, e->obs_cam, e->obs_pt, e->bits);
-  BA_LAUNCH_CHECK();
-  // BA_PAIRS_NO_LIST: no lists, the pair kernel scans the bitmaps every solve (tests of that fallback)
-  if (std::getenv("BA_PAIRS_NO_LIST")) return BA_OK;
-  const int nt = (e->M + kPairTile - 1) / kPairTile;
-  const int64_t n_items = (int64_t)nt * (nt + 1) / 2 * kPairTile * kPairTile;
-  if (n_items >= ((int64_t)1 << 31)) return BA_OK;
-  if (cudaMallocAsync(reinterpret_cast<void**>(&e->pair_ptr), (size_t)(n_items + 1) * sizeof(int64_t), (cudaStream_t)0) != cudaSuccess) {
-    cudaGetLastError();
-    e->pair_ptr = nullptr;
-    return BA_OK;
-  }
-  BA_CUDA(cudaStreamSynchronize((cudaStream_t)0));  // the allocation is ordered on the default stream
-  const unsigned blocks = (unsigned)((n_items + 1 + 7) / 8);
-  pair_count_kernel<<<blocks, 256, 0, s>>>(e->M, e->Wp, n_items, e->bits, e->pair_ptr);
-  BA_LAUNCH_CHECK();
-  {
-    size_t tmp_bytes = 0;
-    BA_CUDA(cub::DeviceScan::ExclusiveSum(nullptr, tmp_bytes, e->pair_ptr, e->pair_ptr, (int)(n_items + 1), s));
-    void* tmp = nullptr;
-    BA_CUDA(cudaMallocAsync(&tmp, tmp_bytes, s));
-    BA_CUDA(cub::DeviceScan::ExclusiveSum(tmp, tmp_bytes, e->pair_ptr, e->pair_ptr, (int)(n_items + 1), s));
-    BA_CUDA(cudaFreeAsync(tmp, s));
-  }
-  int64_t total = 0;
-  BA_CUDA(cudaMemcpyAsync(&total, e->pair_ptr + n_items, sizeof(int64_t), cudaMemcpyDeviceToHost, s));
-  BA_CUDA(cudaStreamSynchronize(s));
-  size_t free_b = 0, total_b = 0;
-  BA_CUDA(cudaMemGetInfo(&free_b, &total_b));
-  const size_t need = (size_t)(total > 0 ? total : 1) * sizeof(int32_t);
-  if (need > free_b / 3 ||
-      cudaMallocAsync(reinterpret_cast<void**>(&e->pair_pts), need, (cudaStream_t)0) != cudaSuccess) {
-    cudaGetLastError();
-    cudaFreeAsync(e->pair_ptr, (cudaStream_t)0);
-    e->pair_ptr = nullptr;
-    e->pair_pts = nullptr;
-    return BA_OK;
-  }
-  BA_CUDA(cudaStreamSynchronize((cudaStream_t)0));
-  e->pair_total = total;
-  pair_fill_kernel<<<(unsigned)((n_items + 7) / 8), 256, 0, s>>>(e->M, e->Wp, n_items, e->bits, e->pair_ptr, e->pair_pts);
-  BA_LAUNCH_CHECK();
-  return BA_OK;
 }
 
 // ---- off-diagonal pairs -------------------------------------------------------------------------
@@ -250,6 +205,67 @@ __device__ __forceinline__ SideJac side_jacobian(const double* __restrict__ c, d
   return s;
 }
 
+// Table rows of cameras i and k into cam[0] and cam[1] (one warp).
+__device__ __forceinline__ void stage_cameras(double (*cam)[20], const double* __restrict__ camtab, int i, int k,
+                                              int lane) {
+  const int which = lane >> 4, c = lane & 15;
+  const double v = camtab[(size_t)(which ? k : i) * kCamTab + c];
+  cam[which][c] = v;
+  __syncwarp();
+  if (c >= 12) cam[which][c + 4] = v;  // 1 / f, u0 / f0, v0 / f0, 1 / f0 (cam_prep_kernel) where side_jacobian reads them
+  __syncwarp();
+}
+
+// The arithmetic of one pair-point, shared by both pair kernels: from the staged rows of cameras i and k
+// and the point's staged row pt, Jc_i's pieces si and the rows t0, t1 of G Jc_k.
+__device__ __forceinline__ void pair_point(const double* __restrict__ cam_i, const double* __restrict__ cam_k,
+                                           const double* __restrict__ pt, SideJac& si, double* t0, double* t1) {
+  const double2 x01 = *reinterpret_cast<const double2*>(pt);
+  const double2 x2v = *reinterpret_cast<const double2*>(pt + 2);  // X2, V00
+  const double2 v12 = *reinterpret_cast<const double2*>(pt + 4);  // V01, V02
+  const double2 v34 = *reinterpret_cast<const double2*>(pt + 6);  // V11, V12
+  const double v22 = pt[8];
+  const double v00 = x2v.y, v01 = v12.x, v02 = v12.y, v11 = v34.x, v12_ = v34.y;
+  si = side_jacobian(cam_i, x01.x, x01.y, x2v.x);
+  const SideJac sk = side_jacobian(cam_k, x01.x, x01.y, x2v.x);
+  // G = 4 Jx_i Vd^-1 Jx_k^T with the four 1 / r^2 factors folded into one scale
+  const double rr = si.r * sk.r;
+  const double rr2 = rr * rr;
+  const double sc = 4.0 * rcp_nr(rr2 * rr2);
+  double g00, g01, g10, g11;
+  {
+    const double m0 = v00 * sk.aX[0] + v01 * sk.aX[1] + v02 * sk.aX[2];
+    const double m1 = v01 * sk.aX[0] + v11 * sk.aX[1] + v12_ * sk.aX[2];
+    const double m2 = v02 * sk.aX[0] + v12_ * sk.aX[1] + v22 * sk.aX[2];
+    g00 = sc * (si.aX[0] * m0 + si.aX[1] * m1 + si.aX[2] * m2);
+    g10 = sc * (si.bX[0] * m0 + si.bX[1] * m1 + si.bX[2] * m2);
+  }
+  {
+    const double m0 = v00 * sk.bX[0] + v01 * sk.bX[1] + v02 * sk.bX[2];
+    const double m1 = v01 * sk.bX[0] + v11 * sk.bX[1] + v12_ * sk.bX[2];
+    const double m2 = v02 * sk.bX[0] + v12_ * sk.bX[1] + v22 * sk.bX[2];
+    g01 = sc * (si.aX[0] * m0 + si.aX[1] * m1 + si.aX[2] * m2);
+    g11 = sc * (si.bX[0] * m0 + si.bX[1] * m1 + si.bX[2] * m2);
+  }
+  // rows of G Jc_k; Jc_k row a = [af, au, 0, -aX, aX x d], row b = [bf, 0, au, -bX, bX x d]
+  t0[0] = g00 * sk.af + g01 * sk.bf;  t1[0] = g10 * sk.af + g11 * sk.bf;
+  t0[1] = g00 * sk.au;                t1[1] = g10 * sk.au;
+  t0[2] = g01 * sk.au;                t1[2] = g11 * sk.au;
+#pragma unroll
+  for (int m = 0; m < 3; ++m) {
+    t0[3 + m] = -(g00 * sk.aX[m] + g01 * sk.bX[m]);
+    t1[3 + m] = -(g10 * sk.aX[m] + g11 * sk.bX[m]);
+  }
+#pragma unroll
+  for (int m = 0; m < 3; ++m) {
+    const int m1 = (m + 1) % 3, m2 = (m + 2) % 3;
+    const double aw = sk.aX[m1] * sk.d[m2] - sk.aX[m2] * sk.d[m1];
+    const double bw = sk.bX[m1] * sk.d[m2] - sk.bX[m2] * sk.d[m1];
+    t0[6 + m] = g00 * aw + g01 * bw;
+    t1[6 + m] = g10 * aw + g11 * bw;
+  }
+}
+
 // ---- bitmap scan (no pair lists) ------------------------------------------------------------------
 // The lanes intersect the two cameras' bitmaps 128 points each per step, a warp prefix sum of the hit
 // counts gives their slots in a ring queue of point ids, and every 32 queued ids make a round.
@@ -263,15 +279,7 @@ schur_pairs_kernel(int M, int axis, int64_t Wp, const uint32_t* __restrict__ bit
   if (!pair_from_linear(blockIdx.x, M, i, k)) return;
   __shared__ __align__(16) PairSmem sm;
   const int lane = threadIdx.x;
-
-  {
-    const int which = lane >> 4, c = lane & 15;
-    const double v = camtab[(size_t)(which ? k : i) * kCamTab + c];
-    sm.cam[which][c] = v;
-    __syncwarp();
-    if (c >= 12) sm.cam[which][c + 4] = v;  // 1 / f, u0 / f0, v0 / f0, 1 / f0 (cam_prep_kernel) where side_jacobian reads them
-    __syncwarp();
-  }
+  stage_cameras(sm.cam, camtab, i, k, lane);
 
   // four bitmap words (128 points) per lane and batch
   const uint4* bi = reinterpret_cast<const uint4*>(bits + (size_t)i * Wp) + lane;
@@ -302,50 +310,9 @@ schur_pairs_kernel(int M, int axis, int64_t Wp, const uint32_t* __restrict__ bit
     double2* t1s = reinterpret_cast<double2*>(sm.tfrag + kFragX + lane * 8);
     const int sw = (lane >> 1) & 3;
     if (lane < cnt) {
-      const double* pt = sm.stage[st] + lane * kPS;
-      const double2 x01 = *reinterpret_cast<const double2*>(pt);
-      const double2 x2v = *reinterpret_cast<const double2*>(pt + 2);  // X2, V00
-      const double2 v12 = *reinterpret_cast<const double2*>(pt + 4);  // V01, V02
-      const double2 v34 = *reinterpret_cast<const double2*>(pt + 6);  // V11, V12
-      const double v22 = pt[8];
-      const double v00 = x2v.y, v01 = v12.x, v02 = v12.y, v11 = v34.x, v12_ = v34.y;
-      const SideJac si = side_jacobian(sm.cam[0], x01.x, x01.y, x2v.x);
+      SideJac si;
       double t0[9], t1[9];
-      {
-        const SideJac sk = side_jacobian(sm.cam[1], x01.x, x01.y, x2v.x);
-        // G = 4 Jx_i Vd^-1 Jx_k^T, with all four 1/r^2 factors folded into one scale
-        const double mk00 = v00 * sk.aX[0] + v01 * sk.aX[1] + v02 * sk.aX[2];
-        const double mk01 = v01 * sk.aX[0] + v11 * sk.aX[1] + v12_ * sk.aX[2];
-        const double mk02 = v02 * sk.aX[0] + v12_ * sk.aX[1] + v22 * sk.aX[2];
-        const double mk10 = v00 * sk.bX[0] + v01 * sk.bX[1] + v02 * sk.bX[2];
-        const double mk11 = v01 * sk.bX[0] + v11 * sk.bX[1] + v12_ * sk.bX[2];
-        const double mk12 = v02 * sk.bX[0] + v12_ * sk.bX[1] + v22 * sk.bX[2];
-        const double rr = si.r * sk.r;
-        const double rr2 = rr * rr;
-        const double sc = 4.0 * rcp_nr(rr2 * rr2);
-        const double g00 = sc * (si.aX[0] * mk00 + si.aX[1] * mk01 + si.aX[2] * mk02);
-        const double g01 = sc * (si.aX[0] * mk10 + si.aX[1] * mk11 + si.aX[2] * mk12);
-        const double g10 = sc * (si.bX[0] * mk00 + si.bX[1] * mk01 + si.bX[2] * mk02);
-        const double g11 = sc * (si.bX[0] * mk10 + si.bX[1] * mk11 + si.bX[2] * mk12);
-        // rows of G Jc_k; Jc_k row a = [af, au, 0, -aX, aX x d], row b = [bf, 0, au, -bX, bX x d]
-        const double aw0 = sk.aX[1] * sk.d[2] - sk.aX[2] * sk.d[1];
-        const double aw1 = sk.aX[2] * sk.d[0] - sk.aX[0] * sk.d[2];
-        const double aw2 = sk.aX[0] * sk.d[1] - sk.aX[1] * sk.d[0];
-        const double bw0 = sk.bX[1] * sk.d[2] - sk.bX[2] * sk.d[1];
-        const double bw1 = sk.bX[2] * sk.d[0] - sk.bX[0] * sk.d[2];
-        const double bw2 = sk.bX[0] * sk.d[1] - sk.bX[1] * sk.d[0];
-        t0[0] = g00 * sk.af + g01 * sk.bf;  t1[0] = g10 * sk.af + g11 * sk.bf;
-        t0[1] = g00 * sk.au;                t1[1] = g10 * sk.au;
-        t0[2] = g01 * sk.au;                t1[2] = g11 * sk.au;
-#pragma unroll
-        for (int m = 0; m < 3; ++m) {
-          t0[3 + m] = -(g00 * sk.aX[m] + g01 * sk.bX[m]);
-          t1[3 + m] = -(g10 * sk.aX[m] + g11 * sk.bX[m]);
-        }
-        t0[6] = g00 * aw0 + g01 * bw0;  t1[6] = g10 * aw0 + g11 * bw0;
-        t0[7] = g00 * aw1 + g01 * bw1;  t1[7] = g10 * aw1 + g11 * bw1;
-        t0[8] = g00 * aw2 + g01 * bw2;  t1[8] = g10 * aw2 + g11 * bw2;
-      }
+      pair_point(sm.cam[0], sm.cam[1], sm.stage[st] + lane * kPS, si, t0, t1);
       double ia[9], ib[9];
       ia[0] = si.af;  ib[0] = si.bf;
       ia[1] = si.au;  ib[1] = 0.0;
@@ -500,7 +467,7 @@ schur_pairs_kernel(int M, int axis, int64_t Wp, const uint32_t* __restrict__ bit
 // shared-memory wavefronts per 32 pair-points.  Here every lane keeps the whole 9 x 9 block of the pair
 // in 81 FP64 registers and adds its point's Jc_i^T (G Jc_k) with 144 DFMAs (the structural zeros of
 // Jc_i skipped): no fragments, no shuffles, 255 registers, eight warps per SM, independent accumulator
-// chains.  The ids of a round come from the static lists (build_pair_index): 32 with one coalesced
+// chains.  The ids of a round come from the static lists (pairs_index): 32 with one coalesced
 // load, fetched a round ahead.
 // The 81 per-lane sums meet once per pair, through shared memory (the staging rows, free by then),
 // in lane order.  Order of summation depends on the data only: bit-reproducible.
@@ -519,14 +486,7 @@ schur_pairs_reg_kernel(int M, int axis, const double* __restrict__ camtab, doubl
   if (!pair_from_linear(blockIdx.x, M, i, k)) return;
   __shared__ __align__(16) PairRegSmem sm;
   const int lane = threadIdx.x;
-  {
-    const int which = lane >> 4, c = lane & 15;
-    const double v = camtab[(size_t)(which ? k : i) * kCamTab + c];
-    sm.cam[which][c] = v;
-    __syncwarp();
-    if (c >= 12) sm.cam[which][c + 4] = v;  // 1 / f, u0 / f0, v0 / f0, 1 / f0 (cam_prep_kernel) where side_jacobian reads them
-    __syncwarp();
-  }
+  stage_cameras(sm.cam, camtab, i, k, lane);
 
   double acc[9][9];
 #pragma unroll
@@ -535,54 +495,9 @@ schur_pairs_reg_kernel(int M, int axis, const double* __restrict__ camtab, doubl
     for (int b = 0; b < 9; ++b) acc[a][b] = 0.0;
 
   auto compute = [&](int st) {
-    const double* pt = sm.stage[st] + lane * kPS;
-    const double2 x01 = *reinterpret_cast<const double2*>(pt);
-    const double2 x2v = *reinterpret_cast<const double2*>(pt + 2);  // X2, V00
-    const double2 v12 = *reinterpret_cast<const double2*>(pt + 4);  // V01, V02
-    const double2 v34 = *reinterpret_cast<const double2*>(pt + 6);  // V11, V12
-    const double v22 = pt[8];
-    const double v00 = x2v.y, v01 = v12.x, v02 = v12.y, v11 = v34.x, v12_ = v34.y;
-    const SideJac si = side_jacobian(sm.cam[0], x01.x, x01.y, x2v.x);
+    SideJac si;
     double t0[9], t1[9];
-    {
-      const SideJac sk = side_jacobian(sm.cam[1], x01.x, x01.y, x2v.x);
-      // G = 4 Jx_i Vd^-1 Jx_k^T with the four 1 / r^2 factors folded into one scale
-      const double rr = si.r * sk.r;
-      const double rr2 = rr * rr;
-      const double sc = 4.0 * rcp_nr(rr2 * rr2);
-      double g00, g01, g10, g11;
-      {
-        const double m0 = v00 * sk.aX[0] + v01 * sk.aX[1] + v02 * sk.aX[2];
-        const double m1 = v01 * sk.aX[0] + v11 * sk.aX[1] + v12_ * sk.aX[2];
-        const double m2 = v02 * sk.aX[0] + v12_ * sk.aX[1] + v22 * sk.aX[2];
-        g00 = sc * (si.aX[0] * m0 + si.aX[1] * m1 + si.aX[2] * m2);
-        g10 = sc * (si.bX[0] * m0 + si.bX[1] * m1 + si.bX[2] * m2);
-      }
-      {
-        const double m0 = v00 * sk.bX[0] + v01 * sk.bX[1] + v02 * sk.bX[2];
-        const double m1 = v01 * sk.bX[0] + v11 * sk.bX[1] + v12_ * sk.bX[2];
-        const double m2 = v02 * sk.bX[0] + v12_ * sk.bX[1] + v22 * sk.bX[2];
-        g01 = sc * (si.aX[0] * m0 + si.aX[1] * m1 + si.aX[2] * m2);
-        g11 = sc * (si.bX[0] * m0 + si.bX[1] * m1 + si.bX[2] * m2);
-      }
-      // rows of G Jc_k; Jc_k row a = [af, au, 0, -aX, aX x d], row b = [bf, 0, au, -bX, bX x d]
-      t0[0] = g00 * sk.af + g01 * sk.bf;  t1[0] = g10 * sk.af + g11 * sk.bf;
-      t0[1] = g00 * sk.au;                t1[1] = g10 * sk.au;
-      t0[2] = g01 * sk.au;                t1[2] = g11 * sk.au;
-#pragma unroll
-      for (int m = 0; m < 3; ++m) {
-        t0[3 + m] = -(g00 * sk.aX[m] + g01 * sk.bX[m]);
-        t1[3 + m] = -(g10 * sk.aX[m] + g11 * sk.bX[m]);
-      }
-#pragma unroll
-      for (int m = 0; m < 3; ++m) {
-        const int m1 = (m + 1) % 3, m2 = (m + 2) % 3;
-        const double aw = sk.aX[m1] * sk.d[m2] - sk.aX[m2] * sk.d[m1];
-        const double bw = sk.bX[m1] * sk.d[m2] - sk.bX[m2] * sk.d[m1];
-        t0[6 + m] = g00 * aw + g01 * bw;
-        t1[6 + m] = g10 * aw + g11 * bw;
-      }
-    }
+    pair_point(sm.cam[0], sm.cam[1], sm.stage[st] + lane * kPS, si, t0, t1);
     // block += Jc_i^T [t0; t1], row by row of Jc_i^T; its structural zeros are skipped
 #pragma unroll
     for (int b = 0; b < 9; ++b) {
@@ -738,6 +653,101 @@ __global__ void schur_diag_finish_kernel(int nchunks, const double* __restrict__
   }
 }
 
+// ---- the camera-pair product: index, choice, launch -------------------------------------------------
+int pairs_prepare(PairProduct* p, int M, int64_t N, cudaStream_t s) {
+  *p = PairProduct();
+  const int nt = (M + kPairTile - 1) / kPairTile;
+  const int64_t n_items = (int64_t)nt * (nt + 1) / 2 * kPairTile * kPairTile;
+  if (n_items >= ((int64_t)1 << 31)) {  // one block per pair item
+    set_error("%d cameras exceed the camera-pair limit: %lld pair items, one launch takes fewer than 2^31 "
+              "(at most %d cameras)", M, (long long)n_items, 2047 * kPairTile);
+    return BA_ERR_INVALID;
+  }
+  p->M = M;
+  p->N = N;
+  p->n_items = n_items;
+  p->Wp = ((N + 31) / 32 + 255) / 256 * 256;  // whole groups of 256 words: 32 lanes x 8 words
+  BA_CUDA(cudaMallocAsync(reinterpret_cast<void**>(&p->bits), (size_t)M * p->Wp * sizeof(uint32_t), s));
+  BA_CUDA(cudaMallocAsync(reinterpret_cast<void**>(&p->PT), (size_t)N * kPT * sizeof(double), s));
+  return BA_OK;
+}
+
+static void free_lists(PairProduct* p, cudaStream_t s) {
+  if (p->pair_ptr) cudaFreeAsync(p->pair_ptr, s);
+  if (p->pair_pts) cudaFreeAsync(p->pair_pts, s);
+  p->pair_ptr = nullptr;
+  p->pair_pts = nullptr;
+  p->kind = PAIRS_SCAN;
+}
+
+int pairs_index(PairProduct* p, int64_t nobs, const int32_t* obs_cam, const int32_t* obs_pt, int num_sms,
+                cudaStream_t s) {
+  free_lists(p, s);
+  BA_CUDA(cudaMemsetAsync(p->bits, 0, (size_t)p->M * p->Wp * sizeof(uint32_t), s));
+  BA_CUDA(cudaMemsetAsync(p->PT, 0, (size_t)p->N * kPT * sizeof(double), s));
+  bitmap_fill_kernel<<<num_sms * 8, 256, 0, s>>>(nobs, p->Wp, obs_cam, obs_pt, p->bits);
+  BA_LAUNCH_CHECK();
+  // BA_PAIRS_NO_LIST: no lists, the pair kernel scans the bitmaps every solve (tests of that fallback)
+  if (std::getenv("BA_PAIRS_NO_LIST")) return BA_OK;
+  const int64_t n_items = p->n_items;
+  if (cudaMallocAsync(reinterpret_cast<void**>(&p->pair_ptr), (size_t)(n_items + 1) * sizeof(int64_t), s) != cudaSuccess) {
+    cudaGetLastError();
+    p->pair_ptr = nullptr;
+    return BA_OK;
+  }
+  const unsigned blocks = (unsigned)((n_items + 1 + 7) / 8);
+  pair_count_kernel<<<blocks, 256, 0, s>>>(p->M, p->Wp, n_items, p->bits, p->pair_ptr);
+  BA_LAUNCH_CHECK();
+  {
+    size_t tmp_bytes = 0;
+    BA_CUDA(cub::DeviceScan::ExclusiveSum(nullptr, tmp_bytes, p->pair_ptr, p->pair_ptr, (int)(n_items + 1), s));
+    void* tmp = nullptr;
+    BA_CUDA(cudaMallocAsync(&tmp, tmp_bytes, s));
+    BA_CUDA(cub::DeviceScan::ExclusiveSum(tmp, tmp_bytes, p->pair_ptr, p->pair_ptr, (int)(n_items + 1), s));
+    BA_CUDA(cudaFreeAsync(tmp, s));
+  }
+  int64_t total = 0;
+  BA_CUDA(cudaMemcpyAsync(&total, p->pair_ptr + n_items, sizeof(int64_t), cudaMemcpyDeviceToHost, s));
+  BA_CUDA(cudaStreamSynchronize(s));
+  size_t free_b = 0, total_b = 0;
+  BA_CUDA(cudaMemGetInfo(&free_b, &total_b));
+  const size_t need = (size_t)(total > 0 ? total : 1) * sizeof(int32_t);
+  if (need > free_b / 3 || cudaMallocAsync(reinterpret_cast<void**>(&p->pair_pts), need, s) != cudaSuccess) {
+    cudaGetLastError();
+    p->pair_pts = nullptr;
+    free_lists(p, s);
+    return BA_OK;
+  }
+  pair_fill_kernel<<<(unsigned)((n_items + 7) / 8), 256, 0, s>>>(p->M, p->Wp, n_items, p->bits, p->pair_ptr,
+                                                                 p->pair_pts);
+  BA_LAUNCH_CHECK();
+  p->kind = PAIRS_LISTS;
+  return BA_OK;
+}
+
+int pairs_launch(const PairProduct* p, const double* camtab, double f0, int axis, double* P, int ld,
+                 const ba_lm_state* ctl, cudaStream_t s) {
+  if (p->kind == PAIRS_LISTS) {
+    BA_CUDA(cudaFuncSetAttribute(schur_pairs_reg_kernel, cudaFuncAttributePreferredSharedMemoryCarveout,
+                                 (int)cudaSharedmemCarveoutMaxShared));
+    schur_pairs_reg_kernel<<<(unsigned)p->n_items, 32, 0, s>>>(p->M, axis, camtab, f0, p->PT, P, ld, ctl, p->pair_ptr,
+                                                              p->pair_pts);
+  } else {
+    BA_CUDA(cudaFuncSetAttribute(schur_pairs_kernel, cudaFuncAttributePreferredSharedMemoryCarveout,
+                                 (int)cudaSharedmemCarveoutMaxShared));
+    schur_pairs_kernel<<<(unsigned)p->n_items, 32, 0, s>>>(p->M, axis, p->Wp, p->bits, camtab, f0, p->PT, P, ld, ctl);
+  }
+  BA_LAUNCH_CHECK();
+  return BA_OK;
+}
+
+void pairs_release(PairProduct* p, cudaStream_t s) {
+  free_lists(p, s);
+  if (p->bits) cudaFreeAsync(p->bits, s);
+  if (p->PT) cudaFreeAsync(p->PT, s);
+  *p = PairProduct();
+}
+
 int launch_schur_sparse(ba_engine* e, const ba_lm_state* ctl, cudaStream_t s) {
   ProfScope ps(e, PG_SYRK, s);
   dim3 dgrid(e->cam_chunks, e->M);
@@ -745,25 +755,7 @@ int launch_schur_sparse(ba_engine* e, const ba_lm_state* ctl, cudaStream_t s) {
   BA_LAUNCH_CHECK();
   schur_diag_finish_kernel<<<e->M, 96, 0, s>>>(e->cam_chunks, e->Upart, e->P(), e->n_pad, e->rhs_row, ctl);
   BA_LAUNCH_CHECK();
-  const int nt = (e->M + kPairTile - 1) / kPairTile;
-  const int64_t n_items = (int64_t)nt * (nt + 1) / 2 * kPairTile * kPairTile;
-  if (n_items >= ((int64_t)1 << 31)) {
-    set_error("too many camera pairs for one launch (M=%d)", e->M);
-    return BA_ERR_INVALID;
-  }
-  if (e->pair_ptr != nullptr && e->pair_pts != nullptr) {
-    BA_CUDA(cudaFuncSetAttribute(schur_pairs_reg_kernel, cudaFuncAttributePreferredSharedMemoryCarveout,
-                                 (int)cudaSharedmemCarveoutMaxShared));
-    schur_pairs_reg_kernel<<<(unsigned)n_items, 32, 0, s>>>(e->M, e->axis, e->camtab[0], e->f0, e->PT, e->P(), e->n_pad,
-                                                           ctl, e->pair_ptr, e->pair_pts);
-  } else {
-    BA_CUDA(cudaFuncSetAttribute(schur_pairs_kernel, cudaFuncAttributePreferredSharedMemoryCarveout,
-                                 (int)cudaSharedmemCarveoutMaxShared));
-    schur_pairs_kernel<<<(unsigned)n_items, 32, 0, s>>>(e->M, e->axis, e->Wp, e->bits, e->camtab[0], e->f0, e->PT,
-                                                       e->P(), e->n_pad, ctl);
-  }
-  BA_LAUNCH_CHECK();
-  return BA_OK;
+  return pairs_launch(&e->pairs, e->camtab[0], e->f0, e->axis, e->P(), e->n_pad, ctl, s);
 }
 
 }  // namespace ba

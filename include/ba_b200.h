@@ -102,7 +102,8 @@ typedef struct ba_iter_record {
 int ba_version(void);
 const char* ba_last_error(void);
 int ba_device_count(void);
-/* BundleAdjuster.__init__ (:11-75) after host-side gauge normalisation. */
+/* BundleAdjuster.__init__ (:11-75) after host-side gauge normalisation.  A list (not dense) problem
+ * of more than 65 504 cameras returns BA_ERR_INVALID: the camera-pair limit of one pair-kernel launch. */
 int ba_create(const ba_problem* problem, ba_engine** out);
 int ba_destroy(ba_engine* e);
 
